@@ -4,6 +4,7 @@
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c5|c4|c1|c2|c3|c2x] [--scale S]
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --impl reference ...      # the CPU arm (oracle port of the reference's C# loops)
+    python bench.py ... --dump-outputs DIR    # also write the last timed step's results as DIR/<workload>_*.npy
 
 A step = one pass of the hot path over one batch of synthetic queries.  `value` = whole-job QPS with
 queries and outputs resident in HBM (CUDA events on the launching stream, max over ranks);
@@ -173,6 +174,17 @@ def dist_env():
 
 def log(s):
     print(s, file=sys.stderr, flush=True)
+
+
+def dump_outputs(out_dir, name: str, scores, ids, counts):
+    """--dump-outputs: what a caller of the timed search receives from its last step, as out_dir/<name>_scores.npy
+    (float32 [nq][k]), <name>_ids.npy and <name>_counts.npy (float64: exact for ids below 2**53), so that two builds
+    can be compared on the same seeded inputs.  nq <= 10,000 and k <= 100 in every workload: at most 13 MB per workload."""
+    if not out_dir:
+        return
+    os.makedirs(out_dir, exist_ok=True)
+    for part, a, dt in (("scores", scores, np.float32), ("ids", ids, np.float64), ("counts", counts, np.float64)):
+        np.save(os.path.join(out_dir, f"{name}_{part}.npy"), np.asarray(a).astype(dt))
 
 
 # ------------------------------------------------------------------------------------------------
@@ -650,6 +662,8 @@ def bench_workload(args, torch, pg, dist, w: dict, steps: int, warmup: int, rank
     value = nq * steps / (ms / 1e3)
     # the result every later check looks at: the merged output of the last timed step
     res_sc, res_rw, res_cn = m_sc.cpu().numpy(), m_rw.cpu().numpy(), m_cn.cpu().numpy()
+    if rank == 0:
+        dump_outputs(args.dump_outputs, w["name"], res_sc, res_rw, res_cn)
 
     # ---- dominant-kernel time (CUDA events inside the library around the scan stage), per launch
     stage_ms = {"total": 0.0, "coarse": 0.0, "scan": 0.0, "merge": 0.0}
@@ -879,10 +893,10 @@ def run_ours(args):
     if args.secondary == "auto":
         args.secondary = "c4" if args.workload == "c5" else "none"
     if args.secondary and args.secondary != "none" and args.secondary != args.workload:
-        # BASELINE config 4 beside the headline config: fewer steps (a C4 step takes ~0.6 s)
+        # BASELINE config 4 beside the headline config
         w2 = workload(args.secondary, args.secondary_scale if args.secondary_scale > 0 else args.scale)
         try:
-            sec = bench_workload(args, torch, pg, dist, w2, min(args.steps, 3), 3, rank, world, local)
+            sec = bench_workload(args, torch, pg, dist, w2, args.steps, args.warmup, rank, world, local)
         except Exception as ex:
             if world > 1:
                 raise
@@ -961,6 +975,7 @@ def run_sharded_entry(args):
         dev_ms += sx.last_search_ms()
     dt = time.perf_counter() - t0
     clocks = sampler.stop()
+    dump_outputs(args.dump_outputs, w["name"], sc.cpu().numpy(), rw.cpu().numpy(), cn.cpu().numpy())
     Qh = Q.cpu().numpy()
     for _ in range(2):
         hs, hr, hc = sx.search(Qh, k, nprobe=nprobe)
@@ -1029,8 +1044,9 @@ def run_reference(args):
     t0 = time.perf_counter()
     for i in range(args.steps):
         off = (i * s) % max(1, len(Qh) - s + 1)
-        _osearch(oidx, Qh[off:off + s], w, threads)
+        ids, scores, counts = _osearch(oidx, Qh[off:off + s], w, threads)
     dt = time.perf_counter() - t0
+    dump_outputs(args.dump_outputs, w["name"], scores, ids, counts)
     value = s * args.steps / dt * (held / w["n"])
     sample = f"{s} of the batch's {len(Qh)} queries per step over {note}, one query per thread"
     line = {"impl": "reference", "metric": METRIC_NAME, "value": round(value, 2), "unit": "QPS", "n_gpus": args.gpus,
@@ -1085,7 +1101,11 @@ def main():
                     help="bracket one extra search step with cudaProfilerStart/Stop (for ncu --profile-from-start off)")
     ap.add_argument("--flat-parity-queries", type=int, default=32,
                     help="queries of a full-size FLAT batch checked against the independent exact top-k")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the results of the last timed step as DIR/<workload>_{scores,ids,counts}.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3  # timing rule: W >= 3
     if args.impl == "reference":
