@@ -262,8 +262,30 @@ int pyrope_sharded_set_codebooks(pyrope_sharded *s, int n_centroids, const float
 int pyrope_sharded_add_batch(pyrope_sharded *s, int64_t n, const float *X, const int64_t *labels,
                              int64_t *first_row_out);
 int pyrope_sharded_delete_row(pyrope_sharded *s, int64_t row);
+/* IVectorIndex.Upsert of an existing row, semantics of pyrope_index_update_row.  FLAT: the owning shard's copy, in place
+ * (un-deletes).  IVF_*: the row must be in the (replicated) write buffer and is updated on every shard; a list row ->
+ * NOT_FOUND, shards that disagree -> INVALID_STATE. */
+int pyrope_sharded_update_row(pyrope_sharded *s, int64_t row, const float *x);
+/* pyrope_index_shadow_row on the shard owning the row's list (FLAT -> INVALID_STATE, no owner -> NOT_FOUND). */
+int pyrope_sharded_shadow_row(pyrope_sharded *s, int64_t row, int shadowed);
+/* pyrope_index_set_labels with global row ordinals (FLAT shards map their local rows through the row blocks). */
+int pyrope_sharded_set_labels(pyrope_sharded *s, int64_t n_rows, const int64_t *labels_by_row);
 int pyrope_sharded_build(pyrope_sharded *s);
 int pyrope_sharded_stats(pyrope_sharded *s, int64_t *live_rows_out);
+/* read from the first shard: the replicas are bit-identical */
+int pyrope_sharded_is_built(pyrope_sharded *s, int *out);
+int pyrope_sharded_get_centroids(pyrope_sharded *s, float *centroids_out, int *n_out);
+int pyrope_sharded_get_codebooks(pyrope_sharded *s, float *codebooks_out, int32_t *ksub_out);
+/* IVectorIndex.Snapshot / Load over N devices.  `path` is a small binary manifest (shape, row count, the FLAT row blocks
+ * and the names of the N shard files); shard i writes path.g<gen>.shard<i> with pyrope_index_snapshot, all in parallel,
+ * the manifest is moved into place last and only then are the previous generation's shard files removed, so the
+ * manifest on disk always names a complete set.  Load is all or nothing: the manifest is checked against the handle
+ * (device count -> INVALID_ARG: no re-sharding on load, nor loading a single-device snapshot; kind / metric / m / k ->
+ * INVALID_ARG, dim -> DIMENSION), every shard then parses and stages its file on its own thread (its shard identity
+ * and row count must match the manifest), and the staged state is committed only when every shard succeeded; on any
+ * failure the live index is left exactly as it was.  Missing file -> NOT_FOUND. */
+int pyrope_sharded_snapshot(pyrope_sharded *s, const char *path);
+int pyrope_sharded_load(pyrope_sharded *s, const char *path);
 /* IVectorIndex.Search for nq queries over all shards: host buffers in / out (H2D of the queries to every device and
  * the D2H of the merged result inside the call). */
 int pyrope_sharded_search_batch(pyrope_sharded *s, int64_t nq, const float *Q, int topk, int64_t max_scans,
@@ -308,6 +330,14 @@ const char *pyrope_peer_last_error(void);
 typedef struct pyrope_delta pyrope_delta;
 /* DeltaVectorIndex..ctor :18-28: dimension / metric mismatch -> INVALID_ARG (ArgumentException). */
 int pyrope_delta_create(pyrope_index *head, pyrope_index *tail, pyrope_delta **out);
+/* The same with a tail sharded over the box's GPUs (IVF_FLAT / IVF_PQ only: a FLAT tail -> UNSUPPORTED; the head must
+ * live on the tail's first device -> else INVALID_ARG).  Every pyrope_delta_* call accepts the result.  Search: the
+ * head's top-k on its stream, the tail through the sharded search (cut to its own top k, as the reference asks the tail
+ * for topK), then one de-duplicating merge; an IVF_PQ tail ignores MaxScans, an IVF_FLAT tail over N > 1 devices refuses
+ * it (UNSUPPORTED); topk <= min(1024, 4096 / N).  Move: the head's live rows go to every shard's replica of the write
+ * buffer (peer copies), the head is tombstoned only after every shard succeeded.  Snapshot: path.tail is the sharded
+ * manifest of pyrope_sharded_snapshot. */
+int pyrope_delta_create_sharded(pyrope_index *head, pyrope_sharded *tail, pyrope_delta **out);
 int pyrope_delta_destroy(pyrope_delta *d);
 /* DeltaVectorIndex.Search :76-122 for nq queries: head top-k and tail top-k with the SAME options (:85,88),
  * merged on the device — the head's copy of a label replaces the tail's, descending score, first topk.
@@ -349,8 +379,13 @@ typedef struct pyrope_vindex pyrope_vindex;
 int pyrope_vindex_create(int kind, int dim, int metric, int nlist, int pq_m, int pq_k, pyrope_vindex **out);
 /* DeltaVectorIndex(head, tail) :18-28; head must be FLAT.  Borrows both (destroy the delta first). */
 int pyrope_vindex_create_delta(pyrope_vindex *head, pyrope_vindex *tail, pyrope_vindex **out);
+/* IvfFlatVectorIndex / IvfPqVectorIndex over n_devices GPUs (devices: CUDA ordinals or NULL for 0..n-1; IVF kinds only):
+ * the row operations go to pyrope_sharded_*.  pyrope_vindex_create_delta takes it as the tail (with a FLAT head on
+ * its first device); pyrope_vindex_native returns NULL for it. */
+int pyrope_vindex_create_sharded(int n_devices, const int *devices, int kind, int dim, int metric, int nlist, int pq_m,
+                                 int pq_k, pyrope_vindex **out);
 int pyrope_vindex_destroy(pyrope_vindex *v);
-int pyrope_vindex_native(pyrope_vindex *v, pyrope_index **out); /* row-ordinal handle (NULL for a delta) */
+int pyrope_vindex_native(pyrope_vindex *v, pyrope_index **out); /* row-ordinal handle (NULL for a delta or a sharded leaf) */
 int pyrope_vindex_set_quantization(pyrope_vindex *v, int enable); /* BruteForceVectorIndex.EnableQuantization */
 int pyrope_vindex_add(pyrope_vindex *v, const char *id, const float *vec, int len);
 int pyrope_vindex_upsert(pyrope_vindex *v, const char *id, const float *vec, int len);

@@ -70,6 +70,14 @@ SIGNATURES = {
     "pyrope_sharded_set_codebooks": (C.c_int, [vp, C.c_int, vp, vp]),
     "pyrope_sharded_add_batch": (C.c_int, [vp, C.c_int64, vp, vp, i64p]),
     "pyrope_sharded_delete_row": (C.c_int, [vp, C.c_int64]),
+    "pyrope_sharded_update_row": (C.c_int, [vp, C.c_int64, vp]),
+    "pyrope_sharded_shadow_row": (C.c_int, [vp, C.c_int64, C.c_int]),
+    "pyrope_sharded_set_labels": (C.c_int, [vp, C.c_int64, vp]),
+    "pyrope_sharded_is_built": (C.c_int, [vp, i32p]),
+    "pyrope_sharded_get_centroids": (C.c_int, [vp, vp, i32p]),
+    "pyrope_sharded_get_codebooks": (C.c_int, [vp, vp, vp]),
+    "pyrope_sharded_snapshot": (C.c_int, [vp, C.c_char_p]),
+    "pyrope_sharded_load": (C.c_int, [vp, C.c_char_p]),
     "pyrope_sharded_build": (C.c_int, [vp]),
     "pyrope_sharded_stats": (C.c_int, [vp, i64p]),
     "pyrope_sharded_search_batch": (C.c_int, [vp, C.c_int64, vp, C.c_int, C.c_int64, C.c_int, vp, vp, vp]),
@@ -106,6 +114,7 @@ SIGNATURES = {
     "pyrope_batcher_last_error": (C.c_char_p, []),
     "pyrope_topk_merge_device": (C.c_int, [C.c_int64, C.c_int, C.c_int, C.c_int, vp, vp, vp, vp, vp, vp]),
     "pyrope_delta_create": (C.c_int, [vp, vp, C.POINTER(vp)]),
+    "pyrope_delta_create_sharded": (C.c_int, [vp, vp, C.POINTER(vp)]),
     "pyrope_delta_destroy": (C.c_int, [vp]),
     "pyrope_delta_search_batch": (C.c_int, [vp, C.c_int64, vp, C.c_int, C.c_int64, C.c_int, vp, vp, vp]),
     "pyrope_delta_search_batch_device": (C.c_int, [vp, C.c_int64, vp, C.c_int, C.c_int64, C.c_int, vp, vp, vp, vp]),
@@ -117,6 +126,7 @@ SIGNATURES = {
     "pyrope_delta_load": (C.c_int, [vp, C.c_char_p]),
     "pyrope_vindex_create": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(vp)]),
     "pyrope_vindex_create_delta": (C.c_int, [vp, vp, C.POINTER(vp)]),
+    "pyrope_vindex_create_sharded": (C.c_int, [C.c_int, i32p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(vp)]),
     "pyrope_vindex_destroy": (C.c_int, [vp]),
     "pyrope_vindex_native": (C.c_int, [vp, C.POINTER(vp)]),
     "pyrope_vindex_set_quantization": (C.c_int, [vp, C.c_int]),
@@ -488,8 +498,47 @@ class ShardedIndex:
         self._ck(rc)
         return True
 
+    def update_row(self, row: int, x):
+        x = _np(x, np.float32).reshape(-1)
+        if x.size != self.dim:
+            raise PyropeGpuError(ERR_DIMENSION, "Vector dimension mismatch")
+        self._ck(load().pyrope_sharded_update_row(self._s, row, _p(x)))
+
+    def shadow_row(self, row: int, shadowed=True):
+        self._ck(load().pyrope_sharded_shadow_row(self._s, row, 1 if shadowed else 0))
+
+    def set_labels(self, labels_by_row):
+        lab = _np(labels_by_row, np.int64)
+        self._ck(load().pyrope_sharded_set_labels(self._s, lab.size, _p(lab)))
+
     def build(self):
         self._ck(load().pyrope_sharded_build(self._s))
+
+    def is_built(self) -> bool:
+        out = C.c_int32(0)
+        self._ck(load().pyrope_sharded_is_built(self._s, C.byref(out)))
+        return bool(out.value)
+
+    def centroids(self):
+        n = C.c_int32(0)
+        self._ck(load().pyrope_sharded_get_centroids(self._s, None, C.byref(n)))
+        if n.value == 0:
+            return None
+        out = np.zeros((n.value, self.dim), np.float32)
+        self._ck(load().pyrope_sharded_get_centroids(self._s, _p(out), C.byref(n)))
+        return out
+
+    def codebooks(self):
+        cb = np.zeros((self.m, self.k, self.dim // self.m), np.float32)
+        ks = np.zeros(self.m, np.int32)
+        self._ck(load().pyrope_sharded_get_codebooks(self._s, _p(cb), _p(ks)))
+        return cb, ks
+
+    def snapshot(self, path: str):
+        self._ck(load().pyrope_sharded_snapshot(self._s, str(path).encode()))
+
+    def load(self, path: str):
+        self._ck(load().pyrope_sharded_load(self._s, str(path).encode()))
 
     def stats(self) -> int:
         out = C.c_int64(0)

@@ -175,6 +175,7 @@ struct TcOperand {
 
 struct pyrope_index {
     int kind = 0, dim = 0, metric = 0, nlist = 0, m = 0, k = 0, sub = 0;
+    int device = 0;  // CUDA ordinal current at creation: every call on this index expects it current
     cudaStream_t stream = nullptr;
     cudaStream_t last_stream = nullptr;
     std::mutex mu;
@@ -1375,6 +1376,7 @@ int pyrope_index_create(int kind, int dim, int metric, int nlist, int pq_m, int 
     h->seg.dim = dim;
     h->seg.cosine = (metric == PYROPE_COSINE);
     h->seg.reuse_slots = (kind != PYROPE_FLAT);
+    cudaGetDevice(&h->device);
     cudaError_t e = cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking);
     if (e != cudaSuccess) {
         delete h;
@@ -1980,9 +1982,20 @@ int parse_snapshot(Index* h, SnapIO& io, const char* path, LoadedSnapshot& L, cu
 }  // namespace
 extern "C" {
 
-int pyrope_index_load(pyrope_index* h, const char* path) {
-    if (!h || !path || !*path) return fail(PYROPE_ERR_INVALID_ARG, "Path cannot be empty");
-    std::lock_guard<std::mutex> g(h->mu);
+}  // extern "C"
+namespace {
+// A snapshot parsed, validated and staged in device memory, ready to be swapped into its index.  load_prepare does
+// everything that can fail (parse, validation, every device allocation); load_commit only swaps and cannot fail.  The
+// sharded index prepares every shard before it commits any (pyrope_sharded_load: all or nothing over N devices).
+struct StagedLoad {
+    LoadedSnapshot L;
+    Segment ns;
+    DevBuf cnorms, list_norms, list_dead, list_off, ksub_d;
+    int64_t list_ndead = 0, max_list_len = 0;
+};
+
+// caller holds h->mu
+int load_prepare(Index* h, const char* path, StagedLoad& S) {
     CK(cudaStreamSynchronize(h->stream));
     if (h->last_stream) CK(cudaStreamSynchronize(h->last_stream));
     SnapIO io;
@@ -1991,17 +2004,16 @@ int pyrope_index_load(pyrope_index* h, const char* path) {
     if (fseek(io.f, 0, SEEK_END) == 0) { io.remaining = (uint64_t)std::max<long>(ftell(io.f), 0); io.bounded = true; }
     rewind(io.f);
     cudaStream_t st = h->stream;
-    LoadedSnapshot L;
+    LoadedSnapshot& L = S.L;
     int rc = parse_snapshot(h, io, path, L, st);
     fclose(io.f);
     if (rc != PYROPE_OK) return rc;  // nothing of the live index was touched
 
-    // ---- commit: device allocations below can still fail (OOM), so the fallible part comes first
+    // device allocations below can still fail (OOM), so they happen before anything is swapped
     const int dim = h->dim;
-    Segment ns;
+    Segment& ns = S.ns;
     ns.dim = dim; ns.cosine = h->seg.cosine; ns.reuse_slots = h->seg.reuse_slots;
     TRY(ns.reserve(std::max<int64_t>(L.nslots, 1), st, true));
-    DevBuf cnorms, list_norms, list_dead, list_off, ksub_d;
     if (L.nslots) {
         CK(cudaMemcpyAsync(ns.X.p, L.X.p, sizeof(float) * (size_t)L.nslots * dim, cudaMemcpyDeviceToDevice, st));
         CK(cudaMemcpyAsync(ns.labels.p, L.labels.p, sizeof(int64_t) * (size_t)L.nslots, cudaMemcpyDeviceToDevice, st));
@@ -2009,31 +2021,35 @@ int pyrope_index_load(pyrope_index* h, const char* path) {
         if (ns.cosine) CK(launch_row_norms_exact(ns.X.as<float>(), L.nslots, dim, dim, ns.norms.as<float>(), st));
     }
     if (h->kind == PYROPE_IVF_PQ && !L.ksub.empty()) {
-        TRY(ksub_d.ensure(sizeof(int32_t) * L.ksub.size(), 0, st, true));
-        CK(cudaMemcpyAsync(ksub_d.p, L.ksub.data(), sizeof(int32_t) * L.ksub.size(), cudaMemcpyHostToDevice, st));
+        TRY(S.ksub_d.ensure(sizeof(int32_t) * L.ksub.size(), 0, st, true));
+        CK(cudaMemcpyAsync(S.ksub_d.p, L.ksub.data(), sizeof(int32_t) * L.ksub.size(), cudaMemcpyHostToDevice, st));
     }
-    int64_t list_ndead = 0, max_list_len = 0;
     if (L.built) {
-        TRY(list_off.ensure(sizeof(int64_t) * L.list_off_h.size(), 0, st, true));
-        CK(cudaMemcpyAsync(list_off.p, L.list_off_h.data(), sizeof(int64_t) * L.list_off_h.size(), cudaMemcpyHostToDevice, st));
-        for (int c = 0; c < L.nc; ++c) max_list_len = std::max(max_list_len, L.list_off_h[(size_t)c + 1] - L.list_off_h[(size_t)c]);
+        TRY(S.list_off.ensure(sizeof(int64_t) * L.list_off_h.size(), 0, st, true));
+        CK(cudaMemcpyAsync(S.list_off.p, L.list_off_h.data(), sizeof(int64_t) * L.list_off_h.size(), cudaMemcpyHostToDevice, st));
+        for (int c = 0; c < L.nc; ++c) S.max_list_len = std::max(S.max_list_len, L.list_off_h[(size_t)c + 1] - L.list_off_h[(size_t)c]);
         if (!L.list_dead_h.empty()) {
-            TRY(list_dead.ensure((size_t)std::max<int64_t>(L.list_total, 1), 0, st, true));
-            CK(cudaMemcpyAsync(list_dead.p, L.list_dead_h.data(), L.list_dead_h.size(), cudaMemcpyHostToDevice, st));
-            for (uint8_t b : L.list_dead_h) list_ndead += b ? 1 : 0;
+            TRY(S.list_dead.ensure((size_t)std::max<int64_t>(L.list_total, 1), 0, st, true));
+            CK(cudaMemcpyAsync(S.list_dead.p, L.list_dead_h.data(), L.list_dead_h.size(), cudaMemcpyHostToDevice, st));
+            for (uint8_t b : L.list_dead_h) S.list_ndead += b ? 1 : 0;
         }
-        TRY(cnorms.ensure(sizeof(float) * (size_t)std::max(L.nc, 1), 0, st, true));
+        TRY(S.cnorms.ensure(sizeof(float) * (size_t)std::max(L.nc, 1), 0, st, true));
         if (h->metric == kCosine) {
-            CK(launch_row_norms_exact(L.centroids.as<float>(), L.nc, dim, dim, cnorms.as<float>(), st));
+            CK(launch_row_norms_exact(L.centroids.as<float>(), L.nc, dim, dim, S.cnorms.as<float>(), st));
             if (h->kind == PYROPE_IVF_FLAT && L.list_total) {
-                TRY(list_norms.ensure(sizeof(float) * (size_t)L.list_total, 0, st, true));
-                CK(launch_row_norms_exact(L.list_payload.as<float>(), L.list_total, dim, dim, list_norms.as<float>(), st));
+                TRY(S.list_norms.ensure(sizeof(float) * (size_t)L.list_total, 0, st, true));
+                CK(launch_row_norms_exact(L.list_payload.as<float>(), L.list_total, dim, dim, S.list_norms.as<float>(), st));
             }
         }
     }
     CK(cudaStreamSynchronize(st));
+    return PYROPE_OK;
+}
 
-    // ---- nothing below can fail: swap the parsed state in
+// caller holds h->mu; nothing here can fail: swap the staged state in
+void load_commit(Index* h, StagedLoad& S) {
+    LoadedSnapshot& L = S.L;
+    Segment& ns = S.ns;
     auto take = [](DevBuf& dst, DevBuf& src) { std::swap(dst.p, src.p); std::swap(dst.bytes, src.bytes); src.release(); };
     Segment& s = h->seg;
     take(s.X, ns.X); take(s.dead, ns.dead); take(s.labels, ns.labels); take(s.norms, ns.norms);
@@ -2048,20 +2064,20 @@ int pyrope_index_load(pyrope_index* h, const char* path) {
     take(h->centroids, L.centroids); take(h->codebook, L.codebook);
     h->cmax_for = nullptr; h->lm_cb16_ok = false;
     h->ksub.swap(L.ksub);
-    if (ksub_d.p) take(h->ksub_d, ksub_d);
+    if (S.ksub_d.p) take(h->ksub_d, S.ksub_d);
     h->list_total = L.list_total;
     h->lists_version++;
-    h->list_ndead = list_ndead;
+    h->list_ndead = S.list_ndead;
     h->list_dead_h.swap(L.list_dead_h);
-    take(h->list_dead, list_dead);
-    h->max_list_len = max_list_len;
+    take(h->list_dead, S.list_dead);
+    h->max_list_len = S.max_list_len;
     if (L.built) {
         h->list_off_h.swap(L.list_off_h);
-        take(h->list_off, list_off); take(h->list_rows, L.list_rows); take(h->list_labels, L.list_labels);
+        take(h->list_off, S.list_off); take(h->list_rows, L.list_rows); take(h->list_labels, L.list_labels);
         if (h->kind == PYROPE_IVF_FLAT) take(h->list_vecs, L.list_payload); else take(h->list_codes, L.list_payload);
         h->lm_codes16_ok = false;
-        take(h->cnorms, cnorms);
-        if (list_norms.p) take(h->list_norms, list_norms);
+        take(h->cnorms, S.cnorms);
+        if (S.list_norms.p) take(h->list_norms, S.list_norms);
     } else {
         h->list_off_h.clear();
     }
@@ -2072,12 +2088,52 @@ int pyrope_index_load(pyrope_index* h, const char* path) {
     // off no loaded row has a quantised form (:312-322 keeps such rows invisible to a later quantised search).
     if (h->kind == PYROPE_FLAT && (h->sq8 || h->x8.p)) {
         h->x8_cap = 0;
-        sq8_rows(h, 0, L.nslots);  // best effort: the rows themselves are already in place
+        sq8_rows(h, 0, h->seg.nslots);  // best effort: the rows themselves are already in place
     }
     h->tc_cent.invalidate();
     if (h->kind != PYROPE_FLAT) { h->row_loc.assign((size_t)h->next_row, -1); h->lists_loc_valid = false; }
+}
+}  // namespace
+extern "C" {
+
+int pyrope_index_load(pyrope_index* h, const char* path) {
+    if (!h || !path || !*path) return fail(PYROPE_ERR_INVALID_ARG, "Path cannot be empty");
+    std::lock_guard<std::mutex> g(h->mu);
+    StagedLoad S;
+    TRY(load_prepare(h, path, S));
+    load_commit(h, S);
     return PYROPE_OK;
 }
+
+// ---- internal (not in the public header): the two halves of pyrope_index_load for pyrope_sharded_load.  _prepare
+// returns an opaque staged snapshot and the shard identity / row count its file records; _commit swaps it in and frees
+// it, _discard frees it unused.  Both run with the index's device current.
+int pyrope_internal_index_load_prepare(pyrope_index* h, const char* path, void** staged_out, int32_t* shard_rank_out,
+                                       int32_t* shard_world_out, int64_t* next_row_out) {
+    if (!h || !path || !*path || !staged_out) return fail(PYROPE_ERR_INVALID_ARG, "Path cannot be empty");
+    *staged_out = nullptr;
+    std::lock_guard<std::mutex> g(h->mu);
+    StagedLoad* S = new (std::nothrow) StagedLoad();
+    if (!S) return fail(PYROPE_ERR_OOM, "out of host memory");
+    int rc = load_prepare(h, path, *S);
+    if (rc != PYROPE_OK) { delete S; return rc; }
+    if (shard_rank_out) *shard_rank_out = S->L.shard_rank;
+    if (shard_world_out) *shard_world_out = S->L.shard_world;
+    if (next_row_out) *next_row_out = S->L.next_row;
+    *staged_out = S;
+    return PYROPE_OK;
+}
+
+void pyrope_internal_index_load_commit(pyrope_index* h, void* staged) {
+    StagedLoad* S = static_cast<StagedLoad*>(staged);
+    {
+        std::lock_guard<std::mutex> g(h->mu);
+        load_commit(h, *S);
+    }
+    delete S;
+}
+
+void pyrope_internal_index_load_discard(void* staged) { delete static_cast<StagedLoad*>(staged); }
 
 // header peek for the string-id layer: rows ever added according to the snapshot (validates the magic only)
 int pyrope_internal_snapshot_next_row(const char* path, int64_t* next_row_out) {
@@ -2233,14 +2289,32 @@ int pyrope_topk_merge_device(int64_t nq, int parts, int k_in, int k_out, const f
 // ---- Head+Tail on device (DeltaVectorIndex.cs) ------------------------------------------------------
 }  // extern "C"
 
+// csrc/sharded.cu (internal, not part of the public header): the pieces of a sharded index a Head+Tail over it uses.
+// The search is pyrope_sharded_search_batch_device whose shards first wait for q_ready (a CUDA event, may be null);
+// absorb is the compaction's "_tail.Add per row" step on every shard (see tail_absorb below).
+extern "C" int pyrope_internal_sharded_search_device(pyrope_sharded* s, int64_t nq, const float* dQ_dev0, int topk,
+                                                     int64_t max_scans, int nprobe, float* d_scores_dev0,
+                                                     int64_t* d_rows_dev0, int32_t* d_counts_dev0, void* q_ready);
+extern "C" int pyrope_internal_sharded_absorb(pyrope_sharded* s, int64_t n, const float* dX, const int64_t* dL, int src_device,
+                                              const int64_t* labels_host, int64_t* tail_rows_out);
+
 struct pyrope_delta {
     pyrope_index* head = nullptr;
-    pyrope_index* tail = nullptr;
+    pyrope_index* tail = nullptr;    // single-device tail, or
+    pyrope_sharded* stail = nullptr;  // a tail sharded over the devices of the box (pyrope_delta_create_sharded)
+    int tail_devices = 1;
     std::mutex mu;
     DevBuf ps, pl, pc, q, os, ol, oc;  // partial (head | tail) results, staged queries, merged outputs
+    cudaEvent_t q_ready = nullptr;     // sharded tail: the queries are in place on the head's stream
 };
 
 namespace {
+
+// an error raised by csrc/sharded.cu: keep its code, copy its message
+int spass(int rc) {
+    if (rc != PYROPE_OK) g_err = pyrope_sharded_last_error();
+    return rc;
+}
 
 // DeltaVectorIndex.Search:76-122 for nq queries: head top-k, tail top-k (same options, :85,88), merge by id with
 // the head's copy winning, descending, Take(topK) — one stream, no host round trip between the three stages.
@@ -2252,12 +2326,24 @@ int delta_search_device(pyrope_delta* d, int64_t nq, const float* dQ, int topk, 
     TRY(d->ps.ensure(sizeof(float) * 2 * per, 0, st));
     TRY(d->pl.ensure(sizeof(int64_t) * 2 * per, 0, st));
     TRY(d->pc.ensure(sizeof(int32_t) * 2 * (size_t)nq, 0, st));
+    if (d->stail) CK(cudaEventRecord(d->q_ready, st));  // before the head's search: the tail does not wait for it
     {
         std::lock_guard<std::mutex> g(hd->mu);
         TRY(search_device(hd, nq, dQ, topk, max_scans, nprobe, d->ps.as<float>(), d->pl.as<int64_t>(),
                           d->pc.as<int32_t>(), st));
     }
-    {
+    if (d->stail) {
+        // The head's top-k is enqueued and overlaps the tail's coarse stage.  The sharded search merges the shards'
+        // lists down to the tail's top k first: the reference asks the tail for topK (:88), so an id the head also
+        // holds costs the result one tail entry, and a single merge of head and per-shard lists would refill that slot
+        // with the tail's (k+1)-th.  An IVF_PQ tail ignores MaxScans (IvfPqVectorIndex.cs), an IVF_FLAT tail over
+        // several devices refuses it (UNSUPPORTED, as pyrope_sharded_search_batch does).
+        Index* t0 = nullptr;
+        TRY(spass(pyrope_sharded_shard(d->stail, 0, &t0, nullptr)));
+        TRY(spass(pyrope_internal_sharded_search_device(d->stail, nq, dQ, topk, t0->kind == PYROPE_IVF_PQ ? -1 : max_scans,
+                                                        nprobe, d->ps.as<float>() + per, d->pl.as<int64_t>() + per,
+                                                        d->pc.as<int32_t>() + nq, d->q_ready)));
+    } else {
         std::lock_guard<std::mutex> g(tl->mu);
         if (tl->kind == PYROPE_IVF_FLAT && max_scans >= 0 && tl->list_ndead > 0) TRY(compact_lists(tl));
         TRY(search_device(tl, nq, dQ, topk, max_scans, nprobe, d->ps.as<float>() + per, d->pl.as<int64_t>() + per,
@@ -2272,9 +2358,14 @@ int delta_validate(pyrope_delta* d, int64_t nq, const float* Q, int topk) {
     if (!d) return fail(PYROPE_ERR_INVALID_ARG, "delta handle is null");
     if (nq < 0 || (nq > 0 && !Q)) return fail(PYROPE_ERR_INVALID_ARG, "query is null");
     if (topk <= 0) return fail(PYROPE_ERR_OUT_OF_RANGE, "topK must be positive.");  // the FLAT head throws first
-    if (2 * topk > kMergeMaxCandidates || topk > kMaxTopK)
-        return fail(PYROPE_ERR_UNSUPPORTED, "topK %d exceeds the supported maximum %d", topk, kMaxTopK);
+    const int lim = std::min(kMaxTopK, kMergeMaxCandidates / std::max(2, d->tail_devices));
+    if (topk > lim) return fail(PYROPE_ERR_UNSUPPORTED, "topK %d exceeds the supported maximum %d", topk, lim);
     return PYROPE_OK;
+}
+
+// the tail's last search ran on the head's stream: do not leave it a handle the head may destroy first
+void delta_forget_stream(pyrope_delta* d, cudaStream_t st) {
+    if (d->tail && d->tail->last_stream == st) d->tail->last_stream = nullptr;
 }
 
 }  // namespace
@@ -2297,11 +2388,41 @@ int pyrope_delta_create(pyrope_index* head, pyrope_index* tail, pyrope_delta** o
     return PYROPE_OK;
 }
 
+int pyrope_delta_create_sharded(pyrope_index* head, pyrope_sharded* tail, pyrope_delta** out) {
+    if (!out) return fail(PYROPE_ERR_INVALID_ARG, "out is null");
+    *out = nullptr;
+    if (!head || !tail) return fail(PYROPE_ERR_INVALID_ARG, "index handle is null");
+    Index* t0 = nullptr;
+    int dev0 = -1, n = 0;
+    TRY(spass(pyrope_sharded_shard(tail, 0, &t0, &dev0)));
+    TRY(spass(pyrope_sharded_device_count(tail, &n)));
+    if (head == t0) return fail(PYROPE_ERR_INVALID_ARG, "Head and Tail must be different indexes");
+    if (head->dim != t0->dim) return fail(PYROPE_ERR_INVALID_ARG, "Head and Tail dimensions must match");
+    if (head->metric != t0->metric) return fail(PYROPE_ERR_INVALID_ARG, "Head and Tail metrics must match");
+    if (head->kind != PYROPE_FLAT) return fail(PYROPE_ERR_UNSUPPORTED, "the head must be a FLAT index");
+    if (head->device != dev0)
+        return fail(PYROPE_ERR_INVALID_ARG, "the head lives on device %d, the sharded tail's first device is %d", head->device, dev0);
+    if (t0->kind == PYROPE_FLAT) return fail(PYROPE_ERR_UNSUPPORTED, "a sharded tail must be IVF_FLAT or IVF_PQ");
+    pyrope_delta* d = new (std::nothrow) pyrope_delta();
+    if (!d) return fail(PYROPE_ERR_OOM, "out of host memory");
+    int cur = 0;
+    cudaGetDevice(&cur);
+    cudaSetDevice(head->device);  // the event is recorded on the head's stream
+    cudaError_t e = cudaEventCreateWithFlags(&d->q_ready, cudaEventDisableTiming);
+    cudaSetDevice(cur);
+    if (e != cudaSuccess) { delete d; return fail(PYROPE_ERR_CUDA, "cudaEventCreate: %s", cudaGetErrorString(e)); }
+    d->head = head;
+    d->stail = tail;
+    d->tail_devices = n;
+    *out = d;
+    return PYROPE_OK;
+}
+
 int pyrope_delta_destroy(pyrope_delta* d) {
     if (!d) return PYROPE_OK;
     cudaStreamSynchronize(d->head->stream);
-    // the tail's last search ran on the head's stream: do not leave it a handle the head may destroy first
-    if (d->tail->last_stream == d->head->stream) d->tail->last_stream = nullptr;
+    delta_forget_stream(d, d->head->stream);
+    if (d->q_ready) cudaEventDestroy(d->q_ready);
     delete d;
     return PYROPE_OK;
 }
@@ -2316,7 +2437,7 @@ int pyrope_delta_search_batch_device(pyrope_delta* d, int64_t nq, const float* d
     TRY(delta_search_device(d, nq, dQ, topk, max_scans, nprobe, d_scores, d_labels, d_counts, st));
     if (!stream) {
         CK(cudaStreamSynchronize(st));
-        if (d->tail->last_stream == st) d->tail->last_stream = nullptr;
+        delta_forget_stream(d, st);
     }
     return PYROPE_OK;
 }
@@ -2340,13 +2461,143 @@ int pyrope_delta_search_batch(pyrope_delta* d, int64_t nq, const float* Q, int t
     CK(cudaMemcpyAsync(labels_out, d->ol.p, sizeof(int64_t) * (size_t)nq * topk, cudaMemcpyDeviceToHost, st));
     CK(cudaMemcpyAsync(counts_out, d->oc.p, sizeof(int32_t) * (size_t)nq, cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
-    if (d->tail->last_stream == st) d->tail->last_stream = nullptr;
+    delta_forget_stream(d, st);
     return PYROPE_OK;
 }
 
 }  // extern "C"
 
 namespace {
+// 1. of DeltaVectorIndex.Build: the head's live rows in scan order (bfHead.Scan(), DeltaVectorIndex.cs:133), gathered on
+// the head's device into mx (n x dim) / ml (labels, also copied to the host as mlab).  Caller holds hd->mu.
+int gather_head_rows(Index* hd, int64_t n, DevBuf& mx, DevBuf& ml, std::vector<int64_t>& mlab, cudaStream_t st) {
+    const Segment& hs = hd->seg;
+    const int dim = hd->dim;
+    std::vector<int64_t> slots;
+    slots.reserve((size_t)n);
+    for (int64_t i = 0; i < hs.nslots; ++i)
+        if (!hs.dead_h[(size_t)i]) slots.push_back(i);
+    DevBuf idx;
+    TRY(idx.ensure(sizeof(int64_t) * (size_t)n, 0, st, true));
+    TRY(mx.ensure(sizeof(float) * (size_t)n * dim, 0, st, true));
+    TRY(ml.ensure(sizeof(int64_t) * (size_t)n, 0, st, true));
+    CK(cudaStreamSynchronize(hd->stream));
+    CK(cudaMemcpyAsync(idx.p, slots.data(), sizeof(int64_t) * (size_t)n, cudaMemcpyHostToDevice, st));
+    CK(launch_gather_rows(hs.X.p, (int64_t)dim * 4, idx.as<int64_t>(), n, mx.p, st));
+    CK(launch_gather_rows(hs.labels.p, 8, idx.as<int64_t>(), n, ml.p, st));
+    mlab.resize((size_t)n);
+    CK(cudaMemcpyAsync(mlab.data(), ml.p, sizeof(int64_t) * (size_t)n, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    return PYROPE_OK;
+}
+
+// 2. of DeltaVectorIndex.Build: _tail.Add(id, vec) per row (:146) for n rows mx / ml (device, on the tail's device; labels
+// also on the host as mlab): an id the tail already buffers is overwritten in place (Dictionary semantics,
+// IvfFlatVectorIndex.cs:47 / IvfPqVectorIndex.cs:42); an id that sits in an inverted list is shadowed by the new buffer
+// row until the tail's Build folds it in.  tail_rows_out (nullable): the tail row ordinal now holding each row.  Caller
+// holds tl->mu with the tail's last search finished.
+int tail_absorb(Index* tl, int64_t n, const float* mx, const int64_t* ml, const int64_t* mlab, int64_t* tail_rows_out) {
+    cudaStream_t st = tl->stream;
+    const int dim = tl->dim;
+    std::vector<int64_t> order((size_t)n);  // moved rows sorted by label
+    for (int64_t i = 0; i < n; ++i) order[(size_t)i] = i;
+    std::sort(order.begin(), order.end(), [&](int64_t a, int64_t b) { return mlab[(size_t)a] < mlab[(size_t)b]; });
+    std::vector<int64_t> sorted((size_t)n);
+    for (int64_t i = 0; i < n; ++i) sorted[(size_t)i] = mlab[(size_t)order[(size_t)i]];
+    std::vector<int64_t> target((size_t)n, -1);  // moved row -> tail buffer slot it overwrites
+    DevBuf dsorted, where;
+    Segment& ts = tl->seg;
+    const bool lists_matter = tl->built && tl->kind == PYROPE_IVF_FLAT && tl->list_total > 0;
+    if (ts.live > 0 || lists_matter) {
+        TRY(dsorted.ensure(sizeof(int64_t) * (size_t)n, 0, st, true));
+        CK(cudaMemcpyAsync(dsorted.p, sorted.data(), sizeof(int64_t) * (size_t)n, cudaMemcpyHostToDevice, st));
+    }
+    if (ts.live > 0) {
+        TRY(where.ensure(sizeof(int64_t) * (size_t)ts.nslots, 0, st, true));
+        CK(launch_find_labels(ts.labels.as<int64_t>(), ts.dead.as<uint8_t>(), ts.nslots, dsorted.as<int64_t>(), n,
+                              where.as<int64_t>(), st));
+        std::vector<int64_t> wh((size_t)ts.nslots);
+        CK(cudaMemcpyAsync(wh.data(), where.p, sizeof(int64_t) * wh.size(), cudaMemcpyDeviceToHost, st));
+        CK(cudaStreamSynchronize(st));
+        for (int64_t s = 0; s < ts.nslots; ++s)
+            if (wh[(size_t)s] >= 0) target[(size_t)order[(size_t)wh[(size_t)s]]] = s;
+    }
+    if (lists_matter) {
+        TRY(ensure_list_dead(tl));
+        TRY(where.ensure(sizeof(int64_t) * (size_t)tl->list_total, 0, st, true));
+        CK(launch_find_labels(tl->list_labels.as<int64_t>(), tl->list_dead.as<uint8_t>(), tl->list_total,
+                              dsorted.as<int64_t>(), n, where.as<int64_t>(), st));
+        std::vector<int64_t> wh((size_t)tl->list_total);
+        CK(cudaMemcpyAsync(wh.data(), where.p, sizeof(int64_t) * wh.size(), cudaMemcpyDeviceToHost, st));
+        CK(cudaStreamSynchronize(st));
+        bool any = false;
+        for (int64_t i = 0; i < tl->list_total; ++i)
+            if (wh[(size_t)i] >= 0) {
+                if (!tl->list_dead_h[(size_t)i]) tl->list_ndead++;
+                tl->lists_version++;
+                tl->list_dead_h[(size_t)i] |= 2;
+                any = true;
+            }
+        if (any)
+            CK(cudaMemcpyAsync(tl->list_dead.p, tl->list_dead_h.data(), (size_t)tl->list_total, cudaMemcpyHostToDevice, st));
+    }
+    std::vector<int64_t> over_src, over_dst, app_src;
+    for (int64_t i = 0; i < n; ++i) {
+        if (target[(size_t)i] >= 0) { over_src.push_back(i); over_dst.push_back(target[(size_t)i]); }
+        else app_src.push_back(i);
+    }
+    if (!over_src.empty()) {
+        const int64_t no = (int64_t)over_src.size();
+        DevBuf a, b, tmp;
+        TRY(a.ensure(sizeof(int64_t) * (size_t)no, 0, st, true));
+        TRY(b.ensure(sizeof(int64_t) * (size_t)no, 0, st, true));
+        TRY(tmp.ensure(sizeof(float) * (size_t)no * dim, 0, st, true));
+        CK(cudaMemcpyAsync(a.p, over_src.data(), sizeof(int64_t) * (size_t)no, cudaMemcpyHostToDevice, st));
+        CK(cudaMemcpyAsync(b.p, over_dst.data(), sizeof(int64_t) * (size_t)no, cudaMemcpyHostToDevice, st));
+        CK(launch_gather_rows(mx, (int64_t)dim * 4, a.as<int64_t>(), no, tmp.p, st));
+        CK(launch_scatter_rows(tmp.p, (int64_t)dim * 4, b.as<int64_t>(), no, ts.X.p, st));
+        if (ts.cosine)
+            for (int64_t i = 0; i < no; ++i)
+                CK(launch_row_norms_exact(ts.X.as<float>() + over_dst[(size_t)i] * dim, 1, dim, dim,
+                                          ts.norms.as<float>() + over_dst[(size_t)i], st));
+        ts.tc_dirty = true;
+        CK(cudaStreamSynchronize(st));
+        if (tl->kind == PYROPE_FLAT)
+            for (int64_t i = 0; i < no; ++i) TRY(sq8_rows(tl, over_dst[(size_t)i], 1));
+        if (tail_rows_out)
+            for (int64_t i = 0; i < no; ++i)
+                tail_rows_out[over_src[(size_t)i]] =
+                    tl->kind == PYROPE_FLAT ? over_dst[(size_t)i] : ts.slot_row[(size_t)over_dst[(size_t)i]];
+    }
+    if (!app_src.empty()) {
+        const int64_t na = (int64_t)app_src.size();
+        const float* ax = mx;
+        const int64_t* al = ml;
+        DevBuf a, tx, tlab;
+        if (na != n) {
+            TRY(a.ensure(sizeof(int64_t) * (size_t)na, 0, st, true));
+            TRY(tx.ensure(sizeof(float) * (size_t)na * dim, 0, st, true));
+            TRY(tlab.ensure(sizeof(int64_t) * (size_t)na, 0, st, true));
+            CK(cudaMemcpyAsync(a.p, app_src.data(), sizeof(int64_t) * (size_t)na, cudaMemcpyHostToDevice, st));
+            CK(launch_gather_rows(mx, (int64_t)dim * 4, a.as<int64_t>(), na, tx.p, st));
+            CK(launch_gather_rows(ml, 8, a.as<int64_t>(), na, tlab.p, st));
+            CK(cudaStreamSynchronize(st));
+            ax = tx.as<float>();
+            al = tlab.as<int64_t>();
+        }
+        const int64_t first = tl->next_row;
+        if (tl->kind != PYROPE_FLAT) tl->row_loc.resize((size_t)(first + na), -1);
+        tl->next_row += na;
+        const int64_t slot0 = ts.nslots;
+        int r = seg_append(tl, na, ax, true, al, true, first);
+        if (r != PYROPE_OK) { tl->next_row = first; return r; }
+        if (tl->kind == PYROPE_FLAT) TRY(sq8_rows(tl, slot0, na));  // a FLAT tail with EnableQuantization
+        if (tail_rows_out)
+            for (int64_t i = 0; i < na; ++i) tail_rows_out[app_src[(size_t)i]] = first + i;
+    }
+    return PYROPE_OK;
+}
+
 // DeltaVectorIndex.Build :124-158 in two steps a caller can take apart: MOVE (head rows -> tail buffer, head tombstoned)
 // and BUILD (the tail's Build).  A host that keeps id tables updates them after the move whatever the build returns.
 int delta_compact_impl(pyrope_delta* d, int64_t* moved_out, int64_t* tail_rows_out, bool do_move, bool do_build) {
@@ -2354,131 +2605,32 @@ int delta_compact_impl(pyrope_delta* d, int64_t* moved_out, int64_t* tail_rows_o
     if (moved_out) *moved_out = 0;
     std::lock_guard<std::mutex> g(d->mu);
     Index* hd = d->head;
-    Index* tl = d->tail;
     std::lock_guard<std::mutex> gh(hd->mu);
-    std::lock_guard<std::mutex> gt(tl->mu);
     if (hd->last_stream) CK(cudaStreamSynchronize(hd->last_stream));
-    if (tl->last_stream) CK(cudaStreamSynchronize(tl->last_stream));
-    cudaStream_t st = tl->stream;
     Segment& hs = hd->seg;
-    const int dim = hd->dim;
     const int64_t n = do_move ? hs.live : 0;
+    if (d->stail) {
+        // sharded tail: the rows are gathered once on the head's device; every shard copies them over (peer copies)
+        // and applies the same step to its replica of the buffer and to the lists it owns
+        if (n > 0) {
+            DevBuf mx, ml;
+            std::vector<int64_t> mlab;
+            TRY(gather_head_rows(hd, n, mx, ml, mlab, hd->stream));
+            TRY(spass(pyrope_internal_sharded_absorb(d->stail, n, mx.as<float>(), ml.as<int64_t>(), hd->device, mlab.data(),
+                                                     tail_rows_out)));
+        }
+    } else {
+        Index* tl = d->tail;
+        std::lock_guard<std::mutex> gt(tl->mu);
+        if (tl->last_stream) CK(cudaStreamSynchronize(tl->last_stream));
+        if (n > 0) {
+            DevBuf mx, ml;
+            std::vector<int64_t> mlab;
+            TRY(gather_head_rows(hd, n, mx, ml, mlab, tl->stream));
+            TRY(tail_absorb(tl, n, mx.as<float>(), ml.as<int64_t>(), mlab.data(), tail_rows_out));
+        }
+    }
     if (n > 0) {
-        // 1. the head's live rows in scan order (bfHead.Scan(), DeltaVectorIndex.cs:133)
-        std::vector<int64_t> slots;
-        slots.reserve((size_t)n);
-        for (int64_t i = 0; i < hs.nslots; ++i)
-            if (!hs.dead_h[(size_t)i]) slots.push_back(i);
-        DevBuf idx, mx, ml;
-        TRY(idx.ensure(sizeof(int64_t) * (size_t)n, 0, st, true));
-        TRY(mx.ensure(sizeof(float) * (size_t)n * dim, 0, st, true));
-        TRY(ml.ensure(sizeof(int64_t) * (size_t)n, 0, st, true));
-        CK(cudaStreamSynchronize(hd->stream));
-        CK(cudaMemcpyAsync(idx.p, slots.data(), sizeof(int64_t) * (size_t)n, cudaMemcpyHostToDevice, st));
-        CK(launch_gather_rows(hs.X.p, (int64_t)dim * 4, idx.as<int64_t>(), n, mx.p, st));
-        CK(launch_gather_rows(hs.labels.p, 8, idx.as<int64_t>(), n, ml.p, st));
-        std::vector<int64_t> mlab((size_t)n);
-        CK(cudaMemcpyAsync(mlab.data(), ml.p, sizeof(int64_t) * (size_t)n, cudaMemcpyDeviceToHost, st));
-        CK(cudaStreamSynchronize(st));
-        // 2. _tail.Add(id, vec) per row (:146): an id the tail already buffers is overwritten in place
-        //    (Dictionary semantics, IvfFlatVectorIndex.cs:47 / IvfPqVectorIndex.cs:42); an id that sits in an
-        //    inverted list is shadowed by the new buffer row until the Build below folds it in.
-        std::vector<int64_t> order((size_t)n);  // moved rows sorted by label
-        for (int64_t i = 0; i < n; ++i) order[(size_t)i] = i;
-        std::sort(order.begin(), order.end(), [&](int64_t a, int64_t b) { return mlab[(size_t)a] < mlab[(size_t)b]; });
-        std::vector<int64_t> sorted((size_t)n);
-        for (int64_t i = 0; i < n; ++i) sorted[(size_t)i] = mlab[(size_t)order[(size_t)i]];
-        std::vector<int64_t> target((size_t)n, -1);  // moved row -> tail buffer slot it overwrites
-        DevBuf dsorted, where;
-        Segment& ts = tl->seg;
-        const bool lists_matter = tl->built && tl->kind == PYROPE_IVF_FLAT && tl->list_total > 0;
-        if (ts.live > 0 || lists_matter) {
-            TRY(dsorted.ensure(sizeof(int64_t) * (size_t)n, 0, st, true));
-            CK(cudaMemcpyAsync(dsorted.p, sorted.data(), sizeof(int64_t) * (size_t)n, cudaMemcpyHostToDevice, st));
-        }
-        if (ts.live > 0) {
-            TRY(where.ensure(sizeof(int64_t) * (size_t)ts.nslots, 0, st, true));
-            CK(launch_find_labels(ts.labels.as<int64_t>(), ts.dead.as<uint8_t>(), ts.nslots, dsorted.as<int64_t>(), n,
-                                  where.as<int64_t>(), st));
-            std::vector<int64_t> wh((size_t)ts.nslots);
-            CK(cudaMemcpyAsync(wh.data(), where.p, sizeof(int64_t) * wh.size(), cudaMemcpyDeviceToHost, st));
-            CK(cudaStreamSynchronize(st));
-            for (int64_t s = 0; s < ts.nslots; ++s)
-                if (wh[(size_t)s] >= 0) target[(size_t)order[(size_t)wh[(size_t)s]]] = s;
-        }
-        if (lists_matter) {
-            TRY(ensure_list_dead(tl));
-            TRY(where.ensure(sizeof(int64_t) * (size_t)tl->list_total, 0, st, true));
-            CK(launch_find_labels(tl->list_labels.as<int64_t>(), tl->list_dead.as<uint8_t>(), tl->list_total,
-                                  dsorted.as<int64_t>(), n, where.as<int64_t>(), st));
-            std::vector<int64_t> wh((size_t)tl->list_total);
-            CK(cudaMemcpyAsync(wh.data(), where.p, sizeof(int64_t) * wh.size(), cudaMemcpyDeviceToHost, st));
-            CK(cudaStreamSynchronize(st));
-            bool any = false;
-            for (int64_t i = 0; i < tl->list_total; ++i)
-                if (wh[(size_t)i] >= 0) {
-                    if (!tl->list_dead_h[(size_t)i]) tl->list_ndead++;
-                    tl->lists_version++;
-                    tl->list_dead_h[(size_t)i] |= 2;
-                    any = true;
-                }
-            if (any)
-                CK(cudaMemcpyAsync(tl->list_dead.p, tl->list_dead_h.data(), (size_t)tl->list_total, cudaMemcpyHostToDevice, st));
-        }
-        std::vector<int64_t> over_src, over_dst, app_src;
-        for (int64_t i = 0; i < n; ++i) {
-            if (target[(size_t)i] >= 0) { over_src.push_back(i); over_dst.push_back(target[(size_t)i]); }
-            else app_src.push_back(i);
-        }
-        if (!over_src.empty()) {
-            const int64_t no = (int64_t)over_src.size();
-            DevBuf a, b, tmp;
-            TRY(a.ensure(sizeof(int64_t) * (size_t)no, 0, st, true));
-            TRY(b.ensure(sizeof(int64_t) * (size_t)no, 0, st, true));
-            TRY(tmp.ensure(sizeof(float) * (size_t)no * dim, 0, st, true));
-            CK(cudaMemcpyAsync(a.p, over_src.data(), sizeof(int64_t) * (size_t)no, cudaMemcpyHostToDevice, st));
-            CK(cudaMemcpyAsync(b.p, over_dst.data(), sizeof(int64_t) * (size_t)no, cudaMemcpyHostToDevice, st));
-            CK(launch_gather_rows(mx.p, (int64_t)dim * 4, a.as<int64_t>(), no, tmp.p, st));
-            CK(launch_scatter_rows(tmp.p, (int64_t)dim * 4, b.as<int64_t>(), no, ts.X.p, st));
-            if (ts.cosine)
-                for (int64_t i = 0; i < no; ++i)
-                    CK(launch_row_norms_exact(ts.X.as<float>() + over_dst[(size_t)i] * dim, 1, dim, dim,
-                                              ts.norms.as<float>() + over_dst[(size_t)i], st));
-            ts.tc_dirty = true;
-            CK(cudaStreamSynchronize(st));
-            if (tl->kind == PYROPE_FLAT)
-                for (int64_t i = 0; i < no; ++i) TRY(sq8_rows(tl, over_dst[(size_t)i], 1));
-            if (tail_rows_out)
-                for (int64_t i = 0; i < no; ++i)
-                    tail_rows_out[over_src[(size_t)i]] =
-                        tl->kind == PYROPE_FLAT ? over_dst[(size_t)i] : ts.slot_row[(size_t)over_dst[(size_t)i]];
-        }
-        if (!app_src.empty()) {
-            const int64_t na = (int64_t)app_src.size();
-            const float* ax = mx.as<float>();
-            const int64_t* al = ml.as<int64_t>();
-            DevBuf a, tx, tlab;
-            if (na != n) {
-                TRY(a.ensure(sizeof(int64_t) * (size_t)na, 0, st, true));
-                TRY(tx.ensure(sizeof(float) * (size_t)na * dim, 0, st, true));
-                TRY(tlab.ensure(sizeof(int64_t) * (size_t)na, 0, st, true));
-                CK(cudaMemcpyAsync(a.p, app_src.data(), sizeof(int64_t) * (size_t)na, cudaMemcpyHostToDevice, st));
-                CK(launch_gather_rows(mx.p, (int64_t)dim * 4, a.as<int64_t>(), na, tx.p, st));
-                CK(launch_gather_rows(ml.p, 8, a.as<int64_t>(), na, tlab.p, st));
-                CK(cudaStreamSynchronize(st));
-                ax = tx.as<float>();
-                al = tlab.as<int64_t>();
-            }
-            const int64_t first = tl->next_row;
-            if (tl->kind != PYROPE_FLAT) tl->row_loc.resize((size_t)(first + na), -1);
-            tl->next_row += na;
-            const int64_t slot0 = ts.nslots;
-            int r = seg_append(tl, na, ax, true, al, true, first);
-            if (r != PYROPE_OK) { tl->next_row = first; return r; }
-            if (tl->kind == PYROPE_FLAT) TRY(sq8_rows(tl, slot0, na));  // a FLAT tail with EnableQuantization
-            if (tail_rows_out)
-                for (int64_t i = 0; i < na; ++i) tail_rows_out[app_src[(size_t)i]] = first + i;
-        }
         // 3. _head.Delete(id) per row (:147): tombstones, slots stay (BruteForceVectorIndex.cs:231-254)
         CK(cudaMemsetAsync(hs.dead.p, 1, (size_t)hs.nslots, hd->stream));
         std::fill(hs.dead_h.begin(), hs.dead_h.end(), (uint8_t)1);
@@ -2490,6 +2642,9 @@ int delta_compact_impl(pyrope_delta* d, int64_t* moved_out, int64_t* tail_rows_o
     }
     // 4. _head.Build() is a no-op for FLAT; _tail.Build() (:151-152)
     if (!do_build) return PYROPE_OK;
+    if (d->stail) return spass(pyrope_sharded_build(d->stail));
+    Index* tl = d->tail;
+    std::lock_guard<std::mutex> gt(tl->mu);
     if (tl->kind == PYROPE_IVF_FLAT) return build_ivfflat(tl);
     if (tl->kind == PYROPE_IVF_PQ) return build_ivfpq(tl);
     return PYROPE_OK;
@@ -2497,6 +2652,25 @@ int delta_compact_impl(pyrope_delta* d, int64_t* moved_out, int64_t* tail_rows_o
 }  // namespace
 
 extern "C" {
+
+// ---- internal (not in the public header): the compaction's per-tail step for csrc/sharded.cu, run on each shard's
+// thread.  _reserve makes room for n more buffer rows before any shard writes; _absorb is tail_absorb above.
+int pyrope_internal_tail_reserve(pyrope_index* tl, int64_t n) {
+    if (!tl || n < 0) return fail(PYROPE_ERR_INVALID_ARG, "bad argument");
+    std::lock_guard<std::mutex> g(tl->mu);
+    TRY(tl->seg.reserve(tl->seg.nslots + n, tl->stream, false));
+    CK(cudaStreamSynchronize(tl->stream));
+    return PYROPE_OK;
+}
+
+int pyrope_internal_tail_absorb(pyrope_index* tl, int64_t n, const float* dX, const int64_t* dL, const int64_t* labels_host,
+                                int64_t* tail_rows_out) {
+    if (!tl || n < 0 || (n > 0 && (!dX || !dL || !labels_host))) return fail(PYROPE_ERR_INVALID_ARG, "bad argument");
+    std::lock_guard<std::mutex> g(tl->mu);
+    if (tl->last_stream) CK(cudaStreamSynchronize(tl->last_stream));
+    if (n == 0) return PYROPE_OK;
+    return tail_absorb(tl, n, dX, dL, labels_host, tail_rows_out);
+}
 
 int pyrope_delta_compact(pyrope_delta* d, int64_t* moved_out, int64_t* tail_rows_out) {
     return delta_compact_impl(d, moved_out, tail_rows_out, true, true);
@@ -2510,6 +2684,12 @@ int pyrope_delta_stats(pyrope_delta* d, int64_t* count_out) {
     if (!d || !count_out) return fail(PYROPE_ERR_INVALID_ARG, "null argument");
     // DeltaVectorIndex.cs:232-236: plain sum of both sides (duplicates counted twice, as in the reference)
     Index* hd = d->head;
+    if (d->stail) {
+        int64_t t = 0;
+        TRY(spass(pyrope_sharded_stats(d->stail, &t)));
+        *count_out = hd->seg.live + t;
+        return PYROPE_OK;
+    }
     Index* tl = d->tail;
     *count_out = hd->seg.live + tl->seg.live + (tl->built ? tl->list_total - tl->list_ndead : 0);
     return PYROPE_OK;
@@ -2520,7 +2700,8 @@ int pyrope_delta_snapshot(pyrope_delta* d, const char* path) {
     if (!path || !*path) return fail(PYROPE_ERR_INVALID_ARG, "Path cannot be empty.");
     const std::string base(path);
     TRY(pyrope_index_snapshot(d->head, (base + ".head").c_str()));
-    TRY(pyrope_index_snapshot(d->tail, (base + ".tail").c_str()));
+    if (d->stail) TRY(spass(pyrope_sharded_snapshot(d->stail, (base + ".tail").c_str())));
+    else TRY(pyrope_index_snapshot(d->tail, (base + ".tail").c_str()));
     const std::string tmp = base + ".tmp";
     FILE* f = fopen(tmp.c_str(), "wb");
     if (!f) return fail(PYROPE_ERR_INVALID_ARG, "cannot open %s for writing", tmp.c_str());
@@ -2541,7 +2722,8 @@ int pyrope_delta_load(pyrope_delta* d, const char* path) {
         FILE* f = fopen(p.c_str(), "rb");
         if (!f) continue;
         fclose(f);
-        TRY(pyrope_index_load(side == 0 ? d->head : d->tail, p.c_str()));
+        if (side == 1 && d->stail) TRY(spass(pyrope_sharded_load(d->stail, p.c_str())));
+        else TRY(pyrope_index_load(side == 0 ? d->head : d->tail, p.c_str()));
     }
     return PYROPE_OK;
 }

@@ -25,9 +25,21 @@
 #include <thread>
 #include <vector>
 
+#include <sys/stat.h>
+
 #include <cuda_runtime.h>
 
 #include "../../include/pyrope_gpu.h"
+
+// api.cu (internal, not part of the public header): the two halves of pyrope_index_load, and the compaction's per-tail
+// step of a Head+Tail (pyrope_delta_*) whose tail is sharded
+extern "C" int pyrope_internal_index_load_prepare(pyrope_index* h, const char* path, void** staged_out, int32_t* shard_rank_out,
+                                                  int32_t* shard_world_out, int64_t* next_row_out);
+extern "C" void pyrope_internal_index_load_commit(pyrope_index* h, void* staged);
+extern "C" void pyrope_internal_index_load_discard(void* staged);
+extern "C" int pyrope_internal_tail_reserve(pyrope_index* tl, int64_t n);
+extern "C" int pyrope_internal_tail_absorb(pyrope_index* tl, int64_t n, const float* dX, const int64_t* dL,
+                                           const int64_t* labels_host, int64_t* tail_rows_out);
 
 namespace {
 
@@ -93,6 +105,7 @@ struct pyrope_sharded {
     struct Seg { int64_t g0, n; int shard; int64_t local0; };
     std::vector<Seg> segs;
     std::vector<int64_t> shard_rows;  // FLAT: rows per shard so far
+    int64_t snap_gen = 0;             // generation of the most recent snapshot written by this handle
     // per-device search buffers (grown on demand), device 0 also holds the gather / merged buffers
     struct Buf { void* p = nullptr; size_t bytes = 0; };
     std::vector<Buf> dQ, pr_local, pr_all, sc, rw, cn;
@@ -353,7 +366,10 @@ int pyrope_sharded_add_batch(pyrope_sharded* s, int64_t n, const float* X, const
     if (rc != PYROPE_OK) return rc;
     for (int r = 0; r < s->n; ++r) {
         const int64_t lo = n * r / s->n, hi = n * (r + 1) / s->n;
-        if (hi > lo) s->segs.push_back({first + lo, hi - lo, r, local0[(size_t)r]});
+        if (hi > lo) {
+            s->segs.push_back({first + lo, hi - lo, r, local0[(size_t)r]});
+            s->shard_rows[(size_t)r] += hi - lo;
+        }
     }
     s->next_row += n;
     return PYROPE_OK;
@@ -411,8 +427,9 @@ int pyrope_sharded_stats(pyrope_sharded* s, int64_t* live_rows_out) {
 
 // queries already on every device?  no: dQ_host / host outputs.  device_io != 0: Q is a DEVICE pointer on device 0 and the
 // outputs are device pointers on device 0 (bench: HBM-resident timing); the queries still travel to the peers over NVLink.
+// q_ready (device_io only, may be null): a CUDA event every shard waits for before it reads the queries.
 static int sharded_search(S* s, int64_t nq, const float* Q, int topk, int64_t max_scans, int nprobe, float* scores_out,
-                          int64_t* rows_out, int32_t* counts_out, int device_io) {
+                          int64_t* rows_out, int32_t* counts_out, int device_io, cudaEvent_t q_ready = nullptr) {
     if (!s) return sfail(PYROPE_ERR_INVALID_ARG, "handle is null");
     if (nq < 0 || (nq > 0 && !Q)) return sfail(PYROPE_ERR_INVALID_ARG, "query is null");
     if (topk <= 0) {
@@ -488,6 +505,7 @@ static int sharded_search(S* s, int64_t nq, const float* Q, int topk, int64_t ma
             if (thr_setup) STRY(pyrope_index_threshold_exchange_attach(s->shard[i], N, r, s->thr_arr.data()));
             if (use_thr) STRY(pyrope_index_threshold_exchange_epoch(s->shard[i], epoch));
             if (device_io) {
+                if (q_ready) SCK(cudaStreamWaitEvent(st, q_ready, 0));
                 if (r == 0) { if (s->dQ[0].p != (const void*)Q) SCK(cudaMemcpyAsync(s->dQ[0].p, Q, qbytes, cudaMemcpyDeviceToDevice, st)); }
                 else SCK(cudaMemcpyPeerAsync(s->dQ[i].p, s->dev[i], Q, s->dev[0], qbytes, st));
                 if (r == 0) SCK(cudaEventRecord(s->ev_t0, st));
@@ -587,6 +605,364 @@ int pyrope_sharded_search_batch_device(pyrope_sharded* s, int64_t nq, const floa
 int pyrope_sharded_last_search_ms(pyrope_sharded* s, float* ms_out) {
     if (!s || !ms_out) return sfail(PYROPE_ERR_INVALID_ARG, "null argument");
     *ms_out = s->last_ms;
+    return PYROPE_OK;
+}
+
+// ---- Upsert / labels / codebooks: each call has the semantics of its pyrope_index_* namesake over the whole index
+
+// FLAT: the segment holding a global row (nullptr if none)
+static const S::Seg* flat_seg(const S* s, int64_t row) {
+    for (const S::Seg& sg : s->segs)
+        if (row >= sg.g0 && row < sg.g0 + sg.n) return &sg;
+    return nullptr;
+}
+
+int pyrope_sharded_update_row(pyrope_sharded* s, int64_t row, const float* x) {
+    if (!s) return sfail(PYROPE_ERR_INVALID_ARG, "handle is null");
+    if (!x) return sfail(PYROPE_ERR_INVALID_ARG, "vector is null");
+    std::lock_guard<std::mutex> g(s->mu);
+    if (row < 0 || row >= s->next_row) return sfail(PYROPE_ERR_NOT_FOUND, "row %lld does not exist", (long long)row);
+    if (s->kind == PYROPE_FLAT) {  // the owner's copy, in place (an Upsert un-deletes)
+        const S::Seg* sg = flat_seg(s, row);
+        if (!sg) return sfail(PYROPE_ERR_NOT_FOUND, "row %lld does not exist", (long long)row);
+        return run_all(s, [&](int r) -> int {
+            if (r == sg->shard) STRY(pyrope_index_update_row(s->shard[(size_t)r], sg->local0 + (row - sg->g0), x));
+            return PYROPE_OK;
+        });
+    }
+    // IVF: only a buffered row can be updated, and the buffer is replicated: every shard must succeed
+    std::vector<int> rcs((size_t)s->n, 0);
+    run_all(s, [&](int r) -> int { rcs[(size_t)r] = pyrope_index_update_row(s->shard[(size_t)r], row, x); return PYROPE_OK; });
+    int ok = 0;
+    for (int rc : rcs) ok += rc == PYROPE_OK;
+    if (ok == s->n) return PYROPE_OK;
+    if (ok == 0) return sfail(rcs[0], "row %lld is not in the write buffer", (long long)row);
+    return sfail(PYROPE_ERR_INVALID_STATE, "row %lld was updated on %d of %d shards", (long long)row, ok, s->n);
+}
+
+int pyrope_sharded_shadow_row(pyrope_sharded* s, int64_t row, int shadowed) {
+    if (!s) return sfail(PYROPE_ERR_INVALID_ARG, "handle is null");
+    if (s->kind == PYROPE_FLAT) return sfail(PYROPE_ERR_INVALID_STATE, "FLAT rows cannot be shadowed");
+    std::lock_guard<std::mutex> g(s->mu);
+    if (row < 0 || row >= s->next_row) return sfail(PYROPE_ERR_NOT_FOUND, "row %lld not found", (long long)row);
+    // a list row lives on the owner of its list only
+    std::vector<int> rcs((size_t)s->n, 0);
+    run_all(s, [&](int r) -> int { rcs[(size_t)r] = pyrope_index_shadow_row(s->shard[(size_t)r], row, shadowed); return PYROPE_OK; });
+    for (int rc : rcs)
+        if (rc == PYROPE_OK) return PYROPE_OK;
+    return sfail(PYROPE_ERR_NOT_FOUND, "row %lld is not in an inverted list", (long long)row);
+}
+
+int pyrope_sharded_set_labels(pyrope_sharded* s, int64_t n_rows, const int64_t* labels_by_row) {
+    if (!s) return sfail(PYROPE_ERR_INVALID_ARG, "handle is null");
+    std::lock_guard<std::mutex> g(s->mu);
+    if (n_rows < s->next_row || (n_rows > 0 && !labels_by_row))
+        return sfail(PYROPE_ERR_INVALID_ARG, "labels for %lld rows needed, %lld given", (long long)s->next_row, (long long)n_rows);
+    if (s->kind != PYROPE_FLAT)
+        return run_all(s, [&](int r) -> int { STRY(pyrope_index_set_labels(s->shard[(size_t)r], n_rows, labels_by_row)); return PYROPE_OK; });
+    // FLAT: a shard's local rows map back to global rows through the segment table
+    return run_all(s, [&](int r) -> int {
+        std::vector<int64_t> L((size_t)s->shard_rows[(size_t)r], -1);
+        for (const S::Seg& sg : s->segs)
+            if (sg.shard == r)
+                for (int64_t i = 0; i < sg.n; ++i) L[(size_t)(sg.local0 + i)] = labels_by_row[(size_t)(sg.g0 + i)];
+        STRY(pyrope_index_set_labels(s->shard[(size_t)r], (int64_t)L.size(), L.data()));
+        return PYROPE_OK;
+    });
+}
+
+// centroids and PQ codebooks are replicated bit for bit: read them from the first shard, on its thread
+int pyrope_sharded_is_built(pyrope_sharded* s, int* out) {
+    if (!s || !out) return sfail(PYROPE_ERR_INVALID_ARG, "null argument");
+    STRY(pyrope_index_is_built(s->shard[0], out));
+    return PYROPE_OK;
+}
+
+int pyrope_sharded_get_centroids(pyrope_sharded* s, float* centroids_out, int* n_out) {
+    if (!s) return sfail(PYROPE_ERR_INVALID_ARG, "handle is null");
+    std::lock_guard<std::mutex> g(s->mu);
+    return run_all(s, [&](int r) -> int {
+        if (r == 0) STRY(pyrope_index_get_centroids(s->shard[0], centroids_out, n_out));
+        return PYROPE_OK;
+    });
+}
+
+int pyrope_sharded_get_codebooks(pyrope_sharded* s, float* codebooks_out, int32_t* ksub_out) {
+    if (!s) return sfail(PYROPE_ERR_INVALID_ARG, "handle is null");
+    std::lock_guard<std::mutex> g(s->mu);
+    return run_all(s, [&](int r) -> int {
+        if (r == 0) STRY(pyrope_index_get_codebooks(s->shard[0], codebooks_out, ksub_out));
+        return PYROPE_OK;
+    });
+}
+
+}  // extern "C"
+
+// ---- snapshot / load ----------------------------------------------------------------------------------------------
+// `path` is a manifest; shard i's state is path.g<gen>.shard<i>, written by pyrope_index_snapshot on that shard's thread.
+// The manifest is written last (tmp + rename) and the previous generation's shard files are removed only after that, so
+// the manifest on disk always names a complete set of shard files.  Manifest, little-endian:
+//   "PYRSHD01", int32 version, n, kind, dim, metric, nlist, m, k, int64 next_row, gen,
+//   uint64 n_segs + n_segs x (int64 g0, int64 n, int32 shard, int64 local0)     (FLAT row blocks, none for IVF)
+//   n x int64 shard_rows (FLAT), n x (uint32 name length, name, uint64 file bytes)   (names relative to the manifest)
+namespace {
+
+constexpr char kManifestMagic[8] = {'P', 'Y', 'R', 'S', 'H', 'D', '0', '1'};
+constexpr int32_t kManifestVersion = 1;
+
+struct Manifest {
+    int32_t n = 0, kind = 0, dim = 0, metric = 0, nlist = 0, m = 0, k = 0;
+    int64_t next_row = 0, gen = 0;
+    std::vector<S::Seg> segs;
+    std::vector<int64_t> shard_rows;
+    std::vector<std::string> names;
+    std::vector<uint64_t> bytes;
+};
+
+std::string dir_of(const std::string& path) {
+    const size_t p = path.rfind('/');
+    return p == std::string::npos ? std::string() : path.substr(0, p + 1);
+}
+
+bool file_bytes(const std::string& path, uint64_t* out) {
+    struct stat st;
+    if (stat(path.c_str(), &st) != 0) return false;
+    *out = (uint64_t)st.st_size;
+    return true;
+}
+
+// parse and check a manifest's own consistency; expect_n > 0: the shard count is checked right after the header (a
+// manifest written by another device count is refused as such, before the rest of it is read)
+int read_manifest(const char* path, Manifest& M, int expect_n = 0) {
+    FILE* f = fopen(path, "rb");
+    if (!f) return sfail(PYROPE_ERR_NOT_FOUND, "Snapshot file not found: %s", path);
+    bool ok = true;
+    auto r = [&](void* p, size_t n) { if (ok && fread(p, 1, n, f) != n) ok = false; };
+    auto rv32 = [&]() { int32_t v = 0; r(&v, 4); return v; };
+    auto rv64 = [&]() { int64_t v = 0; r(&v, 8); return v; };
+    char magic[8] = {0};
+    r(magic, 8);
+    int32_t version = rv32();
+    if (!ok || memcmp(magic, kManifestMagic, 8) != 0 || version != kManifestVersion) {
+        fclose(f);
+        return sfail(PYROPE_ERR_INVALID_ARG, "%s is not a sharded pyrope_gpu snapshot manifest", path);
+    }
+    M.n = rv32(); M.kind = rv32(); M.dim = rv32(); M.metric = rv32(); M.nlist = rv32(); M.m = rv32(); M.k = rv32();
+    M.next_row = rv64(); M.gen = rv64();
+    if (ok && expect_n > 0 && M.n != expect_n) {
+        fclose(f);
+        return sfail(PYROPE_ERR_INVALID_ARG, "snapshot %s was written by %d shards, this index has %d devices (no re-sharding on load)",
+                     path, M.n, expect_n);
+    }
+    const int64_t nsegs = rv64();
+    ok = ok && M.n >= 1 && M.n <= 8 && M.next_row >= 0 && M.gen >= 1 && nsegs >= 0 && nsegs <= M.next_row;
+    for (int64_t i = 0; ok && i < nsegs; ++i) {
+        S::Seg sg;
+        sg.g0 = rv64(); sg.n = rv64(); sg.shard = rv32(); sg.local0 = rv64();
+        M.segs.push_back(sg);
+    }
+    for (int i = 0; ok && i < M.n; ++i) M.shard_rows.push_back(rv64());
+    for (int i = 0; ok && i < M.n; ++i) {
+        uint32_t len = 0;
+        r(&len, 4);
+        if (!ok || len == 0 || len > 4096) { ok = false; break; }
+        std::string name(len, '\0');
+        r(&name[0], len);
+        uint64_t b = 0;
+        r(&b, 8);
+        if (name.find('/') != std::string::npos) ok = false;
+        M.names.push_back(name);
+        M.bytes.push_back(b);
+    }
+    fclose(f);
+    if (!ok) return sfail(PYROPE_ERR_INVALID_ARG, "corrupt or truncated snapshot manifest %s", path);
+    // FLAT row blocks: inside [0, next_row) globally and inside their shard's local rows
+    for (const S::Seg& sg : M.segs)
+        if (sg.shard < 0 || sg.shard >= M.n || sg.n <= 0 || sg.g0 < 0 || sg.g0 + sg.n > M.next_row || sg.local0 < 0 ||
+            sg.local0 + sg.n > M.shard_rows[(size_t)sg.shard])
+            return sfail(PYROPE_ERR_INVALID_ARG, "corrupt snapshot manifest %s: row block table", path);
+    return PYROPE_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int pyrope_sharded_snapshot(pyrope_sharded* s, const char* path) {
+    if (!s) return sfail(PYROPE_ERR_INVALID_ARG, "handle is null");
+    if (!path || !*path) return sfail(PYROPE_ERR_INVALID_ARG, "Path cannot be empty");
+    std::lock_guard<std::mutex> g(s->mu);
+    const std::string base(path), dir = dir_of(base), stem = base.substr(dir.size());
+    Manifest old;
+    const bool have_old = read_manifest(path, old) == PYROPE_OK;
+    // a generation that no manifest at this path names yet, so the files it writes replace none that are still referenced
+    const int64_t gen = std::max(s->snap_gen, have_old ? old.gen : 0) + 1;
+    std::vector<std::string> names((size_t)s->n);
+    for (int r = 0; r < s->n; ++r) names[(size_t)r] = stem + ".g" + std::to_string(gen) + ".shard" + std::to_string(r);
+    int rc = run_all(s, [&](int r) -> int { STRY(pyrope_index_snapshot(s->shard[(size_t)r], (dir + names[(size_t)r]).c_str())); return PYROPE_OK; });
+    std::vector<uint64_t> bytes((size_t)s->n, 0);
+    for (int r = 0; rc == PYROPE_OK && r < s->n; ++r)
+        if (!file_bytes(dir + names[(size_t)r], &bytes[(size_t)r])) rc = sfail(PYROPE_ERR_INVALID_STATE, "shard file %s vanished", names[(size_t)r].c_str());
+    const std::string tmp = base + ".tmp";
+    if (rc == PYROPE_OK) {
+        FILE* f = fopen(tmp.c_str(), "wb");
+        if (!f) {
+            rc = sfail(PYROPE_ERR_INVALID_ARG, "cannot open %s for writing", tmp.c_str());
+        } else {
+            bool ok = true;
+            auto w = [&](const void* p, size_t n) { if (ok && fwrite(p, 1, n, f) != n) ok = false; };
+            auto w32 = [&](int32_t v) { w(&v, 4); };
+            auto w64 = [&](int64_t v) { w(&v, 8); };
+            w(kManifestMagic, 8);
+            w32(kManifestVersion); w32(s->n); w32(s->kind); w32(s->dim); w32(s->metric); w32(s->nlist); w32(s->m); w32(s->k);
+            w64(s->next_row); w64(gen);
+            w64((int64_t)s->segs.size());
+            for (const S::Seg& sg : s->segs) { w64(sg.g0); w64(sg.n); w32(sg.shard); w64(sg.local0); }
+            for (int r = 0; r < s->n; ++r) w64(s->shard_rows[(size_t)r]);
+            for (int r = 0; r < s->n; ++r) {
+                const uint32_t len = (uint32_t)names[(size_t)r].size();
+                w(&len, 4);
+                w(names[(size_t)r].data(), len);
+                w(&bytes[(size_t)r], 8);
+            }
+            if (fclose(f) != 0 || !ok) rc = sfail(PYROPE_ERR_INVALID_STATE, "short write to %s", tmp.c_str());
+            else if (rename(tmp.c_str(), path) != 0) rc = sfail(PYROPE_ERR_INVALID_STATE, "cannot move %s into place", tmp.c_str());
+        }
+    }
+    if (rc != PYROPE_OK) {  // the manifest on disk (if any) still names the previous, complete set
+        remove(tmp.c_str());
+        for (const std::string& nm : names) remove((dir + nm).c_str());
+        return rc;
+    }
+    s->snap_gen = gen;
+    if (have_old)  // the previous generation is no longer referenced
+        for (const std::string& nm : old.names)
+            if (std::find(names.begin(), names.end(), nm) == names.end()) remove((dir + nm).c_str());
+    return PYROPE_OK;
+}
+
+int pyrope_sharded_load(pyrope_sharded* s, const char* path) {
+    if (!s) return sfail(PYROPE_ERR_INVALID_ARG, "handle is null");
+    if (!path || !*path) return sfail(PYROPE_ERR_INVALID_ARG, "Path cannot be empty");
+    std::lock_guard<std::mutex> g(s->mu);
+    Manifest M;
+    {
+        const int rc = read_manifest(path, M, s->n);
+        if (rc == PYROPE_ERR_INVALID_ARG) {  // a single-device snapshot has its own magic: say so
+            FILE* f = fopen(path, "rb");
+            char magic[8] = {0};
+            const bool single = f && fread(magic, 1, 8, f) == 8 && memcmp(magic, "PYRGPU01", 8) == 0;
+            if (f) fclose(f);
+            if (single)
+                return sfail(PYROPE_ERR_INVALID_ARG, "%s is a single-device snapshot; a sharded index loads only a sharded manifest", path);
+        }
+        if (rc != PYROPE_OK) return rc;
+    }
+    if (M.kind != s->kind || M.metric != s->metric || M.m != s->m || M.k != s->k)
+        return sfail(PYROPE_ERR_INVALID_ARG, "snapshot is of a different index type");
+    if (M.dim != s->dim) return sfail(PYROPE_ERR_DIMENSION, "Vector dimension mismatch");
+    if (s->kind != PYROPE_FLAT && !M.segs.empty()) return sfail(PYROPE_ERR_INVALID_ARG, "corrupt snapshot manifest %s: row blocks on an IVF index", path);
+    const std::string dir = dir_of(path);
+    for (int r = 0; r < s->n; ++r) {
+        const std::string f = dir + M.names[(size_t)r];
+        uint64_t b = 0;
+        if (!file_bytes(f, &b)) return sfail(PYROPE_ERR_NOT_FOUND, "Snapshot file not found: %s", f.c_str());
+        if (b != M.bytes[(size_t)r])
+            return sfail(PYROPE_ERR_INVALID_ARG, "shard file %s holds %llu bytes, the manifest recorded %llu", f.c_str(),
+                         (unsigned long long)b, (unsigned long long)M.bytes[(size_t)r]);
+    }
+    // every shard parses and stages its file on its own thread; nothing is committed unless all of them succeed
+    std::vector<void*> staged((size_t)s->n, nullptr);
+    int rc = run_all(s, [&](int r) -> int {
+        int32_t rank = -1, world = 0;
+        int64_t nr = -1;
+        const std::string f = dir + M.names[(size_t)r];
+        STRY(pyrope_internal_index_load_prepare(s->shard[(size_t)r], f.c_str(), &staged[(size_t)r], &rank, &world, &nr));
+        // IVF shards carry their shard identity and the replicated row count; FLAT shards are plain indexes of their rows
+        const bool ivf = s->kind != PYROPE_FLAT;
+        const int want_rank = ivf ? r : 0, want_world = ivf ? s->n : 1;
+        const int64_t want_rows = ivf ? M.next_row : M.shard_rows[(size_t)r];
+        if (rank != want_rank || world != want_world || nr != want_rows)
+            return sfail(PYROPE_ERR_INVALID_ARG, "%s is shard %d of %d with %lld rows, the manifest expects shard %d of %d with %lld rows",
+                         f.c_str(), rank, world, (long long)nr, want_rank, want_world, (long long)want_rows);
+        return PYROPE_OK;
+    });
+    if (rc != PYROPE_OK) {
+        run_all(s, [&](int r) -> int {
+            if (staged[(size_t)r]) pyrope_internal_index_load_discard(staged[(size_t)r]);
+            return PYROPE_OK;
+        });
+        return rc;
+    }
+    run_all(s, [&](int r) -> int { pyrope_internal_index_load_commit(s->shard[(size_t)r], staged[(size_t)r]); return PYROPE_OK; });
+    s->next_row = M.next_row;
+    s->segs = M.segs;
+    s->shard_rows = M.shard_rows;
+    s->snap_gen = std::max(s->snap_gen, M.gen);
+    int b = 0;
+    pyrope_index_is_built(s->shard[0], &b);
+    s->built = s->kind != PYROPE_FLAT && b != 0;
+    return PYROPE_OK;
+}
+
+// ---- internal (not in the public header) ---------------------------------------------------------------------------
+
+// rows ever added according to a sharded snapshot's manifest (the string-id layer sizes its id tables with it)
+int pyrope_internal_sharded_snapshot_next_row(const char* path, int64_t* next_row_out) {
+    Manifest M;
+    const int rc = read_manifest(path, M);
+    if (rc != PYROPE_OK) return rc;
+    *next_row_out = M.next_row;
+    return PYROPE_OK;
+}
+
+// pyrope_sharded_search_batch_device whose shards wait for q_ready (a cudaEvent_t, may be null) before reading the queries
+int pyrope_internal_sharded_search_device(pyrope_sharded* s, int64_t nq, const float* dQ_dev0, int topk, int64_t max_scans,
+                                          int nprobe, float* d_scores_dev0, int64_t* d_rows_dev0, int32_t* d_counts_dev0,
+                                          void* q_ready) {
+    return sharded_search(s, nq, dQ_dev0, topk, max_scans, nprobe, d_scores_dev0, d_rows_dev0, d_counts_dev0, 1,
+                          (cudaEvent_t)q_ready);
+}
+
+// The compaction step of a Head+Tail whose tail is this (IVF) index: n rows (dX n x dim, dL labels: device memory on
+// src_device; labels_host the same labels) join every shard's replica of the write buffer, each shard shadowing the
+// list entries it owns with those labels.  Every shard makes room first, so an allocation failure leaves all of them
+// unchanged; every shard must then report the same row ordinals.
+int pyrope_internal_sharded_absorb(pyrope_sharded* s, int64_t n, const float* dX, const int64_t* dL, int src_device,
+                                   const int64_t* labels_host, int64_t* tail_rows_out) {
+    if (!s || n < 0) return sfail(PYROPE_ERR_INVALID_ARG, "bad argument");
+    if (s->kind == PYROPE_FLAT) return sfail(PYROPE_ERR_UNSUPPORTED, "a sharded FLAT index cannot be a Head+Tail tail");
+    if (n == 0) return PYROPE_OK;
+    std::lock_guard<std::mutex> g(s->mu);
+    const size_t N = (size_t)s->n, xb = sizeof(float) * (size_t)n * s->dim, lb = sizeof(int64_t) * (size_t)n;
+    std::vector<void*> bx(N, nullptr), bl(N, nullptr);
+    std::vector<std::vector<int64_t>> rows(N, std::vector<int64_t>((size_t)n, -1));
+    int rc = run_all(s, [&](int r) -> int {
+        const size_t i = (size_t)r;
+        STRY(pyrope_internal_tail_reserve(s->shard[i], n));
+        SCK(cudaMalloc(&bx[i], xb));
+        SCK(cudaMalloc(&bl[i], lb));
+        SCK(cudaMemcpyPeerAsync(bx[i], s->dev[i], dX, src_device, xb, s->st[i]));
+        SCK(cudaMemcpyPeerAsync(bl[i], s->dev[i], dL, src_device, lb, s->st[i]));
+        SCK(cudaStreamSynchronize(s->st[i]));
+        return PYROPE_OK;
+    });
+    if (rc == PYROPE_OK)
+        rc = run_all(s, [&](int r) -> int {
+            const size_t i = (size_t)r;
+            STRY(pyrope_internal_tail_absorb(s->shard[i], n, (const float*)bx[i], (const int64_t*)bl[i], labels_host, rows[i].data()));
+            return PYROPE_OK;
+        });
+    run_all(s, [&](int r) -> int {
+        if (bx[(size_t)r]) cudaFree(bx[(size_t)r]);
+        if (bl[(size_t)r]) cudaFree(bl[(size_t)r]);
+        return PYROPE_OK;
+    });
+    if (rc != PYROPE_OK) return rc;
+    for (size_t r = 1; r < N; ++r)
+        if (rows[r] != rows[0]) return sfail(PYROPE_ERR_INVALID_STATE, "shard %zu placed the moved rows at other row ordinals than shard 0", r);
+    for (int64_t i = 0; i < n; ++i) s->next_row = std::max(s->next_row, rows[0][(size_t)i] + 1);
+    if (tail_rows_out) memcpy(tail_rows_out, rows[0].data(), lb);
     return PYROPE_OK;
 }
 

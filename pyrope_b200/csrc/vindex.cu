@@ -23,8 +23,10 @@
 
 #include "../../include/pyrope_gpu.h"
 
-// api.cu (internal, not part of the public header): rows ever added according to a snapshot's header
+// api.cu / sharded.cu (internal, not part of the public header): rows ever added according to a snapshot's header /
+// a sharded snapshot's manifest
 extern "C" int pyrope_internal_snapshot_next_row(const char* path, int64_t* next_row_out);
+extern "C" int pyrope_internal_sharded_snapshot_next_row(const char* path, int64_t* next_row_out);
 
 namespace {
 
@@ -44,10 +46,21 @@ int vpass(int rc) {
     if (rc != PYROPE_OK) g_verr = pyrope_last_error();
     return rc;
 }
+// the same for the sharded layer, which keeps its own message
+int spass(int rc) {
+    if (rc != PYROPE_OK) g_verr = pyrope_sharded_last_error();
+    return rc;
+}
 #define VTRY(expr)                            \
     do {                                      \
         int _r = (expr);                      \
         if (_r != PYROPE_OK) return vpass(_r); \
+    } while (0)
+// a status whose message is already in g_verr
+#define LTRY(expr)                       \
+    do {                                 \
+        int _r = (expr);                 \
+        if (_r != PYROPE_OK) return _r;  \
     } while (0)
 
 // process-wide id table: string -> ordinal (the row label), ordinal -> string.  Entries are reference counted — one
@@ -113,7 +126,8 @@ bool blank(const char* id) {  // string.IsNullOrWhiteSpace
 
 struct pyrope_vindex {
     int kind = 0, dim = 0, metric = 0;
-    pyrope_index* h = nullptr;  // null for a delta
+    pyrope_index* h = nullptr;      // one-device leaf (null for a delta)
+    pyrope_sharded* sh = nullptr;   // or a leaf over several devices (pyrope_vindex_create_sharded)
     // delta
     pyrope_vindex* head = nullptr;
     pyrope_vindex* tail = nullptr;
@@ -158,10 +172,37 @@ int check_vec(const V* v, const float* vec, int len) {
     return PYROPE_OK;
 }
 
+// ---- the row-ordinal handle behind a leaf: one device (pyrope_index_*) or several (pyrope_sharded_*).  Errors come
+// back with their message in g_verr.
+int row_add(V* v, int64_t gid, const float* vec, int64_t* row) {
+    return v->sh ? spass(pyrope_sharded_add_batch(v->sh, 1, vec, &gid, row)) : vpass(pyrope_index_add_batch(v->h, 1, vec, &gid, row));
+}
+int row_update(V* v, int64_t row, const float* vec) {
+    return v->sh ? spass(pyrope_sharded_update_row(v->sh, row, vec)) : vpass(pyrope_index_update_row(v->h, row, vec));
+}
+int row_shadow(V* v, int64_t row, int shadowed) {
+    return v->sh ? spass(pyrope_sharded_shadow_row(v->sh, row, shadowed)) : vpass(pyrope_index_shadow_row(v->h, row, shadowed));
+}
+int row_delete(V* v, int64_t row) {
+    return v->sh ? spass(pyrope_sharded_delete_row(v->sh, row)) : vpass(pyrope_index_delete_row(v->h, row));
+}
+int row_build(V* v) { return v->sh ? spass(pyrope_sharded_build(v->sh)) : vpass(pyrope_index_build(v->h)); }
+int row_set_labels(V* v, int64_t n, const int64_t* labels) {
+    return v->sh ? spass(pyrope_sharded_set_labels(v->sh, n, labels)) : vpass(pyrope_index_set_labels(v->h, n, labels));
+}
+int row_snapshot(V* v, const char* path) {
+    return v->sh ? spass(pyrope_sharded_snapshot(v->sh, path)) : vpass(pyrope_index_snapshot(v->h, path));
+}
+int row_load(V* v, const char* path) { return v->sh ? spass(pyrope_sharded_load(v->sh, path)) : vpass(pyrope_index_load(v->h, path)); }
+int row_snapshot_next_row(V* v, const char* path, int64_t* next_row) {
+    return v->sh ? spass(pyrope_internal_sharded_snapshot_next_row(path, next_row))
+                 : vpass(pyrope_internal_snapshot_next_row(path, next_row));
+}
+
 // ---- leaf writes (no locking; callers hold the write lock) ------------------------------------------------
 int leaf_add_new(V* v, int64_t gid, const float* vec) {
     int64_t row = -1;
-    VTRY(pyrope_index_add_batch(v->h, 1, vec, &gid, &row));
+    LTRY(row_add(v, gid, vec, &row));
     v->set_row(gid, row);
     v->note_row(row, gid);
     if (v->kind != PYROPE_FLAT) v->buffered.insert(gid);
@@ -172,11 +213,11 @@ int leaf_add_new(V* v, int64_t gid, const float* vec) {
 int leaf_buffer_set(V* v, int64_t gid, const float* vec) {
     auto it = v->row_of.find(gid);
     if (it == v->row_of.end()) return leaf_add_new(v, gid, vec);
-    if (v->buffered.count(gid)) return vpass(pyrope_index_update_row(v->h, it->second, vec));  // key keeps its slot
+    if (v->buffered.count(gid)) return row_update(v, it->second, vec);  // key keeps its slot
     // the id sits in an inverted list: the buffered copy shadows it (seenIds, IvfFlatVectorIndex.cs:210,
     // IvfPqVectorIndex.cs:170) until the next Build
     const int64_t old = it->second;
-    VTRY(pyrope_index_shadow_row(v->h, old, 1));
+    LTRY(row_shadow(v, old, 1));
     v->shadowed[gid] = old;
     return leaf_add_new(v, gid, vec);
 }
@@ -195,7 +236,7 @@ int leaf_add(V* v, const char* id, const float* vec, int len, bool upsert) {
         if (it == v->row_of.end()) rc = leaf_add_new(v, gid, vec);
         else if (!upsert)  // BruteForceVectorIndex.cs:141-144
             rc = vfail(PYROPE_ERR_INVALID_STATE, "Vector with id '%s' already exists.", id);
-        else rc = vpass(pyrope_index_update_row(v->h, it->second, vec));  // :203-206 in place, scan position kept
+        else rc = row_update(v, it->second, vec);  // :203-206 in place, scan position kept
     }
     if (rc != PYROPE_OK) id_drop_if_unreferenced(gid);
     return rc;
@@ -212,7 +253,7 @@ int leaf_delete(V* v, const char* id, bool* removed) {
     if (it == v->row_of.end()) return PYROPE_OK;
     const int64_t row = it->second;
     if (v->kind == PYROPE_FLAT) {  // BruteForceVectorIndex.cs:231-254: tombstone, id leaves the map
-        VTRY(pyrope_index_delete_row(v->h, row));
+        LTRY(row_delete(v, row));
         v->gid_of_row[(size_t)row] = -1;
         v->drop(it);
         *removed = true;
@@ -221,12 +262,12 @@ int leaf_delete(V* v, const char* id, bool* removed) {
     const bool in_buffer = v->buffered.count(gid) != 0;
     if (v->kind == PYROPE_IVF_PQ) {  // IvfPqVectorIndex.cs:48-53: only the buffer
         if (!in_buffer) return PYROPE_OK;
-        VTRY(pyrope_index_delete_row(v->h, row));
+        LTRY(row_delete(v, row));
         v->gid_of_row[(size_t)row] = -1;
         v->buffered.erase(gid);
         auto sh = v->shadowed.find(gid);
         if (sh != v->shadowed.end()) {  // the encoded copy is visible again
-            VTRY(pyrope_index_shadow_row(v->h, sh->second, 0));
+            LTRY(row_shadow(v, sh->second, 0));
             it->second = sh->second;
             v->shadowed.erase(sh);
         } else {
@@ -236,11 +277,11 @@ int leaf_delete(V* v, const char* id, bool* removed) {
         return PYROPE_OK;
     }
     // IvfFlatVectorIndex.cs:62-83: buffer entry and every list entry with this id
-    VTRY(pyrope_index_delete_row(v->h, row));
+    LTRY(row_delete(v, row));
     v->gid_of_row[(size_t)row] = -1;
     auto sh = v->shadowed.find(gid);
     if (sh != v->shadowed.end()) {
-        VTRY(pyrope_index_delete_row(v->h, sh->second));
+        LTRY(row_delete(v, sh->second));
         v->gid_of_row[(size_t)sh->second] = -1;
         v->shadowed.erase(sh);
     }
@@ -274,7 +315,7 @@ void leaf_after_build(V* v, bool had_buffer) {
 int leaf_build(V* v) {
     if (v->kind == PYROPE_FLAT) return PYROPE_OK;
     const bool had_buffer = !v->buffered.empty();
-    VTRY(pyrope_index_build(v->h));
+    LTRY(row_build(v));
     leaf_after_build(v, had_buffer);
     return PYROPE_OK;
 }
@@ -366,10 +407,10 @@ int leaf_apply_ids(V* v, const LoadedIds& L) {
         if (!row_of.count(kv.first)) { row_of.emplace(kv.first, kv.second); id_ref(kv.first); }
     // the rows in the library's snapshot carry the labels of the process that wrote it: re-label them.  Rows that are
     // gone get -1, which no search returns and no live id ordinal equals.
-    int rc = pyrope_index_set_labels(v->h, L.nrows, gid_of_row.data());
+    int rc = row_set_labels(v, L.nrows, gid_of_row.data());
     if (rc != PYROPE_OK) {
         for (auto& kv : row_of) id_unref(kv.first);
-        return vpass(rc);
+        return rc;
     }
     v->drop_all();
     v->gid_of_row.swap(gid_of_row);
@@ -385,11 +426,11 @@ int leaf_load(V* v, const std::string& path) {
     int r = leaf_parse_ids(path + ".ids", L);
     if (r != PYROPE_OK) return r;
     int64_t next_row = -1;
-    VTRY(pyrope_internal_snapshot_next_row(path.c_str(), &next_row));
+    LTRY(row_snapshot_next_row(v, path.c_str(), &next_row));
     if (L.nrows < next_row)
         return vfail(PYROPE_ERR_INVALID_ARG, "%s.ids covers %lld rows, the snapshot holds %lld", path.c_str(), (long long)L.nrows,
                      (long long)next_row);
-    VTRY(pyrope_index_load(v->h, path.c_str()));
+    LTRY(row_load(v, path.c_str()));
     return leaf_apply_ids(v, L);
 }
 
@@ -414,13 +455,32 @@ int pyrope_vindex_create(int kind, int dim, int metric, int nlist, int pq_m, int
     return PYROPE_OK;
 }
 
+int pyrope_vindex_create_sharded(int n_devices, const int* devices, int kind, int dim, int metric, int nlist, int pq_m, int pq_k,
+                                 pyrope_vindex** out) {
+    if (!out) return vfail(PYROPE_ERR_INVALID_ARG, "out is null");
+    *out = nullptr;
+    if (kind != PYROPE_IVF_FLAT && kind != PYROPE_IVF_PQ) return vfail(PYROPE_ERR_UNSUPPORTED, "a sharded index must be IVF_FLAT or IVF_PQ");
+    V* v = new (std::nothrow) V();
+    if (!v) return vfail(PYROPE_ERR_OOM, "out of host memory");
+    int rc = pyrope_sharded_create(n_devices, devices, kind, dim, metric, nlist, pq_m, pq_k, &v->sh);
+    if (rc != PYROPE_OK) {
+        delete v;
+        return spass(rc);
+    }
+    v->kind = kind; v->dim = dim; v->metric = metric;
+    *out = v;
+    return PYROPE_OK;
+}
+
 int pyrope_vindex_create_delta(pyrope_vindex* head, pyrope_vindex* tail, pyrope_vindex** out) {
     if (!out) return vfail(PYROPE_ERR_INVALID_ARG, "out is null");
     *out = nullptr;
     if (!head || !tail || head->d || tail->d) return vfail(PYROPE_ERR_INVALID_ARG, "head and tail must be leaf indexes");
+    if (head->sh) return vfail(PYROPE_ERR_UNSUPPORTED, "the head must be a one-device FLAT index");
     V* v = new (std::nothrow) V();
     if (!v) return vfail(PYROPE_ERR_OOM, "out of host memory");
-    int rc = pyrope_delta_create(head->h, tail->h, &v->d);  // DeltaVectorIndex..ctor :18-28
+    int rc = tail->sh ? pyrope_delta_create_sharded(head->h, tail->sh, &v->d)  // DeltaVectorIndex..ctor :18-28
+                      : pyrope_delta_create(head->h, tail->h, &v->d);
     if (rc != PYROPE_OK) {
         delete v;
         return vpass(rc);
@@ -435,6 +495,7 @@ int pyrope_vindex_destroy(pyrope_vindex* v) {
     if (!v) return PYROPE_OK;
     if (v->d) pyrope_delta_destroy(v->d);  // the two sides stay alive: they were only borrowed
     if (v->h) pyrope_index_destroy(v->h);
+    if (v->sh) pyrope_sharded_destroy(v->sh);
     v->drop_all();
     delete v;
     return PYROPE_OK;
@@ -537,6 +598,7 @@ int pyrope_vindex_search(pyrope_vindex* v, int64_t nq, const float* Q, int len, 
     }
     std::shared_lock<std::shared_mutex> g(v->lock);
     if (v->d) return vpass(pyrope_delta_search_batch(v->d, nq, Q, topk, max_scans, nprobe, scores_out, gids_out, counts_out));
+    if (v->sh) return spass(pyrope_sharded_search_batch(v->sh, nq, Q, topk, max_scans, nprobe, scores_out, gids_out, counts_out));
     return vpass(pyrope_index_search_batch(v->h, nq, Q, topk, max_scans, nprobe, scores_out, gids_out, counts_out));
 }
 
@@ -595,6 +657,7 @@ int pyrope_vindex_get_centroids(pyrope_vindex* v, float* centroids_out, int* n_o
     V* leaf = v->d ? v->tail : v;  // DeltaVectorIndex.cs:241-252: the tail's, if it has any
     *n_out = 0;
     if (leaf->kind == PYROPE_FLAT) return PYROPE_OK;  // not an ICentroidsProvider -> null
+    if (leaf->sh) return spass(pyrope_sharded_get_centroids(leaf->sh, centroids_out, n_out));
     return vpass(pyrope_index_get_centroids(leaf->h, centroids_out, n_out));
 }
 
@@ -604,7 +667,7 @@ int pyrope_vindex_snapshot(pyrope_vindex* v, const char* path) {
     std::shared_lock<std::shared_mutex> g(v->lock);
     const std::string base(path);
     if (!v->d) {
-        VTRY(pyrope_index_snapshot(v->h, path));
+        LTRY(row_snapshot(v, path));
         return leaf_save_ids(v, base + ".ids");
     }
     VTRY(pyrope_delta_snapshot(v->d, path));

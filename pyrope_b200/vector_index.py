@@ -211,16 +211,34 @@ class _BorrowedGpuIndex(_lib.GpuIndex):
     __del__ = close
 
 
+def _devices(devices):
+    """None -> one device; an int N -> devices 0..N-1; a sequence -> those CUDA ordinals."""
+    if devices is None:
+        return None
+    if isinstance(devices, (int, np.integer)):
+        return list(range(int(devices)))
+    return [int(d) for d in devices]
+
+
 class _Leaf(_VectorIndex):
-    def _create(self, kind, dimension, metric, nlist=100, m=4, k=256):
+    def _create(self, kind, dimension, metric, nlist=100, m=4, k=256, devices=None):
         v = vp()
-        _ck(_lib.load().pyrope_vindex_create(kind, int(dimension), int(metric), int(nlist), int(m), int(k), C.byref(v)))
+        devs = _devices(devices)
+        if devs is None:
+            _ck(_lib.load().pyrope_vindex_create(kind, int(dimension), int(metric), int(nlist), int(m), int(k), C.byref(v)))
+        else:  # the same index over several GPUs of the box (pyrope_sharded_*)
+            dv = np.asarray(devs, np.int32)
+            _ck(_lib.load().pyrope_vindex_create_sharded(len(devs), dv.ctypes.data_as(_lib.i32p), kind, int(dimension),
+                                                         int(metric), int(nlist), int(m), int(k), C.byref(v)))
         self._v, self._dim, self._metric = v, int(dimension), VectorMetric(int(metric))
+        self._devices = devs
 
     def native(self) -> _lib.GpuIndex:
         """Row-ordinal view of the same index (borrowed handle) for bit-exact parity reads."""
         h = vp()
         _ck(_lib.load().pyrope_vindex_native(self._v, C.byref(h)))
+        if not h.value:
+            raise InvalidOperationException("a sharded index has no single row-ordinal handle")
         g = _BorrowedGpuIndex.__new__(_BorrowedGpuIndex)
         g._h, g.kind, g.dim, g.metric = h, self._kind, self._dim, int(self._metric)
         g.nlist, g.m, g.k = self._nlist, self._m, self._k
@@ -247,20 +265,22 @@ class BruteForceVectorIndex(_Leaf):
 
 
 class IvfFlatVectorIndex(_Leaf):
-    """IvfFlatVectorIndex(dimension, metric, nList = 100) — IvfFlatVectorIndex.cs:27-33."""
+    """IvfFlatVectorIndex(dimension, metric, nList = 100) — IvfFlatVectorIndex.cs:27-33.  devices (N or a list of CUDA
+    ordinals) shards the inverted lists over those GPUs; results equal the one-device index's."""
 
-    def __init__(self, dimension: int, metric: VectorMetric = VectorMetric.L2, nList: int = 100):
+    def __init__(self, dimension: int, metric: VectorMetric = VectorMetric.L2, nList: int = 100, devices=None):
         self._kind, self._nlist, self._m, self._k = _lib.IVF_FLAT, nList, 0, 0
-        self._create(_lib.IVF_FLAT, dimension, metric, nlist=nList)
+        self._create(_lib.IVF_FLAT, dimension, metric, nlist=nList, devices=devices)
 
 
 class IvfPqVectorIndex(_Leaf):
-    """IvfPqVectorIndex(dimension, metric, m, k = 256, nList = 100) — IvfPqVectorIndex.cs:27-35."""
+    """IvfPqVectorIndex(dimension, metric, m, k = 256, nList = 100) — IvfPqVectorIndex.cs:27-35.  devices as for
+    IvfFlatVectorIndex."""
 
     def __init__(self, dimension: int, metric: VectorMetric = VectorMetric.L2, m: int = 4, k: int = 256,
-                 nList: int = 100):
+                 nList: int = 100, devices=None):
         self._kind, self._nlist, self._m, self._k = _lib.IVF_PQ, nList, m, k
-        self._create(_lib.IVF_PQ, dimension, metric, nlist=nList, m=m, k=k)
+        self._create(_lib.IVF_PQ, dimension, metric, nlist=nList, m=m, k=k, devices=devices)
 
 
 class DeltaVectorIndex(_VectorIndex):
@@ -276,14 +296,21 @@ class DeltaVectorIndex(_VectorIndex):
 
 def create_index(algorithm: str | None, dimension: int, metric: VectorMetric, params: dict | None = None):
     """VectorIndexRegistry.IndexState..ctor (Services/VectorIndexRegistry.cs:81-113): a BruteForce head over the
-    tail the Algorithm string names (default IVF_FLAT; m 4 / k 256 / nlist 100)."""
+    tail the Algorithm string names (default IVF_FLAT; m 4 / k 256 / nlist 100).  params["devices"] (N, or a list
+    of CUDA ordinals) shards the tail over those GPUs and makes the first of them current for the head; a FLAT tail
+    cannot be sharded (PyropeGpuError, UNSUPPORTED)."""
     params = params or {}
     algo = (algorithm or "IVF_FLAT").upper().replace("GPU_", "")
+    devs = _devices(params.get("devices"))
     if algo == "IVF_PQ":
         tail = IvfPqVectorIndex(dimension, metric, int(params.get("m", 4)), int(params.get("k", 256)),
-                                int(params.get("nlist", 100)))
+                                int(params.get("nlist", 100)), devices=devs)
     elif algo == "FLAT":
+        if devs is not None:
+            raise _lib.PyropeGpuError(_lib.ERR_UNSUPPORTED, "a FLAT tail cannot be sharded over devices")
         tail = BruteForceVectorIndex(dimension, metric)
     else:
-        tail = IvfFlatVectorIndex(dimension, metric, int(params.get("nlist", 100)))
+        tail = IvfFlatVectorIndex(dimension, metric, int(params.get("nlist", 100)), devices=devs)
+    if devs is not None:  # the head lives on the tail's first device
+        _ck(_lib.load().pyrope_gpu_init(devs[0]))
     return DeltaVectorIndex(BruteForceVectorIndex(dimension, metric), tail)
