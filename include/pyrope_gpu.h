@@ -36,6 +36,9 @@ extern "C" {
 #endif
 
 typedef struct pyrope_index pyrope_index; /* opaque */
+typedef struct pyrope_sharded pyrope_sharded;     /* one index over the GPUs of a box, below */
+typedef struct pyrope_delta pyrope_delta;         /* Head+Tail, below */
+typedef struct pyrope_vindex pyrope_vindex;       /* string-id index classes, below */
 
 typedef enum pyrope_status {
     PYROPE_OK = 0,
@@ -210,11 +213,31 @@ int pyrope_index_last_search_scanned(pyrope_index *h, int64_t *codes_out);
 /* ---- host micro-batcher: the reference calls IVectorIndex.Search with ONE query per Garnet session thread
  *      (VectorCommandSet.cs:458, under the read lock of BruteForceVectorIndex.cs:282).  The shim's Search calls
  *      pyrope_batcher_search instead, which blocks while a dispatcher thread gathers the queries that arrive
- *      within max_wait_us (or max_batch of them), issues one pyrope_index_search_batch per group of equal
- *      (topK, MaxScans, NProbe) and returns each caller its own result.  Thread-safe; results are written into
- *      the caller's buffers (topk entries each); errors carry pyrope_batcher_last_error(). */
+ *      within max_wait_us (or max_batch of them), issues one batched search of its target per group of equal
+ *      (MaxScans, NProbe, K) and returns each caller its own result.  K is the topK class: the smallest power of two
+ *      >= topK, capped at the target's limit; a group is searched once at its largest topK and every caller gets
+ *      exactly its own top topK (a Head+Tail merges with a per-query k, pyrope_delta_search_batch_topk).
+ *      Thread-safe; results are written into the caller's buffers (topk entries each); errors carry
+ *      pyrope_batcher_last_error(), with the message of whichever layer raised them.
+ *      The target is borrowed: destroy the batcher first.  It is one of
+ *        pyrope_batcher_create          a pyrope_index: rows_out = row ordinals (or the rows' labels);
+ *        pyrope_batcher_create_sharded  a pyrope_sharded: global row ordinals (labels), dimension from shard 0;
+ *        pyrope_batcher_create_delta    a pyrope_delta (Head+Tail): labels, dimension from the head;
+ *        pyrope_batcher_create_vindex   a pyrope_vindex (string ids): id ORDINALS.  The batch runs under the vindex's
+ *                                       shared lock, as pyrope_vindex_search does.  The shim checks the query length
+ *                                       itself (ValidateDim) before it calls pyrope_batcher_search, holds its read lock
+ *                                       while blocked in it, and turns the ordinals into strings with pyrope_vindex_ids
+ *                                       before it releases that lock.
+ *      A caller's status is the one the direct call on the target would give it alone, and such callers never join a
+ *      batch: topK <= 0 -> OUT_OF_RANGE on a FLAT index, a delta, or a vindex whose search validates like a FLAT head,
+ *      an empty result on an IVF index or leaf; topK above the target's limit (1024 for an index, min(1024, 4096 / N)
+ *      sharded, what pyrope_delta_search_batch accepts for a delta) -> UNSUPPORTED.  A batch that fails reports its
+ *      status and message to every caller in it.  A null target -> INVALID_ARG before any CUDA call. */
 typedef struct pyrope_batcher pyrope_batcher;
 int pyrope_batcher_create(pyrope_index *h, int max_batch, int max_wait_us, pyrope_batcher **out);
+int pyrope_batcher_create_sharded(pyrope_sharded *s, int max_batch, int max_wait_us, pyrope_batcher **out);
+int pyrope_batcher_create_delta(pyrope_delta *d, int max_batch, int max_wait_us, pyrope_batcher **out);
+int pyrope_batcher_create_vindex(pyrope_vindex *v, int max_batch, int max_wait_us, pyrope_batcher **out);
 int pyrope_batcher_destroy(pyrope_batcher *b);
 int pyrope_batcher_search(pyrope_batcher *b, const float *query, int topk, int64_t max_scans, int nprobe,
                           float *scores_out, int64_t *rows_out, int32_t *count_out);
@@ -246,7 +269,6 @@ int pyrope_topk_merge_dedupe_device(int64_t nq, int parts, int k_in, int k_out, 
  *      0's gather buffer and are merged there (one entry per row label).  Results equal the single-GPU index's.
  *      MaxScans (an insertion-/probe-order budget) cannot be split: max_scans >= 0 with N > 1 -> UNSUPPORTED.
  *      Errors: pyrope_sharded_last_error().  Calls on one handle are serialised internally. */
-typedef struct pyrope_sharded pyrope_sharded;
 /* devices: n_devices CUDA ordinals, or NULL for 0..n_devices-1 (1 <= n_devices <= 8; peers must be NVLink/P2P reachable) */
 int pyrope_sharded_create(int n_devices, const int *devices, int kind, int dim, int metric, int nlist, int pq_m,
                           int pq_k, pyrope_sharded **out);
@@ -327,7 +349,6 @@ const char *pyrope_peer_last_error(void);
  *      the label of every row it adds to either side, so "same id" == "same label".  The delta object borrows the
  *      two handles (destroying it leaves them alive); writes keep going to the handles directly
  *      (Add/Upsert -> head, Delete -> both, DeltaVectorIndex.cs:26-74). */
-typedef struct pyrope_delta pyrope_delta;
 /* DeltaVectorIndex..ctor :18-28: dimension / metric mismatch -> INVALID_ARG (ArgumentException). */
 int pyrope_delta_create(pyrope_index *head, pyrope_index *tail, pyrope_delta **out);
 /* The same with a tail sharded over the box's GPUs (IVF_FLAT / IVF_PQ only: a FLAT tail -> UNSUPPORTED; the head must
@@ -345,6 +366,13 @@ int pyrope_delta_destroy(pyrope_delta *d);
  * topk <= 0 -> OUT_OF_RANGE (the FLAT head throws first, BruteForceVectorIndex.cs:278). */
 int pyrope_delta_search_batch(pyrope_delta *d, int64_t nq, const float *Q, int topk, int64_t max_scans,
                               int nprobe, float *scores_out, int64_t *labels_out, int32_t *counts_out);
+/* pyrope_delta_search_batch with topks[i] for query i: outputs have stride max(topks); row i holds counts[i] <= topks[i]
+ * entries, equal to what pyrope_delta_search_batch over the same batch with topk = topks[i] returns for that query.
+ * Head and tail are searched once at max(topks); the de-duplicating merge sees only the first topks[i] entries of
+ * each side for query i, as the reference's Search with topK = topks[i] would.  Any topks[i] that the plain call
+ * rejects fails the whole call with the same status. */
+int pyrope_delta_search_batch_topk(pyrope_delta *d, int64_t nq, const float *Q, const int32_t *topks, int64_t max_scans,
+                                   int nprobe, float *scores_out, int64_t *labels_out, int32_t *counts_out);
 int pyrope_delta_search_batch_device(pyrope_delta *d, int64_t nq, const float *dQ, int topk,
                                      int64_t max_scans, int nprobe, float *d_scores, int64_t *d_labels,
                                      int32_t *d_counts, void *stream);
@@ -375,7 +403,6 @@ int pyrope_delta_load(pyrope_delta *d, const char *path);
  *      empty."), DIMENSION -> ArgumentException("Vector dimension mismatch"), OUT_OF_RANGE ->
  *      ArgumentOutOfRangeException (FLAT topK <= 0), INVALID_STATE -> InvalidOperationException (FLAT duplicate
  *      Add, BruteForceVectorIndex.cs:141-144), NOT_FOUND -> FileNotFoundException (Load). */
-typedef struct pyrope_vindex pyrope_vindex;
 int pyrope_vindex_create(int kind, int dim, int metric, int nlist, int pq_m, int pq_k, pyrope_vindex **out);
 /* DeltaVectorIndex(head, tail) :18-28; head must be FLAT.  Borrows both (destroy the delta first). */
 int pyrope_vindex_create_delta(pyrope_vindex *head, pyrope_vindex *tail, pyrope_vindex **out);

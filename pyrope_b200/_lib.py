@@ -108,6 +108,9 @@ SIGNATURES = {
     "pyrope_index_last_search_scanned": (C.c_int, [vp, i64p]),
     "pyrope_index_last_search_kernel": (C.c_int, [vp, f32p, C.POINTER(C.c_char_p)]),
     "pyrope_batcher_create": (C.c_int, [vp, C.c_int, C.c_int, C.POINTER(vp)]),
+    "pyrope_batcher_create_sharded": (C.c_int, [vp, C.c_int, C.c_int, C.POINTER(vp)]),
+    "pyrope_batcher_create_delta": (C.c_int, [vp, C.c_int, C.c_int, C.POINTER(vp)]),
+    "pyrope_batcher_create_vindex": (C.c_int, [vp, C.c_int, C.c_int, C.POINTER(vp)]),
     "pyrope_batcher_destroy": (C.c_int, [vp]),
     "pyrope_batcher_search": (C.c_int, [vp, vp, C.c_int, C.c_int64, C.c_int, vp, vp, i32p]),
     "pyrope_batcher_stats": (C.c_int, [vp, i64p, i64p]),
@@ -117,6 +120,7 @@ SIGNATURES = {
     "pyrope_delta_create_sharded": (C.c_int, [vp, vp, C.POINTER(vp)]),
     "pyrope_delta_destroy": (C.c_int, [vp]),
     "pyrope_delta_search_batch": (C.c_int, [vp, C.c_int64, vp, C.c_int, C.c_int64, C.c_int, vp, vp, vp]),
+    "pyrope_delta_search_batch_topk": (C.c_int, [vp, C.c_int64, vp, vp, C.c_int64, C.c_int, vp, vp, vp]),
     "pyrope_delta_search_batch_device": (C.c_int, [vp, C.c_int64, vp, C.c_int, C.c_int64, C.c_int, vp, vp, vp, vp]),
     "pyrope_delta_compact": (C.c_int, [vp, i64p, vp]),
     "pyrope_delta_move": (C.c_int, [vp, i64p, vp]),
@@ -566,12 +570,27 @@ class ShardedIndex:
 
 class Batcher:
     """Host micro-batcher (csrc/batcher.cu): search() blocks like IVectorIndex.Search does; concurrent callers
-    share one batched launch.  ctypes drops the GIL during the call, so Python threads batch for real."""
+    share one batched launch.  ctypes drops the GIL during the call, so Python threads batch for real.
 
-    def __init__(self, index: GpuIndex, max_batch: int = 256, max_wait_us: int = 200):
-        b = vp()
-        check(load().pyrope_batcher_create(index._h, max_batch, max_wait_us, C.byref(b)))
-        self._b, self._index = b, index
+    target: a GpuIndex (rows = row ordinals / labels), a ShardedIndex (global row ordinals), a raw pyrope_delta handle
+    (labels) or any vector_index object (id ordinals; vector_index.VectorIndexBatcher turns them into strings).  The
+    batcher borrows the target and keeps a reference to it."""
+
+    def __init__(self, target, max_batch: int = 256, max_wait_us: int = 200):
+        L, b = load(), vp()
+        if isinstance(target, GpuIndex):
+            rc = L.pyrope_batcher_create(target._h, max_batch, max_wait_us, C.byref(b))
+        elif isinstance(target, ShardedIndex):
+            rc = L.pyrope_batcher_create_sharded(target._s, max_batch, max_wait_us, C.byref(b))
+        elif hasattr(target, "_v"):  # a vector_index object (string ids)
+            rc = L.pyrope_batcher_create_vindex(target._v, max_batch, max_wait_us, C.byref(b))
+        elif isinstance(target, (vp, int)):  # a pyrope_delta handle
+            rc = L.pyrope_batcher_create_delta(target, max_batch, max_wait_us, C.byref(b))
+        else:
+            raise TypeError(f"cannot batch searches of {type(target).__name__}")
+        if rc:
+            raise PyropeGpuError(rc, (L.pyrope_batcher_last_error() or b"").decode("utf-8", "replace"))
+        self._b, self._index = b, target
 
     def search(self, q, topk: int, max_scans: int = -1, nprobe: int = -1):
         q = _np(q, np.float32).reshape(-1)

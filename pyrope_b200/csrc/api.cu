@@ -2305,6 +2305,7 @@ struct pyrope_delta {
     int tail_devices = 1;
     std::mutex mu;
     DevBuf ps, pl, pc, q, os, ol, oc;  // partial (head | tail) results, staged queries, merged outputs
+    DevBuf kq;                         // per-query topK of pyrope_delta_search_batch_topk
     cudaEvent_t q_ready = nullptr;     // sharded tail: the queries are in place on the head's stream
 };
 
@@ -2318,8 +2319,12 @@ int spass(int rc) {
 
 // DeltaVectorIndex.Search:76-122 for nq queries: head top-k, tail top-k (same options, :85,88), merge by id with
 // the head's copy winning, descending, Take(topK) — one stream, no host round trip between the three stages.
+// d_kq (nullable, device [nq], every entry <= topk): query i asked for d_kq[i].  Both sides still run once at topk, and
+// the merge keeps only each side's first d_kq[i] entries.  Cutting the merged list at d_kq[i] instead would be wrong:
+// an id the head shares with the tail's top d_kq[i] would let the tail's (d_kq[i]+1)-th entry into the result.
 int delta_search_device(pyrope_delta* d, int64_t nq, const float* dQ, int topk, int64_t max_scans, int nprobe,
-                        float* d_scores, int64_t* d_labels, int32_t* d_counts, cudaStream_t st) {
+                        float* d_scores, int64_t* d_labels, int32_t* d_counts, cudaStream_t st,
+                        const int32_t* d_kq = nullptr) {
     Index* hd = d->head;
     Index* tl = d->tail;
     const size_t per = (size_t)nq * topk;
@@ -2350,15 +2355,18 @@ int delta_search_device(pyrope_delta* d, int64_t nq, const float* dQ, int topk, 
                           d->pc.as<int32_t>() + nq, st));
     }
     CK(launch_merge_pairs(nq, 2, topk, topk, d->ps.as<float>(), d->pl.as<int64_t>(), (int64_t)per, topk, d_scores,
-                          d_labels, d_counts, st, /*dedupe=*/true));
+                          d_labels, d_counts, st, /*dedupe=*/true, d_kq));
     return PYROPE_OK;
 }
+
+// the head's and the tail's lists share one merge of at most kMergeMaxCandidates candidates
+int delta_max_topk(const pyrope_delta* d) { return std::min(kMaxTopK, kMergeMaxCandidates / std::max(2, d->tail_devices)); }
 
 int delta_validate(pyrope_delta* d, int64_t nq, const float* Q, int topk) {
     if (!d) return fail(PYROPE_ERR_INVALID_ARG, "delta handle is null");
     if (nq < 0 || (nq > 0 && !Q)) return fail(PYROPE_ERR_INVALID_ARG, "query is null");
     if (topk <= 0) return fail(PYROPE_ERR_OUT_OF_RANGE, "topK must be positive.");  // the FLAT head throws first
-    const int lim = std::min(kMaxTopK, kMergeMaxCandidates / std::max(2, d->tail_devices));
+    const int lim = delta_max_topk(d);
     if (topk > lim) return fail(PYROPE_ERR_UNSUPPORTED, "topK %d exceeds the supported maximum %d", topk, lim);
     return PYROPE_OK;
 }
@@ -2442,10 +2450,12 @@ int pyrope_delta_search_batch_device(pyrope_delta* d, int64_t nq, const float* d
     return PYROPE_OK;
 }
 
-int pyrope_delta_search_batch(pyrope_delta* d, int64_t nq, const float* Q, int topk, int64_t max_scans, int nprobe,
-                              float* scores_out, int64_t* labels_out, int32_t* counts_out) {
-    TRY(delta_validate(d, nq, Q, topk));
-    if (nq == 0) return PYROPE_OK;
+}  // extern "C"
+
+namespace {
+// host queries in, host results out (stride topk); topks (nullable, host [nq], each <= topk): per-query topK
+int delta_search_host(pyrope_delta* d, int64_t nq, const float* Q, int topk, const int32_t* topks, int64_t max_scans,
+                      int nprobe, float* scores_out, int64_t* labels_out, int32_t* counts_out) {
     if (!scores_out || !labels_out || !counts_out) return fail(PYROPE_ERR_INVALID_ARG, "output buffer is null");
     std::lock_guard<std::mutex> g(d->mu);
     cudaStream_t st = d->head->stream;
@@ -2455,13 +2465,55 @@ int pyrope_delta_search_batch(pyrope_delta* d, int64_t nq, const float* Q, int t
     TRY(d->ol.ensure(sizeof(int64_t) * (size_t)nq * topk, 0, st));
     TRY(d->oc.ensure(sizeof(int32_t) * (size_t)nq, 0, st));
     CK(cudaMemcpyAsync(d->q.p, Q, sizeof(float) * (size_t)nq * dim, cudaMemcpyHostToDevice, st));
+    if (topks) {
+        TRY(d->kq.ensure(sizeof(int32_t) * (size_t)nq, 0, st));
+        CK(cudaMemcpyAsync(d->kq.p, topks, sizeof(int32_t) * (size_t)nq, cudaMemcpyHostToDevice, st));
+    }
     TRY(delta_search_device(d, nq, d->q.as<float>(), topk, max_scans, nprobe, d->os.as<float>(), d->ol.as<int64_t>(),
-                            d->oc.as<int32_t>(), st));
+                            d->oc.as<int32_t>(), st, topks ? d->kq.as<int32_t>() : nullptr));
     CK(cudaMemcpyAsync(scores_out, d->os.p, sizeof(float) * (size_t)nq * topk, cudaMemcpyDeviceToHost, st));
     CK(cudaMemcpyAsync(labels_out, d->ol.p, sizeof(int64_t) * (size_t)nq * topk, cudaMemcpyDeviceToHost, st));
     CK(cudaMemcpyAsync(counts_out, d->oc.p, sizeof(int32_t) * (size_t)nq, cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
     delta_forget_stream(d, st);
+    return PYROPE_OK;
+}
+}  // namespace
+
+extern "C" {
+
+int pyrope_delta_search_batch(pyrope_delta* d, int64_t nq, const float* Q, int topk, int64_t max_scans, int nprobe,
+                              float* scores_out, int64_t* labels_out, int32_t* counts_out) {
+    TRY(delta_validate(d, nq, Q, topk));
+    if (nq == 0) return PYROPE_OK;
+    return delta_search_host(d, nq, Q, topk, nullptr, max_scans, nprobe, scores_out, labels_out, counts_out);
+}
+
+int pyrope_delta_search_batch_topk(pyrope_delta* d, int64_t nq, const float* Q, const int32_t* topks, int64_t max_scans,
+                                   int nprobe, float* scores_out, int64_t* labels_out, int32_t* counts_out) {
+    if (nq > 0 && !topks) return fail(PYROPE_ERR_INVALID_ARG, "topks is null");
+    int kmax = 1;
+    for (int64_t i = 0; i < nq; ++i) {
+        TRY(delta_validate(d, nq, Q, topks[i]));
+        kmax = std::max(kmax, (int)topks[i]);
+    }
+    TRY(delta_validate(d, nq, Q, kmax));
+    if (nq == 0) return PYROPE_OK;
+    return delta_search_host(d, nq, Q, kmax, topks, max_scans, nprobe, scores_out, labels_out, counts_out);
+}
+
+// csrc/batcher.cu (internal): the dimension of a Head+Tail and the largest topK its search accepts
+int pyrope_internal_delta_limits(pyrope_delta* d, int* dim_out, int* max_topk_out) {
+    if (!d) return fail(PYROPE_ERR_INVALID_ARG, "delta handle is null");
+    if (dim_out) *dim_out = d->head->dim;
+    if (max_topk_out) *max_topk_out = delta_max_topk(d);
+    return PYROPE_OK;
+}
+
+// csrc/batcher.cu (internal): FLAT / IVF_FLAT / IVF_PQ of an index (topK <= 0 is an error only on FLAT)
+int pyrope_internal_index_kind(pyrope_index* h, int* kind_out) {
+    if (!h || !kind_out) return fail(PYROPE_ERR_INVALID_ARG, "null argument");
+    *kind_out = h->kind;
     return PYROPE_OK;
 }
 

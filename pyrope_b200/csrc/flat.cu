@@ -201,32 +201,39 @@ __global__ void __launch_bounds__(NT) flat_scan_kernel(FlatScanParams p, int64_t
 
 // ------------------------------------------------------------------------------------------
 // K6 merge: one CTA per query; parts*k_in candidates -> k_out.
+// PER_Q: query q keeps only entries j < k_q = k_per_query[q] of every part (the rest count as empty, for the
+// de-duplication too) and its output is cut at k_q — what the same merge with k_in = k_out = k_q gives, because the
+// sort key (score, part * k_in + j) orders candidates alike for any k_in.
 // ------------------------------------------------------------------------------------------
+template <bool PER_Q>
 __global__ void __launch_bounds__(256) merge_pairs_kernel(int64_t nq, int parts, int k_in, int k_out,
                                                           const float* __restrict__ in_s,
                                                           const int64_t* __restrict__ in_l,
                                                           int64_t part_stride, int64_t q_stride,
                                                           float* out_s, int64_t* out_l,
-                                                          int32_t* out_c, int P, int dedupe) {
+                                                          int32_t* out_c, int P, int dedupe,
+                                                          const int32_t* __restrict__ k_per_query) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     uint64_t* keys = reinterpret_cast<uint64_t*>(smem_raw);
     __shared__ int s_count;
     const int64_t q = blockIdx.x;
     const int tid = threadIdx.x;
     const int total = parts * k_in;
+    const int kq = PER_Q ? min(k_per_query[q], k_in) : k_in;
+    const int kcut = PER_Q ? min(kq, k_out) : k_out;
     if (tid == 0) s_count = 0;
     for (int i = tid; i < P; i += blockDim.x) {
         uint64_t key = 0;
         if (i < total) {
             int part = i / k_in, j = i - part * k_in;
             int64_t a = part * part_stride + q * q_stride + j;
-            const int64_t lab = in_l[a];
+            const int64_t lab = (!PER_Q || j < kq) ? in_l[a] : -1;
             if (lab >= 0) {
                 bool dup = false;
                 if (dedupe) {  // the same id in a lower part (the head) wins
                     for (int pp = 0; pp < part && !dup; ++pp) {
                         const int64_t b = pp * part_stride + q * q_stride;
-                        for (int jj = 0; jj < k_in; ++jj)
+                        for (int jj = 0; jj < kq; ++jj)
                             if (in_l[b + jj] == lab) { dup = true; break; }
                     }
                 }
@@ -239,7 +246,7 @@ __global__ void __launch_bounds__(256) merge_pairs_kernel(int64_t nq, int parts,
     bitonic_sort_desc<false>(keys, P, tid, blockDim.x);
     int local = 0;
     for (int i = tid; i < k_out; i += blockDim.x) {
-        uint64_t key = i < P ? keys[i] : 0ull;
+        uint64_t key = (i < P && (!PER_Q || i < kcut)) ? keys[i] : 0ull;
         if (key) {
             int idx = (int)key_pos(key);
             int part = idx / k_in, j = idx - part * k_in;
@@ -258,30 +265,35 @@ __global__ void __launch_bounds__(256) merge_pairs_kernel(int64_t nq, int parts,
 }
 
 // Few candidates per query (the multi-GPU merge: ranks x k): one WARP per query, eight queries per CTA, no block barriers.
+// PER_Q as for merge_pairs_kernel.
+template <bool PER_Q>
 __global__ void __launch_bounds__(256) merge_pairs_warp_kernel(int64_t nq, int parts, int k_in, int k_out,
                                                                const float* __restrict__ in_s,
                                                                const int64_t* __restrict__ in_l,
                                                                int64_t part_stride, int64_t q_stride,
                                                                float* out_s, int64_t* out_l,
-                                                               int32_t* out_c, int P, int dedupe) {
+                                                               int32_t* out_c, int P, int dedupe,
+                                                               const int32_t* __restrict__ k_per_query) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     uint64_t* keys = reinterpret_cast<uint64_t*>(smem_raw) + (size_t)warp * P;
     const int64_t q = (int64_t)blockIdx.x * (blockDim.x >> 5) + warp;
     if (q >= nq) return;
     const int total = parts * k_in;
+    const int kq = PER_Q ? min(k_per_query[q], k_in) : k_in;
+    const int kcut = PER_Q ? min(kq, k_out) : k_out;
     for (int i = lane; i < P; i += 32) {
         uint64_t key = 0;
         if (i < total) {
             const int part = i / k_in, j = i - part * k_in;
             const int64_t a = part * part_stride + q * q_stride + j;
-            const int64_t lab = in_l[a];
+            const int64_t lab = (!PER_Q || j < kq) ? in_l[a] : -1;
             if (lab >= 0) {
                 bool dup = false;
                 if (dedupe) {  // the same id in a lower part (the head) wins
                     for (int pp = 0; pp < part && !dup; ++pp) {
                         const int64_t b = pp * part_stride + q * q_stride;
-                        for (int jj = 0; jj < k_in; ++jj)
+                        for (int jj = 0; jj < kq; ++jj)
                             if (in_l[b + jj] == lab) { dup = true; break; }
                     }
                 }
@@ -294,7 +306,7 @@ __global__ void __launch_bounds__(256) merge_pairs_warp_kernel(int64_t nq, int p
     bitonic_sort_desc<true>(keys, P, lane, 32);
     int local = 0;
     for (int i = lane; i < k_out; i += 32) {
-        const uint64_t key = i < P ? keys[i] : 0ull;
+        const uint64_t key = (i < P && (!PER_Q || i < kcut)) ? keys[i] : 0ull;
         if (key) {
             const int idx = (int)key_pos(key);
             const int part = idx / k_in, j = idx - part * k_in;
@@ -353,20 +365,33 @@ cudaError_t launch_flat_scan(const FlatScanParams& p, cudaStream_t st) {
 cudaError_t launch_merge_pairs(int64_t nq, int parts, int k_in, int k_out, const float* in_scores,
                                const int64_t* in_labels, int64_t part_stride, int64_t q_stride,
                                float* out_scores, int64_t* out_labels, int32_t* out_counts,
-                               cudaStream_t st, bool dedupe) {
+                               cudaStream_t st, bool dedupe, const int32_t* k_per_query) {
     if (nq <= 0) return cudaSuccess;
     int total = parts * k_in;
     if (total > kMergeMaxCandidates) return cudaErrorInvalidValue;
     int P = next_pow2(total < 2 ? 2 : total);
     if (P <= 256) {
-        merge_pairs_warp_kernel<<<(unsigned)((nq + 7) / 8), 256, sizeof(uint64_t) * (size_t)P * 8, st>>>(
-            nq, parts, k_in, k_out, in_scores, in_labels, part_stride, q_stride, out_scores, out_labels, out_counts, P,
-            dedupe ? 1 : 0);
+        const unsigned grid = (unsigned)((nq + 7) / 8);
+        const size_t smem = sizeof(uint64_t) * (size_t)P * 8;
+        if (k_per_query)
+            merge_pairs_warp_kernel<true><<<grid, 256, smem, st>>>(nq, parts, k_in, k_out, in_scores, in_labels, part_stride,
+                                                                  q_stride, out_scores, out_labels, out_counts, P,
+                                                                  dedupe ? 1 : 0, k_per_query);
+        else
+            merge_pairs_warp_kernel<false><<<grid, 256, smem, st>>>(nq, parts, k_in, k_out, in_scores, in_labels, part_stride,
+                                                                   q_stride, out_scores, out_labels, out_counts, P,
+                                                                   dedupe ? 1 : 0, nullptr);
         return cudaGetLastError();
     }
-    merge_pairs_kernel<<<(unsigned)nq, 256, sizeof(uint64_t) * (size_t)P, st>>>(
-        nq, parts, k_in, k_out, in_scores, in_labels, part_stride, q_stride, out_scores, out_labels,
-        out_counts, P, dedupe ? 1 : 0);
+    const size_t smem = sizeof(uint64_t) * (size_t)P;
+    if (k_per_query)
+        merge_pairs_kernel<true><<<(unsigned)nq, 256, smem, st>>>(nq, parts, k_in, k_out, in_scores, in_labels, part_stride,
+                                                                 q_stride, out_scores, out_labels, out_counts, P,
+                                                                 dedupe ? 1 : 0, k_per_query);
+    else
+        merge_pairs_kernel<false><<<(unsigned)nq, 256, smem, st>>>(nq, parts, k_in, k_out, in_scores, in_labels, part_stride,
+                                                                  q_stride, out_scores, out_labels, out_counts, P,
+                                                                  dedupe ? 1 : 0, nullptr);
     return cudaGetLastError();
 }
 

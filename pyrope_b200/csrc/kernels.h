@@ -130,10 +130,12 @@ cudaError_t launch_sq8_scan(const uint8_t* Q8, int64_t nq, int dpad, const uint8
 // in: candidate (score,label) at address part*part_stride + q*q_stride + j, j < k_in.
 // dedupe: a candidate whose label already occurs in a LOWER part is dropped (DeltaVectorIndex.cs:98-110: the
 // head's copy of an id replaces the tail's).
+// k_per_query (nullable, device [nq]): query q sees only entries j < k_per_query[q] of each part and keeps at most that
+// many, so counts[q] <= k_per_query[q] — the merge a batch whose callers asked for different topK needs.
 cudaError_t launch_merge_pairs(int64_t nq, int parts, int k_in, int k_out, const float* in_scores,
                                const int64_t* in_labels, int64_t part_stride, int64_t q_stride,
                                float* out_scores, int64_t* out_labels, int32_t* out_counts,
-                               cudaStream_t st, bool dedupe = false);
+                               cudaStream_t st, bool dedupe = false, const int32_t* k_per_query = nullptr);
 constexpr int kMergeMaxCandidates = 4096;
 
 // ---- K4: IVF_FLAT inverted-list scan ----------------------------------------------------------

@@ -27,6 +27,8 @@
 // a sharded snapshot's manifest
 extern "C" int pyrope_internal_snapshot_next_row(const char* path, int64_t* next_row_out);
 extern "C" int pyrope_internal_sharded_snapshot_next_row(const char* path, int64_t* next_row_out);
+// api.cu (internal): the dimension and topK limit of a Head+Tail
+extern "C" int pyrope_internal_delta_limits(pyrope_delta* d, int* dim_out, int* max_topk_out);
 
 namespace {
 
@@ -600,6 +602,44 @@ int pyrope_vindex_search(pyrope_vindex* v, int64_t nq, const float* Q, int len, 
     if (v->d) return vpass(pyrope_delta_search_batch(v->d, nq, Q, topk, max_scans, nprobe, scores_out, gids_out, counts_out));
     if (v->sh) return spass(pyrope_sharded_search_batch(v->sh, nq, Q, topk, max_scans, nprobe, scores_out, gids_out, counts_out));
     return vpass(pyrope_index_search_batch(v->h, nq, Q, topk, max_scans, nprobe, scores_out, gids_out, counts_out));
+}
+
+// csrc/batcher.cu (internal): what a Search with topK <= 0 or a large topK gives on this index, so the batcher can answer
+// such a caller alone.  max_topk: the largest topK Search accepts; nonpos_empty: topK <= 0 returns an empty result
+// (an IVF leaf) rather than OUT_OF_RANGE (a FLAT leaf, or a delta whose FLAT head validates first).
+int pyrope_internal_vindex_limits(pyrope_vindex* v, int* dim_out, int* max_topk_out, int* nonpos_empty_out) {
+    if (!v) return vfail(PYROPE_ERR_INVALID_ARG, "index handle is null");
+    int lim = 1024, empty = 0;
+    if (v->d) {
+        VTRY(pyrope_internal_delta_limits(v->d, nullptr, &lim));
+    } else if (v->sh) {
+        int n = 1;
+        LTRY(spass(pyrope_sharded_device_count(v->sh, &n)));
+        lim = std::min(1024, 4096 / n);  // pyrope_sharded_search_batch: n x topK candidates in one merge
+        empty = 1;
+    } else {
+        empty = v->kind != PYROPE_FLAT;
+    }
+    if (dim_out) *dim_out = v->dim;
+    if (max_topk_out) *max_topk_out = lim;
+    if (nonpos_empty_out) *nonpos_empty_out = empty;
+    return PYROPE_OK;
+}
+
+// csrc/batcher.cu (internal): one batched Search under the shared lock, as pyrope_vindex_search runs it, with query i
+// asking for topks[i] (each in 1 .. the limit above).  Outputs have stride max(topks).  A delta merges with the per-query
+// k (pyrope_delta_search_batch_topk); a leaf searches at max(topks), whose first topks[i] entries per query are that
+// query's own top topks[i] — the caller keeps those.
+int pyrope_internal_vindex_search_topk(pyrope_vindex* v, int64_t nq, const float* Q, const int32_t* topks, int64_t max_scans,
+                                       int nprobe, float* scores_out, int64_t* gids_out, int32_t* counts_out) {
+    if (!v) return vfail(PYROPE_ERR_INVALID_ARG, "index handle is null");
+    if (nq > 0 && (!Q || !topks)) return vfail(PYROPE_ERR_INVALID_ARG, "null argument");
+    std::shared_lock<std::shared_mutex> g(v->lock);
+    if (v->d) return vpass(pyrope_delta_search_batch_topk(v->d, nq, Q, topks, max_scans, nprobe, scores_out, gids_out, counts_out));
+    int kmax = 1;
+    for (int64_t i = 0; i < nq; ++i) kmax = std::max(kmax, (int)topks[i]);
+    if (v->sh) return spass(pyrope_sharded_search_batch(v->sh, nq, Q, kmax, max_scans, nprobe, scores_out, gids_out, counts_out));
+    return vpass(pyrope_index_search_batch(v->h, nq, Q, kmax, max_scans, nprobe, scores_out, gids_out, counts_out));
 }
 
 int pyrope_vindex_id(int64_t gid, char* buf, int cap, int* len_out) {

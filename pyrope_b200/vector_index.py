@@ -59,8 +59,12 @@ class IndexStats:  # IVectorIndex.cs:40
     Metric: str
 
 
-def _raise(rc: int):
-    msg = (_lib.load().pyrope_vindex_last_error() or b"").decode("utf-8", "replace")
+def _ck(rc: int):
+    if rc != _lib.OK:
+        _raise(rc)
+
+
+def _raise_msg(rc: int, msg: str):
     if rc == _lib.ERR_INVALID_ARG:
         raise (ArgumentNullException if "cannot be null" in msg else ArgumentException)(msg)
     if rc == _lib.ERR_DIMENSION:
@@ -74,9 +78,8 @@ def _raise(rc: int):
     raise _lib.PyropeGpuError(rc, msg)
 
 
-def _ck(rc: int):
-    if rc != _lib.OK:
-        _raise(rc)
+def _raise(rc: int):
+    _raise_msg(rc, (_lib.load().pyrope_vindex_last_error() or b"").decode("utf-8", "replace"))
 
 
 def _id_string(ordinal: int) -> str:
@@ -104,6 +107,14 @@ def _id_strings(ordinals: np.ndarray) -> list[str]:
 
 def _idb(id_):
     return None if id_ is None else str(id_).encode("utf-8")
+
+
+def _options(options: SearchOptions | None):
+    """(max_scans, nprobe) on the ABI.  null = no budget (-1); a caller's MaxScans <= 0 scans nothing in the reference
+    and must not become "no budget"."""
+    ms = -1 if options is None or options.MaxScans is None else max(int(options.MaxScans), 0)
+    npb = -1 if options is None or options.NProbe is None else int(options.NProbe)
+    return ms, npb
 
 
 class _VectorIndex:
@@ -159,9 +170,7 @@ class _VectorIndex:
         scores = np.zeros((nq, kk), np.float32)
         ids = np.full((nq, kk), -1, np.int64)
         counts = np.zeros(nq, np.int32)
-        # null = no budget (-1 on the ABI); a caller's value <= 0 scans nothing in the reference and must not become "no budget"
-        ms = -1 if options is None or options.MaxScans is None else max(int(options.MaxScans), 0)
-        npb = -1 if options is None or options.NProbe is None else int(options.NProbe)
+        ms, npb = _options(options)
         _ck(_lib.load().pyrope_vindex_search(self._v, nq, _p(Q), ln, int(topK), ms, npb, _p(scores), _p(ids), _p(counts)))
         names = _id_strings(ids.reshape(-1))  # one call, one lock for the whole result list
         out = []
@@ -314,3 +323,37 @@ def create_index(algorithm: str | None, dimension: int, metric: VectorMetric, pa
     if devs is not None:  # the head lives on the tail's first device
         _ck(_lib.load().pyrope_gpu_init(devs[0]))
     return DeltaVectorIndex(BruteForceVectorIndex(dimension, metric), tail)
+
+
+class VectorIndexBatcher:
+    """The Search of the C# shim in front of a micro-batcher (pyrope_batcher_create_vindex): each call enqueues one
+    query and blocks while the dispatcher thread searches it together with the other callers' queries, then turns the
+    id ordinals into strings.  A shim does that translation under the read lock its Search runs under, so an id in the
+    result cannot be deleted and recycled before it is named.  Destroy the batcher (close) before the index."""
+
+    def __init__(self, index: _VectorIndex, max_batch: int = 256, max_wait_us: int = 200):
+        self._index = index
+        self._b = _lib.Batcher(index, max_batch, max_wait_us)
+
+    def Search(self, query, topK: int, options: SearchOptions | None = None) -> list[SearchResult]:
+        if query is None:
+            raise ArgumentNullException("Value cannot be null. (Parameter 'vector')")
+        q = _np(query, np.float32).reshape(-1)
+        if q.size != self._index.Dimension:  # ValidateDim: the batcher reads Dimension floats
+            raise ArgumentException("Vector dimension mismatch")
+        ms, npb = _options(options)
+        kk = max(int(topK), 1)
+        scores, ids, cnt = np.zeros(kk, np.float32), np.full(kk, -1, np.int64), C.c_int32(0)
+        L = _lib.load()
+        rc = L.pyrope_batcher_search(self._b._b, _p(q), int(topK), ms, npb, _p(scores), _p(ids), C.byref(cnt))
+        if rc != _lib.OK:
+            _raise_msg(rc, (L.pyrope_batcher_last_error() or b"").decode("utf-8", "replace"))
+        n = cnt.value
+        names = _id_strings(ids[:n]) if n else []
+        return [SearchResult(names[j], float(scores[j])) for j in range(n)]
+
+    def stats(self) -> dict:
+        return self._b.stats()
+
+    def close(self):
+        self._b.close()
