@@ -115,6 +115,16 @@ int pyrope_index_build(pyrope_index *h);
 /* Bound the training set to the first max_train_rows rows (<=0: all, the reference rule) and the
  * Lloyd iterations (<=0: 10, the reference default).  Opt-in deviation for very large builds. */
 int pyrope_index_set_train_params(pyrope_index *h, int64_t max_train_rows, int max_iter);
+/* Extend (opt-in, no counterpart in the reference): append the write buffer to the inverted lists of a BUILT IVF index
+ * without re-training — FAISS's "add to a trained index".  Every live buffer row, in slot order, goes to its nearest
+ * CURRENT centroid (the bit-exact assignment Build uses); IVF_PQ rows are encoded with the CURRENT codebooks (ksub
+ * honoured).  Each row is appended to the END of its list, rows of one list in slot order, and keeps its row ordinal.
+ * Existing entries keep their positions, row ordinals, labels and dead flags (nothing is compacted, so MaxScans walks
+ * old entries in the same order), except that shadowed entries become deleted: their replacements have just left the
+ * buffer.  The buffer is emptied; centroids, codebooks and next row ordinal are unchanged.  A shard
+ * (pyrope_index_set_shard) appends only to the lists it owns and empties its replica of the buffer.  All or nothing:
+ * on any error the index is exactly as it was.  FLAT -> UNSUPPORTED, not built -> INVALID_STATE, empty buffer -> OK. */
+int pyrope_index_extend(pyrope_index *h);
 /* Freeze codebooks as given inputs: centroids [n_centroids][dim]; pq_codebooks [m][k][dim/m]
  * (NULL for IVF_FLAT).  The next pyrope_index_build only assigns (+ encodes). */
 int pyrope_index_set_codebooks(pyrope_index *h, int n_centroids, const float *centroids,
@@ -293,6 +303,10 @@ int pyrope_sharded_shadow_row(pyrope_sharded *s, int64_t row, int shadowed);
 /* pyrope_index_set_labels with global row ordinals (FLAT shards map their local rows through the row blocks). */
 int pyrope_sharded_set_labels(pyrope_sharded *s, int64_t n_rows, const int64_t *labels_by_row);
 int pyrope_sharded_build(pyrope_sharded *s);
+/* pyrope_index_extend over N devices: every shard prepares on its own thread (assign, encode, merged lists), and the
+ * merges are committed only if all of them prepared and all report the same set of buffered row ordinals (else
+ * INVALID_STATE); on any failure no shard changes. */
+int pyrope_sharded_extend(pyrope_sharded *s);
 int pyrope_sharded_stats(pyrope_sharded *s, int64_t *live_rows_out);
 /* read from the first shard: the replicas are bit-identical */
 int pyrope_sharded_is_built(pyrope_sharded *s, int *out);
@@ -387,6 +401,9 @@ int pyrope_delta_compact(pyrope_delta *d, int64_t *moved_out, int64_t *tail_rows
  * memory while training) leaves every id addressable and can simply be retried. */
 int pyrope_delta_move(pyrope_delta *d, int64_t *moved_out, int64_t *tail_rows_out);
 int pyrope_delta_build_tail(pyrope_delta *d);
+/* The Extend counterpart of pyrope_delta_build_tail (one-device and sharded tails): a compaction by Extend is
+ * pyrope_delta_move followed by this call — the moved rows join the tail's lists without re-training. */
+int pyrope_delta_extend_tail(pyrope_delta *d);
 /* DeltaVectorIndex.GetStats :224-239: head count + tail count (duplicates counted twice, as there). */
 int pyrope_delta_stats(pyrope_delta *d, int64_t *count_out);
 /* DeltaVectorIndex.Snapshot / Load :160-222: path + ".head", path + ".tail" and a manifest at path. */
@@ -418,6 +435,11 @@ int pyrope_vindex_add(pyrope_vindex *v, const char *id, const float *vec, int le
 int pyrope_vindex_upsert(pyrope_vindex *v, const char *id, const float *vec, int len);
 int pyrope_vindex_delete(pyrope_vindex *v, const char *id, int *removed_out);
 int pyrope_vindex_build(pyrope_vindex *v); /* a delta compacts: DeltaVectorIndex.Build :124-158 */
+/* Extend (pyrope_index_extend) with the id bookkeeping: buffered ids become list ids, shadowed list rows are gone, no id
+ * is dropped (an IVF_PQ Build drops the ids it does not re-encode).  A delta compacts like pyrope_vindex_build with
+ * pyrope_delta_extend_tail in place of the tail's Build; a FLAT tail -> UNSUPPORTED and an unbuilt tail -> INVALID_STATE
+ * before any row moves. */
+int pyrope_vindex_extend(pyrope_vindex *v);
 /* nq queries of `len` floats each (len != Dimension -> DIMENSION). */
 int pyrope_vindex_search(pyrope_vindex *v, int64_t nq, const float *Q, int len, int topk, int64_t max_scans,
                          int nprobe, float *scores_out, int64_t *id_ordinals_out, int32_t *counts_out);

@@ -51,6 +51,7 @@ SIGNATURES = {
     "pyrope_index_set_labels": (C.c_int, [vp, C.c_int64, vp]),
     "pyrope_index_set_quantization": (C.c_int, [vp, C.c_int]),
     "pyrope_index_build": (C.c_int, [vp]),
+    "pyrope_index_extend": (C.c_int, [vp]),
     "pyrope_index_set_train_params": (C.c_int, [vp, C.c_int64, C.c_int]),
     "pyrope_index_set_codebooks": (C.c_int, [vp, C.c_int, vp, vp]),
     "pyrope_index_set_shard": (C.c_int, [vp, C.c_int, C.c_int]),
@@ -79,6 +80,7 @@ SIGNATURES = {
     "pyrope_sharded_snapshot": (C.c_int, [vp, C.c_char_p]),
     "pyrope_sharded_load": (C.c_int, [vp, C.c_char_p]),
     "pyrope_sharded_build": (C.c_int, [vp]),
+    "pyrope_sharded_extend": (C.c_int, [vp]),
     "pyrope_sharded_stats": (C.c_int, [vp, i64p]),
     "pyrope_sharded_search_batch": (C.c_int, [vp, C.c_int64, vp, C.c_int, C.c_int64, C.c_int, vp, vp, vp]),
     "pyrope_sharded_search_batch_device": (C.c_int, [vp, C.c_int64, vp, C.c_int, C.c_int64, C.c_int, vp, vp, vp]),
@@ -125,6 +127,7 @@ SIGNATURES = {
     "pyrope_delta_compact": (C.c_int, [vp, i64p, vp]),
     "pyrope_delta_move": (C.c_int, [vp, i64p, vp]),
     "pyrope_delta_build_tail": (C.c_int, [vp]),
+    "pyrope_delta_extend_tail": (C.c_int, [vp]),
     "pyrope_delta_stats": (C.c_int, [vp, i64p]),
     "pyrope_delta_snapshot": (C.c_int, [vp, C.c_char_p]),
     "pyrope_delta_load": (C.c_int, [vp, C.c_char_p]),
@@ -138,6 +141,7 @@ SIGNATURES = {
     "pyrope_vindex_upsert": (C.c_int, [vp, C.c_char_p, vp, C.c_int]),
     "pyrope_vindex_delete": (C.c_int, [vp, C.c_char_p, i32p]),
     "pyrope_vindex_build": (C.c_int, [vp]),
+    "pyrope_vindex_extend": (C.c_int, [vp]),
     "pyrope_vindex_search": (C.c_int, [vp, C.c_int64, vp, C.c_int, C.c_int, C.c_int64, C.c_int, vp, vp, vp]),
     "pyrope_vindex_id": (C.c_int, [C.c_int64, C.c_char_p, C.c_int, i32p]),
     "pyrope_vindex_ids": (C.c_int, [vp, C.c_int64, vp, C.c_int64, vp, i64p]),
@@ -257,6 +261,10 @@ class GpuIndex:
     # ---- build
     def build(self):
         check(load().pyrope_index_build(self._h))
+
+    def extend(self):
+        """Append the write buffer to the built inverted lists without re-training (pyrope_index_extend)."""
+        check(load().pyrope_index_extend(self._h))
 
     def set_train_params(self, max_train_rows=0, max_iter=0):
         check(load().pyrope_index_set_train_params(self._h, max_train_rows, max_iter))
@@ -517,6 +525,10 @@ class ShardedIndex:
 
     def build(self):
         self._ck(load().pyrope_sharded_build(self._s))
+
+    def extend(self):
+        """pyrope_sharded_extend: every shard appends the buffer to the lists it owns, all or nothing."""
+        self._ck(load().pyrope_sharded_extend(self._s))
 
     def is_built(self) -> bool:
         out = C.c_int32(0)

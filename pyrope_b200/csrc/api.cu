@@ -655,21 +655,35 @@ int gather_build_data(Index* h, bool include_lists, BuildData& bd) {
     return PYROPE_OK;
 }
 
-int finish_lists(Index* h, const BuildData& bd, int32_t* d_assign, int nc, SortScratch& sc,
-                 const void* payload, int64_t payload_row_bytes, DevBuf& payload_out) {
+// Stable grouping of n assigned rows by list (sc.vals_out = row order, sc.offs = [nc+1] offsets).  A shard keeps only
+// the lists it owns (l % world == rank): rows of foreign lists sort to the tail and are cut off; kept_out = rows kept.
+int group_rows(Index* h, int32_t* d_assign, int64_t n, int nc, SortScratch& sc, int64_t* kept_out) {
     cudaStream_t st = h->stream;
-    int64_t n = bd.n;
+    *kept_out = n;
     if (h->shard_world > 1) {
         shard_mask_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(d_assign, n, nc, h->shard_rank, h->shard_world);
         CK(cudaGetLastError());
         TRY(group_by_cluster(d_assign, n, nc + 1, sc, st));
-        int64_t kept = 0;
-        CK(cudaMemcpyAsync(&kept, sc.offs.as<int64_t>() + nc, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
+        CK(cudaMemcpyAsync(kept_out, sc.offs.as<int64_t>() + nc, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
         CK(cudaStreamSynchronize(st));
-        n = kept;  // rows of foreign lists sort to the tail and are cut off
     } else {
         TRY(group_by_cluster(d_assign, n, nc, sc, st));
     }
+    return PYROPE_OK;
+}
+
+// the write buffer is consumed by Build (IvfFlatVectorIndex.cs:143, IvfPqVectorIndex.cs:109) and by Extend;
+// give large buffers back to the allocator, keep small ones for the next writes
+void consume_buffer(Index* h) {
+    if ((size_t)h->seg.cap * h->dim * sizeof(float) > ((size_t)256 << 20)) h->seg.release();
+    else h->seg.clear();
+}
+
+int finish_lists(Index* h, const BuildData& bd, int32_t* d_assign, int nc, SortScratch& sc,
+                 const void* payload, int64_t payload_row_bytes, DevBuf& payload_out) {
+    cudaStream_t st = h->stream;
+    int64_t n = bd.n;
+    TRY(group_rows(h, d_assign, bd.n, nc, sc, &n));
     DevBuf order64;
     TRY(order64.ensure(sizeof(int64_t) * (size_t)bd.n, 0, st, true));
     order_to_i64_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(sc.vals_out.as<int32_t>(), n, order64.as<int64_t>());
@@ -697,10 +711,41 @@ int finish_lists(Index* h, const BuildData& bd, int32_t* d_assign, int nc, SortS
     h->built = true;
     h->tc_cent.invalidate();
     h->lists_loc_valid = false;
-    // the write buffer is consumed by Build (IvfFlatVectorIndex.cs:143, IvfPqVectorIndex.cs:109);
-    // give large buffers back to the allocator, keep small ones for the next writes
-    if ((size_t)h->seg.cap * h->dim * sizeof(float) > ((size_t)256 << 20)) h->seg.release();
-    else h->seg.clear();
+    consume_buffer(h);
+    return PYROPE_OK;
+}
+
+// KMeansUtils.FindNearestCentroid against the index's current centroids (cnorms must be current) -> assign[n]
+int assign_to_centroids(Index* h, const float* X, int64_t n, int nc, DevBuf& assign) {
+    cudaStream_t st = h->stream;
+    TRY(assign.ensure(sizeof(int32_t) * (size_t)std::max<int64_t>(n, 1), 0, st, true));
+    AssignScratch as;
+    TRY(assign_rows(h->metric, h->dim, n, X, h->dim, nc, h->centroids.as<float>(), h->cnorms.as<float>(),
+                    assign.as<int32_t>(), as, true, st));
+    CK(cudaStreamSynchronize(st));
+    return PYROPE_OK;
+}
+
+// rows of encoding work per residual chunk
+int64_t pq_encode_chunk(int64_t n) { return std::min<int64_t>(n, (int64_t)4 << 20); }
+
+// IvfPqVectorIndex.cs:82-90: residual to the assigned centroid, ProductQuantizer.Encode with the current codebooks
+// (honouring ksub) -> codes[n][m].  res: scratch of at least pq_encode_chunk(n) rows (grown here if needed).
+int pq_encode_rows(Index* h, const float* X, int64_t n, const int32_t* assign, DevBuf& res, DevBuf& codes) {
+    cudaStream_t st = h->stream;
+    const int dim = h->dim, m = h->m;
+    const int64_t chunk = pq_encode_chunk(n);
+    TRY(res.ensure(sizeof(float) * (size_t)std::max<int64_t>(chunk, 1) * dim, 0, st, true));
+    TRY(h->ksub_d.ensure(sizeof(int32_t) * (size_t)m, 0, st, true));
+    CK(cudaMemcpyAsync(h->ksub_d.p, h->ksub.data(), sizeof(int32_t) * (size_t)m, cudaMemcpyHostToDevice, st));
+    TRY(codes.ensure((size_t)std::max<int64_t>(n, 1) * m, 0, st, true));
+    for (int64_t c0 = 0; c0 < n; c0 += chunk) {
+        int64_t cn = std::min(chunk, n - c0);
+        CK(launch_residuals(X + (size_t)c0 * dim, cn, dim, h->centroids.as<float>(), assign + c0, res.as<float>(), st));
+        CK(launch_pq_encode_exact(res.as<float>(), cn, dim, m, h->k, h->codebook.as<float>(), h->ksub_d.as<int32_t>(),
+                                  codes.as<uint8_t>() + (size_t)c0 * m, st));
+    }
+    CK(cudaStreamSynchronize(st));
     return PYROPE_OK;
 }
 
@@ -730,13 +775,7 @@ int build_ivfflat(Index* h) {
     TRY(h->cnorms.ensure(sizeof(float) * (size_t)nc, 0, st, true));
     if (h->metric == kCosine) CK(launch_row_norms_exact(h->centroids.as<float>(), nc, dim, dim, h->cnorms.as<float>(), st));
     DevBuf assign;
-    TRY(assign.ensure(sizeof(int32_t) * (size_t)bd.n, 0, st, true));
-    {
-        AssignScratch as;
-        TRY(assign_rows(h->metric, dim, bd.n, bd.X, dim, nc, h->centroids.as<float>(), h->cnorms.as<float>(),
-                        assign.as<int32_t>(), as, true, st));
-        CK(cudaStreamSynchronize(st));
-    }
+    TRY(assign_to_centroids(h, bd.X, bd.n, nc, assign));
     SortScratch sc;
     DevBuf newvecs;
     TRY(finish_lists(h, bd, assign.as<int32_t>(), nc, sc, bd.X, (int64_t)dim * 4, newvecs));
@@ -777,15 +816,9 @@ int build_ivfpq(Index* h) {
     TRY(h->cnorms.ensure(sizeof(float) * (size_t)nc, 0, st, true));
     if (h->metric == kCosine) CK(launch_row_norms_exact(h->centroids.as<float>(), nc, dim, dim, h->cnorms.as<float>(), st));
     DevBuf assign;
-    TRY(assign.ensure(sizeof(int32_t) * (size_t)n, 0, st, true));
-    {
-        AssignScratch as;
-        TRY(assign_rows(h->metric, dim, n, bd.X, dim, nc, h->centroids.as<float>(), h->cnorms.as<float>(),
-                        assign.as<int32_t>(), as, true, st));
-        CK(cudaStreamSynchronize(st));
-    }
+    TRY(assign_to_centroids(h, bd.X, n, nc, assign));
     // PQ training on the residuals of the training rows (ProductQuantizer.cs:28-58)
-    const int64_t chunk = std::min<int64_t>(n, (int64_t)4 << 20);
+    const int64_t chunk = pq_encode_chunk(n);
     DevBuf res;
     TRY(res.ensure(sizeof(float) * (size_t)std::max(chunk, h->frozen ? (int64_t)0 : ntrain) * dim, 0, st, true));
     if (!h->frozen) {
@@ -806,18 +839,8 @@ int build_ivfpq(Index* h) {
             CK(cudaStreamSynchronize(st));
         }
     }
-    TRY(h->ksub_d.ensure(sizeof(int32_t) * (size_t)m, 0, st, true));
-    CK(cudaMemcpyAsync(h->ksub_d.p, h->ksub.data(), sizeof(int32_t) * (size_t)m, cudaMemcpyHostToDevice, st));
-    // encode in chunks
     DevBuf codes;
-    TRY(codes.ensure((size_t)n * m, 0, st, true));
-    for (int64_t c0 = 0; c0 < n; c0 += chunk) {
-        int64_t cn = std::min(chunk, n - c0);
-        CK(launch_residuals(bd.X + (size_t)c0 * dim, cn, dim, h->centroids.as<float>(), assign.as<int32_t>() + c0,
-                            res.as<float>(), st));
-        CK(launch_pq_encode_exact(res.as<float>(), cn, dim, m, K, h->codebook.as<float>(), h->ksub_d.as<int32_t>(),
-                                  codes.as<uint8_t>() + (size_t)c0 * m, st));
-    }
+    TRY(pq_encode_rows(h, bd.X, n, assign.as<int32_t>(), res, codes));
     SortScratch sc;
     DevBuf newcodes;
     TRY(finish_lists(h, bd, assign.as<int32_t>(), nc, sc, codes.p, m, newcodes));
@@ -826,6 +849,111 @@ int build_ivfpq(Index* h) {
     h->lm_codes16_ok = false;
     CK(cudaStreamSynchronize(st));
     return PYROPE_OK;
+}
+
+// ---- Extend: append the write buffer to the inverted lists of a built IVF index without re-training.  Every live
+// buffer row (slot order) goes to its nearest CURRENT centroid (assign_rows, as Build), IVF_PQ rows are encoded with the
+// CURRENT codebooks, and each row is appended to the end of its list (rows of one list keep slot order: group_rows is a
+// stable sort).  Old entries keep their order, row ordinals, labels and dead flags, except that shadowed entries (flag 2:
+// their replacement has just left the buffer) become deleted.  A shard appends only to the lists it owns.
+// extend_prepare does everything that can fail and builds the merged arrays aside; extend_commit only swaps them in.
+struct StagedExtend {
+    bool noop = true;
+    std::vector<int64_t> moved;  // row ordinals leaving the buffer, slot order
+    DevBuf payload, rows, labels, dead, norms, off;
+    std::vector<int64_t> off_h;
+    std::vector<uint8_t> dead_h;
+    int64_t total = 0, max_len = 0;
+};
+
+// caller holds h->mu
+int extend_prepare(Index* h, StagedExtend& S) {
+    if (h->kind == PYROPE_FLAT) return fail(PYROPE_ERR_UNSUPPORTED, "Extend needs an IVF index: FLAT has no inverted lists");
+    if (!h->built) return fail(PYROPE_ERR_INVALID_STATE, "Extend needs a built index: call Build first");
+    cudaStream_t st = h->stream;
+    CK(cudaStreamSynchronize(st));
+    if (h->last_stream) CK(cudaStreamSynchronize(h->last_stream));
+    const Segment& s = h->seg;
+    if (s.live == 0) return PYROPE_OK;
+    const int dim = h->dim, nc = h->nc;
+    BuildData bd;
+    TRY(gather_build_data(h, false, bd));  // live buffer slots, slot order
+    const int64_t n = bd.n;
+    S.moved.reserve((size_t)n);
+    for (int64_t i = 0; i < s.nslots; ++i)
+        if (!s.dead_h[(size_t)i]) S.moved.push_back(s.slot_row[(size_t)i]);
+    DevBuf assign, res, codes, nnorm;
+    TRY(assign_to_centroids(h, bd.X, n, nc, assign));
+    const bool pq = h->kind == PYROPE_IVF_PQ, cos_norms = !pq && h->metric == kCosine;
+    const int64_t rb = pq ? h->m : (int64_t)dim * 4;
+    if (pq) TRY(pq_encode_rows(h, bd.X, n, assign.as<int32_t>(), res, codes));
+    if (cos_norms) {
+        TRY(nnorm.ensure(sizeof(float) * (size_t)n, 0, st, true));
+        CK(launch_row_norms_exact(bd.X, n, dim, dim, nnorm.as<float>(), st));
+    }
+    SortScratch sc;
+    int64_t kept = 0;
+    TRY(group_rows(h, assign.as<int32_t>(), n, nc, sc, &kept));
+    std::vector<int64_t> offs_new((size_t)nc + 1);
+    CK(cudaMemcpyAsync(offs_new.data(), sc.offs.p, sizeof(int64_t) * offs_new.size(), cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    S.total = h->list_total + kept;
+    S.off_h.resize((size_t)nc + 1);
+    for (int c = 0; c <= nc; ++c) S.off_h[(size_t)c] = h->list_off_h[(size_t)c] + offs_new[(size_t)c];
+    for (int c = 0; c < nc; ++c) S.max_len = std::max(S.max_len, S.off_h[(size_t)c + 1] - S.off_h[(size_t)c]);
+    const size_t t1 = (size_t)std::max<int64_t>(S.total, 1);
+    TRY(S.off.ensure(sizeof(int64_t) * S.off_h.size(), 0, st, true));
+    CK(cudaMemcpyAsync(S.off.p, S.off_h.data(), sizeof(int64_t) * S.off_h.size(), cudaMemcpyHostToDevice, st));
+    TRY(S.payload.ensure(t1 * (size_t)rb, 0, st, true));
+    TRY(S.rows.ensure(sizeof(int64_t) * t1, 0, st, true));
+    TRY(S.labels.ensure(sizeof(int64_t) * t1, 0, st, true));
+    const bool has_dead = !h->list_dead_h.empty();
+    if (has_dead) TRY(S.dead.ensure(t1, 0, st, true));
+    if (cos_norms) TRY(S.norms.ensure(sizeof(float) * t1, 0, st, true));
+
+    ExtendMergeParams mp{};
+    mp.off_old = h->list_off.as<int64_t>(); mp.offs_new = sc.offs.as<int64_t>(); mp.off_merged = S.off.as<int64_t>();
+    mp.order = sc.vals_out.as<int32_t>(); mp.nc = nc;
+    auto col = [&](const void* old_src, const void* new_src, DevBuf& dst, int64_t row_bytes, int fold) {
+        ExtendMergeColumn& c = mp.col[mp.ncols++];
+        c.old_src = (const uint8_t*)old_src; c.new_src = (const uint8_t*)new_src; c.dst = dst.as<uint8_t>();
+        c.row_bytes = row_bytes; c.fold_flags = fold;
+    };
+    col(pq ? h->list_codes.p : h->list_vecs.p, pq ? codes.p : (const void*)bd.X, S.payload, rb, 0);
+    col(h->list_rows.p, bd.rows.p, S.rows, 8, 0);
+    col(h->list_labels.p, bd.labels.p, S.labels, 8, 0);
+    if (has_dead) col(h->list_dead.p, nullptr, S.dead, 1, 1);
+    if (cos_norms) col(h->list_norms.p, nnorm.p, S.norms, 4, 0);
+    CK(launch_extend_merge(mp, S.total, st));
+    CK(cudaStreamSynchronize(st));
+    if (has_dead) {
+        S.dead_h.assign((size_t)S.total, 0);
+        for (int c = 0; c < nc; ++c) {
+            const int64_t o = h->list_off_h[(size_t)c], len = h->list_off_h[(size_t)c + 1] - o;
+            for (int64_t i = 0; i < len; ++i) S.dead_h[(size_t)(o + offs_new[(size_t)c] + i)] = h->list_dead_h[(size_t)(o + i)] ? 1 : 0;
+        }
+    }
+    S.noop = false;
+    return PYROPE_OK;
+}
+
+// caller holds h->mu; nothing here can fail
+void extend_commit(Index* h, StagedExtend& S) {
+    if (S.noop) return;
+    auto take = [](DevBuf& dst, DevBuf& src) { std::swap(dst.p, src.p); std::swap(dst.bytes, src.bytes); src.release(); };
+    take(h->kind == PYROPE_IVF_PQ ? h->list_codes : h->list_vecs, S.payload);
+    take(h->list_rows, S.rows);
+    take(h->list_labels, S.labels);
+    take(h->list_off, S.off);
+    if (S.dead.p) { take(h->list_dead, S.dead); h->list_dead_h.swap(S.dead_h); }  // list_ndead: non-zero stays non-zero
+    if (S.norms.p) take(h->list_norms, S.norms);
+    h->list_off_h.swap(S.off_h);
+    h->list_total = S.total;
+    h->max_list_len = S.max_len;
+    h->lists_version++;
+    h->lists_loc_valid = false;
+    h->lm_codes16_ok = false;
+    consume_buffer(h);
 }
 
 // A MaxScans budget walks the probed lists entry by entry and never counts a deleted or shadowed entry
@@ -1576,6 +1704,43 @@ int pyrope_index_build(pyrope_index* h) {
     if (h->kind == PYROPE_IVF_FLAT) return build_ivfflat(h);
     return build_ivfpq(h);
 }
+
+int pyrope_index_extend(pyrope_index* h) {
+    if (!h) return fail(PYROPE_ERR_INVALID_ARG, "index handle is null");
+    std::lock_guard<std::mutex> g(h->mu);
+    StagedExtend S;
+    TRY(extend_prepare(h, S));
+    extend_commit(h, S);
+    return PYROPE_OK;
+}
+
+// ---- internal (not in the public header): the two halves of pyrope_index_extend for pyrope_sharded_extend.  _prepare
+// returns an opaque staged merge and the row ordinals that leave the buffer (owned by the staged object); _commit swaps
+// it in and frees it, _discard frees it unused.  Both run with the index's device current.
+int pyrope_internal_index_extend_prepare(pyrope_index* h, void** staged_out, int64_t* n_moved_out, const int64_t** moved_out) {
+    if (!h || !staged_out) return fail(PYROPE_ERR_INVALID_ARG, "index handle is null");
+    *staged_out = nullptr;
+    std::lock_guard<std::mutex> g(h->mu);
+    StagedExtend* S = new (std::nothrow) StagedExtend();
+    if (!S) return fail(PYROPE_ERR_OOM, "out of host memory");
+    int rc = extend_prepare(h, *S);
+    if (rc != PYROPE_OK) { delete S; return rc; }
+    if (n_moved_out) *n_moved_out = (int64_t)S->moved.size();
+    if (moved_out) *moved_out = S->moved.data();
+    *staged_out = S;
+    return PYROPE_OK;
+}
+
+void pyrope_internal_index_extend_commit(pyrope_index* h, void* staged) {
+    StagedExtend* S = static_cast<StagedExtend*>(staged);
+    {
+        std::lock_guard<std::mutex> g(h->mu);
+        extend_commit(h, *S);
+    }
+    delete S;
+}
+
+void pyrope_internal_index_extend_discard(void* staged) { delete static_cast<StagedExtend*>(staged); }
 
 int pyrope_index_set_train_params(pyrope_index* h, int64_t max_train_rows, int max_iter) {
     if (!h) return fail(PYROPE_ERR_INVALID_ARG, "index handle is null");
@@ -2559,7 +2724,9 @@ int tail_absorb(Index* tl, int64_t n, const float* mx, const int64_t* ml, const 
     std::vector<int64_t> target((size_t)n, -1);  // moved row -> tail buffer slot it overwrites
     DevBuf dsorted, where;
     Segment& ts = tl->seg;
-    const bool lists_matter = tl->built && tl->kind == PYROPE_IVF_FLAT && tl->list_total > 0;
+    // both IVF searches skip a list entry whose id is buffered (seenIds, IvfFlatVectorIndex.cs:210, IvfPqVectorIndex.cs:170),
+    // and an Extend that moves the buffered copy into the lists must find the entry it replaces flagged
+    const bool lists_matter = tl->built && tl->kind != PYROPE_FLAT && tl->list_total > 0;
     if (ts.live > 0 || lists_matter) {
         TRY(dsorted.ensure(sizeof(int64_t) * (size_t)n, 0, st, true));
         CK(cudaMemcpyAsync(dsorted.p, sorted.data(), sizeof(int64_t) * (size_t)n, cudaMemcpyHostToDevice, st));
@@ -2651,8 +2818,10 @@ int tail_absorb(Index* tl, int64_t n, const float* mx, const int64_t* ml, const 
 }
 
 // DeltaVectorIndex.Build :124-158 in two steps a caller can take apart: MOVE (head rows -> tail buffer, head tombstoned)
-// and BUILD (the tail's Build).  A host that keeps id tables updates them after the move whatever the build returns.
-int delta_compact_impl(pyrope_delta* d, int64_t* moved_out, int64_t* tail_rows_out, bool do_move, bool do_build) {
+// and BUILD (the tail's Build, or with extend its Extend).  A host that keeps id tables updates them after the move
+// whatever the build returns.
+int delta_compact_impl(pyrope_delta* d, int64_t* moved_out, int64_t* tail_rows_out, bool do_move, bool do_build,
+                       bool extend = false) {
     if (!d) return fail(PYROPE_ERR_INVALID_ARG, "delta handle is null");
     if (moved_out) *moved_out = 0;
     std::lock_guard<std::mutex> g(d->mu);
@@ -2694,9 +2863,15 @@ int delta_compact_impl(pyrope_delta* d, int64_t* moved_out, int64_t* tail_rows_o
     }
     // 4. _head.Build() is a no-op for FLAT; _tail.Build() (:151-152)
     if (!do_build) return PYROPE_OK;
-    if (d->stail) return spass(pyrope_sharded_build(d->stail));
+    if (d->stail) return spass(extend ? pyrope_sharded_extend(d->stail) : pyrope_sharded_build(d->stail));
     Index* tl = d->tail;
     std::lock_guard<std::mutex> gt(tl->mu);
+    if (extend) {
+        StagedExtend S;
+        TRY(extend_prepare(tl, S));
+        extend_commit(tl, S);
+        return PYROPE_OK;
+    }
     if (tl->kind == PYROPE_IVF_FLAT) return build_ivfflat(tl);
     if (tl->kind == PYROPE_IVF_PQ) return build_ivfpq(tl);
     return PYROPE_OK;
@@ -2731,6 +2906,7 @@ int pyrope_delta_move(pyrope_delta* d, int64_t* moved_out, int64_t* tail_rows_ou
     return delta_compact_impl(d, moved_out, tail_rows_out, true, false);
 }
 int pyrope_delta_build_tail(pyrope_delta* d) { return delta_compact_impl(d, nullptr, nullptr, false, true); }
+int pyrope_delta_extend_tail(pyrope_delta* d) { return delta_compact_impl(d, nullptr, nullptr, false, true, true); }
 
 int pyrope_delta_stats(pyrope_delta* d, int64_t* count_out) {
     if (!d || !count_out) return fail(PYROPE_ERR_INVALID_ARG, "null argument");

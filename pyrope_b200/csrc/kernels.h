@@ -254,6 +254,26 @@ cudaError_t launch_scatter_rows(const void* X, int64_t row_bytes, const int64_t*
 cudaError_t launch_find_labels(const int64_t* labels, const uint8_t* skip, int64_t n, const int64_t* sorted,
                                int64_t ns, int64_t* where, cudaStream_t st);
 cudaError_t launch_iota64(int64_t* out, int64_t n, int64_t base, cudaStream_t st);
+
+// ---- Extend: list merge (extend.cu) -----------------------------------------------------------
+// One column = one list-major array (payload, row ordinals, labels, dead flags, norms) of row_bytes per entry.  Merged
+// list c starts at off_merged[c] = off_old[c] + offs_new[c]: old entry i of list c moves to i + offs_new[c], new sorted
+// entry j (0-based within list c) goes to off_old[c + 1] + j, taken from row order[offs_new[c] + j] of new_src (buffer
+// order, [n][row_bytes]; nullptr writes zeros).  fold_flags: every non-zero old byte becomes 1 (shadowed -> deleted).
+constexpr int kExtendMaxColumns = 5;
+struct ExtendMergeColumn {
+    const uint8_t* old_src; const uint8_t* new_src; uint8_t* dst;
+    int64_t row_bytes; int fold_flags;
+    int64_t tile0;                           // set by the launcher
+};
+struct ExtendMergeParams {
+    const int64_t* off_old; const int64_t* offs_new; const int64_t* off_merged;  // [nc + 1] each
+    const int32_t* order; int nc; int ncols;
+    ExtendMergeColumn col[kExtendMaxColumns];
+};
+// CTAs of the merge for one column (16 KiB of merged bytes each)
+int64_t extend_merge_tiles(int64_t merged_rows, int64_t row_bytes);
+cudaError_t launch_extend_merge(ExtendMergeParams p, int64_t merged_rows, cudaStream_t st);
 cudaError_t launch_fill_uniform(float* out, int64_t n, uint64_t seed, uint64_t offset,
                                 cudaStream_t st);
 

@@ -37,6 +37,10 @@ extern "C" int pyrope_internal_index_load_prepare(pyrope_index* h, const char* p
                                                   int32_t* shard_world_out, int64_t* next_row_out);
 extern "C" void pyrope_internal_index_load_commit(pyrope_index* h, void* staged);
 extern "C" void pyrope_internal_index_load_discard(void* staged);
+extern "C" int pyrope_internal_index_extend_prepare(pyrope_index* h, void** staged_out, int64_t* n_moved_out,
+                                                    const int64_t** moved_out);
+extern "C" void pyrope_internal_index_extend_commit(pyrope_index* h, void* staged);
+extern "C" void pyrope_internal_index_extend_discard(void* staged);
 extern "C" int pyrope_internal_tail_reserve(pyrope_index* tl, int64_t n);
 extern "C" int pyrope_internal_tail_absorb(pyrope_index* tl, int64_t n, const float* dX, const int64_t* dL,
                                            const int64_t* labels_host, int64_t* tail_rows_out);
@@ -410,6 +414,38 @@ int pyrope_sharded_build(pyrope_sharded* s) {
         s->built = b != 0;
     }
     return rc;
+}
+
+// Extend on every shard: each prepares on its own thread (assign, encode, merged lists of the lists it owns) and the
+// merges are committed only if all of them prepared and all report the same row ordinals leaving their buffer replica.
+int pyrope_sharded_extend(pyrope_sharded* s) {
+    if (!s) return sfail(PYROPE_ERR_INVALID_ARG, "handle is null");
+    if (s->kind == PYROPE_FLAT) return sfail(PYROPE_ERR_UNSUPPORTED, "Extend needs an IVF index: FLAT has no inverted lists");
+    std::lock_guard<std::mutex> g(s->mu);
+    const size_t N = (size_t)s->n;
+    std::vector<void*> staged(N, nullptr);
+    std::vector<std::vector<int64_t>> moved(N);
+    int rc = run_all(s, [&](int r) -> int {
+        int64_t nm = 0;
+        const int64_t* rows = nullptr;
+        STRY(pyrope_internal_index_extend_prepare(s->shard[(size_t)r], &staged[(size_t)r], &nm, &rows));
+        moved[(size_t)r].assign(rows, rows + nm);
+        std::sort(moved[(size_t)r].begin(), moved[(size_t)r].end());
+        return PYROPE_OK;
+    });
+    for (size_t r = 1; rc == PYROPE_OK && r < N; ++r)
+        if (moved[r] != moved[0])
+            rc = sfail(PYROPE_ERR_INVALID_STATE, "shard %zu and shard 0 would move different buffered rows (%zu vs %zu): the buffer replicas diverged",
+                       r, moved[r].size(), moved[0].size());
+    if (rc != PYROPE_OK) {
+        run_all(s, [&](int r) -> int {
+            if (staged[(size_t)r]) pyrope_internal_index_extend_discard(staged[(size_t)r]);
+            return PYROPE_OK;
+        });
+        return rc;
+    }
+    run_all(s, [&](int r) -> int { pyrope_internal_index_extend_commit(s->shard[(size_t)r], staged[(size_t)r]); return PYROPE_OK; });
+    return PYROPE_OK;
 }
 
 int pyrope_sharded_stats(pyrope_sharded* s, int64_t* live_rows_out) {

@@ -189,6 +189,8 @@ int row_delete(V* v, int64_t row) {
     return v->sh ? spass(pyrope_sharded_delete_row(v->sh, row)) : vpass(pyrope_index_delete_row(v->h, row));
 }
 int row_build(V* v) { return v->sh ? spass(pyrope_sharded_build(v->sh)) : vpass(pyrope_index_build(v->h)); }
+int row_extend(V* v) { return v->sh ? spass(pyrope_sharded_extend(v->sh)) : vpass(pyrope_index_extend(v->h)); }
+int row_is_built(V* v, int* out) { return v->sh ? spass(pyrope_sharded_is_built(v->sh, out)) : vpass(pyrope_index_is_built(v->h, out)); }
 int row_set_labels(V* v, int64_t n, const int64_t* labels) {
     return v->sh ? spass(pyrope_sharded_set_labels(v->sh, n, labels)) : vpass(pyrope_index_set_labels(v->h, n, labels));
 }
@@ -319,6 +321,48 @@ int leaf_build(V* v) {
     const bool had_buffer = !v->buffered.empty();
     LTRY(row_build(v));
     leaf_after_build(v, had_buffer);
+    return PYROPE_OK;
+}
+
+// bookkeeping of a finished Extend: the buffered ids are now list ids under the same row ordinals, the list rows they
+// shadowed are deleted.  Unlike an IVF_PQ Build, no id that was only encoded is dropped.
+void leaf_after_extend(V* v) {
+    for (auto& kv : v->shadowed) v->gid_of_row[(size_t)kv.second] = -1;
+    v->shadowed.clear();
+    v->buffered.clear();
+    if (!v->row_of.empty()) v->built = true;
+}
+
+int leaf_extend(V* v) {
+    LTRY(row_extend(v));  // FLAT -> UNSUPPORTED, not built -> INVALID_STATE
+    leaf_after_extend(v);
+    return PYROPE_OK;
+}
+
+// DeltaVectorIndex.Build's move (:133-147): the head's live rows go to the tail's buffer, the id tables follow them.
+// Caller holds the unique locks of the delta and both sides.
+int delta_move_with_ids(V* v) {
+    V* hd = v->head;
+    V* tl = v->tail;
+    std::vector<int64_t> moved_gids;  // head scan order = row order, live rows only
+    for (size_t r = 0; r < hd->gid_of_row.size(); ++r)
+        if (hd->gid_of_row[r] >= 0) moved_gids.push_back(hd->gid_of_row[r]);
+    std::vector<int64_t> tail_rows(moved_gids.size() + 1, -1);
+    int64_t moved = 0;
+    VTRY(pyrope_delta_move(v->d, &moved, tail_rows.data()));
+    if (moved != (int64_t)moved_gids.size())
+        return vfail(PYROPE_ERR_INVALID_STATE, "compaction moved %lld rows, the id table expected %zu", (long long)moved,
+                     moved_gids.size());
+    for (size_t i = 0; i < moved_gids.size(); ++i) {  // what _tail.Add(id, vec) does to the tail's tables
+        const int64_t gid = moved_gids[i], row = tail_rows[i];
+        auto it = tl->row_of.find(gid);
+        if (it != tl->row_of.end() && !tl->buffered.count(gid) && it->second != row) tl->shadowed[gid] = it->second;
+        tl->set_row(gid, row);
+        tl->note_row(row, gid);
+        if (tl->kind != PYROPE_FLAT) tl->buffered.insert(gid);
+    }
+    std::fill(hd->gid_of_row.begin(), hd->gid_of_row.end(), (int64_t)-1);  // _head.Delete(id) for every moved id
+    hd->drop_all();
     return PYROPE_OK;
 }
 
@@ -561,30 +605,32 @@ int pyrope_vindex_build(pyrope_vindex* v) {
     V* tl = v->tail;
     std::unique_lock<std::shared_mutex> gh(hd->lock);
     std::unique_lock<std::shared_mutex> gt(tl->lock);
-    std::vector<int64_t> moved_gids;  // head scan order = row order, live rows only
-    for (size_t r = 0; r < hd->gid_of_row.size(); ++r)
-        if (hd->gid_of_row[r] >= 0) moved_gids.push_back(hd->gid_of_row[r]);
-    std::vector<int64_t> tail_rows(moved_gids.size() + 1, -1);
-    int64_t moved = 0;
-    const bool had_buffer = !tl->buffered.empty() || !moved_gids.empty();
+    const bool had_buffer = !tl->buffered.empty() || !hd->row_of.empty();
     // move first, book-keeping second, the tail's Build last: if the build fails (out of memory in k-means, say) the id
     // tables already describe where every row is, so Delete / Upsert / Snapshot keep working and Build can be retried
-    VTRY(pyrope_delta_move(v->d, &moved, tail_rows.data()));
-    if (moved != (int64_t)moved_gids.size())
-        return vfail(PYROPE_ERR_INVALID_STATE, "compaction moved %lld rows, the id table expected %zu", (long long)moved,
-                     moved_gids.size());
-    for (size_t i = 0; i < moved_gids.size(); ++i) {  // what _tail.Add(id, vec) does to the tail's tables
-        const int64_t gid = moved_gids[i], row = tail_rows[i];
-        auto it = tl->row_of.find(gid);
-        if (it != tl->row_of.end() && !tl->buffered.count(gid) && it->second != row) tl->shadowed[gid] = it->second;
-        tl->set_row(gid, row);
-        tl->note_row(row, gid);
-        if (tl->kind != PYROPE_FLAT) tl->buffered.insert(gid);
-    }
-    std::fill(hd->gid_of_row.begin(), hd->gid_of_row.end(), (int64_t)-1);  // _head.Delete(id) for every moved id
-    hd->drop_all();
+    LTRY(delta_move_with_ids(v));
     VTRY(pyrope_delta_build_tail(v->d));
     leaf_after_build(tl, had_buffer);
+    return PYROPE_OK;
+}
+
+int pyrope_vindex_extend(pyrope_vindex* v) {
+    if (!v) return vfail(PYROPE_ERR_INVALID_ARG, "index handle is null");
+    std::unique_lock<std::shared_mutex> g(v->lock);
+    if (!v->d) return leaf_extend(v);
+    // compaction by Extend: the move of pyrope_vindex_build, then the tail's Extend instead of its Build
+    V* hd = v->head;
+    V* tl = v->tail;
+    std::unique_lock<std::shared_mutex> gh(hd->lock);
+    std::unique_lock<std::shared_mutex> gt(tl->lock);
+    // a tail that cannot be extended refuses before any row moves
+    if (tl->kind == PYROPE_FLAT) return vfail(PYROPE_ERR_UNSUPPORTED, "Extend needs an IVF tail: FLAT has no inverted lists");
+    int built = 0;
+    LTRY(row_is_built(tl, &built));
+    if (!built) return vfail(PYROPE_ERR_INVALID_STATE, "Extend needs a built tail: call Build first");
+    LTRY(delta_move_with_ids(v));
+    VTRY(pyrope_delta_extend_tail(v->d));
+    leaf_after_extend(tl);
     return PYROPE_OK;
 }
 

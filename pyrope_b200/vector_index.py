@@ -211,6 +211,15 @@ class _VectorIndex:
             pass
 
 
+class _Extendable:
+    """Extend() of the IVF leaves and the Head+Tail (pyrope_vindex_extend; no counterpart in the reference): the write
+    buffer joins the built inverted lists without re-training.  On a DeltaVectorIndex it compacts the head into the tail
+    that way.  Not built -> InvalidOperationException."""
+
+    def Extend(self):
+        _ck(_lib.load().pyrope_vindex_extend(self._v))
+
+
 class _BorrowedGpuIndex(_lib.GpuIndex):
     """Row-ordinal view of a handle the vindex owns: never destroys it."""
 
@@ -273,7 +282,7 @@ class BruteForceVectorIndex(_Leaf):
         self._quant = bool(value)
 
 
-class IvfFlatVectorIndex(_Leaf):
+class IvfFlatVectorIndex(_Extendable, _Leaf):
     """IvfFlatVectorIndex(dimension, metric, nList = 100) — IvfFlatVectorIndex.cs:27-33.  devices (N or a list of CUDA
     ordinals) shards the inverted lists over those GPUs; results equal the one-device index's."""
 
@@ -282,7 +291,7 @@ class IvfFlatVectorIndex(_Leaf):
         self._create(_lib.IVF_FLAT, dimension, metric, nlist=nList, devices=devices)
 
 
-class IvfPqVectorIndex(_Leaf):
+class IvfPqVectorIndex(_Extendable, _Leaf):
     """IvfPqVectorIndex(dimension, metric, m, k = 256, nList = 100) — IvfPqVectorIndex.cs:27-35.  devices as for
     IvfFlatVectorIndex."""
 
@@ -292,7 +301,7 @@ class IvfPqVectorIndex(_Leaf):
         self._create(_lib.IVF_PQ, dimension, metric, nlist=nList, m=m, k=k, devices=devices)
 
 
-class DeltaVectorIndex(_VectorIndex):
+class DeltaVectorIndex(_Extendable, _VectorIndex):
     """DeltaVectorIndex(head, tail) — DeltaVectorIndex.cs:18-28; Search merges on the device, Build compacts
     head -> tail device-to-device."""
 
