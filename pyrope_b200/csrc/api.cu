@@ -429,7 +429,7 @@ int group_by_cluster(const int32_t* d_assign, int64_t n, int nc, SortScratch& sc
 
 // forward declaration (defined with the search helpers below)
 int ensure_tc_operand(TcOperand& op, const float* X, int64_t n, int dim, int metric, const uint8_t* dead,
-                      cudaStream_t st);
+                      cudaStream_t st, const float* norms = nullptr);
 
 struct AssignScratch {
     TcOperand cent;                       // tf32 split + proxy terms of the centroid table
@@ -449,7 +449,7 @@ int assign_rows(int metric, int dim, int64_t n, const float* X, int64_t ldx, int
         return PYROPE_OK;
     }
     if (centroids_changed) sc.cent.invalidate();
-    TRY(ensure_tc_operand(sc.cent, centroids, nc, dim, metric, nullptr, st));
+    TRY(ensure_tc_operand(sc.cent, centroids, nc, dim, metric, nullptr, st, cnorms));
     const int kprime = 1 + flat_tc_margin(1), cap = flat_tc_cap(kprime);
     const int64_t chunk = std::min<int64_t>(n, (int64_t)1 << 20);
     const int64_t chunk_pad = flat_tc_nq_pad(chunk);
@@ -1008,8 +1008,9 @@ int64_t segment_cutoff(const Segment& s, int64_t max_scans) {
     return s.nslots;
 }
 
+// norms (cosine): the exact row norms of X, which decide which rows score 0 (tc_rowterms_kernel)
 int ensure_tc_operand(TcOperand& op, const float* X, int64_t n, int dim, int metric, const uint8_t* dead,
-                      cudaStream_t st) {
+                      cudaStream_t st, const float* norms) {
     if (op.dirty) op.rows_valid = 0;
     const size_t keep_e = (size_t)op.rows_valid * dim * sizeof(float), keep_r = (size_t)op.rows_valid * sizeof(float);
     TRY(op.hi.ensure(sizeof(float) * (size_t)n * dim, keep_e, st));
@@ -1023,7 +1024,7 @@ int ensure_tc_operand(TcOperand& op, const float* X, int64_t n, int dim, int met
     if (op.rows_valid == 0) CK(cudaMemsetAsync(op.amax.p, 0, sizeof(float), st));
     if (op.rows_valid < n) {
         CK(launch_tc_prepare(X, n, dim, metric, dead, op.hi.as<float>(), op.lo.as<float>(), op.scale.as<float>(),
-                             op.bias.as<float>(), op.rows_valid, st));
+                             op.bias.as<float>(), op.rows_valid, st, metric == kCosine ? norms : nullptr));
         CK(launch_tc_amax(X, n, dim, op.scale.as<float>(), op.amax.as<float>(), op.rows_valid, st));
     }
     op.rows_valid = n;
@@ -1150,7 +1151,7 @@ int search_device(Index* h, int64_t nq, const float* dQ, int topk, int64_t max_s
                       const float* xnorm, const int64_t* labels, int kk, PairOut po) -> int {
         if (op.dirty || op.rows_valid < n_rows) ++launches;
         TRY(need_qsplit());
-        TRY(ensure_tc_operand(op, X, n_rows, dim, h->metric, dead, st));
+        TRY(ensure_tc_operand(op, X, n_rows, dim, h->metric, dead, st, xnorm));
         FlatTcParams tp{};
         tp.Q = dQ; tp.Qhi = ws.qhi.as<float>(); tp.Qlo = ws.qlo.as<float>(); tp.nq = nq; tp.dim = dim;
         tp.X = X; tp.Xhi = op.hi.as<float>(); tp.Xlo = op.lo.as<float>(); tp.n_rows = n_rows; tp.n_scan = n_scan_rows;
@@ -1236,7 +1237,7 @@ int search_device(Index* h, int64_t nq, const float* dQ, int topk, int64_t max_s
         TcOperand& op = h->tc_cent;
         if (op.dirty || op.rows_valid < h->nc) ++launches;
         if (op.dirty || op.rows_valid < h->nc) op.h16_rows = 0;
-        TRY(ensure_tc_operand(op, h->centroids.as<float>(), h->nc, dim, h->metric, nullptr, st));
+        TRY(ensure_tc_operand(op, h->centroids.as<float>(), h->nc, dim, h->metric, nullptr, st, h->cnorms.as<float>()));
         TRY(ws.ctc.ensure(coarse_tc_scratch_bytes(nq, h->nc, g_num_sms), 0, st));
         CoarseTcParams cp{};
         // L2 / IP, rows a multiple of 16 bytes in fp16: the tensor passes run on fp16 copies (twice the MMA rate, half the

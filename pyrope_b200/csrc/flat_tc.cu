@@ -772,9 +772,10 @@ __global__ void tc_split_kernel(const float* __restrict__ X, int64_t n_elems, fl
     }
 }
 
-// one warp per row: scale/bias of the proxy score
+// one warp per row: scale/bias of the proxy score.  norms (cosine, may be null): the exact row norms of the re-score
 __global__ void tc_rowterms_kernel(const float* __restrict__ X, int64_t n, int dim, int metric,
-                                   const uint8_t* __restrict__ dead, float* scale, float* bias) {
+                                   const uint8_t* __restrict__ dead, const float* __restrict__ norms, float* scale,
+                                   float* bias) {
     int64_t r = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     int lane = threadIdx.x & 31;
     if (r >= n) return;
@@ -787,7 +788,13 @@ __global__ void tc_rowterms_kernel(const float* __restrict__ X, int64_t n, int d
     if (lane == 0) {
         float sc = 1.f, b = 0.f;
         if (metric == kL2) { sc = 2.f; b = -a; }
-        else if (metric == kCosine) { float nrm = sqrtf(a); sc = nrm < 1e-6f ? 0.f : 1.f / nrm; }
+        else if (metric == kCosine) {
+            // zero or not is decided on the exact norm, as the re-score and the reference (VectorMath.cs) decide it: this
+            // lane-strided sum can land on the other side of 1e-6, and a crowd of rows that score 0 would then push the
+            // scoring rows out of the candidates (or a scoring row would be dropped)
+            const float nrm = sqrtf(a), cut = norms ? norms[r] : nrm;
+            sc = (cut < 1e-6f || nrm == 0.f) ? 0.f : 1.f / nrm;
+        }
         if (dead && dead[r]) b = -INFINITY;
         scale[r] = sc;
         bias[r] = b;
@@ -906,14 +913,16 @@ int flat_tc_pick_splits(int64_t nq, int64_t n_scan, int kprime, int num_sms) {
 }
 
 cudaError_t launch_tc_prepare(const float* X, int64_t n, int dim, int metric, const uint8_t* dead, float* hi, float* lo,
-                              float* scale, float* bias, int64_t from_row, cudaStream_t st) {
+                              float* scale, float* bias, int64_t from_row, cudaStream_t st, const float* norms) {
     if (n <= from_row) return cudaSuccess;
     const int64_t rows = n - from_row;
     const int64_t ne = rows * dim;
     tc_split_kernel<<<(unsigned)((ne / 4 + 256) / 256), 256, 0, st>>>(X + from_row * dim, ne, hi + from_row * dim, lo + from_row * dim);
     if (scale && bias)
         tc_rowterms_kernel<<<(unsigned)((rows * 32 + 255) / 256), 256, 0, st>>>(X + from_row * dim, rows, dim, metric,
-                                                                            dead ? dead + from_row : nullptr, scale + from_row, bias + from_row);
+                                                                            dead ? dead + from_row : nullptr,
+                                                                            norms ? norms + from_row : nullptr, scale + from_row,
+                                                                            bias + from_row);
     return cudaGetLastError();
 }
 
@@ -927,9 +936,9 @@ cudaError_t launch_tc_amax(const float* X, int64_t n, int dim, const float* scal
 }
 
 cudaError_t launch_tc_rowterms(const float* X, int64_t n, int dim, int metric, const uint8_t* dead, float* scale, float* bias,
-                               cudaStream_t st) {
+                               cudaStream_t st, const float* norms) {
     if (n <= 0) return cudaSuccess;
-    tc_rowterms_kernel<<<(unsigned)((n * 32 + 255) / 256), 256, 0, st>>>(X, n, dim, metric, dead, scale, bias);
+    tc_rowterms_kernel<<<(unsigned)((n * 32 + 255) / 256), 256, 0, st>>>(X, n, dim, metric, dead, norms, scale, bias);
     return cudaGetLastError();
 }
 

@@ -70,11 +70,13 @@ int flat_tc_margin(int k);
 int flat_tc_cap(int kprime);
 int flat_tc_pick_splits(int64_t nq, int64_t n_scan, int kprime, int num_sms);
 int64_t flat_tc_nq_pad(int64_t nq);
-// hi = tf32(x) (round to nearest), lo = x - hi for rows [from_row, n); scale/bias may be null
+// hi = tf32(x) (round to nearest), lo = x - hi for rows [from_row, n); scale/bias may be null.  norms (cosine): the
+// exact row norms [n] the re-score divides by; a row's proxy scale is 0 where they are below 1e-6
 cudaError_t launch_tc_prepare(const float* X, int64_t n, int dim, int metric, const uint8_t* dead, float* hi,
-                              float* lo, float* scale, float* bias, int64_t from_row, cudaStream_t st);
+                              float* lo, float* scale, float* bias, int64_t from_row, cudaStream_t st,
+                              const float* norms = nullptr);
 cudaError_t launch_tc_rowterms(const float* X, int64_t n, int dim, int metric, const uint8_t* dead, float* scale,
-                               float* bias, cudaStream_t st);
+                               float* bias, cudaStream_t st, const float* norms = nullptr);
 // amax (device float, zero-initialised) = max(amax, max over rows [from_row, n) of |scale_r| * |x_r|)
 cudaError_t launch_tc_amax(const float* X, int64_t n, int dim, const float* scale, float* amax, int64_t from_row,
                            cudaStream_t st);

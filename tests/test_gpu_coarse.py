@@ -8,6 +8,7 @@ import pytest
 
 from oracle import pyoracle as orc
 from tests.parity import assert_batch_equivalent
+from tests.test_gpu_flat_tc_regimes import in_child  # noqa: F401  (fixture: runs a function in a child process)
 
 pytestmark = pytest.mark.gpu
 
@@ -141,11 +142,42 @@ def test_coarse_probe_values_beyond_fp16(gpu):
     assert_batch_equivalent(ref2.search_batch(Q2, 10, nprobe=16), _s(ix2, Q2, 10, nprobe=16), ctx="centroid beyond fp16")
 
 
-def test_coarse_probe_fp16_and_tf32_passes_agree(gpu, monkeypatch):
+def _coarse_pass_case(gpu):
     rng = np.random.default_rng(44)
     cent = rng.random((30000, 128), dtype=np.float32)
     base = rng.random((80_000, 128), dtype=np.float32)
     ix, ref = _frozen_from(gpu, "L2", cent, base)
     Q = rng.random((300, 128), dtype=np.float32)
+    return ix, ref, Q
+
+
+def _cold_warm(ix, Q):
+    """Search twice: (result, launches of the first search, launches of the second)."""
     a = _s(ix, Q, 10, nprobe=24)
+    cold = ix.last_search_launches()
+    b = _s(ix, Q, 10, nprobe=24)
+    for x, y in zip(a, b):
+        np.testing.assert_array_equal(x, y)
+    return a, cold, ix.last_search_launches()
+
+
+def child_coarse_passes(out):
+    """Child-process side of the test below (PYROPE_COARSE_TF32 is read once per process)."""
+    import pyrope_b200 as pg
+    pg._lib.check(pg.load().pyrope_gpu_init(0))
+    ix, _, Q = _coarse_pass_case(pg)
+    (rows, sc, cnt), cold, warm = _cold_warm(ix, Q)
+    np.savez(out, rows=rows, scores=sc, counts=cnt, cold=cold, warm=warm)
+
+
+def test_coarse_probe_fp16_and_tf32_passes_agree(gpu, in_child):
+    """The same frozen IVF_PQ index probed by the fp16 passes (default) and, in a child process, by the tf32 passes
+    (PYROPE_COARSE_TF32=1): identical results, both the oracle's.  Only the fp16 passes convert the centroid table, on the
+    first search."""
+    ix, ref, Q = _coarse_pass_case(gpu)
+    a, cold, warm = _cold_warm(ix, Q)
     assert_batch_equivalent(ref.search_batch(Q, 10, nprobe=24), a, ctx="fp16 passes")
+    b = in_child({"PYROPE_COARSE_TF32": "1"}, "tests.test_gpu_coarse:child_coarse_passes")
+    for x, y in zip(a, (b["rows"], b["scores"], b["counts"])):
+        np.testing.assert_array_equal(x, y)
+    assert cold - warm == int(b["cold"]) - int(b["warm"]) + 1, (cold, warm, int(b["cold"]), int(b["warm"]))
