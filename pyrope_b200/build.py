@@ -11,7 +11,7 @@ CSRC = os.path.join(HERE, "csrc")
 OBJ = os.path.join(HERE, "build")
 LIB = os.path.join(HERE, "libpyrope_gpu.so")
 SOURCES = ["api.cu", "flat.cu", "ivf.cu", "pq.cu", "pq_lm.cu", "ivf_lm.cu", "build.cu", "flat_tc.cu", "coarse_tc.cu", "batcher.cu", "vindex.cu", "formats.cu", "sq8.cu", "sharded.cu", "peer.cu", "extend.cu"]
-HEADERS = ["common.cuh", "kernels.h", "exact_arith.cuh", "dotnet_random.h", "../../include/pyrope_gpu.h"]
+HEADERS = ["common.cuh", "internal.h", "kernels.h", "exact_arith.cuh", "dotnet_random.h", "../../include/pyrope_gpu.h"]
 
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 EXTRA = os.environ.get("PYROPE_NVCC_EXTRA", "").split()  # extra nvcc flags for experiments (e.g. a -D switch)

@@ -4,16 +4,18 @@
 // HBM layout (one index, one GPU):
 //   Segment (FLAT rows / IVF pre-build buffer): X[cap][dim] fp32 row-major, dead[cap] u8,
 //     labels[cap] i64, norms[cap] fp32 (Cosine only).  Scan order = slot order.
-//   IVF lists: list_off[nc+1] i64; entries list-major: list_vecs[total][dim] fp32 (IVF_FLAT) or
-//     list_codes[total][m] u8 (IVF_PQ), list_rows/list_labels[total] i64, list_dead[total] u8
-//     (allocated on first delete), list_norms (Cosine IVF_FLAT); centroids[nc][dim], cnorms[nc],
-//     codebook[m][k][dim/m] fp32 zero padded, ksub[m].
+//   IVF lists (IvfLists): off[nc+1] i64; entries list-major: payload[total][dim] fp32 (IVF_FLAT) or
+//     payload[total][m] u8 (IVF_PQ), rows/labels[total] i64, dead[total] u8 (allocated on first delete),
+//     norms (Cosine IVF_FLAT); centroids[nc][dim], cnorms[nc], codebook[m][k][dim/m] fp32 zero padded, ksub[m].
+// Build, Extend and Load replace the lists (and Build / Load the trained quantisers) the same way: a *_prepare that only
+// reads the index stages everything that can fail in a Staged, then install swaps it in and cannot fail.
 #include <cub/cub.cuh>
 
 #include <algorithm>
 #include <cstdarg>
 #include <cstdio>
 #include <cstring>
+#include <memory>
 #include <mutex>
 #include <string>
 #include <vector>
@@ -22,6 +24,7 @@
 #include "../../include/pyrope_gpu.h"
 #include "common.cuh"
 #include "dotnet_random.h"
+#include "internal.h"
 #include "kernels.h"
 
 using namespace pyrope;
@@ -68,10 +71,22 @@ int ensure_init() {
     return PYROPE_OK;
 }
 
-// grow-only device buffer
+// grow-only device buffer; owns its memory, so it moves but does not copy
 struct DevBuf {
     void* p = nullptr;
     size_t bytes = 0;
+    DevBuf() = default;
+    DevBuf(const DevBuf&) = delete;
+    DevBuf& operator=(const DevBuf&) = delete;
+    DevBuf(DevBuf&& o) noexcept : p(o.p), bytes(o.bytes) { o.p = nullptr; o.bytes = 0; }
+    DevBuf& operator=(DevBuf&& o) noexcept {
+        if (this != &o) {
+            release();
+            std::swap(p, o.p);
+            std::swap(bytes, o.bytes);
+        }
+        return *this;
+    }
     ~DevBuf() { release(); }
     void release() {
         if (p) cudaFree(p);
@@ -171,6 +186,16 @@ struct TcOperand {
     void invalidate() { dirty = true; h16_rows = 0; }
 };
 
+// The inverted lists of an IVF index.  Entry i of list c sits at off_h[c] <= i < off_h[c + 1]; payload rows are dim * 4
+// bytes (IVF_FLAT vectors) or m bytes (IVF_PQ codes).  dead[i]: bit 0 deleted, bit 1 shadowed by a buffered row; dead /
+// dead_h stay empty until the first flag is set, ndead counts the flagged entries.
+struct IvfLists {
+    DevBuf off, rows, labels, payload, dead, norms;
+    std::vector<int64_t> off_h;
+    std::vector<uint8_t> dead_h;
+    int64_t total = 0, ndead = 0, max_len = 0;
+};
+
 }  // namespace
 
 struct pyrope_index {
@@ -186,24 +211,20 @@ struct pyrope_index {
     // IVF state
     bool built = false;
     int nc = 0;
-    DevBuf centroids, cnorms, codebook, list_off, list_rows, list_labels, list_dead, list_vecs, list_codes,
-        list_norms;
-    std::vector<int64_t> list_off_h;
-    std::vector<uint8_t> list_dead_h;
-    int64_t list_total = 0, list_ndead = 0, max_list_len = 0;
+    DevBuf centroids, cnorms, codebook;
+    IvfLists lists;  // replaced only by install
     // compacted view of the lists for MaxScans-budgeted IVF_FLAT searches (compact_lists)
     DevBuf bv_vecs, bv_labels, bv_norms, bv_off;
     uint64_t lists_version = 1, bv_version = 0;  // lists_version moves whenever lists or their dead flags change
     // shape of the most recent list-major IVF_PQ search (for pyrope_index_last_search_scanned)
     int64_t lm_nq = 0; int lm_P = 0, lm_k = 0;
     std::vector<int32_t> ksub;
-    DevBuf ksub_d;
     // list-major IVF_PQ with m < 16: the equivalent 16-table quantiser (kernels.h, IvfPqScanParams::lm_codebook) and the
     // codes repeated to 16 bytes per row; rebuilt lazily after the codebook / the lists were replaced
     DevBuf lm_cb16, lm_codes16;
     bool lm_cb16_ok = false, lm_codes16_ok = false;
-    DevBuf pq_cmax;                    // list-major IVF_PQ: max codeword norm per sub-quantiser, valid for codebook_ptr
-    const void* cmax_for = nullptr;    // codebook buffer the cached bound was computed from (reset whenever it is rewritten)
+    DevBuf pq_cmax;            // list-major IVF_PQ: max codeword norm per sub-quantiser of the table the scan reads
+    bool pq_cmax_ok = false;   // reset whenever that table is rewritten
     bool frozen = false;  // codebooks supplied by the caller
     int64_t max_train_rows = 0;
     int max_iter = 0;
@@ -348,11 +369,12 @@ int add_common(Index* h, int64_t n, const float* X, bool dev, const int64_t* lab
 int rebuild_row_loc(Index* h) {
     if (h->lists_loc_valid) return PYROPE_OK;
     std::fill(h->row_loc.begin(), h->row_loc.end(), (int64_t)-1);
-    if (h->list_total > 0) {
-        std::vector<int64_t> rows((size_t)h->list_total);
-        CK(cudaMemcpy(rows.data(), h->list_rows.p, sizeof(int64_t) * rows.size(), cudaMemcpyDeviceToHost));
-        for (int64_t i = 0; i < h->list_total; ++i)
-            if (h->list_dead_h.empty() || !(h->list_dead_h[(size_t)i] & 1)) h->row_loc[(size_t)rows[(size_t)i]] = -2 - i;
+    const IvfLists& L = h->lists;
+    if (L.total > 0) {
+        std::vector<int64_t> rows((size_t)L.total);
+        CK(cudaMemcpy(rows.data(), L.rows.p, sizeof(int64_t) * rows.size(), cudaMemcpyDeviceToHost));
+        for (int64_t i = 0; i < L.total; ++i)
+            if (L.dead_h.empty() || !(L.dead_h[(size_t)i] & 1)) h->row_loc[(size_t)rows[(size_t)i]] = -2 - i;
     }
     for (int64_t s = 0; s < h->seg.nslots; ++s)
         if (!h->seg.dead_h[(size_t)s]) h->row_loc[(size_t)h->seg.slot_row[(size_t)s]] = s;
@@ -361,11 +383,30 @@ int rebuild_row_loc(Index* h) {
 }
 
 int ensure_list_dead(Index* h) {
-    if (h->list_dead.p && h->list_dead_h.size() == (size_t)h->list_total) return PYROPE_OK;
-    TRY(h->list_dead.ensure((size_t)std::max<int64_t>(h->list_total, 1), 0, h->stream, true));
-    CK(cudaMemsetAsync(h->list_dead.p, 0, (size_t)std::max<int64_t>(h->list_total, 1), h->stream));
-    h->list_dead_h.assign((size_t)h->list_total, 0);
-    h->list_ndead = 0;
+    IvfLists& L = h->lists;
+    if (L.dead.p && L.dead_h.size() == (size_t)L.total) return PYROPE_OK;
+    TRY(L.dead.ensure((size_t)std::max<int64_t>(L.total, 1), 0, h->stream, true));
+    CK(cudaMemsetAsync(L.dead.p, 0, (size_t)std::max<int64_t>(L.total, 1), h->stream));
+    L.dead_h.assign((size_t)L.total, 0);
+    L.ndead = 0;
+    return PYROPE_OK;
+}
+
+// Sets (set = true) or clears flag bits on the list entries at pos (ascending), keeping the host and device flags, the
+// count of flagged entries and lists_version in step.  Caller synchronises the stream.
+int set_list_flag(Index* h, const std::vector<int64_t>& pos, uint8_t bits, bool set) {
+    if (pos.empty()) return PYROPE_OK;
+    TRY(ensure_list_dead(h));
+    IvfLists& L = h->lists;
+    for (int64_t p : pos) {
+        uint8_t& f = L.dead_h[(size_t)p];
+        const uint8_t nv = set ? (f | bits) : (f & ~bits);
+        L.ndead += (nv != 0) - (f != 0);
+        f = nv;
+    }
+    h->lists_version++;
+    const size_t lo = (size_t)pos.front(), n = (size_t)pos.back() + 1 - lo;
+    CK(cudaMemcpyAsync(L.dead.as<uint8_t>() + lo, L.dead_h.data() + lo, n, cudaMemcpyHostToDevice, h->stream));
     return PYROPE_OK;
 }
 
@@ -539,26 +580,27 @@ struct BuildData {
 
 // Collect the rows a Build sees, in the reference's order: live list entries (list order) then
 // live buffer slots (slot order).  IVF_PQ passes lists=false (IvfPqVectorIndex.cs:64).
-int gather_build_data(Index* h, bool include_lists, BuildData& bd) {
-    cudaStream_t st = h->stream;
-    Segment& s = h->seg;
-    const int dim = h->dim;
+int gather_build_data(const Index& h, bool include_lists, BuildData& bd) {
+    cudaStream_t st = h.stream;
+    const Segment& s = h.seg;
+    const IvfLists& L = h.lists;
+    const int dim = h.dim;
     // uniqueData (IvfFlatVectorIndex.cs:91-108) is a Dictionary filled from the lists first, then from the buffer:
     // an indexed id that was re-added through the buffer KEEPS its list position and takes the buffer's vector.
     // A shadowed list entry (flag 2) is matched to the live buffer slot carrying the same label; callers that do
     // not pass labels get the buffer row appended at the end instead (their labels differ by construction).
     std::unordered_map<int64_t, int64_t> repl_at;  // list position -> buffer slot that replaces it
     std::vector<uint8_t> slot_used;
-    if (include_lists && h->built && !h->list_dead_h.empty() && s.live > 0) {
+    if (include_lists && h.built && !L.dead_h.empty() && s.live > 0) {
         std::vector<int64_t> sh;
-        for (int64_t i = 0; i < h->list_total; ++i)
-            if (h->list_dead_h[(size_t)i] == 2) sh.push_back(i);
+        for (int64_t i = 0; i < L.total; ++i)
+            if (L.dead_h[(size_t)i] == 2) sh.push_back(i);
         if (!sh.empty()) {
             DevBuf di, dl;
             TRY(di.ensure(sizeof(int64_t) * sh.size(), 0, st, true));
             TRY(dl.ensure(sizeof(int64_t) * sh.size(), 0, st, true));
             CK(cudaMemcpyAsync(di.p, sh.data(), sizeof(int64_t) * sh.size(), cudaMemcpyHostToDevice, st));
-            CK(launch_gather_rows(h->list_labels.p, 8, di.as<int64_t>(), (int64_t)sh.size(), dl.p, st));
+            CK(launch_gather_rows(L.labels.p, 8, di.as<int64_t>(), (int64_t)sh.size(), dl.p, st));
             std::vector<int64_t> shl(sh.size()), bl((size_t)s.nslots);
             CK(cudaMemcpyAsync(shl.data(), dl.p, sizeof(int64_t) * sh.size(), cudaMemcpyDeviceToHost, st));
             CK(cudaMemcpyAsync(bl.data(), s.labels.p, sizeof(int64_t) * (size_t)s.nslots, cudaMemcpyDeviceToHost, st));
@@ -577,10 +619,10 @@ int gather_build_data(Index* h, bool include_lists, BuildData& bd) {
     }
     std::vector<int64_t> list_pos;
     std::vector<int64_t> repl_out, repl_slot;  // output index <- buffer slot
-    if (include_lists && h->built) {
-        list_pos.reserve((size_t)h->list_total);
-        for (int64_t i = 0; i < h->list_total; ++i) {
-            if (h->list_dead_h.empty() || !h->list_dead_h[(size_t)i]) list_pos.push_back(i);
+    if (include_lists && h.built) {
+        list_pos.reserve((size_t)L.total);
+        for (int64_t i = 0; i < L.total; ++i) {
+            if (L.dead_h.empty() || !L.dead_h[(size_t)i]) list_pos.push_back(i);
             else if (!repl_at.empty()) {
                 auto it = repl_at.find(i);
                 if (it == repl_at.end()) continue;
@@ -617,9 +659,9 @@ int gather_build_data(Index* h, bool include_lists, BuildData& bd) {
     TRY(idx.ensure(sizeof(int64_t) * (size_t)std::max(nl, nb), 0, st, true));
     if (nl) {
         CK(cudaMemcpyAsync(idx.p, list_pos.data(), sizeof(int64_t) * (size_t)nl, cudaMemcpyHostToDevice, st));
-        CK(launch_gather_rows(h->list_vecs.p, (int64_t)dim * 4, idx.as<int64_t>(), nl, bd.Xown.p, st));
-        CK(launch_gather_rows(h->list_rows.p, 8, idx.as<int64_t>(), nl, bd.rows.p, st));
-        CK(launch_gather_rows(h->list_labels.p, 8, idx.as<int64_t>(), nl, bd.labels.p, st));
+        CK(launch_gather_rows(L.payload.p, (int64_t)dim * 4, idx.as<int64_t>(), nl, bd.Xown.p, st));
+        CK(launch_gather_rows(L.rows.p, 8, idx.as<int64_t>(), nl, bd.rows.p, st));
+        CK(launch_gather_rows(L.labels.p, 8, idx.as<int64_t>(), nl, bd.labels.p, st));
         CK(cudaStreamSynchronize(st));
     }
     if (!repl_out.empty()) {  // replaced entries: the buffer's vector and row ordinal at the list entry's place
@@ -657,11 +699,11 @@ int gather_build_data(Index* h, bool include_lists, BuildData& bd) {
 
 // Stable grouping of n assigned rows by list (sc.vals_out = row order, sc.offs = [nc+1] offsets).  A shard keeps only
 // the lists it owns (l % world == rank): rows of foreign lists sort to the tail and are cut off; kept_out = rows kept.
-int group_rows(Index* h, int32_t* d_assign, int64_t n, int nc, SortScratch& sc, int64_t* kept_out) {
-    cudaStream_t st = h->stream;
+int group_rows(const Index& h, int32_t* d_assign, int64_t n, int nc, SortScratch& sc, int64_t* kept_out) {
+    cudaStream_t st = h.stream;
     *kept_out = n;
-    if (h->shard_world > 1) {
-        shard_mask_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(d_assign, n, nc, h->shard_rank, h->shard_world);
+    if (h.shard_world > 1) {
+        shard_mask_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(d_assign, n, nc, h.shard_rank, h.shard_world);
         CK(cudaGetLastError());
         TRY(group_by_cluster(d_assign, n, nc + 1, sc, st));
         CK(cudaMemcpyAsync(kept_out, sc.offs.as<int64_t>() + nc, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
@@ -679,49 +721,119 @@ void consume_buffer(Index* h) {
     else h->seg.clear();
 }
 
-int finish_lists(Index* h, const BuildData& bd, int32_t* d_assign, int nc, SortScratch& sc,
-                 const void* payload, int64_t payload_row_bytes, DevBuf& payload_out) {
-    cudaStream_t st = h->stream;
+// Staged::moved of a Build or an Extend: the row ordinals of the live buffer slots in slot order.  Only a shard of a
+// sharded index needs them (every replica must move the same rows), so only a shard pays this host pass over the buffer
+std::vector<int64_t> buffered_rows(const Index& h) {
+    std::vector<int64_t> rows;
+    if (h.shard_world == 1) return rows;
+    const Segment& s = h.seg;
+    rows.reserve((size_t)s.live);
+    for (int64_t i = 0; i < s.nslots; ++i)
+        if (!s.dead_h[(size_t)i]) rows.push_back(s.slot_row[(size_t)i]);
+    return rows;
+}
+
+// What a Build, an Extend or a Load replaces in an index.  Its *_prepare fills it while only reading the index, and does
+// everything that can fail there; install then swaps it in.
+struct Staged {
+    explicit Staged(const Index& h) : nc(h.nc), built(h.built), frozen(h.frozen) {}
+    bool noop = true;  // an empty Build / Extend: nothing to install
+    IvfLists lists;
+    // quantiser: new centroids and (IVF_PQ) codebooks / ksub, from a Build that trains them or from a Load.  cnorms, when
+    // present, replaces the centroid norms
+    bool quantiser = false;
+    DevBuf centroids, cnorms, codebook;
+    std::vector<int32_t> ksub;
+    int nc;
+    bool built, frozen;
+    // load: the write buffer and the counters the file holds replace the index's; otherwise the buffer moved into the
+    // lists and is consumed (moved: its row ordinals in slot order, on a shard of a sharded index)
+    bool load = false;
+    Segment seg;
+    int nlist = 0;
+    int64_t next_row = 0;
+    int32_t shard_rank = 0, shard_world = 1;
+    std::vector<int64_t> moved;
+};
+
+// The only function that swaps trained state into an index, and the one place that resets what is derived from it.
+// Cannot fail.  Caller holds h->mu.
+void install(Index* h, Staged& S) {
+    if (S.noop) return;
+    h->lists = std::move(S.lists);
+    h->lists_version++;
+    h->lists_loc_valid = false;
+    h->lm_codes16_ok = false;
+    if (S.quantiser) {
+        h->centroids = std::move(S.centroids);
+        h->codebook = std::move(S.codebook);
+        h->ksub.swap(S.ksub);
+        h->lm_cb16_ok = false;
+        h->pq_cmax_ok = false;
+    }
+    if (S.quantiser || S.cnorms.p) h->tc_cent.invalidate();
+    if (S.cnorms.p) h->cnorms = std::move(S.cnorms);
+    h->nc = S.nc;
+    h->built = S.built;
+    h->frozen = S.frozen;
+    if (!S.load) {
+        consume_buffer(h);
+        return;
+    }
+    h->seg = std::move(S.seg);
+    h->tc_seg.invalidate();
+    h->nlist = S.nlist;
+    h->next_row = S.next_row;
+    h->shard_rank = S.shard_rank;
+    h->shard_world = S.shard_world;
+    if (h->kind != PYROPE_FLAT) h->row_loc.assign((size_t)h->next_row, -1);
+    // SQ8 (FLAT): the reference's Load re-adds every row through InternalAdd (BruteForceVectorIndex.cs:93-97 ->
+    // :162-184), which quantises it iff the LOADING index has EnableQuantization on at that moment — the flag is a
+    // property of the object, not of the file.  Same here: with the flag on every loaded row gets its byte copy
+    // (ScalarQuantizer is deterministic, so re-quantising reproduces the bytes the snapshotting index held), with it
+    // off no loaded row has a quantised form (:312-322 keeps such rows invisible to a later quantised search).
+    if (h->kind == PYROPE_FLAT && (h->sq8 || h->x8.p)) {
+        h->x8_cap = 0;
+        sq8_rows(h, 0, h->seg.nslots);  // best effort: the rows themselves are already in place
+    }
+}
+
+// New lists in S.lists for the bd.n rows of a Build, assigned to nc lists; payload: one row of payload_row_bytes per row
+int finish_lists(const Index& h, const BuildData& bd, int32_t* d_assign, int nc, const void* payload,
+                 int64_t payload_row_bytes, Staged& S) {
+    cudaStream_t st = h.stream;
+    IvfLists& L = S.lists;
+    SortScratch sc;
     int64_t n = bd.n;
     TRY(group_rows(h, d_assign, bd.n, nc, sc, &n));
     DevBuf order64;
     TRY(order64.ensure(sizeof(int64_t) * (size_t)bd.n, 0, st, true));
     order_to_i64_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(sc.vals_out.as<int32_t>(), n, order64.as<int64_t>());
     CK(cudaGetLastError());
-    TRY(payload_out.ensure((size_t)std::max<int64_t>(n, 1) * (size_t)payload_row_bytes, 0, st, true));
-    CK(launch_gather_rows(payload, payload_row_bytes, order64.as<int64_t>(), n, payload_out.p, st));
-    TRY(h->list_rows.ensure(sizeof(int64_t) * (size_t)std::max<int64_t>(n, 1), 0, st, true));
-    TRY(h->list_labels.ensure(sizeof(int64_t) * (size_t)std::max<int64_t>(n, 1), 0, st, true));
-    widen_rows_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(sc.vals_out.as<int32_t>(), bd.rows.as<int64_t>(), n, h->list_rows.as<int64_t>());
-    widen_rows_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(sc.vals_out.as<int32_t>(), bd.labels.as<int64_t>(), n, h->list_labels.as<int64_t>());
+    TRY(L.payload.ensure((size_t)std::max<int64_t>(n, 1) * (size_t)payload_row_bytes, 0, st, true));
+    CK(launch_gather_rows(payload, payload_row_bytes, order64.as<int64_t>(), n, L.payload.p, st));
+    TRY(L.rows.ensure(sizeof(int64_t) * (size_t)std::max<int64_t>(n, 1), 0, st, true));
+    TRY(L.labels.ensure(sizeof(int64_t) * (size_t)std::max<int64_t>(n, 1), 0, st, true));
+    widen_rows_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(sc.vals_out.as<int32_t>(), bd.rows.as<int64_t>(), n, L.rows.as<int64_t>());
+    widen_rows_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(sc.vals_out.as<int32_t>(), bd.labels.as<int64_t>(), n, L.labels.as<int64_t>());
     CK(cudaGetLastError());
-    TRY(h->list_off.ensure(sizeof(int64_t) * ((size_t)nc + 1), 0, st, true));
-    CK(cudaMemcpyAsync(h->list_off.p, sc.offs.p, sizeof(int64_t) * ((size_t)nc + 1), cudaMemcpyDeviceToDevice, st));
-    h->list_off_h.resize((size_t)nc + 1);
-    CK(cudaMemcpyAsync(h->list_off_h.data(), sc.offs.p, sizeof(int64_t) * ((size_t)nc + 1), cudaMemcpyDeviceToHost, st));
+    TRY(L.off.ensure(sizeof(int64_t) * ((size_t)nc + 1), 0, st, true));
+    CK(cudaMemcpyAsync(L.off.p, sc.offs.p, sizeof(int64_t) * ((size_t)nc + 1), cudaMemcpyDeviceToDevice, st));
+    L.off_h.resize((size_t)nc + 1);
+    CK(cudaMemcpyAsync(L.off_h.data(), sc.offs.p, sizeof(int64_t) * ((size_t)nc + 1), cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
-    h->list_total = n;
-    h->max_list_len = 0;
-    for (int c = 0; c < nc; ++c) h->max_list_len = std::max(h->max_list_len, h->list_off_h[(size_t)c + 1] - h->list_off_h[(size_t)c]);
-    h->list_dead_h.clear();
-    h->list_dead.release();
-    h->list_ndead = 0;
-    h->lists_version++;
-    h->nc = nc;
-    h->built = true;
-    h->tc_cent.invalidate();
-    h->lists_loc_valid = false;
-    consume_buffer(h);
+    L.total = n;
+    for (int c = 0; c < nc; ++c) L.max_len = std::max(L.max_len, L.off_h[(size_t)c + 1] - L.off_h[(size_t)c]);
     return PYROPE_OK;
 }
 
-// KMeansUtils.FindNearestCentroid against the index's current centroids (cnorms must be current) -> assign[n]
-int assign_to_centroids(Index* h, const float* X, int64_t n, int nc, DevBuf& assign) {
-    cudaStream_t st = h->stream;
+// KMeansUtils.FindNearestCentroid against nc centroids (cnorms: their norms, read for Cosine) -> assign[n]
+int assign_to_centroids(const Index& h, const float* centroids, const float* cnorms, int nc, const float* X, int64_t n,
+                        DevBuf& assign) {
+    cudaStream_t st = h.stream;
     TRY(assign.ensure(sizeof(int32_t) * (size_t)std::max<int64_t>(n, 1), 0, st, true));
     AssignScratch as;
-    TRY(assign_rows(h->metric, h->dim, n, X, h->dim, nc, h->centroids.as<float>(), h->cnorms.as<float>(),
-                    assign.as<int32_t>(), as, true, st));
+    TRY(assign_rows(h.metric, h.dim, n, X, h.dim, nc, centroids, cnorms, assign.as<int32_t>(), as, true, st));
     CK(cudaStreamSynchronize(st));
     return PYROPE_OK;
 }
@@ -729,125 +841,92 @@ int assign_to_centroids(Index* h, const float* X, int64_t n, int nc, DevBuf& ass
 // rows of encoding work per residual chunk
 int64_t pq_encode_chunk(int64_t n) { return std::min<int64_t>(n, (int64_t)4 << 20); }
 
-// IvfPqVectorIndex.cs:82-90: residual to the assigned centroid, ProductQuantizer.Encode with the current codebooks
+// IvfPqVectorIndex.cs:82-90: residual to the assigned centroid, ProductQuantizer.Encode with the given codebooks
 // (honouring ksub) -> codes[n][m].  res: scratch of at least pq_encode_chunk(n) rows (grown here if needed).
-int pq_encode_rows(Index* h, const float* X, int64_t n, const int32_t* assign, DevBuf& res, DevBuf& codes) {
-    cudaStream_t st = h->stream;
-    const int dim = h->dim, m = h->m;
+int pq_encode_rows(const Index& h, const float* centroids, const float* codebook, const std::vector<int32_t>& ksub,
+                   const float* X, int64_t n, const int32_t* assign, DevBuf& res, DevBuf& codes) {
+    cudaStream_t st = h.stream;
+    const int dim = h.dim, m = h.m;
     const int64_t chunk = pq_encode_chunk(n);
     TRY(res.ensure(sizeof(float) * (size_t)std::max<int64_t>(chunk, 1) * dim, 0, st, true));
-    TRY(h->ksub_d.ensure(sizeof(int32_t) * (size_t)m, 0, st, true));
-    CK(cudaMemcpyAsync(h->ksub_d.p, h->ksub.data(), sizeof(int32_t) * (size_t)m, cudaMemcpyHostToDevice, st));
+    DevBuf ksub_d;
+    TRY(ksub_d.ensure(sizeof(int32_t) * (size_t)m, 0, st, true));
+    CK(cudaMemcpyAsync(ksub_d.p, ksub.data(), sizeof(int32_t) * (size_t)m, cudaMemcpyHostToDevice, st));
     TRY(codes.ensure((size_t)std::max<int64_t>(n, 1) * m, 0, st, true));
     for (int64_t c0 = 0; c0 < n; c0 += chunk) {
         int64_t cn = std::min(chunk, n - c0);
-        CK(launch_residuals(X + (size_t)c0 * dim, cn, dim, h->centroids.as<float>(), assign + c0, res.as<float>(), st));
-        CK(launch_pq_encode_exact(res.as<float>(), cn, dim, m, h->k, h->codebook.as<float>(), h->ksub_d.as<int32_t>(),
+        CK(launch_residuals(X + (size_t)c0 * dim, cn, dim, centroids, assign + c0, res.as<float>(), st));
+        CK(launch_pq_encode_exact(res.as<float>(), cn, dim, m, h.k, codebook, ksub_d.as<int32_t>(),
                                   codes.as<uint8_t>() + (size_t)c0 * m, st));
     }
     CK(cudaStreamSynchronize(st));
     return PYROPE_OK;
 }
 
-int build_ivfflat(Index* h) {
-    cudaStream_t st = h->stream;
-    const int dim = h->dim;
+// ---- Build (IvfFlatVectorIndex.cs:87-143, IvfPqVectorIndex.cs:56-109): k-means over the rows Build sees trains new
+// centroids (and, IVF_PQ, codebooks on the residuals) unless the caller froze them; every row is assigned, encoded and
+// grouped into new lists.  IVF_FLAT sees its live list entries then its buffer, IVF_PQ its buffer alone (:64).
+int build_prepare(const Index& h, Staged& S) {
+    if (h.last_stream) CK(cudaStreamSynchronize(h.last_stream));
+    if (h.kind == PYROPE_FLAT) return PYROPE_OK;  // BruteForceVectorIndex.cs:56
+    cudaStream_t st = h.stream;
+    const int dim = h.dim, m = h.m, K = h.k, sub = h.sub;
+    const bool pq = h.kind == PYROPE_IVF_PQ;
     BuildData bd;
-    TRY(gather_build_data(h, true, bd));
-    if (bd.n == 0) return PYROPE_OK;  // IvfFlatVectorIndex.cs:112
-    int nc;
-    if (h->frozen) {
-        nc = h->nc;
-    } else {
-        int k = (int)std::min<int64_t>(h->nlist, bd.n);
-        if (k <= 0) k = 1;
-        int64_t ntrain = (h->max_train_rows > 0) ? std::min<int64_t>(h->max_train_rows, bd.n) : bd.n;
-        if (k > ntrain) k = (int)ntrain;
-        DevBuf cent;
-        TRY(cent.ensure(sizeof(float) * (size_t)k * dim, 0, st, true));
-        int iters = 0;
-        TRY(kmeans_train_device(h->metric, dim, ntrain, dim, bd.X, k, h->max_iter > 0 ? h->max_iter : 10, 42,
-                                cent.as<float>(), &nc, &iters, st));
-        TRY(h->centroids.ensure(sizeof(float) * (size_t)nc * dim, 0, st, true));
-        CK(cudaMemcpyAsync(h->centroids.p, cent.p, sizeof(float) * (size_t)nc * dim, cudaMemcpyDeviceToDevice, st));
-        CK(cudaStreamSynchronize(st));
-    }
-    TRY(h->cnorms.ensure(sizeof(float) * (size_t)nc, 0, st, true));
-    if (h->metric == kCosine) CK(launch_row_norms_exact(h->centroids.as<float>(), nc, dim, dim, h->cnorms.as<float>(), st));
-    DevBuf assign;
-    TRY(assign_to_centroids(h, bd.X, bd.n, nc, assign));
-    SortScratch sc;
-    DevBuf newvecs;
-    TRY(finish_lists(h, bd, assign.as<int32_t>(), nc, sc, bd.X, (int64_t)dim * 4, newvecs));
-    std::swap(h->list_vecs.p, newvecs.p);
-    std::swap(h->list_vecs.bytes, newvecs.bytes);
-    if (h->metric == kCosine) {
-        TRY(h->list_norms.ensure(sizeof(float) * (size_t)std::max<int64_t>(h->list_total, 1), 0, st, true));
-        CK(launch_row_norms_exact(h->list_vecs.as<float>(), h->list_total, dim, dim, h->list_norms.as<float>(), st));
-    }
-    CK(cudaStreamSynchronize(st));
-    return PYROPE_OK;
-}
-
-int build_ivfpq(Index* h) {
-    cudaStream_t st = h->stream;
-    const int dim = h->dim, m = h->m, K = h->k, sub = h->sub;
-    BuildData bd;
-    TRY(gather_build_data(h, false, bd));
-    if (bd.n == 0) return PYROPE_OK;  // IvfPqVectorIndex.cs:62,65
+    TRY(gather_build_data(h, !pq, bd));
     const int64_t n = bd.n;
-    int nc;
-    const int64_t ntrain = (h->max_train_rows > 0) ? std::min<int64_t>(h->max_train_rows, n) : n;
-    const int iters_max = h->max_iter > 0 ? h->max_iter : 10;
-    if (h->frozen) {
-        nc = h->nc;
-    } else {
-        int k = (int)std::min<int64_t>(h->nlist, n);
+    if (n == 0) return PYROPE_OK;  // IvfFlatVectorIndex.cs:112, IvfPqVectorIndex.cs:62,65
+    const int64_t ntrain = (h.max_train_rows > 0) ? std::min<int64_t>(h.max_train_rows, n) : n;
+    if (!h.frozen) {
+        int k = (int)std::min<int64_t>(h.nlist, n);
         if (k > ntrain) k = (int)ntrain;
         if (k <= 0) k = 1;
-        DevBuf cent;
-        TRY(cent.ensure(sizeof(float) * (size_t)k * dim, 0, st, true));
+        TRY(S.centroids.ensure(sizeof(float) * (size_t)k * dim, 0, st, true));
         int iters = 0;
-        TRY(kmeans_train_device(h->metric, dim, ntrain, dim, bd.X, k, iters_max, 123, cent.as<float>(), &nc, &iters, st));
-        TRY(h->centroids.ensure(sizeof(float) * (size_t)nc * dim, 0, st, true));
-        CK(cudaMemcpyAsync(h->centroids.p, cent.p, sizeof(float) * (size_t)nc * dim, cudaMemcpyDeviceToDevice, st));
-        CK(cudaStreamSynchronize(st));
+        TRY(kmeans_train_device(h.metric, dim, ntrain, dim, bd.X, k, h.max_iter > 0 ? h.max_iter : 10, pq ? 123 : 42,
+                                S.centroids.as<float>(), &S.nc, &iters, st));
+        S.quantiser = true;
     }
-    TRY(h->cnorms.ensure(sizeof(float) * (size_t)nc, 0, st, true));
-    if (h->metric == kCosine) CK(launch_row_norms_exact(h->centroids.as<float>(), nc, dim, dim, h->cnorms.as<float>(), st));
+    const float* cent = (h.frozen ? h.centroids : S.centroids).as<float>();
+    TRY(S.cnorms.ensure(sizeof(float) * (size_t)S.nc, 0, st, true));
+    if (h.metric == kCosine) CK(launch_row_norms_exact(cent, S.nc, dim, dim, S.cnorms.as<float>(), st));
     DevBuf assign;
-    TRY(assign_to_centroids(h, bd.X, n, nc, assign));
-    // PQ training on the residuals of the training rows (ProductQuantizer.cs:28-58)
-    const int64_t chunk = pq_encode_chunk(n);
-    DevBuf res;
-    TRY(res.ensure(sizeof(float) * (size_t)std::max(chunk, h->frozen ? (int64_t)0 : ntrain) * dim, 0, st, true));
-    if (!h->frozen) {
-        CK(launch_residuals(bd.X, ntrain, dim, h->centroids.as<float>(), assign.as<int32_t>(), res.as<float>(), st));
-        TRY(h->codebook.ensure(sizeof(float) * (size_t)m * K * sub, 0, st, true));
-        CK(cudaMemsetAsync(h->codebook.p, 0, sizeof(float) * (size_t)m * K * sub, st));
-        h->cmax_for = nullptr; h->lm_cb16_ok = false;
-        h->ksub.assign((size_t)m, 0);
-        DevBuf cb1;
-        TRY(cb1.ensure(sizeof(float) * (size_t)K * sub, 0, st, true));
-        for (int mi = 0; mi < m; ++mi) {
-            int kk = 0, iters = 0;
-            TRY(kmeans_train_device(kL2, sub, ntrain, dim, res.as<float>() + (size_t)mi * sub, K, 10, 42 + mi,
-                                    cb1.as<float>(), &kk, &iters, st));
-            h->ksub[(size_t)mi] = kk;
-            CK(cudaMemcpyAsync(h->codebook.as<float>() + (size_t)mi * K * sub, cb1.p, sizeof(float) * (size_t)kk * sub,
-                               cudaMemcpyDeviceToDevice, st));
-            CK(cudaStreamSynchronize(st));
+    TRY(assign_to_centroids(h, cent, S.cnorms.as<float>(), S.nc, bd.X, n, assign));
+    const void* payload = bd.X;
+    DevBuf res, codes;
+    if (pq) {
+        TRY(res.ensure(sizeof(float) * (size_t)std::max(pq_encode_chunk(n), h.frozen ? (int64_t)0 : ntrain) * dim, 0, st, true));
+        if (!h.frozen) {  // PQ training on the residuals of the training rows (ProductQuantizer.cs:28-58)
+            CK(launch_residuals(bd.X, ntrain, dim, cent, assign.as<int32_t>(), res.as<float>(), st));
+            TRY(S.codebook.ensure(sizeof(float) * (size_t)m * K * sub, 0, st, true));
+            CK(cudaMemsetAsync(S.codebook.p, 0, sizeof(float) * (size_t)m * K * sub, st));
+            S.ksub.assign((size_t)m, 0);
+            DevBuf cb1;
+            TRY(cb1.ensure(sizeof(float) * (size_t)K * sub, 0, st, true));
+            for (int mi = 0; mi < m; ++mi) {
+                int kk = 0, iters = 0;
+                TRY(kmeans_train_device(kL2, sub, ntrain, dim, res.as<float>() + (size_t)mi * sub, K, 10, 42 + mi,
+                                        cb1.as<float>(), &kk, &iters, st));
+                S.ksub[(size_t)mi] = kk;
+                CK(cudaMemcpyAsync(S.codebook.as<float>() + (size_t)mi * K * sub, cb1.p, sizeof(float) * (size_t)kk * sub,
+                                   cudaMemcpyDeviceToDevice, st));
+                CK(cudaStreamSynchronize(st));
+            }
         }
+        TRY(pq_encode_rows(h, cent, (h.frozen ? h.codebook : S.codebook).as<float>(), h.frozen ? h.ksub : S.ksub, bd.X, n,
+                           assign.as<int32_t>(), res, codes));
+        payload = codes.p;
     }
-    DevBuf codes;
-    TRY(pq_encode_rows(h, bd.X, n, assign.as<int32_t>(), res, codes));
-    SortScratch sc;
-    DevBuf newcodes;
-    TRY(finish_lists(h, bd, assign.as<int32_t>(), nc, sc, codes.p, m, newcodes));
-    std::swap(h->list_codes.p, newcodes.p);
-    std::swap(h->list_codes.bytes, newcodes.bytes);
-    h->lm_codes16_ok = false;
+    TRY(finish_lists(h, bd, assign.as<int32_t>(), S.nc, payload, pq ? m : (int64_t)dim * 4, S));
+    IvfLists& L = S.lists;
+    if (!pq && h.metric == kCosine) {
+        TRY(L.norms.ensure(sizeof(float) * (size_t)std::max<int64_t>(L.total, 1), 0, st, true));
+        CK(launch_row_norms_exact(L.payload.as<float>(), L.total, dim, dim, L.norms.as<float>(), st));
+    }
     CK(cudaStreamSynchronize(st));
+    S.built = true;
+    S.moved = buffered_rows(h);
+    S.noop = false;
     return PYROPE_OK;
 }
 
@@ -856,37 +935,25 @@ int build_ivfpq(Index* h) {
 // CURRENT codebooks, and each row is appended to the end of its list (rows of one list keep slot order: group_rows is a
 // stable sort).  Old entries keep their order, row ordinals, labels and dead flags, except that shadowed entries (flag 2:
 // their replacement has just left the buffer) become deleted.  A shard appends only to the lists it owns.
-// extend_prepare does everything that can fail and builds the merged arrays aside; extend_commit only swaps them in.
-struct StagedExtend {
-    bool noop = true;
-    std::vector<int64_t> moved;  // row ordinals leaving the buffer, slot order
-    DevBuf payload, rows, labels, dead, norms, off;
-    std::vector<int64_t> off_h;
-    std::vector<uint8_t> dead_h;
-    int64_t total = 0, max_len = 0;
-};
-
-// caller holds h->mu
-int extend_prepare(Index* h, StagedExtend& S) {
-    if (h->kind == PYROPE_FLAT) return fail(PYROPE_ERR_UNSUPPORTED, "Extend needs an IVF index: FLAT has no inverted lists");
-    if (!h->built) return fail(PYROPE_ERR_INVALID_STATE, "Extend needs a built index: call Build first");
-    cudaStream_t st = h->stream;
+int extend_prepare(const Index& h, Staged& S) {
+    if (h.kind == PYROPE_FLAT) return fail(PYROPE_ERR_UNSUPPORTED, "Extend needs an IVF index: FLAT has no inverted lists");
+    if (!h.built) return fail(PYROPE_ERR_INVALID_STATE, "Extend needs a built index: call Build first");
+    cudaStream_t st = h.stream;
     CK(cudaStreamSynchronize(st));
-    if (h->last_stream) CK(cudaStreamSynchronize(h->last_stream));
-    const Segment& s = h->seg;
+    if (h.last_stream) CK(cudaStreamSynchronize(h.last_stream));
+    const Segment& s = h.seg;
     if (s.live == 0) return PYROPE_OK;
-    const int dim = h->dim, nc = h->nc;
+    const IvfLists& O = h.lists;
+    IvfLists& L = S.lists;
+    const int dim = h.dim, nc = h.nc;
     BuildData bd;
     TRY(gather_build_data(h, false, bd));  // live buffer slots, slot order
     const int64_t n = bd.n;
-    S.moved.reserve((size_t)n);
-    for (int64_t i = 0; i < s.nslots; ++i)
-        if (!s.dead_h[(size_t)i]) S.moved.push_back(s.slot_row[(size_t)i]);
     DevBuf assign, res, codes, nnorm;
-    TRY(assign_to_centroids(h, bd.X, n, nc, assign));
-    const bool pq = h->kind == PYROPE_IVF_PQ, cos_norms = !pq && h->metric == kCosine;
-    const int64_t rb = pq ? h->m : (int64_t)dim * 4;
-    if (pq) TRY(pq_encode_rows(h, bd.X, n, assign.as<int32_t>(), res, codes));
+    TRY(assign_to_centroids(h, h.centroids.as<float>(), h.cnorms.as<float>(), nc, bd.X, n, assign));
+    const bool pq = h.kind == PYROPE_IVF_PQ, cos_norms = !pq && h.metric == kCosine;
+    const int64_t rb = pq ? h.m : (int64_t)dim * 4;
+    if (pq) TRY(pq_encode_rows(h, h.centroids.as<float>(), h.codebook.as<float>(), h.ksub, bd.X, n, assign.as<int32_t>(), res, codes));
     if (cos_norms) {
         TRY(nnorm.ensure(sizeof(float) * (size_t)n, 0, st, true));
         CK(launch_row_norms_exact(bd.X, n, dim, dim, nnorm.as<float>(), st));
@@ -897,63 +964,46 @@ int extend_prepare(Index* h, StagedExtend& S) {
     std::vector<int64_t> offs_new((size_t)nc + 1);
     CK(cudaMemcpyAsync(offs_new.data(), sc.offs.p, sizeof(int64_t) * offs_new.size(), cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
-    S.total = h->list_total + kept;
-    S.off_h.resize((size_t)nc + 1);
-    for (int c = 0; c <= nc; ++c) S.off_h[(size_t)c] = h->list_off_h[(size_t)c] + offs_new[(size_t)c];
-    for (int c = 0; c < nc; ++c) S.max_len = std::max(S.max_len, S.off_h[(size_t)c + 1] - S.off_h[(size_t)c]);
-    const size_t t1 = (size_t)std::max<int64_t>(S.total, 1);
-    TRY(S.off.ensure(sizeof(int64_t) * S.off_h.size(), 0, st, true));
-    CK(cudaMemcpyAsync(S.off.p, S.off_h.data(), sizeof(int64_t) * S.off_h.size(), cudaMemcpyHostToDevice, st));
-    TRY(S.payload.ensure(t1 * (size_t)rb, 0, st, true));
-    TRY(S.rows.ensure(sizeof(int64_t) * t1, 0, st, true));
-    TRY(S.labels.ensure(sizeof(int64_t) * t1, 0, st, true));
-    const bool has_dead = !h->list_dead_h.empty();
-    if (has_dead) TRY(S.dead.ensure(t1, 0, st, true));
-    if (cos_norms) TRY(S.norms.ensure(sizeof(float) * t1, 0, st, true));
+    L.total = O.total + kept;
+    L.off_h.resize((size_t)nc + 1);
+    for (int c = 0; c <= nc; ++c) L.off_h[(size_t)c] = O.off_h[(size_t)c] + offs_new[(size_t)c];
+    for (int c = 0; c < nc; ++c) L.max_len = std::max(L.max_len, L.off_h[(size_t)c + 1] - L.off_h[(size_t)c]);
+    const size_t t1 = (size_t)std::max<int64_t>(L.total, 1);
+    TRY(L.off.ensure(sizeof(int64_t) * L.off_h.size(), 0, st, true));
+    CK(cudaMemcpyAsync(L.off.p, L.off_h.data(), sizeof(int64_t) * L.off_h.size(), cudaMemcpyHostToDevice, st));
+    TRY(L.payload.ensure(t1 * (size_t)rb, 0, st, true));
+    TRY(L.rows.ensure(sizeof(int64_t) * t1, 0, st, true));
+    TRY(L.labels.ensure(sizeof(int64_t) * t1, 0, st, true));
+    const bool has_dead = !O.dead_h.empty();
+    if (has_dead) TRY(L.dead.ensure(t1, 0, st, true));
+    if (cos_norms) TRY(L.norms.ensure(sizeof(float) * t1, 0, st, true));
 
     ExtendMergeParams mp{};
-    mp.off_old = h->list_off.as<int64_t>(); mp.offs_new = sc.offs.as<int64_t>(); mp.off_merged = S.off.as<int64_t>();
+    mp.off_old = O.off.as<int64_t>(); mp.offs_new = sc.offs.as<int64_t>(); mp.off_merged = L.off.as<int64_t>();
     mp.order = sc.vals_out.as<int32_t>(); mp.nc = nc;
     auto col = [&](const void* old_src, const void* new_src, DevBuf& dst, int64_t row_bytes, int fold) {
         ExtendMergeColumn& c = mp.col[mp.ncols++];
         c.old_src = (const uint8_t*)old_src; c.new_src = (const uint8_t*)new_src; c.dst = dst.as<uint8_t>();
         c.row_bytes = row_bytes; c.fold_flags = fold;
     };
-    col(pq ? h->list_codes.p : h->list_vecs.p, pq ? codes.p : (const void*)bd.X, S.payload, rb, 0);
-    col(h->list_rows.p, bd.rows.p, S.rows, 8, 0);
-    col(h->list_labels.p, bd.labels.p, S.labels, 8, 0);
-    if (has_dead) col(h->list_dead.p, nullptr, S.dead, 1, 1);
-    if (cos_norms) col(h->list_norms.p, nnorm.p, S.norms, 4, 0);
-    CK(launch_extend_merge(mp, S.total, st));
+    col(O.payload.p, pq ? codes.p : (const void*)bd.X, L.payload, rb, 0);
+    col(O.rows.p, bd.rows.p, L.rows, 8, 0);
+    col(O.labels.p, bd.labels.p, L.labels, 8, 0);
+    if (has_dead) col(O.dead.p, nullptr, L.dead, 1, 1);
+    if (cos_norms) col(O.norms.p, nnorm.p, L.norms, 4, 0);
+    CK(launch_extend_merge(mp, L.total, st));
     CK(cudaStreamSynchronize(st));
     if (has_dead) {
-        S.dead_h.assign((size_t)S.total, 0);
+        L.dead_h.assign((size_t)L.total, 0);
         for (int c = 0; c < nc; ++c) {
-            const int64_t o = h->list_off_h[(size_t)c], len = h->list_off_h[(size_t)c + 1] - o;
-            for (int64_t i = 0; i < len; ++i) S.dead_h[(size_t)(o + offs_new[(size_t)c] + i)] = h->list_dead_h[(size_t)(o + i)] ? 1 : 0;
+            const int64_t o = O.off_h[(size_t)c], len = O.off_h[(size_t)c + 1] - o;
+            for (int64_t i = 0; i < len; ++i) L.dead_h[(size_t)(o + offs_new[(size_t)c] + i)] = O.dead_h[(size_t)(o + i)] ? 1 : 0;
         }
+        L.ndead = O.ndead;  // a flagged entry stays flagged (shadowed becomes deleted), appended entries carry no flag
     }
+    S.moved = buffered_rows(h);
     S.noop = false;
     return PYROPE_OK;
-}
-
-// caller holds h->mu; nothing here can fail
-void extend_commit(Index* h, StagedExtend& S) {
-    if (S.noop) return;
-    auto take = [](DevBuf& dst, DevBuf& src) { std::swap(dst.p, src.p); std::swap(dst.bytes, src.bytes); src.release(); };
-    take(h->kind == PYROPE_IVF_PQ ? h->list_codes : h->list_vecs, S.payload);
-    take(h->list_rows, S.rows);
-    take(h->list_labels, S.labels);
-    take(h->list_off, S.off);
-    if (S.dead.p) { take(h->list_dead, S.dead); h->list_dead_h.swap(S.dead_h); }  // list_ndead: non-zero stays non-zero
-    if (S.norms.p) take(h->list_norms, S.norms);
-    h->list_off_h.swap(S.off_h);
-    h->list_total = S.total;
-    h->max_list_len = S.max_len;
-    h->lists_version++;
-    h->lists_loc_valid = false;
-    h->lm_codes16_ok = false;
-    consume_buffer(h);
 }
 
 // A MaxScans budget walks the probed lists entry by entry and never counts a deleted or shadowed entry
@@ -961,14 +1011,14 @@ void extend_commit(Index* h, StagedExtend& S) {
 // compacted VIEW of them (dead entries squeezed out, offsets recomputed).  The lists themselves are left alone:
 // a shadowed entry's position still decides where its replacement lands at the next Build (:91-108).
 int compact_lists(Index* h) {
-    if (h->list_ndead == 0 || h->bv_version == h->lists_version) return PYROPE_OK;
+    if (h->lists.ndead == 0 || h->bv_version == h->lists_version) return PYROPE_OK;
     cudaStream_t st = h->stream;
     std::vector<int64_t> keep;
-    keep.reserve((size_t)h->list_total);
+    keep.reserve((size_t)h->lists.total);
     std::vector<int64_t> noff((size_t)h->nc + 1, 0);
     for (int c = 0; c < h->nc; ++c) {
-        for (int64_t i = h->list_off_h[(size_t)c]; i < h->list_off_h[(size_t)c + 1]; ++i)
-            if (!h->list_dead_h[(size_t)i]) keep.push_back(i);
+        for (int64_t i = h->lists.off_h[(size_t)c]; i < h->lists.off_h[(size_t)c + 1]; ++i)
+            if (!h->lists.dead_h[(size_t)i]) keep.push_back(i);
         noff[(size_t)c + 1] = (int64_t)keep.size();
     }
     const int64_t n = (int64_t)keep.size();
@@ -979,11 +1029,11 @@ int compact_lists(Index* h) {
     TRY(h->bv_vecs.ensure(sizeof(float) * n1 * h->dim, 0, st));
     TRY(h->bv_labels.ensure(sizeof(int64_t) * n1, 0, st));
     TRY(h->bv_off.ensure(sizeof(int64_t) * noff.size(), 0, st));
-    CK(launch_gather_rows(h->list_vecs.p, (int64_t)h->dim * 4, idx.as<int64_t>(), n, h->bv_vecs.p, st));
-    CK(launch_gather_rows(h->list_labels.p, 8, idx.as<int64_t>(), n, h->bv_labels.p, st));
+    CK(launch_gather_rows(h->lists.payload.p, (int64_t)h->dim * 4, idx.as<int64_t>(), n, h->bv_vecs.p, st));
+    CK(launch_gather_rows(h->lists.labels.p, 8, idx.as<int64_t>(), n, h->bv_labels.p, st));
     if (h->metric == kCosine) {
         TRY(h->bv_norms.ensure(sizeof(float) * n1, 0, st));
-        CK(launch_gather_rows(h->list_norms.p, 4, idx.as<int64_t>(), n, h->bv_norms.p, st));
+        CK(launch_gather_rows(h->lists.norms.p, 4, idx.as<int64_t>(), n, h->bv_norms.p, st));
     }
     CK(cudaMemcpyAsync(h->bv_off.p, noff.data(), sizeof(int64_t) * noff.size(), cudaMemcpyHostToDevice, st));
     CK(cudaStreamSynchronize(st));
@@ -1078,7 +1128,7 @@ int search_device(Index* h, int64_t nq, const float* dQ, int topk, int64_t max_s
 
     int P = 0;  // probes
     bool scan_lists = false;
-    if (ivf && h->built && h->nc > 0 && h->list_total > 0) {
+    if (ivf && h->built && h->nc > 0 && h->lists.total > 0) {
         int np = nprobe >= 0 ? nprobe : (h->kind == PYROPE_IVF_FLAT ? 3 : 1);
         P = std::min(np, h->nc);
         scan_lists = P > 0;
@@ -1100,9 +1150,9 @@ int search_device(Index* h, int64_t nq, const float* dQ, int topk, int64_t max_s
         groups = (int)std::max<int64_t>(1, std::min<int64_t>(want, P));
     }
     const bool use_lm = scan_lists && h->kind == PYROPE_IVF_PQ && !h->pq_force_generic && h->pq_lm_mode != 0 &&
-                        ivfpq_lm_supported(dim, h->m, h->k, P, k, nq, h->list_total, h->max_list_len);
+                        ivfpq_lm_supported(dim, h->m, h->k, P, k, nq, h->lists.total, h->lists.max_len);
     const bool use_flm = scan_lists && h->kind == PYROPE_IVF_FLAT && h->pq_lm_mode != 0 && nq >= 64 &&
-                         ivfflat_lm_supported(dim, h->metric, P, k, nq, h->list_total, max_scans >= 0);
+                         ivfflat_lm_supported(dim, h->metric, P, k, nq, h->lists.total, max_scans >= 0);
     if (use_lm || use_flm) groups = 1;
     int max_parts = kMergeMaxCandidates / k;
     if (max_parts < 1) max_parts = 1;
@@ -1342,23 +1392,23 @@ int search_device(Index* h, int64_t nq, const float* dQ, int topk, int64_t max_s
     }
     // ---- list scan
     if (scan_lists) {
-        const uint8_t* ldead = h->list_ndead > 0 ? h->list_dead.as<uint8_t>() : nullptr;
+        const uint8_t* ldead = h->lists.ndead > 0 ? h->lists.dead.as<uint8_t>() : nullptr;
         if (h->kind == PYROPE_IVF_FLAT) {
             const int32_t* allow = nullptr;
-            const bool budget_view = max_scans >= 0 && h->list_ndead > 0;
+            const bool budget_view = max_scans >= 0 && h->lists.ndead > 0;
             if (budget_view && h->bv_version != h->lists_version)
                 return fail(PYROPE_ERR_INVALID_STATE, "budgeted IVF_FLAT search without a compacted list view");
             if (max_scans >= 0) {
                 TRY(ws.allow.ensure(sizeof(int32_t) * (size_t)nq * P, 0, st));
-                CK(launch_probe_allow(probes_dev, nq, P, (budget_view ? h->bv_off : h->list_off).as<int64_t>(),
+                CK(launch_probe_allow(probes_dev, nq, P, (budget_view ? h->bv_off : h->lists.off).as<int64_t>(),
                                       max_scans - seg_live_scanned, ws.allow.as<int32_t>(), st));
                 ++launches;
                 allow = ws.allow.as<int32_t>();
             }
             IvfFlatScanParams ip{};
             ip.Q = dQ; ip.nq = nq; ip.dim = dim; ip.probes = probes_dev; ip.nprobe = P; ip.allow = allow;
-            ip.list_off = h->list_off.as<int64_t>(); ip.vecs = h->list_vecs.as<float>(); ip.dead = ldead;
-            ip.norms = h->list_norms.as<float>(); ip.labels = h->list_labels.as<int64_t>(); ip.qnorm = qnorm;
+            ip.list_off = h->lists.off.as<int64_t>(); ip.vecs = h->lists.payload.as<float>(); ip.dead = ldead;
+            ip.norms = h->lists.norms.as<float>(); ip.labels = h->lists.labels.as<int64_t>(); ip.qnorm = qnorm;
             if (budget_view) {
                 ip.list_off = h->bv_off.as<int64_t>(); ip.vecs = h->bv_vecs.as<float>(); ip.dead = nullptr;
                 ip.norms = h->bv_norms.as<float>(); ip.labels = h->bv_labels.as<int64_t>();
@@ -1379,9 +1429,9 @@ int search_device(Index* h, int64_t nq, const float* dQ, int topk, int64_t max_s
         } else {
             IvfPqScanParams pp{};
             pp.Q = dQ; pp.nq = nq; pp.dim = dim; pp.probes = probes_dev; pp.nprobe = P;
-            pp.list_off = h->list_off.as<int64_t>(); pp.nlist = h->nc; pp.centroids = h->centroids.as<float>();
+            pp.list_off = h->lists.off.as<int64_t>(); pp.nlist = h->nc; pp.centroids = h->centroids.as<float>();
             pp.codebook = h->codebook.as<float>(); pp.m = h->m; pp.ksub = h->k;
-            pp.codes = h->list_codes.as<uint8_t>(); pp.dead = ldead; pp.labels = h->list_labels.as<int64_t>();
+            pp.codes = h->lists.payload.as<uint8_t>(); pp.dead = ldead; pp.labels = h->lists.labels.as<int64_t>();
             pp.k = k; pp.groups = groups; pp.force_generic = h->pq_force_generic;
             pp.out = out; pp.out.part_base = seg_splits;
             if (use_lm && parts == 1) {  // the only part: the final kernel writes the search's output itself, no merge pass
@@ -1405,27 +1455,27 @@ int search_device(Index* h, int64_t nq, const float* dQ, int topk, int64_t max_s
                         TRY(h->lm_cb16.ensure(sizeof(float) * (size_t)h->k * dim, 0, st, true));
                         CK(launch_pq_lm_expand_codebook(h->codebook.as<float>(), h->m, h->k, dim, h->lm_cb16.as<float>(), st));
                         h->lm_cb16_ok = true;
-                        h->cmax_for = nullptr;
+                        h->pq_cmax_ok = false;
                         ++launches;
                     }
                     if (!h->lm_codes16_ok) {
-                        TRY(h->lm_codes16.ensure((size_t)std::max<int64_t>(h->list_total, 1) * 16, 0, st, true));
-                        CK(launch_pq_lm_expand_codes(h->list_codes.as<uint8_t>(), h->list_total, h->m, h->lm_codes16.as<uint8_t>(), st));
+                        TRY(h->lm_codes16.ensure((size_t)std::max<int64_t>(h->lists.total, 1) * 16, 0, st, true));
+                        CK(launch_pq_lm_expand_codes(h->lists.payload.as<uint8_t>(), h->lists.total, h->m, h->lm_codes16.as<uint8_t>(), st));
                         h->lm_codes16_ok = true;
                         ++launches;
                     }
                     pp.lm_codebook = h->lm_cb16.as<float>();
                     pp.lm_codes = h->lm_codes16.as<uint8_t>();
                 }
-                if (h->cmax_for != h->codebook.p || !h->pq_cmax.p) {  // once per codebook
+                if (!h->pq_cmax_ok) {  // once per codebook
                     TRY(h->pq_cmax.ensure(sizeof(float) * 16, 0, st, true));
                     CK(launch_pq_cmax(pp.lm_codebook ? pp.lm_codebook : h->codebook.as<float>(), h->k, dim / 16, h->pq_cmax.as<float>(), st));
-                    h->cmax_for = h->codebook.p;
+                    h->pq_cmax_ok = true;
                     ++launches;
                 }
                 pp.cmax = h->pq_cmax.as<float>();
-                TRY(ws.lm.ensure(ivfpq_lm_scratch_bytes(nq, P, k, h->nc, dim, h->max_list_len), 0, st));
-                pp.max_list_len = h->max_list_len;
+                TRY(ws.lm.ensure(ivfpq_lm_scratch_bytes(nq, P, k, h->nc, dim, h->lists.max_len), 0, st));
+                pp.max_list_len = h->lists.max_len;
                 pp.ev_k0 = h->evk[0]; pp.ev_k1 = h->evk[1];
                 pp.aux_stream = h->aux; pp.ev_fork = h->evf[0]; pp.ev_join = h->evf[1];
                 h->evk_valid = true;
@@ -1618,12 +1668,7 @@ int pyrope_index_delete_row(pyrope_index* h, int64_t row) {
     } else {
         if (h->kind == PYROPE_IVF_PQ)  // IvfPqVectorIndex.cs:48-53: Delete only touches the buffer
             return fail(PYROPE_ERR_NOT_FOUND, "row %lld is encoded in a list; IVF_PQ deletes only buffered rows", (long long)row);
-        int64_t pos = -2 - loc;
-        TRY(ensure_list_dead(h));
-        if (!(h->list_dead_h[(size_t)pos])) h->list_ndead++;
-        h->list_dead_h[(size_t)pos] |= 1;
-        h->lists_version++;
-        CK(cudaMemcpyAsync(h->list_dead.as<uint8_t>() + pos, &h->list_dead_h[(size_t)pos], 1, cudaMemcpyHostToDevice, st));
+        TRY(set_list_flag(h, {-2 - loc}, 1, true));
         h->row_loc[(size_t)row] = -1;
     }
     CK(cudaStreamSynchronize(st));
@@ -1639,15 +1684,7 @@ int pyrope_index_shadow_row(pyrope_index* h, int64_t row, int shadowed) {
     TRY(rebuild_row_loc(h));
     int64_t loc = h->row_loc[(size_t)row];
     if (loc > -2) return fail(PYROPE_ERR_NOT_FOUND, "row %lld is not in an inverted list", (long long)row);
-    int64_t pos = -2 - loc;
-    TRY(ensure_list_dead(h));
-    uint8_t old = h->list_dead_h[(size_t)pos];
-    uint8_t nv = shadowed ? (old | 2) : (old & ~2);
-    if (!old && nv) h->list_ndead++;
-    if (old && !nv) h->list_ndead--;
-    h->list_dead_h[(size_t)pos] = nv;
-    h->lists_version++;
-    CK(cudaMemcpyAsync(h->list_dead.as<uint8_t>() + pos, &h->list_dead_h[(size_t)pos], 1, cudaMemcpyHostToDevice, h->stream));
+    TRY(set_list_flag(h, {-2 - loc}, 2, shadowed != 0));
     CK(cudaStreamSynchronize(h->stream));
     return PYROPE_OK;
 }
@@ -1669,11 +1706,11 @@ int pyrope_index_set_labels(pyrope_index* h, int64_t n_rows, const int64_t* labe
         CK(cudaMemcpyAsync(s.labels.p, L.data(), sizeof(int64_t) * L.size(), cudaMemcpyHostToDevice, st));
         CK(cudaStreamSynchronize(st));
     }
-    if (h->kind != PYROPE_FLAT && h->list_total > 0) {
+    if (h->kind != PYROPE_FLAT && h->lists.total > 0) {
         DevBuf dl;
         TRY(dl.ensure(sizeof(int64_t) * (size_t)n_rows, 0, st, true));
         CK(cudaMemcpyAsync(dl.p, labels_by_row, sizeof(int64_t) * (size_t)n_rows, cudaMemcpyHostToDevice, st));
-        CK(launch_gather_rows(dl.p, 8, h->list_rows.as<int64_t>(), h->list_total, h->list_labels.p, st));
+        CK(launch_gather_rows(dl.p, 8, h->lists.rows.as<int64_t>(), h->lists.total, h->lists.labels.p, st));
         CK(cudaStreamSynchronize(st));
     }
     return PYROPE_OK;
@@ -1700,48 +1737,20 @@ int pyrope_index_set_quantization(pyrope_index* h, int enable) {
 int pyrope_index_build(pyrope_index* h) {
     if (!h) return fail(PYROPE_ERR_INVALID_ARG, "index handle is null");
     std::lock_guard<std::mutex> g(h->mu);
-    if (h->last_stream) CK(cudaStreamSynchronize(h->last_stream));
-    if (h->kind == PYROPE_FLAT) return PYROPE_OK;  // BruteForceVectorIndex.cs:56
-    if (h->kind == PYROPE_IVF_FLAT) return build_ivfflat(h);
-    return build_ivfpq(h);
+    Staged S(*h);
+    TRY(build_prepare(*h, S));
+    install(h, S);
+    return PYROPE_OK;
 }
 
 int pyrope_index_extend(pyrope_index* h) {
     if (!h) return fail(PYROPE_ERR_INVALID_ARG, "index handle is null");
     std::lock_guard<std::mutex> g(h->mu);
-    StagedExtend S;
-    TRY(extend_prepare(h, S));
-    extend_commit(h, S);
+    Staged S(*h);
+    TRY(extend_prepare(*h, S));
+    install(h, S);
     return PYROPE_OK;
 }
-
-// ---- internal (not in the public header): the two halves of pyrope_index_extend for pyrope_sharded_extend.  _prepare
-// returns an opaque staged merge and the row ordinals that leave the buffer (owned by the staged object); _commit swaps
-// it in and frees it, _discard frees it unused.  Both run with the index's device current.
-int pyrope_internal_index_extend_prepare(pyrope_index* h, void** staged_out, int64_t* n_moved_out, const int64_t** moved_out) {
-    if (!h || !staged_out) return fail(PYROPE_ERR_INVALID_ARG, "index handle is null");
-    *staged_out = nullptr;
-    std::lock_guard<std::mutex> g(h->mu);
-    StagedExtend* S = new (std::nothrow) StagedExtend();
-    if (!S) return fail(PYROPE_ERR_OOM, "out of host memory");
-    int rc = extend_prepare(h, *S);
-    if (rc != PYROPE_OK) { delete S; return rc; }
-    if (n_moved_out) *n_moved_out = (int64_t)S->moved.size();
-    if (moved_out) *moved_out = S->moved.data();
-    *staged_out = S;
-    return PYROPE_OK;
-}
-
-void pyrope_internal_index_extend_commit(pyrope_index* h, void* staged) {
-    StagedExtend* S = static_cast<StagedExtend*>(staged);
-    {
-        std::lock_guard<std::mutex> g(h->mu);
-        extend_commit(h, *S);
-    }
-    delete S;
-}
-
-void pyrope_internal_index_extend_discard(void* staged) { delete static_cast<StagedExtend*>(staged); }
 
 int pyrope_index_set_train_params(pyrope_index* h, int64_t max_train_rows, int max_iter) {
     if (!h) return fail(PYROPE_ERR_INVALID_ARG, "index handle is null");
@@ -1763,7 +1772,7 @@ int pyrope_index_set_codebooks(pyrope_index* h, int n_centroids, const float* ce
         size_t cb = sizeof(float) * (size_t)h->m * h->k * h->sub;
         TRY(h->codebook.ensure(cb, 0, st, true));
         CK(cudaMemcpyAsync(h->codebook.p, pq_codebooks, cb, cudaMemcpyDefault, st));
-        h->cmax_for = nullptr; h->lm_cb16_ok = false;
+        h->pq_cmax_ok = false; h->lm_cb16_ok = false;
         h->ksub.assign((size_t)h->m, h->k);
     }
     CK(cudaStreamSynchronize(st));
@@ -1912,12 +1921,12 @@ int pyrope_index_get_lists(pyrope_index* h, int64_t* offsets_out, int64_t* rows_
         if (total_out) *total_out = 0;
         return PYROPE_OK;
     }
-    if (total_out) *total_out = h->list_total;
-    if (offsets_out) memcpy(offsets_out, h->list_off_h.data(), sizeof(int64_t) * ((size_t)h->nc + 1));
-    if (rows_out && h->list_total)
-        CK(cudaMemcpy(rows_out, h->list_rows.p, sizeof(int64_t) * (size_t)h->list_total, cudaMemcpyDeviceToHost));
-    if (codes_out && h->list_total && h->kind == PYROPE_IVF_PQ)
-        CK(cudaMemcpy(codes_out, h->list_codes.p, (size_t)h->list_total * h->m, cudaMemcpyDeviceToHost));
+    if (total_out) *total_out = h->lists.total;
+    if (offsets_out) memcpy(offsets_out, h->lists.off_h.data(), sizeof(int64_t) * ((size_t)h->nc + 1));
+    if (rows_out && h->lists.total)
+        CK(cudaMemcpy(rows_out, h->lists.rows.p, sizeof(int64_t) * (size_t)h->lists.total, cudaMemcpyDeviceToHost));
+    if (codes_out && h->lists.total && h->kind == PYROPE_IVF_PQ)
+        CK(cudaMemcpy(codes_out, h->lists.payload.p, (size_t)h->lists.total * h->m, cudaMemcpyDeviceToHost));
     return PYROPE_OK;
 }
 
@@ -2006,14 +2015,14 @@ int pyrope_index_snapshot(pyrope_index* h, const char* path) {
         const bool have_cb = h->kind == PYROPE_IVF_PQ && h->codebook.p && !h->ksub.empty();
         TRY(io.wdev(h->codebook.p, have_cb ? sizeof(float) * (size_t)h->m * h->k * h->sub : 0));
         io.wvec(h->ksub);
-        io.wv<int64_t>(h->built ? h->list_total : 0);
+        io.wv<int64_t>(h->built ? h->lists.total : 0);
         if (h->built) {
-            io.wvec(h->list_off_h);
-            TRY(io.wdev(h->list_rows.p, sizeof(int64_t) * (size_t)h->list_total));
-            TRY(io.wdev(h->list_labels.p, sizeof(int64_t) * (size_t)h->list_total));
-            if (h->kind == PYROPE_IVF_FLAT) TRY(io.wdev(h->list_vecs.p, sizeof(float) * (size_t)h->list_total * h->dim));
-            else TRY(io.wdev(h->list_codes.p, (size_t)h->list_total * h->m));
-            io.wvec(h->list_dead_h);
+            io.wvec(h->lists.off_h);
+            TRY(io.wdev(h->lists.rows.p, sizeof(int64_t) * (size_t)h->lists.total));
+            TRY(io.wdev(h->lists.labels.p, sizeof(int64_t) * (size_t)h->lists.total));
+            const size_t per = h->kind == PYROPE_IVF_FLAT ? sizeof(float) * (size_t)h->dim : (size_t)h->m;
+            TRY(io.wdev(h->lists.payload.p, (size_t)h->lists.total * per));
+            io.wvec(h->lists.dead_h);
         }
         return PYROPE_OK;
     };
@@ -2058,7 +2067,7 @@ int check_i64_range(const DevBuf& b, int64_t n, int64_t lo, int64_t hi, bool all
     return PYROPE_OK;
 }
 
-int parse_snapshot(Index* h, SnapIO& io, const char* path, LoadedSnapshot& L, cudaStream_t st) {
+int parse_snapshot(const Index* h, SnapIO& io, const char* path, LoadedSnapshot& L, cudaStream_t st) {
     auto bad = [&](const char* what) { return fail(PYROPE_ERR_INVALID_ARG, "corrupt or truncated snapshot %s: %s", path, what); };
     char magic[8];
     io.r(magic, 8);
@@ -2145,40 +2154,27 @@ int parse_snapshot(Index* h, SnapIO& io, const char* path, LoadedSnapshot& L, cu
     if (!io.ok) return bad("short read");
     return PYROPE_OK;
 }
-}  // namespace
-extern "C" {
 
-}  // extern "C"
-namespace {
-// A snapshot parsed, validated and staged in device memory, ready to be swapped into its index.  load_prepare does
-// everything that can fail (parse, validation, every device allocation); load_commit only swaps and cannot fail.  The
-// sharded index prepares every shard before it commits any (pyrope_sharded_load: all or nothing over N devices).
-struct StagedLoad {
-    LoadedSnapshot L;
-    Segment ns;
-    DevBuf cnorms, list_norms, list_dead, list_off, ksub_d;
-    int64_t list_ndead = 0, max_list_len = 0;
-};
-
-// caller holds h->mu
-int load_prepare(Index* h, const char* path, StagedLoad& S) {
-    CK(cudaStreamSynchronize(h->stream));
-    if (h->last_stream) CK(cudaStreamSynchronize(h->last_stream));
+// Load: everything that can fail (parse, validation, every device allocation) stages the file aside, so a truncated or
+// corrupt file or an OOM leaves the index as it was.  The sharded index prepares every shard before it installs any
+// (pyrope_sharded_load: all or nothing over N devices).
+int load_prepare(const Index& h, const char* path, Staged& S) {
+    CK(cudaStreamSynchronize(h.stream));
+    if (h.last_stream) CK(cudaStreamSynchronize(h.last_stream));
     SnapIO io;
     io.f = fopen(path, "rb");
     if (!io.f) return fail(PYROPE_ERR_NOT_FOUND, "Snapshot file not found: %s", path);  // FileNotFoundException
     if (fseek(io.f, 0, SEEK_END) == 0) { io.remaining = (uint64_t)std::max<long>(ftell(io.f), 0); io.bounded = true; }
     rewind(io.f);
-    cudaStream_t st = h->stream;
-    LoadedSnapshot& L = S.L;
-    int rc = parse_snapshot(h, io, path, L, st);
+    cudaStream_t st = h.stream;
+    LoadedSnapshot L;
+    int rc = parse_snapshot(&h, io, path, L, st);
     fclose(io.f);
-    if (rc != PYROPE_OK) return rc;  // nothing of the live index was touched
+    if (rc != PYROPE_OK) return rc;
 
-    // device allocations below can still fail (OOM), so they happen before anything is swapped
-    const int dim = h->dim;
-    Segment& ns = S.ns;
-    ns.dim = dim; ns.cosine = h->seg.cosine; ns.reuse_slots = h->seg.reuse_slots;
+    const int dim = h.dim;
+    Segment& ns = S.seg;
+    ns.dim = dim; ns.cosine = h.seg.cosine; ns.reuse_slots = h.seg.reuse_slots;
     TRY(ns.reserve(std::max<int64_t>(L.nslots, 1), st, true));
     if (L.nslots) {
         CK(cudaMemcpyAsync(ns.X.p, L.X.p, sizeof(float) * (size_t)L.nslots * dim, cudaMemcpyDeviceToDevice, st));
@@ -2186,78 +2182,65 @@ int load_prepare(Index* h, const char* path, StagedLoad& S) {
         CK(cudaMemcpyAsync(ns.dead.p, L.dead_h.data(), (size_t)L.nslots, cudaMemcpyHostToDevice, st));
         if (ns.cosine) CK(launch_row_norms_exact(ns.X.as<float>(), L.nslots, dim, dim, ns.norms.as<float>(), st));
     }
-    if (h->kind == PYROPE_IVF_PQ && !L.ksub.empty()) {
-        TRY(S.ksub_d.ensure(sizeof(int32_t) * L.ksub.size(), 0, st, true));
-        CK(cudaMemcpyAsync(S.ksub_d.p, L.ksub.data(), sizeof(int32_t) * L.ksub.size(), cudaMemcpyHostToDevice, st));
-    }
+    ns.nslots = L.nslots; ns.live = L.live; ns.ndead = L.ndead;
+    ns.dead_h.swap(L.dead_h); ns.slot_row.swap(L.slot_row); ns.free_stack.swap(L.free_stack);
+    IvfLists& T = S.lists;
     if (L.built) {
-        TRY(S.list_off.ensure(sizeof(int64_t) * L.list_off_h.size(), 0, st, true));
-        CK(cudaMemcpyAsync(S.list_off.p, L.list_off_h.data(), sizeof(int64_t) * L.list_off_h.size(), cudaMemcpyHostToDevice, st));
-        for (int c = 0; c < L.nc; ++c) S.max_list_len = std::max(S.max_list_len, L.list_off_h[(size_t)c + 1] - L.list_off_h[(size_t)c]);
+        T.total = L.list_total;
+        T.rows = std::move(L.list_rows);
+        T.labels = std::move(L.list_labels);
+        T.payload = std::move(L.list_payload);
+        T.off_h.swap(L.list_off_h);
+        TRY(T.off.ensure(sizeof(int64_t) * T.off_h.size(), 0, st, true));
+        CK(cudaMemcpyAsync(T.off.p, T.off_h.data(), sizeof(int64_t) * T.off_h.size(), cudaMemcpyHostToDevice, st));
+        for (int c = 0; c < L.nc; ++c) T.max_len = std::max(T.max_len, T.off_h[(size_t)c + 1] - T.off_h[(size_t)c]);
         if (!L.list_dead_h.empty()) {
-            TRY(S.list_dead.ensure((size_t)std::max<int64_t>(L.list_total, 1), 0, st, true));
-            CK(cudaMemcpyAsync(S.list_dead.p, L.list_dead_h.data(), L.list_dead_h.size(), cudaMemcpyHostToDevice, st));
-            for (uint8_t b : L.list_dead_h) S.list_ndead += b ? 1 : 0;
+            T.dead_h.swap(L.list_dead_h);
+            TRY(T.dead.ensure((size_t)std::max<int64_t>(T.total, 1), 0, st, true));
+            CK(cudaMemcpyAsync(T.dead.p, T.dead_h.data(), T.dead_h.size(), cudaMemcpyHostToDevice, st));
+            for (uint8_t b : T.dead_h) T.ndead += b ? 1 : 0;
         }
         TRY(S.cnorms.ensure(sizeof(float) * (size_t)std::max(L.nc, 1), 0, st, true));
-        if (h->metric == kCosine) {
+        if (h.metric == kCosine) {
             CK(launch_row_norms_exact(L.centroids.as<float>(), L.nc, dim, dim, S.cnorms.as<float>(), st));
-            if (h->kind == PYROPE_IVF_FLAT && L.list_total) {
-                TRY(S.list_norms.ensure(sizeof(float) * (size_t)L.list_total, 0, st, true));
-                CK(launch_row_norms_exact(L.list_payload.as<float>(), L.list_total, dim, dim, S.list_norms.as<float>(), st));
+            if (h.kind == PYROPE_IVF_FLAT && T.total) {
+                TRY(T.norms.ensure(sizeof(float) * (size_t)T.total, 0, st, true));
+                CK(launch_row_norms_exact(T.payload.as<float>(), T.total, dim, dim, T.norms.as<float>(), st));
             }
         }
     }
     CK(cudaStreamSynchronize(st));
+    S.quantiser = true;
+    S.centroids = std::move(L.centroids);
+    S.codebook = std::move(L.codebook);
+    S.ksub.swap(L.ksub);
+    S.nc = L.nc; S.built = L.built; S.frozen = L.frozen;
+    S.load = true;
+    S.nlist = L.nlist;
+    S.next_row = L.next_row;
+    S.shard_rank = L.shard_rank; S.shard_world = L.shard_world;
+    S.noop = false;
     return PYROPE_OK;
 }
 
-// caller holds h->mu; nothing here can fail: swap the staged state in
-void load_commit(Index* h, StagedLoad& S) {
-    LoadedSnapshot& L = S.L;
-    Segment& ns = S.ns;
-    auto take = [](DevBuf& dst, DevBuf& src) { std::swap(dst.p, src.p); std::swap(dst.bytes, src.bytes); src.release(); };
-    Segment& s = h->seg;
-    take(s.X, ns.X); take(s.dead, ns.dead); take(s.labels, ns.labels); take(s.norms, ns.norms);
-    s.cap = ns.cap; s.nslots = L.nslots; s.live = L.live; s.ndead = L.ndead;
-    s.dead_h.swap(L.dead_h); s.slot_row.swap(L.slot_row); s.free_stack.swap(L.free_stack);
-    s.tc_dirty = true;
-    h->tc_seg.invalidate();
-    h->nlist = L.nlist;
-    h->next_row = L.next_row;
-    h->built = L.built; h->frozen = L.frozen; h->nc = L.nc;
-    h->shard_rank = L.shard_rank; h->shard_world = L.shard_world;
-    take(h->centroids, L.centroids); take(h->codebook, L.codebook);
-    h->cmax_for = nullptr; h->lm_cb16_ok = false;
-    h->ksub.swap(L.ksub);
-    if (S.ksub_d.p) take(h->ksub_d, S.ksub_d);
-    h->list_total = L.list_total;
-    h->lists_version++;
-    h->list_ndead = S.list_ndead;
-    h->list_dead_h.swap(L.list_dead_h);
-    take(h->list_dead, S.list_dead);
-    h->max_list_len = S.max_list_len;
-    if (L.built) {
-        h->list_off_h.swap(L.list_off_h);
-        take(h->list_off, S.list_off); take(h->list_rows, L.list_rows); take(h->list_labels, L.list_labels);
-        if (h->kind == PYROPE_IVF_FLAT) take(h->list_vecs, L.list_payload); else take(h->list_codes, L.list_payload);
-        h->lm_codes16_ok = false;
-        take(h->cnorms, S.cnorms);
-        if (S.list_norms.p) take(h->list_norms, S.list_norms);
-    } else {
-        h->list_off_h.clear();
+// the first half of pyrope_internal_index_prepare_*: a Staged on the heap that the caller commits or discards
+template <typename Prepare>
+int prepare_detached(pyrope_index* h, void** staged_out, pyrope_internal_staged_info* info, Prepare prepare) {
+    if (!h || !staged_out) return fail(PYROPE_ERR_INVALID_ARG, "index handle is null");
+    *staged_out = nullptr;
+    std::lock_guard<std::mutex> g(h->mu);
+    std::unique_ptr<Staged> S(new (std::nothrow) Staged(*h));
+    if (!S) return fail(PYROPE_ERR_OOM, "out of host memory");
+    TRY(prepare(*h, *S));
+    if (info) {
+        info->n_moved = (int64_t)S->moved.size();
+        info->moved = S->moved.data();
+        info->shard_rank = S->shard_rank;
+        info->shard_world = S->shard_world;
+        info->next_row = S->next_row;
     }
-    // SQ8 (FLAT): the reference's Load re-adds every row through InternalAdd (BruteForceVectorIndex.cs:93-97 ->
-    // :162-184), which quantises it iff the LOADING index has EnableQuantization on at that moment — the flag is a
-    // property of the object, not of the file.  Same here: with the flag on every loaded row gets its byte copy
-    // (ScalarQuantizer is deterministic, so re-quantising reproduces the bytes the snapshotting index held), with it
-    // off no loaded row has a quantised form (:312-322 keeps such rows invisible to a later quantised search).
-    if (h->kind == PYROPE_FLAT && (h->sq8 || h->x8.p)) {
-        h->x8_cap = 0;
-        sq8_rows(h, 0, h->seg.nslots);  // best effort: the rows themselves are already in place
-    }
-    h->tc_cent.invalidate();
-    if (h->kind != PYROPE_FLAT) { h->row_loc.assign((size_t)h->next_row, -1); h->lists_loc_valid = false; }
+    *staged_out = S.release();
+    return PYROPE_OK;
 }
 }  // namespace
 extern "C" {
@@ -2265,41 +2248,32 @@ extern "C" {
 int pyrope_index_load(pyrope_index* h, const char* path) {
     if (!h || !path || !*path) return fail(PYROPE_ERR_INVALID_ARG, "Path cannot be empty");
     std::lock_guard<std::mutex> g(h->mu);
-    StagedLoad S;
-    TRY(load_prepare(h, path, S));
-    load_commit(h, S);
+    Staged S(*h);
+    TRY(load_prepare(*h, path, S));
+    install(h, S);
     return PYROPE_OK;
 }
 
-// ---- internal (not in the public header): the two halves of pyrope_index_load for pyrope_sharded_load.  _prepare
-// returns an opaque staged snapshot and the shard identity / row count its file records; _commit swaps it in and frees
-// it, _discard frees it unused.  Both run with the index's device current.
-int pyrope_internal_index_load_prepare(pyrope_index* h, const char* path, void** staged_out, int32_t* shard_rank_out,
-                                       int32_t* shard_world_out, int64_t* next_row_out) {
-    if (!h || !path || !*path || !staged_out) return fail(PYROPE_ERR_INVALID_ARG, "Path cannot be empty");
-    *staged_out = nullptr;
+int pyrope_internal_index_prepare_build(pyrope_index* h, void** staged_out, pyrope_internal_staged_info* info) {
+    return prepare_detached(h, staged_out, info, build_prepare);
+}
+
+int pyrope_internal_index_prepare_extend(pyrope_index* h, void** staged_out, pyrope_internal_staged_info* info) {
+    return prepare_detached(h, staged_out, info, extend_prepare);
+}
+
+int pyrope_internal_index_prepare_load(pyrope_index* h, const char* path, void** staged_out, pyrope_internal_staged_info* info) {
+    if (!path || !*path) return fail(PYROPE_ERR_INVALID_ARG, "Path cannot be empty");
+    return prepare_detached(h, staged_out, info, [path](const Index& x, Staged& S) { return load_prepare(x, path, S); });
+}
+
+void pyrope_internal_index_commit(pyrope_index* h, void* staged) {
+    std::unique_ptr<Staged> S(static_cast<Staged*>(staged));
     std::lock_guard<std::mutex> g(h->mu);
-    StagedLoad* S = new (std::nothrow) StagedLoad();
-    if (!S) return fail(PYROPE_ERR_OOM, "out of host memory");
-    int rc = load_prepare(h, path, *S);
-    if (rc != PYROPE_OK) { delete S; return rc; }
-    if (shard_rank_out) *shard_rank_out = S->L.shard_rank;
-    if (shard_world_out) *shard_world_out = S->L.shard_world;
-    if (next_row_out) *next_row_out = S->L.next_row;
-    *staged_out = S;
-    return PYROPE_OK;
+    install(h, *S);
 }
 
-void pyrope_internal_index_load_commit(pyrope_index* h, void* staged) {
-    StagedLoad* S = static_cast<StagedLoad*>(staged);
-    {
-        std::lock_guard<std::mutex> g(h->mu);
-        load_commit(h, *S);
-    }
-    delete S;
-}
-
-void pyrope_internal_index_load_discard(void* staged) { delete static_cast<StagedLoad*>(staged); }
+void pyrope_internal_index_discard(void* staged) { delete static_cast<Staged*>(staged); }
 
 // header peek for the string-id layer: rows ever added according to the snapshot (validates the magic only)
 int pyrope_internal_snapshot_next_row(const char* path, int64_t* next_row_out) {
@@ -2318,7 +2292,7 @@ int pyrope_internal_snapshot_next_row(const char* path, int64_t* next_row_out) {
 
 int pyrope_index_stats(pyrope_index* h, int64_t* live_rows, int64_t* buffer_rows, int* dim, int* metric) {
     if (!h) return fail(PYROPE_ERR_INVALID_ARG, "index handle is null");
-    if (live_rows) *live_rows = h->seg.live + (h->built ? h->list_total - h->list_ndead : 0);
+    if (live_rows) *live_rows = h->seg.live + (h->built ? h->lists.total - h->lists.ndead : 0);
     if (buffer_rows) *buffer_rows = h->seg.live;
     if (dim) *dim = h->dim;
     if (metric) *metric = h->metric;
@@ -2330,7 +2304,7 @@ int pyrope_index_search_batch_device(pyrope_index* h, int64_t nq, const float* d
     TRY(validate_search(h, nq, dQ, topk));
     if (nq == 0) return PYROPE_OK;
     std::lock_guard<std::mutex> g(h->mu);
-    if (h->kind == PYROPE_IVF_FLAT && max_scans >= 0 && h->list_ndead > 0) TRY(compact_lists(h));
+    if (h->kind == PYROPE_IVF_FLAT && max_scans >= 0 && h->lists.ndead > 0) TRY(compact_lists(h));
     cudaStream_t st = stream ? (cudaStream_t)stream : h->stream;
     TRY(search_device(h, nq, dQ, topk, max_scans, nprobe, d_scores, d_rows, d_counts, st));
     if (!stream) CK(cudaStreamSynchronize(st));
@@ -2358,7 +2332,7 @@ int pyrope_index_search_batch_probed_device(pyrope_index* h, int64_t nq, const f
     if (!d_probes) return fail(PYROPE_ERR_INVALID_ARG, "probes is null");
     if (nq == 0) return PYROPE_OK;
     std::lock_guard<std::mutex> g(h->mu);
-    if (h->kind == PYROPE_IVF_FLAT && max_scans >= 0 && h->list_ndead > 0) TRY(compact_lists(h));
+    if (h->kind == PYROPE_IVF_FLAT && max_scans >= 0 && h->lists.ndead > 0) TRY(compact_lists(h));
     cudaStream_t st = stream ? (cudaStream_t)stream : h->stream;
     TRY(search_device(h, nq, dQ, topk, max_scans, nprobe, d_scores, d_rows, d_counts, st, d_probes, nullptr));
     if (!stream) CK(cudaStreamSynchronize(st));
@@ -2371,7 +2345,7 @@ int pyrope_index_search_batch(pyrope_index* h, int64_t nq, const float* Q, int t
     if (nq == 0) return PYROPE_OK;
     if (!scores_out || !rows_out || !counts_out) return fail(PYROPE_ERR_INVALID_ARG, "output buffer is null");
     std::lock_guard<std::mutex> g(h->mu);
-    if (h->kind == PYROPE_IVF_FLAT && max_scans >= 0 && h->list_ndead > 0) TRY(compact_lists(h));
+    if (h->kind == PYROPE_IVF_FLAT && max_scans >= 0 && h->lists.ndead > 0) TRY(compact_lists(h));
     cudaStream_t st = h->stream;
     Workspace& ws = h->ws;
     const int kk = std::max(topk, 1);
@@ -2430,7 +2404,7 @@ int pyrope_index_last_search_scanned(pyrope_index* h, int64_t* codes_out) {
     if (h->kind == PYROPE_IVF_FLAT)
         CK(ivfflat_lm_scanned_rows(h->ws.lm.p, h->lm_nq, h->lm_P, h->lm_k, h->nc, &v, h->last_stream ? h->last_stream : h->stream));
     else
-        CK(ivfpq_lm_scanned_codes(h->ws.lm.p, h->lm_nq, h->lm_P, h->lm_k, h->nc, h->dim, h->max_list_len, &v,
+        CK(ivfpq_lm_scanned_codes(h->ws.lm.p, h->lm_nq, h->lm_P, h->lm_k, h->nc, h->dim, h->lists.max_len, &v,
                                   h->last_stream ? h->last_stream : h->stream));
     *codes_out = (int64_t)v;
     return PYROPE_OK;
@@ -2454,15 +2428,6 @@ int pyrope_topk_merge_device(int64_t nq, int parts, int k_in, int k_out, const f
 
 // ---- Head+Tail on device (DeltaVectorIndex.cs) ------------------------------------------------------
 }  // extern "C"
-
-// csrc/sharded.cu (internal, not part of the public header): the pieces of a sharded index a Head+Tail over it uses.
-// The search is pyrope_sharded_search_batch_device whose shards first wait for q_ready (a CUDA event, may be null);
-// absorb is the compaction's "_tail.Add per row" step on every shard (see tail_absorb below).
-extern "C" int pyrope_internal_sharded_search_device(pyrope_sharded* s, int64_t nq, const float* dQ_dev0, int topk,
-                                                     int64_t max_scans, int nprobe, float* d_scores_dev0,
-                                                     int64_t* d_rows_dev0, int32_t* d_counts_dev0, void* q_ready);
-extern "C" int pyrope_internal_sharded_absorb(pyrope_sharded* s, int64_t n, const float* dX, const int64_t* dL, int src_device,
-                                              const int64_t* labels_host, int64_t* tail_rows_out);
 
 struct pyrope_delta {
     pyrope_index* head = nullptr;
@@ -2516,7 +2481,7 @@ int delta_search_device(pyrope_delta* d, int64_t nq, const float* dQ, int topk, 
                                                         d->pc.as<int32_t>() + nq, d->q_ready)));
     } else {
         std::lock_guard<std::mutex> g(tl->mu);
-        if (tl->kind == PYROPE_IVF_FLAT && max_scans >= 0 && tl->list_ndead > 0) TRY(compact_lists(tl));
+        if (tl->kind == PYROPE_IVF_FLAT && max_scans >= 0 && tl->lists.ndead > 0) TRY(compact_lists(tl));
         TRY(search_device(tl, nq, dQ, topk, max_scans, nprobe, d->ps.as<float>() + per, d->pl.as<int64_t>() + per,
                           d->pc.as<int32_t>() + nq, st));
     }
@@ -2727,7 +2692,7 @@ int tail_absorb(Index* tl, int64_t n, const float* mx, const int64_t* ml, const 
     Segment& ts = tl->seg;
     // both IVF searches skip a list entry whose id is buffered (seenIds, IvfFlatVectorIndex.cs:210, IvfPqVectorIndex.cs:170),
     // and an Extend that moves the buffered copy into the lists must find the entry it replaces flagged
-    const bool lists_matter = tl->built && tl->kind != PYROPE_FLAT && tl->list_total > 0;
+    const bool lists_matter = tl->built && tl->kind != PYROPE_FLAT && tl->lists.total > 0;
     if (ts.live > 0 || lists_matter) {
         TRY(dsorted.ensure(sizeof(int64_t) * (size_t)n, 0, st, true));
         CK(cudaMemcpyAsync(dsorted.p, sorted.data(), sizeof(int64_t) * (size_t)n, cudaMemcpyHostToDevice, st));
@@ -2744,22 +2709,16 @@ int tail_absorb(Index* tl, int64_t n, const float* mx, const int64_t* ml, const 
     }
     if (lists_matter) {
         TRY(ensure_list_dead(tl));
-        TRY(where.ensure(sizeof(int64_t) * (size_t)tl->list_total, 0, st, true));
-        CK(launch_find_labels(tl->list_labels.as<int64_t>(), tl->list_dead.as<uint8_t>(), tl->list_total,
+        TRY(where.ensure(sizeof(int64_t) * (size_t)tl->lists.total, 0, st, true));
+        CK(launch_find_labels(tl->lists.labels.as<int64_t>(), tl->lists.dead.as<uint8_t>(), tl->lists.total,
                               dsorted.as<int64_t>(), n, where.as<int64_t>(), st));
-        std::vector<int64_t> wh((size_t)tl->list_total);
+        std::vector<int64_t> wh((size_t)tl->lists.total);
         CK(cudaMemcpyAsync(wh.data(), where.p, sizeof(int64_t) * wh.size(), cudaMemcpyDeviceToHost, st));
         CK(cudaStreamSynchronize(st));
-        bool any = false;
-        for (int64_t i = 0; i < tl->list_total; ++i)
-            if (wh[(size_t)i] >= 0) {
-                if (!tl->list_dead_h[(size_t)i]) tl->list_ndead++;
-                tl->lists_version++;
-                tl->list_dead_h[(size_t)i] |= 2;
-                any = true;
-            }
-        if (any)
-            CK(cudaMemcpyAsync(tl->list_dead.p, tl->list_dead_h.data(), (size_t)tl->list_total, cudaMemcpyHostToDevice, st));
+        std::vector<int64_t> shadow;
+        for (int64_t i = 0; i < tl->lists.total; ++i)
+            if (wh[(size_t)i] >= 0) shadow.push_back(i);
+        TRY(set_list_flag(tl, shadow, 2, true));
     }
     std::vector<int64_t> over_src, over_dst, app_src;
     for (int64_t i = 0; i < n; ++i) {
@@ -2867,14 +2826,9 @@ int delta_compact_impl(pyrope_delta* d, int64_t* moved_out, int64_t* tail_rows_o
     if (d->stail) return spass(extend ? pyrope_sharded_extend(d->stail) : pyrope_sharded_build(d->stail));
     Index* tl = d->tail;
     std::lock_guard<std::mutex> gt(tl->mu);
-    if (extend) {
-        StagedExtend S;
-        TRY(extend_prepare(tl, S));
-        extend_commit(tl, S);
-        return PYROPE_OK;
-    }
-    if (tl->kind == PYROPE_IVF_FLAT) return build_ivfflat(tl);
-    if (tl->kind == PYROPE_IVF_PQ) return build_ivfpq(tl);
+    Staged S(*tl);
+    TRY(extend ? extend_prepare(*tl, S) : build_prepare(*tl, S));
+    install(tl, S);
     return PYROPE_OK;
 }
 }  // namespace
@@ -2920,7 +2874,7 @@ int pyrope_delta_stats(pyrope_delta* d, int64_t* count_out) {
         return PYROPE_OK;
     }
     Index* tl = d->tail;
-    *count_out = hd->seg.live + tl->seg.live + (tl->built ? tl->list_total - tl->list_ndead : 0);
+    *count_out = hd->seg.live + tl->seg.live + (tl->built ? tl->lists.total - tl->lists.ndead : 0);
     return PYROPE_OK;
 }
 

@@ -27,14 +27,7 @@
 #include <vector>
 
 #include "../../include/pyrope_gpu.h"
-
-// api.cu / vindex.cu (internal, not part of the public header)
-extern "C" int pyrope_internal_index_kind(pyrope_index* h, int* kind_out);
-extern "C" int pyrope_internal_delta_limits(pyrope_delta* d, int* dim_out, int* max_topk_out);
-extern "C" int pyrope_internal_vindex_limits(pyrope_vindex* v, int* dim_out, int* max_topk_out, int* nonpos_empty_out);
-extern "C" int pyrope_internal_vindex_search_topk(pyrope_vindex* v, int64_t nq, const float* Q, const int32_t* topks,
-                                                  int64_t max_scans, int nprobe, float* scores_out, int64_t* gids_out,
-                                                  int32_t* counts_out);
+#include "internal.h"
 
 namespace {
 

@@ -30,20 +30,7 @@
 #include <cuda_runtime.h>
 
 #include "../../include/pyrope_gpu.h"
-
-// api.cu (internal, not part of the public header): the two halves of pyrope_index_load, and the compaction's per-tail
-// step of a Head+Tail (pyrope_delta_*) whose tail is sharded
-extern "C" int pyrope_internal_index_load_prepare(pyrope_index* h, const char* path, void** staged_out, int32_t* shard_rank_out,
-                                                  int32_t* shard_world_out, int64_t* next_row_out);
-extern "C" void pyrope_internal_index_load_commit(pyrope_index* h, void* staged);
-extern "C" void pyrope_internal_index_load_discard(void* staged);
-extern "C" int pyrope_internal_index_extend_prepare(pyrope_index* h, void** staged_out, int64_t* n_moved_out,
-                                                    const int64_t** moved_out);
-extern "C" void pyrope_internal_index_extend_commit(pyrope_index* h, void* staged);
-extern "C" void pyrope_internal_index_extend_discard(void* staged);
-extern "C" int pyrope_internal_tail_reserve(pyrope_index* tl, int64_t n);
-extern "C" int pyrope_internal_tail_absorb(pyrope_index* tl, int64_t n, const float* dX, const int64_t* dL,
-                                           const int64_t* labels_host, int64_t* tail_rows_out);
+#include "internal.h"
 
 namespace {
 
@@ -205,6 +192,42 @@ int grow_pinned(void** p, size_t* have, size_t need) {
     SCK(cudaMallocHost(p, need));
     *have = need;
     return PYROPE_OK;
+}
+
+// Build, Extend or Load on every shard, all or nothing: prepare(r, &staged) stages shard r's operation on its own thread,
+// then check() compares what the shards staged.  Only if every shard prepared and the check passed does every shard
+// install its staged state; otherwise every staged state is dropped and every shard is left as it was.
+int stage_all(S* s, const std::function<int(int, void**)>& prepare, const std::function<int()>& check) {
+    std::vector<void*> staged((size_t)s->n, nullptr);
+    int rc = run_all(s, [&](int r) -> int { return prepare(r, &staged[(size_t)r]); });
+    if (rc == PYROPE_OK) rc = check();
+    if (rc != PYROPE_OK) {
+        run_all(s, [&](int r) -> int { pyrope_internal_index_discard(staged[(size_t)r]); return PYROPE_OK; });
+        return rc;
+    }
+    run_all(s, [&](int r) -> int { pyrope_internal_index_commit(s->shard[(size_t)r], staged[(size_t)r]); return PYROPE_OK; });
+    return PYROPE_OK;
+}
+
+// Build and Extend consume every shard's replica of the write buffer: they go ahead only if every shard moves the same
+// buffered row ordinals into its lists
+int stage_consuming(S* s, int (*prepare)(pyrope_index*, void**, pyrope_internal_staged_info*)) {
+    std::vector<std::vector<int64_t>> moved((size_t)s->n);
+    auto prep = [&](int r, void** staged) -> int {
+        pyrope_internal_staged_info info{};
+        STRY(prepare(s->shard[(size_t)r], staged, &info));
+        moved[(size_t)r].assign(info.moved, info.moved + info.n_moved);
+        std::sort(moved[(size_t)r].begin(), moved[(size_t)r].end());
+        return PYROPE_OK;
+    };
+    auto same = [&]() -> int {
+        for (size_t r = 1; r < moved.size(); ++r)
+            if (moved[r] != moved[0])
+                return sfail(PYROPE_ERR_INVALID_STATE, "shard %zu and shard 0 would move different buffered rows (%zu vs %zu): the buffer replicas diverged",
+                             r, moved[r].size(), moved[0].size());
+        return PYROPE_OK;
+    };
+    return stage_all(s, prep, same);
 }
 
 }  // namespace
@@ -407,7 +430,7 @@ int pyrope_sharded_delete_row(pyrope_sharded* s, int64_t row) {
 int pyrope_sharded_build(pyrope_sharded* s) {
     if (!s) return sfail(PYROPE_ERR_INVALID_ARG, "handle is null");
     std::lock_guard<std::mutex> g(s->mu);
-    int rc = run_all(s, [&](int r) -> int { STRY(pyrope_index_build(s->shard[(size_t)r])); return PYROPE_OK; });
+    const int rc = stage_consuming(s, pyrope_internal_index_prepare_build);
     if (rc == PYROPE_OK && s->kind != PYROPE_FLAT) {
         int b = 0;
         pyrope_index_is_built(s->shard[0], &b);
@@ -416,36 +439,11 @@ int pyrope_sharded_build(pyrope_sharded* s) {
     return rc;
 }
 
-// Extend on every shard: each prepares on its own thread (assign, encode, merged lists of the lists it owns) and the
-// merges are committed only if all of them prepared and all report the same row ordinals leaving their buffer replica.
 int pyrope_sharded_extend(pyrope_sharded* s) {
     if (!s) return sfail(PYROPE_ERR_INVALID_ARG, "handle is null");
     if (s->kind == PYROPE_FLAT) return sfail(PYROPE_ERR_UNSUPPORTED, "Extend needs an IVF index: FLAT has no inverted lists");
     std::lock_guard<std::mutex> g(s->mu);
-    const size_t N = (size_t)s->n;
-    std::vector<void*> staged(N, nullptr);
-    std::vector<std::vector<int64_t>> moved(N);
-    int rc = run_all(s, [&](int r) -> int {
-        int64_t nm = 0;
-        const int64_t* rows = nullptr;
-        STRY(pyrope_internal_index_extend_prepare(s->shard[(size_t)r], &staged[(size_t)r], &nm, &rows));
-        moved[(size_t)r].assign(rows, rows + nm);
-        std::sort(moved[(size_t)r].begin(), moved[(size_t)r].end());
-        return PYROPE_OK;
-    });
-    for (size_t r = 1; rc == PYROPE_OK && r < N; ++r)
-        if (moved[r] != moved[0])
-            rc = sfail(PYROPE_ERR_INVALID_STATE, "shard %zu and shard 0 would move different buffered rows (%zu vs %zu): the buffer replicas diverged",
-                       r, moved[r].size(), moved[0].size());
-    if (rc != PYROPE_OK) {
-        run_all(s, [&](int r) -> int {
-            if (staged[(size_t)r]) pyrope_internal_index_extend_discard(staged[(size_t)r]);
-            return PYROPE_OK;
-        });
-        return rc;
-    }
-    run_all(s, [&](int r) -> int { pyrope_internal_index_extend_commit(s->shard[(size_t)r], staged[(size_t)r]); return PYROPE_OK; });
-    return PYROPE_OK;
+    return stage_consuming(s, pyrope_internal_index_prepare_extend);
 }
 
 int pyrope_sharded_stats(pyrope_sharded* s, int64_t* live_rows_out) {
@@ -907,30 +905,22 @@ int pyrope_sharded_load(pyrope_sharded* s, const char* path) {
             return sfail(PYROPE_ERR_INVALID_ARG, "shard file %s holds %llu bytes, the manifest recorded %llu", f.c_str(),
                          (unsigned long long)b, (unsigned long long)M.bytes[(size_t)r]);
     }
-    // every shard parses and stages its file on its own thread; nothing is committed unless all of them succeed
-    std::vector<void*> staged((size_t)s->n, nullptr);
-    int rc = run_all(s, [&](int r) -> int {
-        int32_t rank = -1, world = 0;
-        int64_t nr = -1;
+    // every shard parses and stages its file on its own thread; nothing is installed unless all of them succeed
+    const int rc = stage_all(s, [&](int r, void** staged) -> int {
+        pyrope_internal_staged_info info{};
         const std::string f = dir + M.names[(size_t)r];
-        STRY(pyrope_internal_index_load_prepare(s->shard[(size_t)r], f.c_str(), &staged[(size_t)r], &rank, &world, &nr));
+        STRY(pyrope_internal_index_prepare_load(s->shard[(size_t)r], f.c_str(), staged, &info));
         // IVF shards carry their shard identity and the replicated row count; FLAT shards are plain indexes of their rows
         const bool ivf = s->kind != PYROPE_FLAT;
         const int want_rank = ivf ? r : 0, want_world = ivf ? s->n : 1;
         const int64_t want_rows = ivf ? M.next_row : M.shard_rows[(size_t)r];
-        if (rank != want_rank || world != want_world || nr != want_rows)
+        if (info.shard_rank != want_rank || info.shard_world != want_world || info.next_row != want_rows)
             return sfail(PYROPE_ERR_INVALID_ARG, "%s is shard %d of %d with %lld rows, the manifest expects shard %d of %d with %lld rows",
-                         f.c_str(), rank, world, (long long)nr, want_rank, want_world, (long long)want_rows);
+                         f.c_str(), info.shard_rank, info.shard_world, (long long)info.next_row, want_rank, want_world,
+                         (long long)want_rows);
         return PYROPE_OK;
-    });
-    if (rc != PYROPE_OK) {
-        run_all(s, [&](int r) -> int {
-            if (staged[(size_t)r]) pyrope_internal_index_load_discard(staged[(size_t)r]);
-            return PYROPE_OK;
-        });
-        return rc;
-    }
-    run_all(s, [&](int r) -> int { pyrope_internal_index_load_commit(s->shard[(size_t)r], staged[(size_t)r]); return PYROPE_OK; });
+    }, [] { return PYROPE_OK; });
+    if (rc != PYROPE_OK) return rc;
     s->next_row = M.next_row;
     s->segs = M.segs;
     s->shard_rows = M.shard_rows;

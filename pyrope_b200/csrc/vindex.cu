@@ -22,13 +22,7 @@
 #include <vector>
 
 #include "../../include/pyrope_gpu.h"
-
-// api.cu / sharded.cu (internal, not part of the public header): rows ever added according to a snapshot's header /
-// a sharded snapshot's manifest
-extern "C" int pyrope_internal_snapshot_next_row(const char* path, int64_t* next_row_out);
-extern "C" int pyrope_internal_sharded_snapshot_next_row(const char* path, int64_t* next_row_out);
-// api.cu (internal): the dimension and topK limit of a Head+Tail
-extern "C" int pyrope_internal_delta_limits(pyrope_delta* d, int* dim_out, int* max_topk_out);
+#include "internal.h"
 
 namespace {
 

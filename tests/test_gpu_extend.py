@@ -286,6 +286,37 @@ def test_extend_sharded_equals_one_device_and_snapshot(gpu, kind, tmp_path):
         sx.close()
 
 
+@pytest.mark.gpu
+def test_sharded_build_and_extend_are_all_or_nothing(gpu):
+    """Build and Extend consume every shard's replica of the buffer: when one replica diverged, both refuse and leave
+    every shard's lists and buffer as they were."""
+    n = max(_counts(gpu))
+    if n < 2:
+        pytest.skip("needs 2 GPUs")
+    rng = np.random.default_rng(35)
+    X = rng.standard_normal((2600, DIM)).astype(np.float32)
+    sx = gpu.ShardedIndex(n, gpu.IVF_FLAT, DIM, gpu.L2, nlist=20, m=8, k=K)
+    sx.add(X[:2000])
+    sx.build()
+    before = [sx.shard(r)[0].lists() for r in range(n)]
+    sx.add(X[2000:2500])
+    sh0, _ = sx.shard(0)
+    sh0.add(X[2500:])  # only shard 0's replica holds these rows
+    for op in (sx.build, sx.extend):
+        with pytest.raises(gpu._lib.PyropeGpuError) as e:
+            op()
+        assert e.value.code == gpu._lib.ERR_INVALID_STATE, e.value.message
+        for r in range(n):
+            sh, _ = sx.shard(r)
+            off, rows, _ = sh.lists()
+            np.testing.assert_array_equal(off, before[r][0], err_msg=f"{op.__name__}: shard {r} offsets")
+            np.testing.assert_array_equal(rows, before[r][1], err_msg=f"{op.__name__}: shard {r} rows")
+            assert sh.stats()["buffer"] == (600 if r == 0 else 500), f"{op.__name__}: shard {r} buffer"
+            del sh
+    del sh0
+    sx.close()
+
+
 # ---- Head+Tail with string ids: a CPU model of compaction by Extend ------------------------------------------------
 class RefExtendDelta:
     """DeltaVectorIndex whose compaction is Extend, over the oracle: the head is an oracle FLAT index; the tail is kept
