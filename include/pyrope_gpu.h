@@ -9,9 +9,11 @@
  * Gpu*VectorIndex : IVectorIndex P/Invokes the functions below (stub in INTEGRATION.md).
  *
  * Conventions
- *  - every function returns a pyrope_status (0 ok, <0 error); pyrope_last_error() returns a
- *    thread-local message.  The library never aborts/exits (VectorCommandSet.cs:547-554 turns any
- *    exception into "-ERR <message>"; the shim maps codes to the .NET exception types named below).
+ *  - every function returns a pyrope_status (0 ok, <0 error); pyrope_last_error() returns the calling
+ *    thread's message of its most recent failure, whichever module raised it.  The per-module readers
+ *    (pyrope_sharded_, _peer_, _batcher_, _vindex_, _formats_last_error) return the same message.  The
+ *    library never aborts/exits (VectorCommandSet.cs:547-554 turns any exception into "-ERR <message>";
+ *    the shim maps codes to the .NET exception types named below).
  *  - host pointers unless the function name ends in _device.  Inputs are only read during the call
  *    (the library copies, as BruteForceVectorIndex.Add does, BruteForceVectorIndex.cs:147-148).
  *  - string ids stay host-side in the shim (List<string>/Dictionary<string,long> exactly like
@@ -227,8 +229,7 @@ int pyrope_index_last_search_scanned(pyrope_index *h, int64_t *codes_out);
  *      (MaxScans, NProbe, K) and returns each caller its own result.  K is the topK class: the smallest power of two
  *      >= topK, capped at the target's limit; a group is searched once at its largest topK and every caller gets
  *      exactly its own top topK (a Head+Tail merges with a per-query k, pyrope_delta_search_batch_topk).
- *      Thread-safe; results are written into the caller's buffers (topk entries each); errors carry
- *      pyrope_batcher_last_error(), with the message of whichever layer raised them.
+ *      Thread-safe; results are written into the caller's buffers (topk entries each).
  *      The target is borrowed: destroy the batcher first.  It is one of
  *        pyrope_batcher_create          a pyrope_index: rows_out = row ordinals (or the rows' labels);
  *        pyrope_batcher_create_sharded  a pyrope_sharded: global row ordinals (labels), dimension from shard 0;
@@ -278,7 +279,7 @@ int pyrope_topk_merge_dedupe_device(int64_t nq, int parts, int k_in, int k_out, 
  *      IVF_PQ scan kernels exchange thresholds through peer memory while they run; local top-k lists land in device
  *      0's gather buffer and are merged there (one entry per row label).  Results equal the single-GPU index's.
  *      MaxScans (an insertion-/probe-order budget) cannot be split: max_scans >= 0 with N > 1 -> UNSUPPORTED.
- *      Errors: pyrope_sharded_last_error().  Calls on one handle are serialised internally. */
+ *      Calls on one handle are serialised internally. */
 /* devices: n_devices CUDA ordinals, or NULL for 0..n_devices-1 (1 <= n_devices <= 8; peers must be NVLink/P2P reachable) */
 int pyrope_sharded_create(int n_devices, const int *devices, int kind, int dim, int metric, int nlist, int pq_m,
                           int pq_k, pyrope_sharded **out);
@@ -343,7 +344,7 @@ const char *pyrope_sharded_last_error(void);
  *      of 16) into every rank's buffer, a release of this call's epoch to the peers, and a wait for theirs; work
  *      enqueued after it on the same stream sees *d_gathered_out = [world][bytes_per_rank].  The area is double-buffered
  *      by call parity: consume the gathered data (on that stream) before the next-but-one call on the same slot.
- *      A rank whose peers never arrive faults after ~20 s instead of hanging the device.  Errors: pyrope_peer_last_error(). */
+ *      A rank whose peers never arrive faults after ~20 s instead of hanging the device. */
 typedef struct pyrope_peer_group pyrope_peer_group;
 int pyrope_peer_group_create(int world, int rank, size_t slot_bytes, int n_slots, pyrope_peer_group **out);
 int pyrope_peer_group_destroy(pyrope_peer_group *g);
@@ -415,7 +416,7 @@ int pyrope_delta_load(pyrope_delta *d, const char *path);
  *      DeltaVectorIndex over two of them; it keeps the id dictionaries those classes keep and maps their
  *      Add / Upsert / Delete / Build / Search semantics onto the row-ordinal entry points above, so the C# class
  *      behind IVectorIndex is a one-line forwarder per method.  Search returns id ORDINALS (process-wide, the
- *      row labels); pyrope_vindex_id turns one into its UTF-8 string.  Errors: pyrope_vindex_last_error().
+ *      row labels); pyrope_vindex_id turns one into its UTF-8 string.
  *      Status codes map to the exceptions the reference throws: INVALID_ARG -> ArgumentException ("Id cannot be
  *      empty."), DIMENSION -> ArgumentException("Vector dimension mismatch"), OUT_OF_RANGE ->
  *      ArgumentOutOfRangeException (FLAT topK <= 0), INVALID_STATE -> InvalidOperationException (FLAT duplicate
@@ -459,7 +460,7 @@ int pyrope_vindex_snapshot(pyrope_vindex *v, const char *path); /* index file(s)
 int pyrope_vindex_load(pyrope_vindex *v, const char *path);
 const char *pyrope_vindex_last_error(void);
 
-/* ---- data formats either side of the path (csrc/formats.cu; host only).  Errors: pyrope_formats_last_error().
+/* ---- data formats either side of the path (csrc/formats.cu; host only).
  *      pyrope_parse_vector = VectorParsing.ParseVector (Utils/VectorParsing.cs:10-35): a VEC.ADD / VEC.SEARCH payload
  *      is tried as a JSON array, then as ',' / ' ' separated text, then taken as raw little-endian float32 (length a
  *      multiple of 4) — the binary form is what the benchmark client sends (VectorEncoding.ToLittleEndianBytes,

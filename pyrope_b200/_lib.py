@@ -406,38 +406,32 @@ class PeerGroup:
     def __init__(self, world: int, rank: int, slot_bytes: int, n_slots: int = 1):
         g = vp()
         self._g = None
-        self._ck(load().pyrope_peer_group_create(world, rank, slot_bytes, n_slots, C.byref(g)))
+        check(load().pyrope_peer_group_create(world, rank, slot_bytes, n_slots, C.byref(g)))
         self._g = g
         self.world, self.rank = world, rank
 
-    @staticmethod
-    def _ck(rc: int):
-        if rc != OK:
-            msg = load().pyrope_peer_last_error()
-            raise PyropeGpuError(rc, msg.decode("utf-8", "replace") if msg else "")
-
     def handle(self) -> bytes:
         buf = C.create_string_buffer(64)
-        self._ck(load().pyrope_peer_group_handle(self._g, buf))
+        check(load().pyrope_peer_group_handle(self._g, buf))
         return buf.raw
 
     def open(self, handles: bytes):
         assert len(handles) == 64 * self.world
-        self._ck(load().pyrope_peer_group_open(self._g, C.create_string_buffer(handles, len(handles))))
+        check(load().pyrope_peer_group_open(self._g, C.create_string_buffer(handles, len(handles))))
 
     def buffer(self) -> int:
         out = vp()
-        self._ck(load().pyrope_peer_group_buffer(self._g, C.byref(out)))
+        check(load().pyrope_peer_group_buffer(self._g, C.byref(out)))
         return out.value
 
     def attach(self, buffers):
         arr = (vp * self.world)(*[vp(int(b)) if b else vp() for b in buffers])
-        self._ck(load().pyrope_peer_group_attach(self._g, arr))
+        check(load().pyrope_peer_group_attach(self._g, arr))
 
     def allgather(self, slot: int, src_ptr: int, bytes_per_rank: int, stream: int = 0) -> int:
         """Enqueue the exchange on `stream`; returns the device address of [world][bytes_per_rank]."""
         out = vp()
-        self._ck(load().pyrope_peer_allgather_device(self._g, slot, vp(src_ptr), bytes_per_rank, C.byref(out), vp(stream)))
+        check(load().pyrope_peer_allgather_device(self._g, slot, vp(src_ptr), bytes_per_rank, C.byref(out), vp(stream)))
         return out.value
 
     def close(self):
@@ -455,15 +449,9 @@ class ShardedIndex:
                  devices=None):
         s = vp()
         dv = _np(devices, np.int32) if devices is not None else None
-        self._ck(load().pyrope_sharded_create(n_devices, dv.ctypes.data_as(i32p) if dv is not None else None, kind, dim,
-                                              metric, nlist, m, k, C.byref(s)))
+        check(load().pyrope_sharded_create(n_devices, dv.ctypes.data_as(i32p) if dv is not None else None, kind, dim,
+                                          metric, nlist, m, k, C.byref(s)))
         self._s, self.n, self.kind, self.dim, self.metric, self.nlist, self.m, self.k = s, n_devices, kind, dim, metric, nlist, m, k
-
-    @staticmethod
-    def _ck(rc):
-        if rc != OK:
-            msg = load().pyrope_sharded_last_error()
-            raise PyropeGpuError(rc, msg.decode("utf-8", "replace") if msg else "")
 
     def close(self):
         if getattr(self, "_s", None):
@@ -475,22 +463,22 @@ class ShardedIndex:
     def shard(self, i: int):
         """(borrowed GpuIndex view of shard i, its CUDA device ordinal)"""
         h, dev = vp(), C.c_int32(0)
-        self._ck(load().pyrope_sharded_shard(self._s, i, C.byref(h), C.byref(dev)))
+        check(load().pyrope_sharded_shard(self._s, i, C.byref(h), C.byref(dev)))
         g = _BorrowedIndex.__new__(_BorrowedIndex)
         g._h, g.kind, g.dim, g.metric, g.nlist, g.m, g.k = h, self.kind, self.dim, self.metric, self.nlist, self.m, self.k
         g._owner = self  # keep the sharded object alive while the view is in use
         return g, dev.value
 
     def note_rows(self, total: int):
-        self._ck(load().pyrope_sharded_note_rows(self._s, total))
+        check(load().pyrope_sharded_note_rows(self._s, total))
 
     def set_train_params(self, max_train_rows=0, max_iter=0):
-        self._ck(load().pyrope_sharded_set_train_params(self._s, max_train_rows, max_iter))
+        check(load().pyrope_sharded_set_train_params(self._s, max_train_rows, max_iter))
 
     def set_codebooks(self, centroids, pq_codebooks=None):
         c = _np(centroids, np.float32)
         cb = _np(pq_codebooks, np.float32) if pq_codebooks is not None else None
-        self._ck(load().pyrope_sharded_set_codebooks(self._s, c.shape[0], _p(c), _p(cb)))
+        check(load().pyrope_sharded_set_codebooks(self._s, c.shape[0], _p(c), _p(cb)))
 
     def add(self, X, labels=None) -> int:
         X = _np(X, np.float32)
@@ -500,65 +488,65 @@ class ShardedIndex:
             raise PyropeGpuError(ERR_DIMENSION, "Vector dimension mismatch")
         lab = _np(labels, np.int64) if labels is not None else None
         first = C.c_int64(-1)
-        self._ck(load().pyrope_sharded_add_batch(self._s, X.shape[0], _p(X), _p(lab), C.byref(first)))
+        check(load().pyrope_sharded_add_batch(self._s, X.shape[0], _p(X), _p(lab), C.byref(first)))
         return first.value
 
     def delete_row(self, row: int) -> bool:
         rc = load().pyrope_sharded_delete_row(self._s, row)
         if rc == ERR_NOT_FOUND:
             return False
-        self._ck(rc)
+        check(rc)
         return True
 
     def update_row(self, row: int, x):
         x = _np(x, np.float32).reshape(-1)
         if x.size != self.dim:
             raise PyropeGpuError(ERR_DIMENSION, "Vector dimension mismatch")
-        self._ck(load().pyrope_sharded_update_row(self._s, row, _p(x)))
+        check(load().pyrope_sharded_update_row(self._s, row, _p(x)))
 
     def shadow_row(self, row: int, shadowed=True):
-        self._ck(load().pyrope_sharded_shadow_row(self._s, row, 1 if shadowed else 0))
+        check(load().pyrope_sharded_shadow_row(self._s, row, 1 if shadowed else 0))
 
     def set_labels(self, labels_by_row):
         lab = _np(labels_by_row, np.int64)
-        self._ck(load().pyrope_sharded_set_labels(self._s, lab.size, _p(lab)))
+        check(load().pyrope_sharded_set_labels(self._s, lab.size, _p(lab)))
 
     def build(self):
-        self._ck(load().pyrope_sharded_build(self._s))
+        check(load().pyrope_sharded_build(self._s))
 
     def extend(self):
         """pyrope_sharded_extend: every shard appends the buffer to the lists it owns, all or nothing."""
-        self._ck(load().pyrope_sharded_extend(self._s))
+        check(load().pyrope_sharded_extend(self._s))
 
     def is_built(self) -> bool:
         out = C.c_int32(0)
-        self._ck(load().pyrope_sharded_is_built(self._s, C.byref(out)))
+        check(load().pyrope_sharded_is_built(self._s, C.byref(out)))
         return bool(out.value)
 
     def centroids(self):
         n = C.c_int32(0)
-        self._ck(load().pyrope_sharded_get_centroids(self._s, None, C.byref(n)))
+        check(load().pyrope_sharded_get_centroids(self._s, None, C.byref(n)))
         if n.value == 0:
             return None
         out = np.zeros((n.value, self.dim), np.float32)
-        self._ck(load().pyrope_sharded_get_centroids(self._s, _p(out), C.byref(n)))
+        check(load().pyrope_sharded_get_centroids(self._s, _p(out), C.byref(n)))
         return out
 
     def codebooks(self):
         cb = np.zeros((self.m, self.k, self.dim // self.m), np.float32)
         ks = np.zeros(self.m, np.int32)
-        self._ck(load().pyrope_sharded_get_codebooks(self._s, _p(cb), _p(ks)))
+        check(load().pyrope_sharded_get_codebooks(self._s, _p(cb), _p(ks)))
         return cb, ks
 
     def snapshot(self, path: str):
-        self._ck(load().pyrope_sharded_snapshot(self._s, str(path).encode()))
+        check(load().pyrope_sharded_snapshot(self._s, str(path).encode()))
 
     def load(self, path: str):
-        self._ck(load().pyrope_sharded_load(self._s, str(path).encode()))
+        check(load().pyrope_sharded_load(self._s, str(path).encode()))
 
     def stats(self) -> int:
         out = C.c_int64(0)
-        self._ck(load().pyrope_sharded_stats(self._s, C.byref(out)))
+        check(load().pyrope_sharded_stats(self._s, C.byref(out)))
         return out.value
 
     def search(self, Q, topk: int, max_scans: int = -1, nprobe: int = -1):
@@ -567,16 +555,16 @@ class ShardedIndex:
             Q = Q[None, :]
         nq, kk = Q.shape[0], max(topk, 1)
         scores, rows, counts = np.zeros((nq, kk), np.float32), np.full((nq, kk), -1, np.int64), np.zeros(nq, np.int32)
-        self._ck(load().pyrope_sharded_search_batch(self._s, nq, _p(Q), topk, max_scans, nprobe, _p(scores), _p(rows), _p(counts)))
+        check(load().pyrope_sharded_search_batch(self._s, nq, _p(Q), topk, max_scans, nprobe, _p(scores), _p(rows), _p(counts)))
         return scores, rows, counts
 
     def search_device(self, q_ptr: int, nq: int, topk: int, scores_ptr: int, rows_ptr: int, counts_ptr: int, nprobe: int = -1):
-        self._ck(load().pyrope_sharded_search_batch_device(self._s, nq, vp(q_ptr), topk, -1, nprobe, vp(scores_ptr), vp(rows_ptr),
-                                                           vp(counts_ptr)))
+        check(load().pyrope_sharded_search_batch_device(self._s, nq, vp(q_ptr), topk, -1, nprobe, vp(scores_ptr), vp(rows_ptr),
+                                                       vp(counts_ptr)))
 
     def last_search_ms(self) -> float:
         out = C.c_float(0)
-        self._ck(load().pyrope_sharded_last_search_ms(self._s, C.byref(out)))
+        check(load().pyrope_sharded_last_search_ms(self._s, C.byref(out)))
         return out.value
 
 
@@ -600,17 +588,14 @@ class Batcher:
             rc = L.pyrope_batcher_create_delta(target, max_batch, max_wait_us, C.byref(b))
         else:
             raise TypeError(f"cannot batch searches of {type(target).__name__}")
-        if rc:
-            raise PyropeGpuError(rc, (L.pyrope_batcher_last_error() or b"").decode("utf-8", "replace"))
+        check(rc)
         self._b, self._index = b, target
 
     def search(self, q, topk: int, max_scans: int = -1, nprobe: int = -1):
         q = _np(q, np.float32).reshape(-1)
         kk = max(topk, 1)
         scores, rows, cnt = np.zeros(kk, np.float32), np.full(kk, -1, np.int64), C.c_int32(0)
-        rc = load().pyrope_batcher_search(self._b, _p(q), topk, max_scans, nprobe, _p(scores), _p(rows), C.byref(cnt))
-        if rc:
-            raise PyropeGpuError(rc, (load().pyrope_batcher_last_error() or b"").decode())
+        check(load().pyrope_batcher_search(self._b, _p(q), topk, max_scans, nprobe, _p(scores), _p(rows), C.byref(cnt)))
         return scores[:cnt.value], rows[:cnt.value]
 
     def stats(self):

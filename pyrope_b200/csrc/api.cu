@@ -29,9 +29,7 @@
 
 using namespace pyrope;
 
-namespace {
-
-thread_local std::string g_err;
+static thread_local std::string g_err;  // the library's error message, one per thread (internal.h)
 
 int fail(int code, const char* fmt, ...) {
     char buf[512];
@@ -43,19 +41,7 @@ int fail(int code, const char* fmt, ...) {
     return code;
 }
 
-#define CK(expr)                                                                                   \
-    do {                                                                                           \
-        cudaError_t _e = (expr);                                                                   \
-        if (_e != cudaSuccess)                                                                     \
-            return fail(_e == cudaErrorMemoryAllocation ? PYROPE_ERR_OOM : PYROPE_ERR_CUDA,        \
-                        "CUDA error %s at %s:%d: %s", cudaGetErrorName(_e), __FILE__, __LINE__,    \
-                        cudaGetErrorString(_e));                                                   \
-    } while (0)
-#define TRY(expr)                 \
-    do {                          \
-        int _r = (expr);          \
-        if (_r != PYROPE_OK) return _r; \
-    } while (0)
+namespace {
 
 int g_num_sms = 148;
 bool g_inited = false;
@@ -1516,6 +1502,12 @@ int validate_search(Index* h, int64_t nq, const float* Q, int topk) {
 extern "C" {
 
 const char* pyrope_last_error(void) { return g_err.c_str(); }
+// kept for shims that bind the per-module readers: every module reports through the one channel
+const char* pyrope_sharded_last_error(void) { return g_err.c_str(); }
+const char* pyrope_peer_last_error(void) { return g_err.c_str(); }
+const char* pyrope_batcher_last_error(void) { return g_err.c_str(); }
+const char* pyrope_vindex_last_error(void) { return g_err.c_str(); }
+const char* pyrope_formats_last_error(void) { return g_err.c_str(); }
 int pyrope_version(void) { return 100; }
 
 int pyrope_gpu_device_count(int* out) {
@@ -2442,12 +2434,6 @@ struct pyrope_delta {
 
 namespace {
 
-// an error raised by csrc/sharded.cu: keep its code, copy its message
-int spass(int rc) {
-    if (rc != PYROPE_OK) g_err = pyrope_sharded_last_error();
-    return rc;
-}
-
 // DeltaVectorIndex.Search:76-122 for nq queries: head top-k, tail top-k (same options, :85,88), merge by id with
 // the head's copy winning, descending, Take(topK) — one stream, no host round trip between the three stages.
 // d_kq (nullable, device [nq], every entry <= topk): query i asked for d_kq[i].  Both sides still run once at topk, and
@@ -2475,10 +2461,10 @@ int delta_search_device(pyrope_delta* d, int64_t nq, const float* dQ, int topk, 
         // with the tail's (k+1)-th.  An IVF_PQ tail ignores MaxScans (IvfPqVectorIndex.cs), an IVF_FLAT tail over
         // several devices refuses it (UNSUPPORTED, as pyrope_sharded_search_batch does).
         Index* t0 = nullptr;
-        TRY(spass(pyrope_sharded_shard(d->stail, 0, &t0, nullptr)));
-        TRY(spass(pyrope_internal_sharded_search_device(d->stail, nq, dQ, topk, t0->kind == PYROPE_IVF_PQ ? -1 : max_scans,
-                                                        nprobe, d->ps.as<float>() + per, d->pl.as<int64_t>() + per,
-                                                        d->pc.as<int32_t>() + nq, d->q_ready)));
+        TRY(pyrope_sharded_shard(d->stail, 0, &t0, nullptr));
+        TRY(pyrope_internal_sharded_search_device(d->stail, nq, dQ, topk, t0->kind == PYROPE_IVF_PQ ? -1 : max_scans,
+                                                  nprobe, d->ps.as<float>() + per, d->pl.as<int64_t>() + per,
+                                                  d->pc.as<int32_t>() + nq, d->q_ready));
     } else {
         std::lock_guard<std::mutex> g(tl->mu);
         if (tl->kind == PYROPE_IVF_FLAT && max_scans >= 0 && tl->lists.ndead > 0) TRY(compact_lists(tl));
@@ -2533,8 +2519,8 @@ int pyrope_delta_create_sharded(pyrope_index* head, pyrope_sharded* tail, pyrope
     if (!head || !tail) return fail(PYROPE_ERR_INVALID_ARG, "index handle is null");
     Index* t0 = nullptr;
     int dev0 = -1, n = 0;
-    TRY(spass(pyrope_sharded_shard(tail, 0, &t0, &dev0)));
-    TRY(spass(pyrope_sharded_device_count(tail, &n)));
+    TRY(pyrope_sharded_shard(tail, 0, &t0, &dev0));
+    TRY(pyrope_sharded_device_count(tail, &n));
     if (head == t0) return fail(PYROPE_ERR_INVALID_ARG, "Head and Tail must be different indexes");
     if (head->dim != t0->dim) return fail(PYROPE_ERR_INVALID_ARG, "Head and Tail dimensions must match");
     if (head->metric != t0->metric) return fail(PYROPE_ERR_INVALID_ARG, "Head and Tail metrics must match");
@@ -2797,8 +2783,8 @@ int delta_compact_impl(pyrope_delta* d, int64_t* moved_out, int64_t* tail_rows_o
             DevBuf mx, ml;
             std::vector<int64_t> mlab;
             TRY(gather_head_rows(hd, n, mx, ml, mlab, hd->stream));
-            TRY(spass(pyrope_internal_sharded_absorb(d->stail, n, mx.as<float>(), ml.as<int64_t>(), hd->device, mlab.data(),
-                                                     tail_rows_out)));
+            TRY(pyrope_internal_sharded_absorb(d->stail, n, mx.as<float>(), ml.as<int64_t>(), hd->device, mlab.data(),
+                                               tail_rows_out));
         }
     } else {
         Index* tl = d->tail;
@@ -2823,7 +2809,7 @@ int delta_compact_impl(pyrope_delta* d, int64_t* moved_out, int64_t* tail_rows_o
     }
     // 4. _head.Build() is a no-op for FLAT; _tail.Build() (:151-152)
     if (!do_build) return PYROPE_OK;
-    if (d->stail) return spass(extend ? pyrope_sharded_extend(d->stail) : pyrope_sharded_build(d->stail));
+    if (d->stail) return extend ? pyrope_sharded_extend(d->stail) : pyrope_sharded_build(d->stail);
     Index* tl = d->tail;
     std::lock_guard<std::mutex> gt(tl->mu);
     Staged S(*tl);
@@ -2869,7 +2855,7 @@ int pyrope_delta_stats(pyrope_delta* d, int64_t* count_out) {
     Index* hd = d->head;
     if (d->stail) {
         int64_t t = 0;
-        TRY(spass(pyrope_sharded_stats(d->stail, &t)));
+        TRY(pyrope_sharded_stats(d->stail, &t));
         *count_out = hd->seg.live + t;
         return PYROPE_OK;
     }
@@ -2883,7 +2869,7 @@ int pyrope_delta_snapshot(pyrope_delta* d, const char* path) {
     if (!path || !*path) return fail(PYROPE_ERR_INVALID_ARG, "Path cannot be empty.");
     const std::string base(path);
     TRY(pyrope_index_snapshot(d->head, (base + ".head").c_str()));
-    if (d->stail) TRY(spass(pyrope_sharded_snapshot(d->stail, (base + ".tail").c_str())));
+    if (d->stail) TRY(pyrope_sharded_snapshot(d->stail, (base + ".tail").c_str()));
     else TRY(pyrope_index_snapshot(d->tail, (base + ".tail").c_str()));
     const std::string tmp = base + ".tmp";
     FILE* f = fopen(tmp.c_str(), "wb");
@@ -2905,7 +2891,7 @@ int pyrope_delta_load(pyrope_delta* d, const char* path) {
         FILE* f = fopen(p.c_str(), "rb");
         if (!f) continue;
         fclose(f);
-        if (side == 1 && d->stail) TRY(spass(pyrope_sharded_load(d->stail, p.c_str())));
+        if (side == 1 && d->stail) TRY(pyrope_sharded_load(d->stail, p.c_str()));
         else TRY(pyrope_index_load(side == 0 ? d->head : d->tail, p.c_str()));
     }
     return PYROPE_OK;

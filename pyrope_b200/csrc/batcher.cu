@@ -18,7 +18,6 @@
 #include <algorithm>
 #include <chrono>
 #include <condition_variable>
-#include <cstdio>
 #include <cstring>
 #include <deque>
 #include <mutex>
@@ -48,13 +47,6 @@ struct Request {
     std::chrono::steady_clock::time_point t_in;
 };
 
-thread_local std::string g_berr;
-
-int bfail(int code, const char* msg) {
-    g_berr = msg;
-    return code;
-}
-
 }  // namespace
 
 struct pyrope_batcher {
@@ -76,29 +68,20 @@ struct pyrope_batcher {
         return std::min(c, max_topk);
     }
 
-    // one batched search; outputs have stride max(topks); on failure err holds the raising layer's message
+    // one batched search; outputs have stride max(topks)
     int search(int64_t nb, const float* Q, const int32_t* topks, int kmax, int64_t max_scans, int nprobe, float* S,
-               int64_t* R, int32_t* C, std::string& err) {
-        int rc = PYROPE_OK;
+               int64_t* R, int32_t* C) {
         switch (target) {
             case kIndex:
-                rc = pyrope_index_search_batch((pyrope_index*)handle, nb, Q, kmax, max_scans, nprobe, S, R, C);
-                if (rc) err = pyrope_last_error();
-                break;
+                return pyrope_index_search_batch((pyrope_index*)handle, nb, Q, kmax, max_scans, nprobe, S, R, C);
             case kSharded:
-                rc = pyrope_sharded_search_batch((pyrope_sharded*)handle, nb, Q, kmax, max_scans, nprobe, S, R, C);
-                if (rc) err = pyrope_sharded_last_error();
-                break;
+                return pyrope_sharded_search_batch((pyrope_sharded*)handle, nb, Q, kmax, max_scans, nprobe, S, R, C);
             case kDelta:
-                rc = pyrope_delta_search_batch_topk((pyrope_delta*)handle, nb, Q, topks, max_scans, nprobe, S, R, C);
-                if (rc) err = pyrope_last_error();
-                break;
+                return pyrope_delta_search_batch_topk((pyrope_delta*)handle, nb, Q, topks, max_scans, nprobe, S, R, C);
             case kVindex:
-                rc = pyrope_internal_vindex_search_topk((pyrope_vindex*)handle, nb, Q, topks, max_scans, nprobe, S, R, C);
-                if (rc) err = pyrope_vindex_last_error();
-                break;
+                return pyrope_internal_vindex_search_topk((pyrope_vindex*)handle, nb, Q, topks, max_scans, nprobe, S, R, C);
         }
-        return rc;
+        return PYROPE_OK;
     }
 
     void run() {
@@ -141,8 +124,9 @@ struct pyrope_batcher {
             R.assign(nb * kk, -1);
             C.assign(nb, 0);
             for (size_t i = 0; i < nb; ++i) memcpy(&Q[i * (size_t)dim], batch[i]->query, sizeof(float) * (size_t)dim);
-            std::string err;
-            const int rc = search((int64_t)nb, Q.data(), K.data(), kmax, max_scans, nprobe, S.data(), R.data(), C.data(), err);
+            const int rc = search((int64_t)nb, Q.data(), K.data(), kmax, max_scans, nprobe, S.data(), R.data(), C.data());
+            // the message is on this thread: every caller takes a copy back to its own
+            const std::string err = rc ? pyrope_last_error() : "";
             for (size_t i = 0; i < nb; ++i) {
                 Request* r = batch[i];
                 r->status = rc;
@@ -167,7 +151,7 @@ namespace {
 int start(Target t, void* handle, int dim, int max_topk, bool nonpos_empty, int max_batch, int max_wait_us,
           pyrope_batcher** out) {
     pyrope_batcher* b = new (std::nothrow) pyrope_batcher();
-    if (!b) return bfail(PYROPE_ERR_OOM, "out of host memory");
+    if (!b) return fail(PYROPE_ERR_OOM, "out of host memory");
     b->target = t;
     b->handle = handle;
     b->dim = dim;
@@ -185,40 +169,35 @@ int start(Target t, void* handle, int dim, int max_topk, bool nonpos_empty, int 
 extern "C" {
 
 int pyrope_batcher_create(pyrope_index* h, int max_batch, int max_wait_us, pyrope_batcher** out) {
-    if (!h || !out) return bfail(PYROPE_ERR_INVALID_ARG, "null argument");
+    if (!h || !out) return fail(PYROPE_ERR_INVALID_ARG, "null argument");
     int dim = 0, kind = 0;
-    int rc = pyrope_index_stats(h, nullptr, nullptr, &dim, nullptr);
-    if (!rc) rc = pyrope_internal_index_kind(h, &kind);
-    if (rc) return bfail(rc, pyrope_last_error());
+    TRY(pyrope_index_stats(h, nullptr, nullptr, &dim, nullptr));
+    TRY(pyrope_internal_index_kind(h, &kind));
     return start(kIndex, h, dim, 1024, kind != PYROPE_FLAT, max_batch, max_wait_us, out);
 }
 
 int pyrope_batcher_create_sharded(pyrope_sharded* s, int max_batch, int max_wait_us, pyrope_batcher** out) {
-    if (!s || !out) return bfail(PYROPE_ERR_INVALID_ARG, "null argument");
+    if (!s || !out) return fail(PYROPE_ERR_INVALID_ARG, "null argument");
     pyrope_index* s0 = nullptr;
     int n = 0, dim = 0, kind = 0;
-    int rc = pyrope_sharded_device_count(s, &n);
-    if (!rc) rc = pyrope_sharded_shard(s, 0, &s0, nullptr);
-    if (rc) return bfail(rc, pyrope_sharded_last_error());
-    rc = pyrope_index_stats(s0, nullptr, nullptr, &dim, nullptr);
-    if (!rc) rc = pyrope_internal_index_kind(s0, &kind);
-    if (rc) return bfail(rc, pyrope_last_error());
+    TRY(pyrope_sharded_device_count(s, &n));
+    TRY(pyrope_sharded_shard(s, 0, &s0, nullptr));
+    TRY(pyrope_index_stats(s0, nullptr, nullptr, &dim, nullptr));
+    TRY(pyrope_internal_index_kind(s0, &kind));
     return start(kSharded, s, dim, std::min(1024, 4096 / n), kind != PYROPE_FLAT, max_batch, max_wait_us, out);
 }
 
 int pyrope_batcher_create_delta(pyrope_delta* d, int max_batch, int max_wait_us, pyrope_batcher** out) {
-    if (!d || !out) return bfail(PYROPE_ERR_INVALID_ARG, "null argument");
+    if (!d || !out) return fail(PYROPE_ERR_INVALID_ARG, "null argument");
     int dim = 0, lim = 0;
-    const int rc = pyrope_internal_delta_limits(d, &dim, &lim);
-    if (rc) return bfail(rc, pyrope_last_error());
+    TRY(pyrope_internal_delta_limits(d, &dim, &lim));
     return start(kDelta, d, dim, lim, false, max_batch, max_wait_us, out);
 }
 
 int pyrope_batcher_create_vindex(pyrope_vindex* v, int max_batch, int max_wait_us, pyrope_batcher** out) {
-    if (!v || !out) return bfail(PYROPE_ERR_INVALID_ARG, "null argument");
+    if (!v || !out) return fail(PYROPE_ERR_INVALID_ARG, "null argument");
     int dim = 0, lim = 0, empty = 0;
-    const int rc = pyrope_internal_vindex_limits(v, &dim, &lim, &empty);
-    if (rc) return bfail(rc, pyrope_vindex_last_error());
+    TRY(pyrope_internal_vindex_limits(v, &dim, &lim, &empty));
     return start(kVindex, v, dim, lim, empty != 0, max_batch, max_wait_us, out);
 }
 
@@ -236,33 +215,26 @@ int pyrope_batcher_destroy(pyrope_batcher* b) {
 
 int pyrope_batcher_search(pyrope_batcher* b, const float* query, int topk, int64_t max_scans, int nprobe,
                           float* scores_out, int64_t* rows_out, int32_t* count_out) {
-    if (!b || !query || !scores_out || !rows_out || !count_out) return PYROPE_ERR_INVALID_ARG;
+    if (!b || !query || !scores_out || !rows_out || !count_out) return fail(PYROPE_ERR_INVALID_ARG, "null argument");
     *count_out = 0;
     // what the target's own search answers this caller alone, whatever the rest of the batch asks
-    if (topk <= 0) return b->nonpos_empty ? PYROPE_OK : bfail(PYROPE_ERR_OUT_OF_RANGE, "topK must be positive.");
-    if (topk > b->max_topk) {
-        char msg[96];
-        snprintf(msg, sizeof msg, "topK %d exceeds the supported maximum %d", topk, b->max_topk);
-        return bfail(PYROPE_ERR_UNSUPPORTED, msg);
-    }
+    if (topk <= 0) return b->nonpos_empty ? PYROPE_OK : fail(PYROPE_ERR_OUT_OF_RANGE, "topK must be positive.");
+    if (topk > b->max_topk) return fail(PYROPE_ERR_UNSUPPORTED, "topK %d exceeds the supported maximum %d", topk, b->max_topk);
     Request r;
     r.query = query; r.topk = topk; r.k_class = b->k_class(topk); r.max_scans = max_scans; r.nprobe = nprobe;
     r.scores = scores_out; r.rows = rows_out; r.count = count_out;
     r.t_in = std::chrono::steady_clock::now();
     std::unique_lock<std::mutex> lk(b->mu);
-    if (b->stop) return PYROPE_ERR_INVALID_STATE;
+    if (b->stop) return fail(PYROPE_ERR_INVALID_STATE, "the batcher is shutting down");
     b->queue.push_back(&r);
     b->cv_work.notify_one();
     b->cv_done.wait(lk, [&] { return r.done; });
     lk.unlock();
-    if (r.status) g_berr = r.error;
-    return r.status;
+    return r.status ? fail(r.status, "%s", r.error.c_str()) : PYROPE_OK;
 }
 
-const char* pyrope_batcher_last_error(void) { return g_berr.c_str(); }
-
 int pyrope_batcher_stats(pyrope_batcher* b, int64_t* batches_out, int64_t* queries_out) {
-    if (!b) return PYROPE_ERR_INVALID_ARG;
+    if (!b) return fail(PYROPE_ERR_INVALID_ARG, "batcher handle is null");
     std::lock_guard<std::mutex> g(b->mu);
     if (batches_out) *batches_out = b->n_batches;
     if (queries_out) *queries_out = b->n_queries;

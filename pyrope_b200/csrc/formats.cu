@@ -5,7 +5,6 @@
 //     straight into an index's device storage.
 #include <cerrno>
 #include <cmath>
-#include <cstdarg>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -13,20 +12,9 @@
 #include <vector>
 
 #include "../../include/pyrope_gpu.h"
+#include "internal.h"
 
 namespace {
-
-thread_local std::string g_ferr;
-
-int ffail(int code, const char* fmt, ...) {
-    char buf[512];
-    va_list ap;
-    va_start(ap, fmt);
-    vsnprintf(buf, sizeof buf, fmt, ap);
-    va_end(ap);
-    g_ferr = buf;
-    return code;
-}
 
 // char.IsWhiteSpace restricted to what a single UTF-8 byte can encode
 inline bool ws(unsigned char c) { return c == ' ' || (c >= 9 && c <= 13); }
@@ -174,19 +162,17 @@ bool parse_csv(const unsigned char* p, int64_t n, std::vector<float>& out) {
 
 extern "C" {
 
-const char* pyrope_formats_last_error(void) { return g_ferr.c_str(); }
-
 int pyrope_parse_vector(const uint8_t* data, int64_t len, float* out, int64_t cap, int64_t* n_out) {
     if (n_out) *n_out = 0;
-    if (!data || len <= 0) return ffail(PYROPE_ERR_INVALID_ARG, "Vector payload is empty. (Parameter 'data')");
+    if (!data || len <= 0) return fail(PYROPE_ERR_INVALID_ARG, "Vector payload is empty. (Parameter 'data')");
     std::vector<float> v;
     const int js = parse_json(data, len, v);
-    if (js < 0) return ffail(PYROPE_ERR_INVALID_ARG, "Either the JSON value is not in a supported format, or is out of bounds for a Single.");
+    if (js < 0) return fail(PYROPE_ERR_INVALID_ARG, "Either the JSON value is not in a supported format, or is out of bounds for a Single.");
     if (js == 0) {
         v.clear();
         if (!parse_csv(data, len, v)) {
             v.clear();
-            if (len % 4 != 0) return ffail(PYROPE_ERR_INVALID_ARG, "Unsupported vector format.");
+            if (len % 4 != 0) return fail(PYROPE_ERR_INVALID_ARG, "Unsupported vector format.");
             v.resize((size_t)(len / 4));  // ParseBinaryVector :93-99: the bytes ARE the floats
             memcpy(v.data(), data, (size_t)len);
         }
@@ -197,8 +183,8 @@ int pyrope_parse_vector(const uint8_t* data, int64_t len, float* out, int64_t ca
 }
 
 int pyrope_encode_vector(const float* vec, int64_t n, uint8_t* out, int64_t cap_bytes) {
-    if (!vec && n > 0) return ffail(PYROPE_ERR_INVALID_ARG, "Value cannot be null. (Parameter 'vector')");
-    if (n < 0 || cap_bytes < n * 4) return ffail(PYROPE_ERR_INVALID_ARG, "destination holds %lld bytes, %lld needed", (long long)cap_bytes, (long long)n * 4);
+    if (!vec && n > 0) return fail(PYROPE_ERR_INVALID_ARG, "Value cannot be null. (Parameter 'vector')");
+    if (n < 0 || cap_bytes < n * 4) return fail(PYROPE_ERR_INVALID_ARG, "destination holds %lld bytes, %lld needed", (long long)cap_bytes, (long long)n * 4);
     if (n > 0) memcpy(out, vec, (size_t)n * 4);  // VectorEncoding.ToLittleEndianBytes: x86-64 / aarch64 are little-endian
     return PYROPE_OK;
 }
@@ -209,10 +195,10 @@ int pyrope_fvecs_read(const char* path, int64_t limit, int64_t skip, float* out,
                       int* dim_out) {
     if (count_out) *count_out = 0;
     if (dim_out) *dim_out = 0;
-    if (!path) return ffail(PYROPE_ERR_INVALID_ARG, "Value cannot be null. (Parameter 'path')");
+    if (!path) return fail(PYROPE_ERR_INVALID_ARG, "Value cannot be null. (Parameter 'path')");
     if (limit == 0) return PYROPE_OK;
     FILE* f = fopen(path, "rb");
-    if (!f) return ffail(PYROPE_ERR_NOT_FOUND, "Could not find file '%s'.", path);
+    if (!f) return fail(PYROPE_ERR_NOT_FOUND, "Could not find file '%s'.", path);
     int64_t count = 0, seen = 0, written = 0;
     int dim0 = 0;
     int rc = PYROPE_OK;
@@ -221,11 +207,11 @@ int pyrope_fvecs_read(const char* path, int64_t limit, int64_t skip, float* out,
         if (limit > 0 && count >= limit) break;
         int32_t d = 0;
         if (fread(&d, 1, 4, f) != 4) break;  // end of file, or a torn header: ReadInt32 throws EndOfStream -> yield break
-        if (d <= 0) { rc = ffail(PYROPE_ERR_INVALID_ARG, "Invalid vector dimension %d in fvecs file.", d); break; }
+        if (d <= 0) { rc = fail(PYROPE_ERR_INVALID_ARG, "Invalid vector dimension %d in fvecs file.", d); break; }
         if (dim0 == 0) dim0 = d;
-        if (d != dim0) { rc = ffail(PYROPE_ERR_DIMENSION, "Vector dimension mismatch"); break; }
+        if (d != dim0) { rc = fail(PYROPE_ERR_DIMENSION, "Vector dimension mismatch"); break; }
         rec.resize((size_t)d);
-        if (fread(rec.data(), 4, (size_t)d, f) != (size_t)d) { rc = ffail(PYROPE_ERR_INVALID_ARG, "Truncated fvecs record."); break; }
+        if (fread(rec.data(), 4, (size_t)d, f) != (size_t)d) { rc = fail(PYROPE_ERR_INVALID_ARG, "Truncated fvecs record."); break; }
         if (seen++ < skip) continue;
         if (out && written + d <= cap_floats) {
             memcpy(out + written, rec.data(), sizeof(float) * (size_t)d);
@@ -243,32 +229,31 @@ int pyrope_fvecs_read(const char* path, int64_t limit, int64_t skip, float* out,
 // Stream an fvecs file into an index: 64 MiB batches through pyrope_index_add_batch (labels = row ordinals).
 int pyrope_index_add_fvecs(pyrope_index* h, const char* path, int64_t limit, int64_t* added_out) {
     if (added_out) *added_out = 0;
-    if (!h) return ffail(PYROPE_ERR_INVALID_ARG, "index handle is null");
-    if (!path) return ffail(PYROPE_ERR_INVALID_ARG, "Value cannot be null. (Parameter 'path')");
+    if (!h) return fail(PYROPE_ERR_INVALID_ARG, "index handle is null");
+    if (!path) return fail(PYROPE_ERR_INVALID_ARG, "Value cannot be null. (Parameter 'path')");
     if (limit == 0) return PYROPE_OK;
     int dim = 0;
-    int rc = pyrope_index_stats(h, nullptr, nullptr, &dim, nullptr);
-    if (rc != PYROPE_OK) { g_ferr = pyrope_last_error(); return rc; }
+    TRY(pyrope_index_stats(h, nullptr, nullptr, &dim, nullptr));
     FILE* f = fopen(path, "rb");
-    if (!f) return ffail(PYROPE_ERR_NOT_FOUND, "Could not find file '%s'.", path);
+    if (!f) return fail(PYROPE_ERR_NOT_FOUND, "Could not find file '%s'.", path);
     const int64_t batch_rows = std::max<int64_t>(1, ((int64_t)64 << 20) / ((int64_t)dim * 4));
     std::vector<float> buf((size_t)batch_rows * dim);
     int64_t added = 0, in_batch = 0;
     auto flush = [&]() -> int {
         if (in_batch == 0) return PYROPE_OK;
-        int r = pyrope_index_add_batch(h, in_batch, buf.data(), nullptr, nullptr);
-        if (r != PYROPE_OK) g_ferr = pyrope_last_error();
-        else added += in_batch;
+        const int r = pyrope_index_add_batch(h, in_batch, buf.data(), nullptr, nullptr);
+        if (r == PYROPE_OK) added += in_batch;
         in_batch = 0;
         return r;
     };
+    int rc = PYROPE_OK;
     for (;;) {
         if (limit > 0 && added + in_batch >= limit) break;
         int32_t d = 0;
         if (fread(&d, 1, 4, f) != 4) break;
-        if (d <= 0) { rc = ffail(PYROPE_ERR_INVALID_ARG, "Invalid vector dimension %d in fvecs file.", d); break; }
-        if (d != dim) { rc = ffail(PYROPE_ERR_DIMENSION, "Vector dimension mismatch"); break; }
-        if (fread(buf.data() + (size_t)in_batch * dim, 4, (size_t)d, f) != (size_t)d) { rc = ffail(PYROPE_ERR_INVALID_ARG, "Truncated fvecs record."); break; }
+        if (d <= 0) { rc = fail(PYROPE_ERR_INVALID_ARG, "Invalid vector dimension %d in fvecs file.", d); break; }
+        if (d != dim) { rc = fail(PYROPE_ERR_DIMENSION, "Vector dimension mismatch"); break; }
+        if (fread(buf.data() + (size_t)in_batch * dim, 4, (size_t)d, f) != (size_t)d) { rc = fail(PYROPE_ERR_INVALID_ARG, "Truncated fvecs record."); break; }
         if (++in_batch == batch_rows && (rc = flush()) != PYROPE_OK) break;
     }
     fclose(f);

@@ -5,6 +5,27 @@
 #include "../../include/pyrope_gpu.h"
 
 #ifdef __cplusplus
+// ---- api.cu: the library's one error channel.  fail() formats the message into the calling thread's slot, which every
+// pyrope_*_last_error() returns, and returns code.  A message crosses threads only where a worker's failure is handed
+// back to the caller explicitly (sharded.cu run_all, batcher.cu Request::error).
+int fail(int code, const char* fmt, ...) __attribute__((format(printf, 2, 3)));
+
+// a failing CUDA call: OOM for an allocation, CUDA otherwise, with the call site in the message
+#define CK(expr)                                                                                   \
+    do {                                                                                           \
+        cudaError_t _e = (expr);                                                                   \
+        if (_e != cudaSuccess)                                                                     \
+            return fail(_e == cudaErrorMemoryAllocation ? PYROPE_ERR_OOM : PYROPE_ERR_CUDA,        \
+                        "CUDA error %s at %s:%d: %s", cudaGetErrorName(_e), __FILE__, __LINE__,    \
+                        cudaGetErrorString(_e));                                                   \
+    } while (0)
+// a failing library call: its status and its message pass through unchanged
+#define TRY(expr)                       \
+    do {                                \
+        int _r = (expr);                \
+        if (_r != PYROPE_OK) return _r; \
+    } while (0)
+
 extern "C" {
 #endif
 

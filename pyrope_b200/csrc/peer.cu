@@ -18,35 +18,15 @@
 // same stream, before the next call, which is how a search step uses it.
 // Every rank must issue the same sequence of calls (slot, size): the epoch is a per-slot call counter.
 #include <algorithm>
-#include <cstdarg>
-#include <cstdio>
 #include <cstring>
-#include <string>
 #include <vector>
 
 #include <cuda_runtime.h>
 
 #include "../../include/pyrope_gpu.h"
+#include "internal.h"
 
 namespace {
-
-thread_local std::string g_perr;
-int pfail(int code, const char* fmt, ...) {
-    char buf[512];
-    va_list ap;
-    va_start(ap, fmt);
-    vsnprintf(buf, sizeof buf, fmt, ap);
-    va_end(ap);
-    g_perr = buf;
-    return code;
-}
-#define PCK(expr)                                                                                                   \
-    do {                                                                                                            \
-        cudaError_t _e = (expr);                                                                                    \
-        if (_e != cudaSuccess)                                                                                      \
-            return pfail(_e == cudaErrorMemoryAllocation ? PYROPE_ERR_OOM : PYROPE_ERR_CUDA, "CUDA error %s at %s:%d: %s", \
-                         cudaGetErrorName(_e), __FILE__, __LINE__, cudaGetErrorString(_e));                         \
-    } while (0)
 
 constexpr int kMaxWorld = 8;
 constexpr int kMaxSlots = 8;
@@ -96,15 +76,13 @@ struct pyrope_peer_group {
 
 extern "C" {
 
-const char* pyrope_peer_last_error(void) { return g_perr.c_str(); }
-
 int pyrope_peer_group_create(int world, int rank, size_t slot_bytes, int n_slots, pyrope_peer_group** out) {
-    if (!out) return pfail(PYROPE_ERR_INVALID_ARG, "out is null");
+    if (!out) return fail(PYROPE_ERR_INVALID_ARG, "out is null");
     *out = nullptr;
-    if (world < 2 || world > kMaxWorld || rank < 0 || rank >= world) return pfail(PYROPE_ERR_INVALID_ARG, "world must be 2..8, rank below it");
-    if (n_slots < 1 || n_slots > kMaxSlots || slot_bytes == 0) return pfail(PYROPE_ERR_INVALID_ARG, "1..8 slots of at least one byte");
+    if (world < 2 || world > kMaxWorld || rank < 0 || rank >= world) return fail(PYROPE_ERR_INVALID_ARG, "world must be 2..8, rank below it");
+    if (n_slots < 1 || n_slots > kMaxSlots || slot_bytes == 0) return fail(PYROPE_ERR_INVALID_ARG, "1..8 slots of at least one byte");
     pyrope_peer_group* g = new (std::nothrow) pyrope_peer_group();
-    if (!g) return pfail(PYROPE_ERR_OOM, "out of host memory");
+    if (!g) return fail(PYROPE_ERR_OOM, "out of host memory");
     g->world = world; g->rank = rank; g->n_slots = n_slots;
     g->slot_bytes = (slot_bytes + 255) & ~(size_t)255;
     g->total = kFlagBytes + (size_t)n_slots * 2 * world * g->slot_bytes;
@@ -116,8 +94,8 @@ int pyrope_peer_group_create(int world, int rank, size_t slot_bytes, int n_slots
         const size_t want = g->total;
         if (g->local) cudaFree(g->local);
         delete g;
-        return pfail(e == cudaErrorMemoryAllocation ? PYROPE_ERR_OOM : PYROPE_ERR_CUDA, "peer group buffer (%zu bytes): %s", want,
-                     cudaGetErrorString(e));
+        return fail(e == cudaErrorMemoryAllocation ? PYROPE_ERR_OOM : PYROPE_ERR_CUDA, "peer group buffer (%zu bytes): %s", want,
+                    cudaGetErrorString(e));
     }
     g->peers[rank] = g->local;
     *out = g;
@@ -140,23 +118,23 @@ int pyrope_peer_group_destroy(pyrope_peer_group* g) {
 }
 
 int pyrope_peer_group_handle(pyrope_peer_group* g, void* handle_out) {
-    if (!g || !handle_out) return pfail(PYROPE_ERR_INVALID_ARG, "null argument");
+    if (!g || !handle_out) return fail(PYROPE_ERR_INVALID_ARG, "null argument");
     static_assert(sizeof(cudaIpcMemHandle_t) == 64, "handle size");
     cudaIpcMemHandle_t hd;
-    PCK(cudaIpcGetMemHandle(&hd, g->local));
+    CK(cudaIpcGetMemHandle(&hd, g->local));
     memcpy(handle_out, &hd, sizeof hd);
     return PYROPE_OK;
 }
 
 int pyrope_peer_group_buffer(pyrope_peer_group* g, void** d_buffer_out) {
-    if (!g || !d_buffer_out) return pfail(PYROPE_ERR_INVALID_ARG, "null argument");
+    if (!g || !d_buffer_out) return fail(PYROPE_ERR_INVALID_ARG, "null argument");
     *d_buffer_out = g->local;
     return PYROPE_OK;
 }
 
 int pyrope_peer_group_open(pyrope_peer_group* g, const void* handles) {
-    if (!g || !handles) return pfail(PYROPE_ERR_INVALID_ARG, "null argument");
-    if (g->attached) return pfail(PYROPE_ERR_INVALID_STATE, "peers are already attached");
+    if (!g || !handles) return fail(PYROPE_ERR_INVALID_ARG, "null argument");
+    if (g->attached) return fail(PYROPE_ERR_INVALID_STATE, "peers are already attached");
     for (int r = 0; r < g->world; ++r) {
         if (r == g->rank) continue;
         cudaIpcMemHandle_t hd;
@@ -167,7 +145,7 @@ int pyrope_peer_group_open(pyrope_peer_group* g, const void* handles) {
             cudaGetLastError();
             for (int rr = 0; rr < r; ++rr)
                 if (rr != g->rank && g->peers[rr]) { cudaIpcCloseMemHandle(g->peers[rr]); g->peers[rr] = nullptr; }
-            return pfail(PYROPE_ERR_UNSUPPORTED, "cannot map the buffer of rank %d: %s", r, cudaGetErrorString(e));
+            return fail(PYROPE_ERR_UNSUPPORTED, "cannot map the buffer of rank %d: %s", r, cudaGetErrorString(e));
         }
         g->peers[r] = static_cast<unsigned char*>(p);
     }
@@ -177,11 +155,11 @@ int pyrope_peer_group_open(pyrope_peer_group* g, const void* handles) {
 }
 
 int pyrope_peer_group_attach(pyrope_peer_group* g, void* const* buffers) {
-    if (!g || !buffers) return pfail(PYROPE_ERR_INVALID_ARG, "null argument");
-    if (g->attached) return pfail(PYROPE_ERR_INVALID_STATE, "peers are already attached");
+    if (!g || !buffers) return fail(PYROPE_ERR_INVALID_ARG, "null argument");
+    if (g->attached) return fail(PYROPE_ERR_INVALID_STATE, "peers are already attached");
     for (int r = 0; r < g->world; ++r) {
         if (r == g->rank) continue;
-        if (!buffers[r]) return pfail(PYROPE_ERR_INVALID_ARG, "buffer of rank %d is null", r);
+        if (!buffers[r]) return fail(PYROPE_ERR_INVALID_ARG, "buffer of rank %d is null", r);
         g->peers[r] = static_cast<unsigned char*>(buffers[r]);
     }
     g->attached = true;
@@ -191,11 +169,11 @@ int pyrope_peer_group_attach(pyrope_peer_group* g, void* const* buffers) {
 
 int pyrope_peer_allgather_device(pyrope_peer_group* g, int slot, const void* d_src, size_t bytes_per_rank, const void** d_gathered_out,
                                  void* stream) {
-    if (!g || !d_src || !d_gathered_out) return pfail(PYROPE_ERR_INVALID_ARG, "null argument");
-    if (!g->attached) return pfail(PYROPE_ERR_INVALID_STATE, "attach or open the peers first");
-    if (slot < 0 || slot >= g->n_slots) return pfail(PYROPE_ERR_INVALID_ARG, "slot %d of %d", slot, g->n_slots);
+    if (!g || !d_src || !d_gathered_out) return fail(PYROPE_ERR_INVALID_ARG, "null argument");
+    if (!g->attached) return fail(PYROPE_ERR_INVALID_STATE, "attach or open the peers first");
+    if (slot < 0 || slot >= g->n_slots) return fail(PYROPE_ERR_INVALID_ARG, "slot %d of %d", slot, g->n_slots);
     if (bytes_per_rank == 0 || bytes_per_rank > g->slot_bytes || (bytes_per_rank & 15) || (reinterpret_cast<uintptr_t>(d_src) & 15))
-        return pfail(PYROPE_ERR_INVALID_ARG, "contribution must be 16-byte aligned, a multiple of 16 bytes and at most %zu bytes", g->slot_bytes);
+        return fail(PYROPE_ERR_INVALID_ARG, "contribution must be 16-byte aligned, a multiple of 16 bytes and at most %zu bytes", g->slot_bytes);
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     const unsigned long long epoch = g->epoch[slot] + 1;  // committed below, once both kernels are enqueued
     // [slot][parity][rank][bytes_per_rank]: the ranks' contributions are contiguous, like an all-gather's output
@@ -207,7 +185,7 @@ int pyrope_peer_allgather_device(pyrope_peer_group* g, int slot, const void* d_s
     peer_scatter_kernel<<<dim3(chunks, (unsigned)g->world), 256, 0, st>>>(pp, half + (size_t)g->rank * bytes_per_rank,
                                                                         static_cast<const uint4*>(d_src), n16);
     peer_signal_wait_kernel<<<1, 32, 0, st>>>(pp, g->world, g->rank, slot, epoch);
-    PCK(cudaGetLastError());
+    CK(cudaGetLastError());
     g->epoch[slot] = epoch;
     *d_gathered_out = g->local + half;
     return PYROPE_OK;

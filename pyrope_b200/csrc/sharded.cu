@@ -16,7 +16,6 @@
 #include <algorithm>
 #include <atomic>
 #include <condition_variable>
-#include <cstdarg>
 #include <cstdio>
 #include <cstring>
 #include <functional>
@@ -33,17 +32,6 @@
 #include "internal.h"
 
 namespace {
-
-thread_local std::string g_serr;
-int sfail(int code, const char* fmt, ...) {
-    char buf[512];
-    va_list ap;
-    va_start(ap, fmt);
-    vsnprintf(buf, sizeof buf, fmt, ap);
-    va_end(ap);
-    g_serr = buf;
-    return code;
-}
 
 // reusable barrier for the worker threads of one job
 struct HostBarrier {
@@ -134,7 +122,8 @@ void worker_main(Worker* w, int device) {
     }
 }
 
-// run fn(r) on every shard's thread, wait for all; returns the first non-zero status (with its message)
+// run fn(r) on every shard's thread, wait for all; returns the first non-zero status, with the message its fn left on
+// that shard's thread
 int run_all(S* s, const std::function<int(int)>& fn) {
     std::vector<int> rc((size_t)s->n, 0);
     std::vector<std::string> msg((size_t)s->n);
@@ -144,7 +133,7 @@ int run_all(S* s, const std::function<int(int)>& fn) {
             std::lock_guard<std::mutex> g(w->mu);
             w->job = [&, r] {
                 rc[(size_t)r] = fn(r);
-                if (rc[(size_t)r] != PYROPE_OK) msg[(size_t)r] = g_serr.empty() ? pyrope_last_error() : g_serr;
+                if (rc[(size_t)r] != PYROPE_OK) msg[(size_t)r] = pyrope_last_error();
             };
             w->has_job = true;
             w->done = false;
@@ -157,29 +146,16 @@ int run_all(S* s, const std::function<int(int)>& fn) {
         w->cv.wait(g, [&] { return w->done; });
     }
     for (int r = 0; r < s->n; ++r)
-        if (rc[(size_t)r] != PYROPE_OK) return sfail(rc[(size_t)r], "shard %d (device %d): %s", r, s->dev[(size_t)r], msg[(size_t)r].c_str());
+        if (rc[(size_t)r] != PYROPE_OK) return fail(rc[(size_t)r], "shard %d (device %d): %s", r, s->dev[(size_t)r], msg[(size_t)r].c_str());
     return PYROPE_OK;
 }
-
-#define SCK(expr)                                                                                      \
-    do {                                                                                               \
-        cudaError_t _e = (expr);                                                                       \
-        if (_e != cudaSuccess)                                                                         \
-            return sfail(_e == cudaErrorMemoryAllocation ? PYROPE_ERR_OOM : PYROPE_ERR_CUDA,           \
-                         "CUDA error %s at %s:%d: %s", cudaGetErrorName(_e), __FILE__, __LINE__, cudaGetErrorString(_e)); \
-    } while (0)
-#define STRY(expr)                                   \
-    do {                                             \
-        int _r = (expr);                             \
-        if (_r != PYROPE_OK) { g_serr = pyrope_last_error(); return _r; } \
-    } while (0)
 
 int grow(S::Buf& b, size_t need) {  // on the current device
     if (need <= b.bytes) return PYROPE_OK;
     if (b.p) cudaFree(b.p);
     b.p = nullptr;
     b.bytes = 0;
-    SCK(cudaMalloc(&b.p, need));
+    CK(cudaMalloc(&b.p, need));
     b.bytes = need;
     return PYROPE_OK;
 }
@@ -189,7 +165,7 @@ int grow_pinned(void** p, size_t* have, size_t need) {
     if (*p) cudaFreeHost(*p);
     *p = nullptr;
     *have = 0;
-    SCK(cudaMallocHost(p, need));
+    CK(cudaMallocHost(p, need));
     *have = need;
     return PYROPE_OK;
 }
@@ -215,7 +191,7 @@ int stage_consuming(S* s, int (*prepare)(pyrope_index*, void**, pyrope_internal_
     std::vector<std::vector<int64_t>> moved((size_t)s->n);
     auto prep = [&](int r, void** staged) -> int {
         pyrope_internal_staged_info info{};
-        STRY(prepare(s->shard[(size_t)r], staged, &info));
+        TRY(prepare(s->shard[(size_t)r], staged, &info));
         moved[(size_t)r].assign(info.moved, info.moved + info.n_moved);
         std::sort(moved[(size_t)r].begin(), moved[(size_t)r].end());
         return PYROPE_OK;
@@ -223,8 +199,8 @@ int stage_consuming(S* s, int (*prepare)(pyrope_index*, void**, pyrope_internal_
     auto same = [&]() -> int {
         for (size_t r = 1; r < moved.size(); ++r)
             if (moved[r] != moved[0])
-                return sfail(PYROPE_ERR_INVALID_STATE, "shard %zu and shard 0 would move different buffered rows (%zu vs %zu): the buffer replicas diverged",
-                             r, moved[r].size(), moved[0].size());
+                return fail(PYROPE_ERR_INVALID_STATE, "shard %zu and shard 0 would move different buffered rows (%zu vs %zu): the buffer replicas diverged",
+                            r, moved[r].size(), moved[0].size());
         return PYROPE_OK;
     };
     return stage_all(s, prep, same);
@@ -234,23 +210,21 @@ int stage_consuming(S* s, int (*prepare)(pyrope_index*, void**, pyrope_internal_
 
 extern "C" {
 
-const char* pyrope_sharded_last_error(void) { return g_serr.c_str(); }
-
 int pyrope_sharded_create(int n_devices, const int* devices, int kind, int dim, int metric, int nlist, int pq_m, int pq_k,
                           pyrope_sharded** out) {
-    if (!out) return sfail(PYROPE_ERR_INVALID_ARG, "out is null");
+    if (!out) return fail(PYROPE_ERR_INVALID_ARG, "out is null");
     *out = nullptr;
     int have = 0;
-    SCK(cudaGetDeviceCount(&have));
-    if (n_devices < 1 || n_devices > 8) return sfail(PYROPE_ERR_INVALID_ARG, "n_devices must be 1..8");
-    if (n_devices > have) return sfail(PYROPE_ERR_INVALID_ARG, "%d devices requested, %d visible", n_devices, have);
+    CK(cudaGetDeviceCount(&have));
+    if (n_devices < 1 || n_devices > 8) return fail(PYROPE_ERR_INVALID_ARG, "n_devices must be 1..8");
+    if (n_devices > have) return fail(PYROPE_ERR_INVALID_ARG, "%d devices requested, %d visible", n_devices, have);
     S* s = new (std::nothrow) S();
-    if (!s) return sfail(PYROPE_ERR_OOM, "out of host memory");
+    if (!s) return fail(PYROPE_ERR_OOM, "out of host memory");
     s->n = n_devices; s->kind = kind; s->dim = dim; s->metric = metric; s->nlist = nlist; s->m = pq_m; s->k = pq_k;
     s->bar.n = n_devices;
     for (int r = 0; r < n_devices; ++r) {
         const int d = devices ? devices[r] : r;
-        if (d < 0 || d >= have) { delete s; return sfail(PYROPE_ERR_INVALID_ARG, "device %d does not exist", d); }
+        if (d < 0 || d >= have) { delete s; return fail(PYROPE_ERR_INVALID_ARG, "device %d does not exist", d); }
         s->dev.push_back(d);
     }
     const size_t N = (size_t)n_devices;
@@ -264,23 +238,23 @@ int pyrope_sharded_create(int n_devices, const int* devices, int kind, int dim, 
         s->workers.push_back(w);
     }
     int rc = run_all(s, [&](int r) -> int {
-        STRY(pyrope_gpu_init(s->dev[(size_t)r]));
+        TRY(pyrope_gpu_init(s->dev[(size_t)r]));
         for (int p = 0; p < s->n; ++p) {  // NVLink peer access to every other shard's device
             if (p == r) continue;
             int can = 0;
-            SCK(cudaDeviceCanAccessPeer(&can, s->dev[(size_t)r], s->dev[(size_t)p]));
-            if (!can) return sfail(PYROPE_ERR_UNSUPPORTED, "device %d cannot access device %d", s->dev[(size_t)r], s->dev[(size_t)p]);
+            CK(cudaDeviceCanAccessPeer(&can, s->dev[(size_t)r], s->dev[(size_t)p]));
+            if (!can) return fail(PYROPE_ERR_UNSUPPORTED, "device %d cannot access device %d", s->dev[(size_t)r], s->dev[(size_t)p]);
             cudaError_t e = cudaDeviceEnablePeerAccess(s->dev[(size_t)p], 0);
             if (e != cudaSuccess && e != cudaErrorPeerAccessAlreadyEnabled)
-                return sfail(PYROPE_ERR_CUDA, "cudaDeviceEnablePeerAccess: %s", cudaGetErrorString(e));
+                return fail(PYROPE_ERR_CUDA, "cudaDeviceEnablePeerAccess: %s", cudaGetErrorString(e));
             cudaGetLastError();
         }
-        STRY(pyrope_index_create(kind, dim, metric, nlist, pq_m, pq_k, &s->shard[(size_t)r]));
-        if (kind != PYROPE_FLAT && s->n > 1) STRY(pyrope_index_set_shard(s->shard[(size_t)r], r, s->n));
-        SCK(cudaStreamCreateWithFlags(&s->st[(size_t)r], cudaStreamNonBlocking));
-        SCK(cudaEventCreateWithFlags(&s->ev_probe[(size_t)r], cudaEventDisableTiming));
-        SCK(cudaEventCreateWithFlags(&s->ev_res[(size_t)r], cudaEventDisableTiming));
-        if (r == 0) { SCK(cudaEventCreate(&s->ev_t0)); SCK(cudaEventCreate(&s->ev_t1)); }
+        TRY(pyrope_index_create(kind, dim, metric, nlist, pq_m, pq_k, &s->shard[(size_t)r]));
+        if (kind != PYROPE_FLAT && s->n > 1) TRY(pyrope_index_set_shard(s->shard[(size_t)r], r, s->n));
+        CK(cudaStreamCreateWithFlags(&s->st[(size_t)r], cudaStreamNonBlocking));
+        CK(cudaEventCreateWithFlags(&s->ev_probe[(size_t)r], cudaEventDisableTiming));
+        CK(cudaEventCreateWithFlags(&s->ev_res[(size_t)r], cudaEventDisableTiming));
+        if (r == 0) { CK(cudaEventCreate(&s->ev_t0)); CK(cudaEventCreate(&s->ev_t1)); }
         return PYROPE_OK;
     });
     if (rc != PYROPE_OK) { pyrope_sharded_destroy(s); return rc; }
@@ -325,43 +299,43 @@ int pyrope_sharded_destroy(pyrope_sharded* s) {
 }
 
 int pyrope_sharded_device_count(pyrope_sharded* s, int* out) {
-    if (!s || !out) return sfail(PYROPE_ERR_INVALID_ARG, "null argument");
+    if (!s || !out) return fail(PYROPE_ERR_INVALID_ARG, "null argument");
     *out = s->n;
     return PYROPE_OK;
 }
 
 int pyrope_sharded_shard(pyrope_sharded* s, int i, pyrope_index** index_out, int* device_out) {
-    if (!s || i < 0 || i >= s->n) return sfail(PYROPE_ERR_INVALID_ARG, "no such shard");
+    if (!s || i < 0 || i >= s->n) return fail(PYROPE_ERR_INVALID_ARG, "no such shard");
     if (index_out) *index_out = s->shard[(size_t)i];
     if (device_out) *device_out = s->dev[(size_t)i];
     return PYROPE_OK;
 }
 
 int pyrope_sharded_set_train_params(pyrope_sharded* s, int64_t max_train_rows, int max_iter) {
-    if (!s) return sfail(PYROPE_ERR_INVALID_ARG, "handle is null");
-    for (pyrope_index* h : s->shard) STRY(pyrope_index_set_train_params(h, max_train_rows, max_iter));
+    if (!s) return fail(PYROPE_ERR_INVALID_ARG, "handle is null");
+    for (pyrope_index* h : s->shard) TRY(pyrope_index_set_train_params(h, max_train_rows, max_iter));
     return PYROPE_OK;
 }
 
 int pyrope_sharded_set_codebooks(pyrope_sharded* s, int n_centroids, const float* centroids, const float* pq_codebooks) {
-    if (!s) return sfail(PYROPE_ERR_INVALID_ARG, "handle is null");
+    if (!s) return fail(PYROPE_ERR_INVALID_ARG, "handle is null");
     std::lock_guard<std::mutex> g(s->mu);
     return run_all(s, [&](int r) -> int {
-        STRY(pyrope_index_set_codebooks(s->shard[(size_t)r], n_centroids, centroids, pq_codebooks));
+        TRY(pyrope_index_set_codebooks(s->shard[(size_t)r], n_centroids, centroids, pq_codebooks));
         return PYROPE_OK;
     });
 }
 
 // Rows added through the shard handles directly (device-resident feeds): tell the sharded object how many global rows exist.
 int pyrope_sharded_note_rows(pyrope_sharded* s, int64_t total_rows) {
-    if (!s || total_rows < 0) return sfail(PYROPE_ERR_INVALID_ARG, "bad argument");
+    if (!s || total_rows < 0) return fail(PYROPE_ERR_INVALID_ARG, "bad argument");
     s->next_row = total_rows;
     return PYROPE_OK;
 }
 
 int pyrope_sharded_add_batch(pyrope_sharded* s, int64_t n, const float* X, const int64_t* labels, int64_t* first_row_out) {
-    if (!s) return sfail(PYROPE_ERR_INVALID_ARG, "handle is null");
-    if (n < 0 || (n > 0 && !X)) return sfail(PYROPE_ERR_INVALID_ARG, "vector is null");
+    if (!s) return fail(PYROPE_ERR_INVALID_ARG, "handle is null");
+    if (n < 0 || (n > 0 && !X)) return fail(PYROPE_ERR_INVALID_ARG, "vector is null");
     std::lock_guard<std::mutex> g(s->mu);
     const int64_t first = s->next_row;
     if (first_row_out) *first_row_out = first;
@@ -370,8 +344,8 @@ int pyrope_sharded_add_batch(pyrope_sharded* s, int64_t n, const float* X, const
         // every shard sees every row (same row ordinals everywhere); Build keeps the lists a shard owns
         int rc = run_all(s, [&](int r) -> int {
             int64_t fr = -1;
-            STRY(pyrope_index_add_batch(s->shard[(size_t)r], n, X, labels, &fr));
-            if (fr != first) return sfail(PYROPE_ERR_INVALID_STATE, "shard %d row ordinals diverged (%lld vs %lld)", r, (long long)fr, (long long)first);
+            TRY(pyrope_index_add_batch(s->shard[(size_t)r], n, X, labels, &fr));
+            if (fr != first) return fail(PYROPE_ERR_INVALID_STATE, "shard %d row ordinals diverged (%lld vs %lld)", r, (long long)fr, (long long)first);
             return PYROPE_OK;
         });
         if (rc == PYROPE_OK) s->next_row += n;
@@ -387,7 +361,7 @@ int pyrope_sharded_add_batch(pyrope_sharded* s, int64_t n, const float* X, const
     std::vector<int64_t> local0((size_t)s->n, -1);
     int rc = run_all(s, [&](int r) -> int {
         const int64_t lo = n * r / s->n, hi = n * (r + 1) / s->n;
-        if (hi > lo) STRY(pyrope_index_add_batch(s->shard[(size_t)r], hi - lo, X + (size_t)lo * s->dim, labels + lo, &local0[(size_t)r]));
+        if (hi > lo) TRY(pyrope_index_add_batch(s->shard[(size_t)r], hi - lo, X + (size_t)lo * s->dim, labels + lo, &local0[(size_t)r]));
         return PYROPE_OK;
     });
     if (rc != PYROPE_OK) return rc;
@@ -403,32 +377,33 @@ int pyrope_sharded_add_batch(pyrope_sharded* s, int64_t n, const float* X, const
 }
 
 int pyrope_sharded_delete_row(pyrope_sharded* s, int64_t row) {
-    if (!s) return sfail(PYROPE_ERR_INVALID_ARG, "handle is null");
+    if (!s) return fail(PYROPE_ERR_INVALID_ARG, "handle is null");
     std::lock_guard<std::mutex> g(s->mu);
-    if (row < 0 || row >= s->next_row) return sfail(PYROPE_ERR_NOT_FOUND, "row %lld not found", (long long)row);
+    if (row < 0 || row >= s->next_row) return fail(PYROPE_ERR_NOT_FOUND, "row %lld not found", (long long)row);
     if (s->kind == PYROPE_FLAT) {
         for (const S::Seg& sg : s->segs)
             if (row >= sg.g0 && row < sg.g0 + sg.n) {
-                int rc = PYROPE_OK;
-                run_all(s, [&](int r) -> int {
-                    if (r == sg.shard) rc = pyrope_index_delete_row(s->shard[(size_t)r], sg.local0 + (row - sg.g0));
-                    return PYROPE_OK;
+                const int rc = run_all(s, [&](int r) -> int {
+                    return r == sg.shard ? pyrope_index_delete_row(s->shard[(size_t)r], sg.local0 + (row - sg.g0)) : PYROPE_OK;
                 });
-                if (rc != PYROPE_OK) g_serr = "row not found";
-                return rc;
+                return rc == PYROPE_ERR_NOT_FOUND ? fail(rc, "row not found") : rc;
             }
-        return sfail(PYROPE_ERR_NOT_FOUND, "row %lld not found", (long long)row);
+        return fail(PYROPE_ERR_NOT_FOUND, "row %lld not found", (long long)row);
     }
-    // IVF: a buffered row lives on every shard, a list row on its owner only
+    // IVF: a buffered row lives on every shard, a list row on its owner only.  A shard without the row answers NOT_FOUND;
+    // any other failure reaches the caller with that shard's message.
     std::vector<int> rcs((size_t)s->n, 0);
-    run_all(s, [&](int r) -> int { rcs[(size_t)r] = pyrope_index_delete_row(s->shard[(size_t)r], row); return PYROPE_OK; });
-    for (int rc : rcs)
-        if (rc == PYROPE_OK) return PYROPE_OK;
-    return sfail(rcs[0], "row %lld not found", (long long)row);
+    const int rc = run_all(s, [&](int r) -> int {
+        rcs[(size_t)r] = pyrope_index_delete_row(s->shard[(size_t)r], row);
+        return rcs[(size_t)r] == PYROPE_ERR_NOT_FOUND ? PYROPE_OK : rcs[(size_t)r];
+    });
+    for (int c : rcs)
+        if (c == PYROPE_OK) return PYROPE_OK;
+    return rc != PYROPE_OK ? rc : fail(PYROPE_ERR_NOT_FOUND, "row %lld not found", (long long)row);
 }
 
 int pyrope_sharded_build(pyrope_sharded* s) {
-    if (!s) return sfail(PYROPE_ERR_INVALID_ARG, "handle is null");
+    if (!s) return fail(PYROPE_ERR_INVALID_ARG, "handle is null");
     std::lock_guard<std::mutex> g(s->mu);
     const int rc = stage_consuming(s, pyrope_internal_index_prepare_build);
     if (rc == PYROPE_OK && s->kind != PYROPE_FLAT) {
@@ -440,18 +415,18 @@ int pyrope_sharded_build(pyrope_sharded* s) {
 }
 
 int pyrope_sharded_extend(pyrope_sharded* s) {
-    if (!s) return sfail(PYROPE_ERR_INVALID_ARG, "handle is null");
-    if (s->kind == PYROPE_FLAT) return sfail(PYROPE_ERR_UNSUPPORTED, "Extend needs an IVF index: FLAT has no inverted lists");
+    if (!s) return fail(PYROPE_ERR_INVALID_ARG, "handle is null");
+    if (s->kind == PYROPE_FLAT) return fail(PYROPE_ERR_UNSUPPORTED, "Extend needs an IVF index: FLAT has no inverted lists");
     std::lock_guard<std::mutex> g(s->mu);
     return stage_consuming(s, pyrope_internal_index_prepare_extend);
 }
 
 int pyrope_sharded_stats(pyrope_sharded* s, int64_t* live_rows_out) {
-    if (!s || !live_rows_out) return sfail(PYROPE_ERR_INVALID_ARG, "null argument");
+    if (!s || !live_rows_out) return fail(PYROPE_ERR_INVALID_ARG, "null argument");
     int64_t tot = 0;
     for (int r = 0; r < s->n; ++r) {
         int64_t live = 0, buf = 0;
-        STRY(pyrope_index_stats(s->shard[(size_t)r], &live, &buf, nullptr, nullptr));
+        TRY(pyrope_index_stats(s->shard[(size_t)r], &live, &buf, nullptr, nullptr));
         // IVF: buffered rows are replicated on every shard, list rows are not
         tot += (s->kind == PYROPE_FLAT || r == 0) ? live : live - buf;
     }
@@ -464,23 +439,23 @@ int pyrope_sharded_stats(pyrope_sharded* s, int64_t* live_rows_out) {
 // q_ready (device_io only, may be null): a CUDA event every shard waits for before it reads the queries.
 static int sharded_search(S* s, int64_t nq, const float* Q, int topk, int64_t max_scans, int nprobe, float* scores_out,
                           int64_t* rows_out, int32_t* counts_out, int device_io, cudaEvent_t q_ready = nullptr) {
-    if (!s) return sfail(PYROPE_ERR_INVALID_ARG, "handle is null");
-    if (nq < 0 || (nq > 0 && !Q)) return sfail(PYROPE_ERR_INVALID_ARG, "query is null");
+    if (!s) return fail(PYROPE_ERR_INVALID_ARG, "handle is null");
+    if (nq < 0 || (nq > 0 && !Q)) return fail(PYROPE_ERR_INVALID_ARG, "query is null");
     if (topk <= 0) {
-        if (s->kind == PYROPE_FLAT) return sfail(PYROPE_ERR_OUT_OF_RANGE, "topK must be positive.");
+        if (s->kind == PYROPE_FLAT) return fail(PYROPE_ERR_OUT_OF_RANGE, "topK must be positive.");
         for (int64_t i = 0; !device_io && i < nq; ++i) counts_out[i] = 0;
         return PYROPE_OK;
     }
     if (nq == 0) return PYROPE_OK;
-    if (!scores_out || !rows_out || !counts_out) return sfail(PYROPE_ERR_INVALID_ARG, "output buffer is null");
+    if (!scores_out || !rows_out || !counts_out) return fail(PYROPE_ERR_INVALID_ARG, "output buffer is null");
     if (max_scans >= 0 && s->n > 1)
-        return sfail(PYROPE_ERR_UNSUPPORTED, "MaxScans walks rows in insertion / probe order and cannot be split over devices");
-    if ((int64_t)s->n * topk > 4096) return sfail(PYROPE_ERR_UNSUPPORTED, "topK %d too large for %d shards", topk, s->n);
+        return fail(PYROPE_ERR_UNSUPPORTED, "MaxScans walks rows in insertion / probe order and cannot be split over devices");
+    if ((int64_t)s->n * topk > 4096) return fail(PYROPE_ERR_UNSUPPORTED, "topK %d too large for %d shards", topk, s->n);
     std::lock_guard<std::mutex> g(s->mu);
     const int N = s->n, dim = s->dim, k = topk;
     const bool ivf = s->kind != PYROPE_FLAT;
     int built = 0;
-    if (ivf) STRY(pyrope_index_is_built(s->shard[0], &built));
+    if (ivf) TRY(pyrope_index_is_built(s->shard[0], &built));
     const bool split = ivf && built && N > 1;
     const int P = nprobe >= 0 ? std::min(nprobe, std::max(s->nlist, 1)) : (s->kind == PYROPE_IVF_FLAT ? 3 : 1);
     const int64_t per = (nq + N - 1) / N;  // coarse slice per shard
@@ -500,67 +475,67 @@ static int sharded_search(S* s, int64_t nq, const float* Q, int topk, int64_t ma
         auto phase = [&](const std::function<int()>& body) {
             if (failed.load() || myrc != PYROPE_OK) return;
             myrc = body();
-            if (myrc != PYROPE_OK) { mymsg = g_serr; failed.store(true); }
+            if (myrc != PYROPE_OK) { mymsg = pyrope_last_error(); failed.store(true); }
         };
         const size_t per_s = sizeof(float) * (size_t)nq * k, per_r = sizeof(int64_t) * (size_t)nq * k;
         // ---- phase 1: buffers, staging, threshold-exchange arrays
         phase([&]() -> int {
-            STRY(grow(s->dQ[i], qbytes));
-            STRY(grow(s->sc[i], per_s));
-            STRY(grow(s->rw[i], per_r));
-            STRY(grow(s->cn[i], sizeof(int32_t) * (size_t)nq));
+            TRY(grow(s->dQ[i], qbytes));
+            TRY(grow(s->sc[i], per_s));
+            TRY(grow(s->rw[i], per_r));
+            TRY(grow(s->cn[i], sizeof(int32_t) * (size_t)nq));
             if (split) {
-                STRY(grow(s->pr_local[i], sizeof(int64_t) * (size_t)per * P));
-                STRY(grow(s->pr_all[i], sizeof(int64_t) * (size_t)per * N * P));
+                TRY(grow(s->pr_local[i], sizeof(int64_t) * (size_t)per * P));
+                TRY(grow(s->pr_all[i], sizeof(int64_t) * (size_t)per * N * P));
             }
             if (r == 0) {
-                STRY(grow(s->g_sc, per_s * (size_t)N));
-                STRY(grow(s->g_rw, per_r * (size_t)N));
-                STRY(grow(s->m_sc, per_s));
-                STRY(grow(s->m_rw, per_r));
-                STRY(grow(s->m_cn, sizeof(int32_t) * (size_t)nq));
+                TRY(grow(s->g_sc, per_s * (size_t)N));
+                TRY(grow(s->g_rw, per_r * (size_t)N));
+                TRY(grow(s->m_sc, per_s));
+                TRY(grow(s->m_rw, per_r));
+                TRY(grow(s->m_cn, sizeof(int32_t) * (size_t)nq));
                 if (!device_io) {
-                    STRY(grow_pinned(&s->hQ, &s->hQ_bytes, qbytes));
-                    STRY(grow_pinned(&s->hOut, &s->hOut_bytes, per_s + per_r + (size_t)nq * 4));
+                    TRY(grow_pinned(&s->hQ, &s->hQ_bytes, qbytes));
+                    TRY(grow_pinned(&s->hOut, &s->hOut_bytes, per_s + per_r + (size_t)nq * 4));
                     memcpy(s->hQ, Q, qbytes);
                 }
             }
-            if (thr_setup && s->exchange) STRY(pyrope_index_threshold_exchange_close(s->shard[i]));
+            if (thr_setup && s->exchange) TRY(pyrope_index_threshold_exchange_close(s->shard[i]));
             return PYROPE_OK;
         });
         s->bar.wait();  // nobody publishes into an array that is about to be replaced
         phase([&]() -> int {
-            if (thr_setup) STRY(pyrope_index_threshold_exchange_array(s->shard[i], std::max<int64_t>(nq, 16384), &s->thr_arr[i]));
+            if (thr_setup) TRY(pyrope_index_threshold_exchange_array(s->shard[i], std::max<int64_t>(nq, 16384), &s->thr_arr[i]));
             return PYROPE_OK;
         });
         s->bar.wait();  // buffers and arrays of every shard exist (peers write into them), staging is filled
         // ---- phase 2: queries, coarse slice, probe lists to every peer
         phase([&]() -> int {
-            if (thr_setup) STRY(pyrope_index_threshold_exchange_attach(s->shard[i], N, r, s->thr_arr.data()));
-            if (use_thr) STRY(pyrope_index_threshold_exchange_epoch(s->shard[i], epoch));
+            if (thr_setup) TRY(pyrope_index_threshold_exchange_attach(s->shard[i], N, r, s->thr_arr.data()));
+            if (use_thr) TRY(pyrope_index_threshold_exchange_epoch(s->shard[i], epoch));
             if (device_io) {
-                if (q_ready) SCK(cudaStreamWaitEvent(st, q_ready, 0));
-                if (r == 0) { if (s->dQ[0].p != (const void*)Q) SCK(cudaMemcpyAsync(s->dQ[0].p, Q, qbytes, cudaMemcpyDeviceToDevice, st)); }
-                else SCK(cudaMemcpyPeerAsync(s->dQ[i].p, s->dev[i], Q, s->dev[0], qbytes, st));
-                if (r == 0) SCK(cudaEventRecord(s->ev_t0, st));
+                if (q_ready) CK(cudaStreamWaitEvent(st, q_ready, 0));
+                if (r == 0) { if (s->dQ[0].p != (const void*)Q) CK(cudaMemcpyAsync(s->dQ[0].p, Q, qbytes, cudaMemcpyDeviceToDevice, st)); }
+                else CK(cudaMemcpyPeerAsync(s->dQ[i].p, s->dev[i], Q, s->dev[0], qbytes, st));
+                if (r == 0) CK(cudaEventRecord(s->ev_t0, st));
             } else {
-                if (r == 0) SCK(cudaEventRecord(s->ev_t0, st));
-                SCK(cudaMemcpyAsync(s->dQ[i].p, s->hQ, qbytes, cudaMemcpyHostToDevice, st));
+                if (r == 0) CK(cudaEventRecord(s->ev_t0, st));
+                CK(cudaMemcpyAsync(s->dQ[i].p, s->hQ, qbytes, cudaMemcpyHostToDevice, st));
             }
             if (split) {
                 const float* dQ = reinterpret_cast<const float*>(s->dQ[i].p);
                 const int64_t qlo = std::min<int64_t>(nq, per * r), qhi = std::min<int64_t>(nq, qlo + per);
                 int64_t* pl = reinterpret_cast<int64_t*>(s->pr_local[i].p);
                 if (qhi > qlo) {
-                    STRY(pyrope_index_coarse_probe_device(s->shard[i], qhi - qlo, dQ + (size_t)qlo * dim, P, pl, st));
+                    TRY(pyrope_index_coarse_probe_device(s->shard[i], qhi - qlo, dQ + (size_t)qlo * dim, P, pl, st));
                     int64_t* d[8] = {nullptr};
                     for (int p = 0; p < N; ++p) d[p] = reinterpret_cast<int64_t*>(s->pr_all[(size_t)p].p);
                     const int64_t words = (qhi - qlo) * P;
                     scatter_words_kernel<<<(unsigned)((words + 255) / 256), 256, 0, st>>>(pl, words, d[0], d[1], d[2], d[3], d[4], d[5],
                                                                                       d[6], d[7], qlo * P);
-                    SCK(cudaGetLastError());
+                    CK(cudaGetLastError());
                 }
-                SCK(cudaEventRecord(s->ev_probe[i], st));
+                CK(cudaEventRecord(s->ev_probe[i], st));
             }
             return PYROPE_OK;
         });
@@ -573,45 +548,45 @@ static int sharded_search(S* s, int64_t nq, const float* Q, int topk, int64_t ma
             int32_t* cn = reinterpret_cast<int32_t*>(s->cn[i].p);
             if (split) {
                 for (int p = 0; p < N; ++p)
-                    if (p != r) SCK(cudaStreamWaitEvent(st, s->ev_probe[(size_t)p], 0));
-                STRY(pyrope_index_search_batch_probed_device(s->shard[i], nq, dQ, k, -1, P,
-                                                             reinterpret_cast<const int64_t*>(s->pr_all[i].p), sc, rw, cn, st));
+                    if (p != r) CK(cudaStreamWaitEvent(st, s->ev_probe[(size_t)p], 0));
+                TRY(pyrope_index_search_batch_probed_device(s->shard[i], nq, dQ, k, -1, P,
+                                                            reinterpret_cast<const int64_t*>(s->pr_all[i].p), sc, rw, cn, st));
             } else {
-                STRY(pyrope_index_search_batch_device(s->shard[i], nq, dQ, k, N > 1 ? -1 : max_scans, nprobe, sc, rw, cn, st));
+                TRY(pyrope_index_search_batch_device(s->shard[i], nq, dQ, k, N > 1 ? -1 : max_scans, nprobe, sc, rw, cn, st));
             }
             if (r == 0) {
-                SCK(cudaMemcpyAsync(s->g_sc.p, sc, per_s, cudaMemcpyDeviceToDevice, st));
-                SCK(cudaMemcpyAsync(s->g_rw.p, rw, per_r, cudaMemcpyDeviceToDevice, st));
+                CK(cudaMemcpyAsync(s->g_sc.p, sc, per_s, cudaMemcpyDeviceToDevice, st));
+                CK(cudaMemcpyAsync(s->g_rw.p, rw, per_r, cudaMemcpyDeviceToDevice, st));
             } else {
-                SCK(cudaMemcpyPeerAsync((char*)s->g_sc.p + per_s * i, s->dev[0], sc, s->dev[i], per_s, st));
-                SCK(cudaMemcpyPeerAsync((char*)s->g_rw.p + per_r * i, s->dev[0], rw, s->dev[i], per_r, st));
+                CK(cudaMemcpyPeerAsync((char*)s->g_sc.p + per_s * i, s->dev[0], sc, s->dev[i], per_s, st));
+                CK(cudaMemcpyPeerAsync((char*)s->g_rw.p + per_r * i, s->dev[0], rw, s->dev[i], per_r, st));
             }
-            SCK(cudaEventRecord(s->ev_res[i], st));
+            CK(cudaEventRecord(s->ev_res[i], st));
             return PYROPE_OK;
         });
         s->bar.wait();  // every shard's result event is recorded
         // ---- phase 4: merge on the first shard's device
         phase([&]() -> int {
             if (r != 0) return PYROPE_OK;
-            for (int p = 1; p < N; ++p) SCK(cudaStreamWaitEvent(st, s->ev_res[(size_t)p], 0));
+            for (int p = 1; p < N; ++p) CK(cudaStreamWaitEvent(st, s->ev_res[(size_t)p], 0));
             float* ms = device_io ? scores_out : reinterpret_cast<float*>(s->m_sc.p);
             int64_t* mr = device_io ? rows_out : reinterpret_cast<int64_t*>(s->m_rw.p);
             int32_t* mc = device_io ? counts_out : reinterpret_cast<int32_t*>(s->m_cn.p);
-            STRY(pyrope_topk_merge_dedupe_device(nq, N, k, k, reinterpret_cast<const float*>(s->g_sc.p),
-                                                 reinterpret_cast<const int64_t*>(s->g_rw.p), ms, mr, mc, ivf ? 1 : 0, st));
+            TRY(pyrope_topk_merge_dedupe_device(nq, N, k, k, reinterpret_cast<const float*>(s->g_sc.p),
+                                                reinterpret_cast<const int64_t*>(s->g_rw.p), ms, mr, mc, ivf ? 1 : 0, st));
             if (!device_io) {
                 char* ho = reinterpret_cast<char*>(s->hOut);
-                SCK(cudaMemcpyAsync(ho, ms, per_s, cudaMemcpyDeviceToHost, st));
-                SCK(cudaMemcpyAsync(ho + per_s, mr, per_r, cudaMemcpyDeviceToHost, st));
-                SCK(cudaMemcpyAsync(ho + per_s + per_r, mc, sizeof(int32_t) * (size_t)nq, cudaMemcpyDeviceToHost, st));
+                CK(cudaMemcpyAsync(ho, ms, per_s, cudaMemcpyDeviceToHost, st));
+                CK(cudaMemcpyAsync(ho + per_s, mr, per_r, cudaMemcpyDeviceToHost, st));
+                CK(cudaMemcpyAsync(ho + per_s + per_r, mc, sizeof(int32_t) * (size_t)nq, cudaMemcpyDeviceToHost, st));
             }
-            SCK(cudaEventRecord(s->ev_t1, st));
+            CK(cudaEventRecord(s->ev_t1, st));
             return PYROPE_OK;
         });
         cudaStreamSynchronize(st);  // the call is synchronous: every shard is idle when it returns
         s->bar.wait();               // ... and the first shard has consumed every peer's result
-        if (myrc != PYROPE_OK) g_serr = mymsg;
-        return myrc;
+        if (myrc != PYROPE_OK) return fail(myrc, "%s", mymsg.c_str());
+        return PYROPE_OK;
     });
     if (rc != PYROPE_OK) return rc;
     if (use_thr) { s->exchange = true; s->thr_cap = std::max<int64_t>(s->thr_cap, std::max<int64_t>(nq, 16384)); }
@@ -637,7 +612,7 @@ int pyrope_sharded_search_batch_device(pyrope_sharded* s, int64_t nq, const floa
 }
 
 int pyrope_sharded_last_search_ms(pyrope_sharded* s, float* ms_out) {
-    if (!s || !ms_out) return sfail(PYROPE_ERR_INVALID_ARG, "null argument");
+    if (!s || !ms_out) return fail(PYROPE_ERR_INVALID_ARG, "null argument");
     *ms_out = s->last_ms;
     return PYROPE_OK;
 }
@@ -652,80 +627,80 @@ static const S::Seg* flat_seg(const S* s, int64_t row) {
 }
 
 int pyrope_sharded_update_row(pyrope_sharded* s, int64_t row, const float* x) {
-    if (!s) return sfail(PYROPE_ERR_INVALID_ARG, "handle is null");
-    if (!x) return sfail(PYROPE_ERR_INVALID_ARG, "vector is null");
+    if (!s) return fail(PYROPE_ERR_INVALID_ARG, "handle is null");
+    if (!x) return fail(PYROPE_ERR_INVALID_ARG, "vector is null");
     std::lock_guard<std::mutex> g(s->mu);
-    if (row < 0 || row >= s->next_row) return sfail(PYROPE_ERR_NOT_FOUND, "row %lld does not exist", (long long)row);
+    if (row < 0 || row >= s->next_row) return fail(PYROPE_ERR_NOT_FOUND, "row %lld does not exist", (long long)row);
     if (s->kind == PYROPE_FLAT) {  // the owner's copy, in place (an Upsert un-deletes)
         const S::Seg* sg = flat_seg(s, row);
-        if (!sg) return sfail(PYROPE_ERR_NOT_FOUND, "row %lld does not exist", (long long)row);
+        if (!sg) return fail(PYROPE_ERR_NOT_FOUND, "row %lld does not exist", (long long)row);
         return run_all(s, [&](int r) -> int {
-            if (r == sg->shard) STRY(pyrope_index_update_row(s->shard[(size_t)r], sg->local0 + (row - sg->g0), x));
+            if (r == sg->shard) TRY(pyrope_index_update_row(s->shard[(size_t)r], sg->local0 + (row - sg->g0), x));
             return PYROPE_OK;
         });
     }
     // IVF: only a buffered row can be updated, and the buffer is replicated: every shard must succeed
     std::vector<int> rcs((size_t)s->n, 0);
-    run_all(s, [&](int r) -> int { rcs[(size_t)r] = pyrope_index_update_row(s->shard[(size_t)r], row, x); return PYROPE_OK; });
+    const int rc = run_all(s, [&](int r) -> int { return rcs[(size_t)r] = pyrope_index_update_row(s->shard[(size_t)r], row, x); });
     int ok = 0;
-    for (int rc : rcs) ok += rc == PYROPE_OK;
+    for (int c : rcs) ok += c == PYROPE_OK;
     if (ok == s->n) return PYROPE_OK;
-    if (ok == 0) return sfail(rcs[0], "row %lld is not in the write buffer", (long long)row);
-    return sfail(PYROPE_ERR_INVALID_STATE, "row %lld was updated on %d of %d shards", (long long)row, ok, s->n);
+    if (ok > 0) return fail(PYROPE_ERR_INVALID_STATE, "row %lld was updated on %d of %d shards", (long long)row, ok, s->n);
+    return rcs[0] == PYROPE_ERR_NOT_FOUND ? fail(rcs[0], "row %lld is not in the write buffer", (long long)row) : rc;
 }
 
 int pyrope_sharded_shadow_row(pyrope_sharded* s, int64_t row, int shadowed) {
-    if (!s) return sfail(PYROPE_ERR_INVALID_ARG, "handle is null");
-    if (s->kind == PYROPE_FLAT) return sfail(PYROPE_ERR_INVALID_STATE, "FLAT rows cannot be shadowed");
+    if (!s) return fail(PYROPE_ERR_INVALID_ARG, "handle is null");
+    if (s->kind == PYROPE_FLAT) return fail(PYROPE_ERR_INVALID_STATE, "FLAT rows cannot be shadowed");
     std::lock_guard<std::mutex> g(s->mu);
-    if (row < 0 || row >= s->next_row) return sfail(PYROPE_ERR_NOT_FOUND, "row %lld not found", (long long)row);
+    if (row < 0 || row >= s->next_row) return fail(PYROPE_ERR_NOT_FOUND, "row %lld not found", (long long)row);
     // a list row lives on the owner of its list only
     std::vector<int> rcs((size_t)s->n, 0);
     run_all(s, [&](int r) -> int { rcs[(size_t)r] = pyrope_index_shadow_row(s->shard[(size_t)r], row, shadowed); return PYROPE_OK; });
     for (int rc : rcs)
         if (rc == PYROPE_OK) return PYROPE_OK;
-    return sfail(PYROPE_ERR_NOT_FOUND, "row %lld is not in an inverted list", (long long)row);
+    return fail(PYROPE_ERR_NOT_FOUND, "row %lld is not in an inverted list", (long long)row);
 }
 
 int pyrope_sharded_set_labels(pyrope_sharded* s, int64_t n_rows, const int64_t* labels_by_row) {
-    if (!s) return sfail(PYROPE_ERR_INVALID_ARG, "handle is null");
+    if (!s) return fail(PYROPE_ERR_INVALID_ARG, "handle is null");
     std::lock_guard<std::mutex> g(s->mu);
     if (n_rows < s->next_row || (n_rows > 0 && !labels_by_row))
-        return sfail(PYROPE_ERR_INVALID_ARG, "labels for %lld rows needed, %lld given", (long long)s->next_row, (long long)n_rows);
+        return fail(PYROPE_ERR_INVALID_ARG, "labels for %lld rows needed, %lld given", (long long)s->next_row, (long long)n_rows);
     if (s->kind != PYROPE_FLAT)
-        return run_all(s, [&](int r) -> int { STRY(pyrope_index_set_labels(s->shard[(size_t)r], n_rows, labels_by_row)); return PYROPE_OK; });
+        return run_all(s, [&](int r) -> int { TRY(pyrope_index_set_labels(s->shard[(size_t)r], n_rows, labels_by_row)); return PYROPE_OK; });
     // FLAT: a shard's local rows map back to global rows through the segment table
     return run_all(s, [&](int r) -> int {
         std::vector<int64_t> L((size_t)s->shard_rows[(size_t)r], -1);
         for (const S::Seg& sg : s->segs)
             if (sg.shard == r)
                 for (int64_t i = 0; i < sg.n; ++i) L[(size_t)(sg.local0 + i)] = labels_by_row[(size_t)(sg.g0 + i)];
-        STRY(pyrope_index_set_labels(s->shard[(size_t)r], (int64_t)L.size(), L.data()));
+        TRY(pyrope_index_set_labels(s->shard[(size_t)r], (int64_t)L.size(), L.data()));
         return PYROPE_OK;
     });
 }
 
 // centroids and PQ codebooks are replicated bit for bit: read them from the first shard, on its thread
 int pyrope_sharded_is_built(pyrope_sharded* s, int* out) {
-    if (!s || !out) return sfail(PYROPE_ERR_INVALID_ARG, "null argument");
-    STRY(pyrope_index_is_built(s->shard[0], out));
+    if (!s || !out) return fail(PYROPE_ERR_INVALID_ARG, "null argument");
+    TRY(pyrope_index_is_built(s->shard[0], out));
     return PYROPE_OK;
 }
 
 int pyrope_sharded_get_centroids(pyrope_sharded* s, float* centroids_out, int* n_out) {
-    if (!s) return sfail(PYROPE_ERR_INVALID_ARG, "handle is null");
+    if (!s) return fail(PYROPE_ERR_INVALID_ARG, "handle is null");
     std::lock_guard<std::mutex> g(s->mu);
     return run_all(s, [&](int r) -> int {
-        if (r == 0) STRY(pyrope_index_get_centroids(s->shard[0], centroids_out, n_out));
+        if (r == 0) TRY(pyrope_index_get_centroids(s->shard[0], centroids_out, n_out));
         return PYROPE_OK;
     });
 }
 
 int pyrope_sharded_get_codebooks(pyrope_sharded* s, float* codebooks_out, int32_t* ksub_out) {
-    if (!s) return sfail(PYROPE_ERR_INVALID_ARG, "handle is null");
+    if (!s) return fail(PYROPE_ERR_INVALID_ARG, "handle is null");
     std::lock_guard<std::mutex> g(s->mu);
     return run_all(s, [&](int r) -> int {
-        if (r == 0) STRY(pyrope_index_get_codebooks(s->shard[0], codebooks_out, ksub_out));
+        if (r == 0) TRY(pyrope_index_get_codebooks(s->shard[0], codebooks_out, ksub_out));
         return PYROPE_OK;
     });
 }
@@ -769,7 +744,7 @@ bool file_bytes(const std::string& path, uint64_t* out) {
 // manifest written by another device count is refused as such, before the rest of it is read)
 int read_manifest(const char* path, Manifest& M, int expect_n = 0) {
     FILE* f = fopen(path, "rb");
-    if (!f) return sfail(PYROPE_ERR_NOT_FOUND, "Snapshot file not found: %s", path);
+    if (!f) return fail(PYROPE_ERR_NOT_FOUND, "Snapshot file not found: %s", path);
     bool ok = true;
     auto r = [&](void* p, size_t n) { if (ok && fread(p, 1, n, f) != n) ok = false; };
     auto rv32 = [&]() { int32_t v = 0; r(&v, 4); return v; };
@@ -779,14 +754,14 @@ int read_manifest(const char* path, Manifest& M, int expect_n = 0) {
     int32_t version = rv32();
     if (!ok || memcmp(magic, kManifestMagic, 8) != 0 || version != kManifestVersion) {
         fclose(f);
-        return sfail(PYROPE_ERR_INVALID_ARG, "%s is not a sharded pyrope_gpu snapshot manifest", path);
+        return fail(PYROPE_ERR_INVALID_ARG, "%s is not a sharded pyrope_gpu snapshot manifest", path);
     }
     M.n = rv32(); M.kind = rv32(); M.dim = rv32(); M.metric = rv32(); M.nlist = rv32(); M.m = rv32(); M.k = rv32();
     M.next_row = rv64(); M.gen = rv64();
     if (ok && expect_n > 0 && M.n != expect_n) {
         fclose(f);
-        return sfail(PYROPE_ERR_INVALID_ARG, "snapshot %s was written by %d shards, this index has %d devices (no re-sharding on load)",
-                     path, M.n, expect_n);
+        return fail(PYROPE_ERR_INVALID_ARG, "snapshot %s was written by %d shards, this index has %d devices (no re-sharding on load)",
+                    path, M.n, expect_n);
     }
     const int64_t nsegs = rv64();
     ok = ok && M.n >= 1 && M.n <= 8 && M.next_row >= 0 && M.gen >= 1 && nsegs >= 0 && nsegs <= M.next_row;
@@ -809,12 +784,12 @@ int read_manifest(const char* path, Manifest& M, int expect_n = 0) {
         M.bytes.push_back(b);
     }
     fclose(f);
-    if (!ok) return sfail(PYROPE_ERR_INVALID_ARG, "corrupt or truncated snapshot manifest %s", path);
+    if (!ok) return fail(PYROPE_ERR_INVALID_ARG, "corrupt or truncated snapshot manifest %s", path);
     // FLAT row blocks: inside [0, next_row) globally and inside their shard's local rows
     for (const S::Seg& sg : M.segs)
         if (sg.shard < 0 || sg.shard >= M.n || sg.n <= 0 || sg.g0 < 0 || sg.g0 + sg.n > M.next_row || sg.local0 < 0 ||
             sg.local0 + sg.n > M.shard_rows[(size_t)sg.shard])
-            return sfail(PYROPE_ERR_INVALID_ARG, "corrupt snapshot manifest %s: row block table", path);
+            return fail(PYROPE_ERR_INVALID_ARG, "corrupt snapshot manifest %s: row block table", path);
     return PYROPE_OK;
 }
 
@@ -823,8 +798,8 @@ int read_manifest(const char* path, Manifest& M, int expect_n = 0) {
 extern "C" {
 
 int pyrope_sharded_snapshot(pyrope_sharded* s, const char* path) {
-    if (!s) return sfail(PYROPE_ERR_INVALID_ARG, "handle is null");
-    if (!path || !*path) return sfail(PYROPE_ERR_INVALID_ARG, "Path cannot be empty");
+    if (!s) return fail(PYROPE_ERR_INVALID_ARG, "handle is null");
+    if (!path || !*path) return fail(PYROPE_ERR_INVALID_ARG, "Path cannot be empty");
     std::lock_guard<std::mutex> g(s->mu);
     const std::string base(path), dir = dir_of(base), stem = base.substr(dir.size());
     Manifest old;
@@ -833,15 +808,15 @@ int pyrope_sharded_snapshot(pyrope_sharded* s, const char* path) {
     const int64_t gen = std::max(s->snap_gen, have_old ? old.gen : 0) + 1;
     std::vector<std::string> names((size_t)s->n);
     for (int r = 0; r < s->n; ++r) names[(size_t)r] = stem + ".g" + std::to_string(gen) + ".shard" + std::to_string(r);
-    int rc = run_all(s, [&](int r) -> int { STRY(pyrope_index_snapshot(s->shard[(size_t)r], (dir + names[(size_t)r]).c_str())); return PYROPE_OK; });
+    int rc = run_all(s, [&](int r) -> int { TRY(pyrope_index_snapshot(s->shard[(size_t)r], (dir + names[(size_t)r]).c_str())); return PYROPE_OK; });
     std::vector<uint64_t> bytes((size_t)s->n, 0);
     for (int r = 0; rc == PYROPE_OK && r < s->n; ++r)
-        if (!file_bytes(dir + names[(size_t)r], &bytes[(size_t)r])) rc = sfail(PYROPE_ERR_INVALID_STATE, "shard file %s vanished", names[(size_t)r].c_str());
+        if (!file_bytes(dir + names[(size_t)r], &bytes[(size_t)r])) rc = fail(PYROPE_ERR_INVALID_STATE, "shard file %s vanished", names[(size_t)r].c_str());
     const std::string tmp = base + ".tmp";
     if (rc == PYROPE_OK) {
         FILE* f = fopen(tmp.c_str(), "wb");
         if (!f) {
-            rc = sfail(PYROPE_ERR_INVALID_ARG, "cannot open %s for writing", tmp.c_str());
+            rc = fail(PYROPE_ERR_INVALID_ARG, "cannot open %s for writing", tmp.c_str());
         } else {
             bool ok = true;
             auto w = [&](const void* p, size_t n) { if (ok && fwrite(p, 1, n, f) != n) ok = false; };
@@ -859,8 +834,8 @@ int pyrope_sharded_snapshot(pyrope_sharded* s, const char* path) {
                 w(names[(size_t)r].data(), len);
                 w(&bytes[(size_t)r], 8);
             }
-            if (fclose(f) != 0 || !ok) rc = sfail(PYROPE_ERR_INVALID_STATE, "short write to %s", tmp.c_str());
-            else if (rename(tmp.c_str(), path) != 0) rc = sfail(PYROPE_ERR_INVALID_STATE, "cannot move %s into place", tmp.c_str());
+            if (fclose(f) != 0 || !ok) rc = fail(PYROPE_ERR_INVALID_STATE, "short write to %s", tmp.c_str());
+            else if (rename(tmp.c_str(), path) != 0) rc = fail(PYROPE_ERR_INVALID_STATE, "cannot move %s into place", tmp.c_str());
         }
     }
     if (rc != PYROPE_OK) {  // the manifest on disk (if any) still names the previous, complete set
@@ -876,8 +851,8 @@ int pyrope_sharded_snapshot(pyrope_sharded* s, const char* path) {
 }
 
 int pyrope_sharded_load(pyrope_sharded* s, const char* path) {
-    if (!s) return sfail(PYROPE_ERR_INVALID_ARG, "handle is null");
-    if (!path || !*path) return sfail(PYROPE_ERR_INVALID_ARG, "Path cannot be empty");
+    if (!s) return fail(PYROPE_ERR_INVALID_ARG, "handle is null");
+    if (!path || !*path) return fail(PYROPE_ERR_INVALID_ARG, "Path cannot be empty");
     std::lock_guard<std::mutex> g(s->mu);
     Manifest M;
     {
@@ -888,36 +863,36 @@ int pyrope_sharded_load(pyrope_sharded* s, const char* path) {
             const bool single = f && fread(magic, 1, 8, f) == 8 && memcmp(magic, "PYRGPU01", 8) == 0;
             if (f) fclose(f);
             if (single)
-                return sfail(PYROPE_ERR_INVALID_ARG, "%s is a single-device snapshot; a sharded index loads only a sharded manifest", path);
+                return fail(PYROPE_ERR_INVALID_ARG, "%s is a single-device snapshot; a sharded index loads only a sharded manifest", path);
         }
         if (rc != PYROPE_OK) return rc;
     }
     if (M.kind != s->kind || M.metric != s->metric || M.m != s->m || M.k != s->k)
-        return sfail(PYROPE_ERR_INVALID_ARG, "snapshot is of a different index type");
-    if (M.dim != s->dim) return sfail(PYROPE_ERR_DIMENSION, "Vector dimension mismatch");
-    if (s->kind != PYROPE_FLAT && !M.segs.empty()) return sfail(PYROPE_ERR_INVALID_ARG, "corrupt snapshot manifest %s: row blocks on an IVF index", path);
+        return fail(PYROPE_ERR_INVALID_ARG, "snapshot is of a different index type");
+    if (M.dim != s->dim) return fail(PYROPE_ERR_DIMENSION, "Vector dimension mismatch");
+    if (s->kind != PYROPE_FLAT && !M.segs.empty()) return fail(PYROPE_ERR_INVALID_ARG, "corrupt snapshot manifest %s: row blocks on an IVF index", path);
     const std::string dir = dir_of(path);
     for (int r = 0; r < s->n; ++r) {
         const std::string f = dir + M.names[(size_t)r];
         uint64_t b = 0;
-        if (!file_bytes(f, &b)) return sfail(PYROPE_ERR_NOT_FOUND, "Snapshot file not found: %s", f.c_str());
+        if (!file_bytes(f, &b)) return fail(PYROPE_ERR_NOT_FOUND, "Snapshot file not found: %s", f.c_str());
         if (b != M.bytes[(size_t)r])
-            return sfail(PYROPE_ERR_INVALID_ARG, "shard file %s holds %llu bytes, the manifest recorded %llu", f.c_str(),
-                         (unsigned long long)b, (unsigned long long)M.bytes[(size_t)r]);
+            return fail(PYROPE_ERR_INVALID_ARG, "shard file %s holds %llu bytes, the manifest recorded %llu", f.c_str(),
+                        (unsigned long long)b, (unsigned long long)M.bytes[(size_t)r]);
     }
     // every shard parses and stages its file on its own thread; nothing is installed unless all of them succeed
     const int rc = stage_all(s, [&](int r, void** staged) -> int {
         pyrope_internal_staged_info info{};
         const std::string f = dir + M.names[(size_t)r];
-        STRY(pyrope_internal_index_prepare_load(s->shard[(size_t)r], f.c_str(), staged, &info));
+        TRY(pyrope_internal_index_prepare_load(s->shard[(size_t)r], f.c_str(), staged, &info));
         // IVF shards carry their shard identity and the replicated row count; FLAT shards are plain indexes of their rows
         const bool ivf = s->kind != PYROPE_FLAT;
         const int want_rank = ivf ? r : 0, want_world = ivf ? s->n : 1;
         const int64_t want_rows = ivf ? M.next_row : M.shard_rows[(size_t)r];
         if (info.shard_rank != want_rank || info.shard_world != want_world || info.next_row != want_rows)
-            return sfail(PYROPE_ERR_INVALID_ARG, "%s is shard %d of %d with %lld rows, the manifest expects shard %d of %d with %lld rows",
-                         f.c_str(), info.shard_rank, info.shard_world, (long long)info.next_row, want_rank, want_world,
-                         (long long)want_rows);
+            return fail(PYROPE_ERR_INVALID_ARG, "%s is shard %d of %d with %lld rows, the manifest expects shard %d of %d with %lld rows",
+                        f.c_str(), info.shard_rank, info.shard_world, (long long)info.next_row, want_rank, want_world,
+                        (long long)want_rows);
         return PYROPE_OK;
     }, [] { return PYROPE_OK; });
     if (rc != PYROPE_OK) return rc;
@@ -956,8 +931,8 @@ int pyrope_internal_sharded_search_device(pyrope_sharded* s, int64_t nq, const f
 // unchanged; every shard must then report the same row ordinals.
 int pyrope_internal_sharded_absorb(pyrope_sharded* s, int64_t n, const float* dX, const int64_t* dL, int src_device,
                                    const int64_t* labels_host, int64_t* tail_rows_out) {
-    if (!s || n < 0) return sfail(PYROPE_ERR_INVALID_ARG, "bad argument");
-    if (s->kind == PYROPE_FLAT) return sfail(PYROPE_ERR_UNSUPPORTED, "a sharded FLAT index cannot be a Head+Tail tail");
+    if (!s || n < 0) return fail(PYROPE_ERR_INVALID_ARG, "bad argument");
+    if (s->kind == PYROPE_FLAT) return fail(PYROPE_ERR_UNSUPPORTED, "a sharded FLAT index cannot be a Head+Tail tail");
     if (n == 0) return PYROPE_OK;
     std::lock_guard<std::mutex> g(s->mu);
     const size_t N = (size_t)s->n, xb = sizeof(float) * (size_t)n * s->dim, lb = sizeof(int64_t) * (size_t)n;
@@ -965,18 +940,18 @@ int pyrope_internal_sharded_absorb(pyrope_sharded* s, int64_t n, const float* dX
     std::vector<std::vector<int64_t>> rows(N, std::vector<int64_t>((size_t)n, -1));
     int rc = run_all(s, [&](int r) -> int {
         const size_t i = (size_t)r;
-        STRY(pyrope_internal_tail_reserve(s->shard[i], n));
-        SCK(cudaMalloc(&bx[i], xb));
-        SCK(cudaMalloc(&bl[i], lb));
-        SCK(cudaMemcpyPeerAsync(bx[i], s->dev[i], dX, src_device, xb, s->st[i]));
-        SCK(cudaMemcpyPeerAsync(bl[i], s->dev[i], dL, src_device, lb, s->st[i]));
-        SCK(cudaStreamSynchronize(s->st[i]));
+        TRY(pyrope_internal_tail_reserve(s->shard[i], n));
+        CK(cudaMalloc(&bx[i], xb));
+        CK(cudaMalloc(&bl[i], lb));
+        CK(cudaMemcpyPeerAsync(bx[i], s->dev[i], dX, src_device, xb, s->st[i]));
+        CK(cudaMemcpyPeerAsync(bl[i], s->dev[i], dL, src_device, lb, s->st[i]));
+        CK(cudaStreamSynchronize(s->st[i]));
         return PYROPE_OK;
     });
     if (rc == PYROPE_OK)
         rc = run_all(s, [&](int r) -> int {
             const size_t i = (size_t)r;
-            STRY(pyrope_internal_tail_absorb(s->shard[i], n, (const float*)bx[i], (const int64_t*)bl[i], labels_host, rows[i].data()));
+            TRY(pyrope_internal_tail_absorb(s->shard[i], n, (const float*)bx[i], (const int64_t*)bl[i], labels_host, rows[i].data()));
             return PYROPE_OK;
         });
     run_all(s, [&](int r) -> int {
@@ -986,7 +961,7 @@ int pyrope_internal_sharded_absorb(pyrope_sharded* s, int64_t n, const float* dX
     });
     if (rc != PYROPE_OK) return rc;
     for (size_t r = 1; r < N; ++r)
-        if (rows[r] != rows[0]) return sfail(PYROPE_ERR_INVALID_STATE, "shard %zu placed the moved rows at other row ordinals than shard 0", r);
+        if (rows[r] != rows[0]) return fail(PYROPE_ERR_INVALID_STATE, "shard %zu placed the moved rows at other row ordinals than shard 0", r);
     for (int64_t i = 0; i < n; ++i) s->next_row = std::max(s->next_row, rows[0][(size_t)i] + 1);
     if (tail_rows_out) memcpy(tail_rows_out, rows[0].data(), lb);
     return PYROPE_OK;

@@ -11,7 +11,6 @@
 // created separately (as DeltaVectorIndexTests.cs and VectorIndexRegistry.cs:110-111 do) agree on identity and
 // the Head+Tail merge can de-duplicate on the device.
 #include <algorithm>
-#include <cstdarg>
 #include <cstdio>
 #include <cstring>
 #include <mutex>
@@ -25,39 +24,6 @@
 #include "internal.h"
 
 namespace {
-
-thread_local std::string g_verr;
-
-int vfail(int code, const char* fmt, ...) {
-    char buf[512];
-    va_list ap;
-    va_start(ap, fmt);
-    vsnprintf(buf, sizeof buf, fmt, ap);
-    va_end(ap);
-    g_verr = buf;
-    return code;
-}
-// an error raised by the row-ordinal layer: keep its code, copy its message
-int vpass(int rc) {
-    if (rc != PYROPE_OK) g_verr = pyrope_last_error();
-    return rc;
-}
-// the same for the sharded layer, which keeps its own message
-int spass(int rc) {
-    if (rc != PYROPE_OK) g_verr = pyrope_sharded_last_error();
-    return rc;
-}
-#define VTRY(expr)                            \
-    do {                                      \
-        int _r = (expr);                      \
-        if (_r != PYROPE_OK) return vpass(_r); \
-    } while (0)
-// a status whose message is already in g_verr
-#define LTRY(expr)                       \
-    do {                                 \
-        int _r = (expr);                 \
-        if (_r != PYROPE_OK) return _r;  \
-    } while (0)
 
 // process-wide id table: string -> ordinal (the row label), ordinal -> string.  Entries are reference counted — one
 // reference per leaf index whose row_of holds the id — and an ordinal whose count drops to zero is recycled, so a
@@ -163,44 +129,43 @@ namespace {
 typedef pyrope_vindex V;
 
 int check_vec(const V* v, const float* vec, int len) {
-    if (!vec) return vfail(PYROPE_ERR_INVALID_ARG, "Value cannot be null. (Parameter 'vector')");
-    if (len != v->dim) return vfail(PYROPE_ERR_DIMENSION, "Vector dimension mismatch");
+    if (!vec) return fail(PYROPE_ERR_INVALID_ARG, "Value cannot be null. (Parameter 'vector')");
+    if (len != v->dim) return fail(PYROPE_ERR_DIMENSION, "Vector dimension mismatch");
     return PYROPE_OK;
 }
 
-// ---- the row-ordinal handle behind a leaf: one device (pyrope_index_*) or several (pyrope_sharded_*).  Errors come
-// back with their message in g_verr.
+// ---- the row-ordinal handle behind a leaf: one device (pyrope_index_*) or several (pyrope_sharded_*)
 int row_add(V* v, int64_t gid, const float* vec, int64_t* row) {
-    return v->sh ? spass(pyrope_sharded_add_batch(v->sh, 1, vec, &gid, row)) : vpass(pyrope_index_add_batch(v->h, 1, vec, &gid, row));
+    return v->sh ? pyrope_sharded_add_batch(v->sh, 1, vec, &gid, row) : pyrope_index_add_batch(v->h, 1, vec, &gid, row);
 }
 int row_update(V* v, int64_t row, const float* vec) {
-    return v->sh ? spass(pyrope_sharded_update_row(v->sh, row, vec)) : vpass(pyrope_index_update_row(v->h, row, vec));
+    return v->sh ? pyrope_sharded_update_row(v->sh, row, vec) : pyrope_index_update_row(v->h, row, vec);
 }
 int row_shadow(V* v, int64_t row, int shadowed) {
-    return v->sh ? spass(pyrope_sharded_shadow_row(v->sh, row, shadowed)) : vpass(pyrope_index_shadow_row(v->h, row, shadowed));
+    return v->sh ? pyrope_sharded_shadow_row(v->sh, row, shadowed) : pyrope_index_shadow_row(v->h, row, shadowed);
 }
 int row_delete(V* v, int64_t row) {
-    return v->sh ? spass(pyrope_sharded_delete_row(v->sh, row)) : vpass(pyrope_index_delete_row(v->h, row));
+    return v->sh ? pyrope_sharded_delete_row(v->sh, row) : pyrope_index_delete_row(v->h, row);
 }
-int row_build(V* v) { return v->sh ? spass(pyrope_sharded_build(v->sh)) : vpass(pyrope_index_build(v->h)); }
-int row_extend(V* v) { return v->sh ? spass(pyrope_sharded_extend(v->sh)) : vpass(pyrope_index_extend(v->h)); }
-int row_is_built(V* v, int* out) { return v->sh ? spass(pyrope_sharded_is_built(v->sh, out)) : vpass(pyrope_index_is_built(v->h, out)); }
+int row_build(V* v) { return v->sh ? pyrope_sharded_build(v->sh) : pyrope_index_build(v->h); }
+int row_extend(V* v) { return v->sh ? pyrope_sharded_extend(v->sh) : pyrope_index_extend(v->h); }
+int row_is_built(V* v, int* out) { return v->sh ? pyrope_sharded_is_built(v->sh, out) : pyrope_index_is_built(v->h, out); }
 int row_set_labels(V* v, int64_t n, const int64_t* labels) {
-    return v->sh ? spass(pyrope_sharded_set_labels(v->sh, n, labels)) : vpass(pyrope_index_set_labels(v->h, n, labels));
+    return v->sh ? pyrope_sharded_set_labels(v->sh, n, labels) : pyrope_index_set_labels(v->h, n, labels);
 }
 int row_snapshot(V* v, const char* path) {
-    return v->sh ? spass(pyrope_sharded_snapshot(v->sh, path)) : vpass(pyrope_index_snapshot(v->h, path));
+    return v->sh ? pyrope_sharded_snapshot(v->sh, path) : pyrope_index_snapshot(v->h, path);
 }
-int row_load(V* v, const char* path) { return v->sh ? spass(pyrope_sharded_load(v->sh, path)) : vpass(pyrope_index_load(v->h, path)); }
+int row_load(V* v, const char* path) { return v->sh ? pyrope_sharded_load(v->sh, path) : pyrope_index_load(v->h, path); }
 int row_snapshot_next_row(V* v, const char* path, int64_t* next_row) {
-    return v->sh ? spass(pyrope_internal_sharded_snapshot_next_row(path, next_row))
-                 : vpass(pyrope_internal_snapshot_next_row(path, next_row));
+    return v->sh ? pyrope_internal_sharded_snapshot_next_row(path, next_row)
+                 : pyrope_internal_snapshot_next_row(path, next_row);
 }
 
 // ---- leaf writes (no locking; callers hold the write lock) ------------------------------------------------
 int leaf_add_new(V* v, int64_t gid, const float* vec) {
     int64_t row = -1;
-    LTRY(row_add(v, gid, vec, &row));
+    TRY(row_add(v, gid, vec, &row));
     v->set_row(gid, row);
     v->note_row(row, gid);
     if (v->kind != PYROPE_FLAT) v->buffered.insert(gid);
@@ -215,15 +180,15 @@ int leaf_buffer_set(V* v, int64_t gid, const float* vec) {
     // the id sits in an inverted list: the buffered copy shadows it (seenIds, IvfFlatVectorIndex.cs:210,
     // IvfPqVectorIndex.cs:170) until the next Build
     const int64_t old = it->second;
-    LTRY(row_shadow(v, old, 1));
+    TRY(row_shadow(v, old, 1));
     v->shadowed[gid] = old;
     return leaf_add_new(v, gid, vec);
 }
 
 int leaf_add(V* v, const char* id, const float* vec, int len, bool upsert) {
     if (v->kind != PYROPE_IVF_PQ && blank(id))  // IvfPqVectorIndex.Add validates nothing (:36-45)
-        return vfail(PYROPE_ERR_INVALID_ARG, v->kind == PYROPE_FLAT ? "Id cannot be empty. (Parameter 'id')" : "Id empty");
-    if (!id) return vfail(PYROPE_ERR_INVALID_ARG, "Value cannot be null. (Parameter 'key')");
+        return fail(PYROPE_ERR_INVALID_ARG, v->kind == PYROPE_FLAT ? "Id cannot be empty. (Parameter 'id')" : "Id empty");
+    if (!id) return fail(PYROPE_ERR_INVALID_ARG, "Value cannot be null. (Parameter 'key')");
     int r = check_vec(v, vec, len);  // IVF_PQ stores any array and fails at Build; the device copy cannot
     if (r != PYROPE_OK) return r;
     const int64_t gid = intern_id(id);
@@ -233,7 +198,7 @@ int leaf_add(V* v, const char* id, const float* vec, int len, bool upsert) {
         auto it = v->row_of.find(gid);
         if (it == v->row_of.end()) rc = leaf_add_new(v, gid, vec);
         else if (!upsert)  // BruteForceVectorIndex.cs:141-144
-            rc = vfail(PYROPE_ERR_INVALID_STATE, "Vector with id '%s' already exists.", id);
+            rc = fail(PYROPE_ERR_INVALID_STATE, "Vector with id '%s' already exists.", id);
         else rc = row_update(v, it->second, vec);  // :203-206 in place, scan position kept
     }
     if (rc != PYROPE_OK) id_drop_if_unreferenced(gid);
@@ -243,15 +208,15 @@ int leaf_add(V* v, const char* id, const float* vec, int len, bool upsert) {
 int leaf_delete(V* v, const char* id, bool* removed) {
     *removed = false;
     if (v->kind != PYROPE_IVF_PQ && blank(id))
-        return vfail(PYROPE_ERR_INVALID_ARG, v->kind == PYROPE_FLAT ? "Id cannot be empty. (Parameter 'id')" : "Id empty");
-    if (!id) return vfail(PYROPE_ERR_INVALID_ARG, "Value cannot be null. (Parameter 'key')");
+        return fail(PYROPE_ERR_INVALID_ARG, v->kind == PYROPE_FLAT ? "Id cannot be empty. (Parameter 'id')" : "Id empty");
+    if (!id) return fail(PYROPE_ERR_INVALID_ARG, "Value cannot be null. (Parameter 'key')");
     const int64_t gid = lookup_id(id);
     if (gid < 0) return PYROPE_OK;
     auto it = v->row_of.find(gid);
     if (it == v->row_of.end()) return PYROPE_OK;
     const int64_t row = it->second;
     if (v->kind == PYROPE_FLAT) {  // BruteForceVectorIndex.cs:231-254: tombstone, id leaves the map
-        LTRY(row_delete(v, row));
+        TRY(row_delete(v, row));
         v->gid_of_row[(size_t)row] = -1;
         v->drop(it);
         *removed = true;
@@ -260,12 +225,12 @@ int leaf_delete(V* v, const char* id, bool* removed) {
     const bool in_buffer = v->buffered.count(gid) != 0;
     if (v->kind == PYROPE_IVF_PQ) {  // IvfPqVectorIndex.cs:48-53: only the buffer
         if (!in_buffer) return PYROPE_OK;
-        LTRY(row_delete(v, row));
+        TRY(row_delete(v, row));
         v->gid_of_row[(size_t)row] = -1;
         v->buffered.erase(gid);
         auto sh = v->shadowed.find(gid);
         if (sh != v->shadowed.end()) {  // the encoded copy is visible again
-            LTRY(row_shadow(v, sh->second, 0));
+            TRY(row_shadow(v, sh->second, 0));
             it->second = sh->second;
             v->shadowed.erase(sh);
         } else {
@@ -275,11 +240,11 @@ int leaf_delete(V* v, const char* id, bool* removed) {
         return PYROPE_OK;
     }
     // IvfFlatVectorIndex.cs:62-83: buffer entry and every list entry with this id
-    LTRY(row_delete(v, row));
+    TRY(row_delete(v, row));
     v->gid_of_row[(size_t)row] = -1;
     auto sh = v->shadowed.find(gid);
     if (sh != v->shadowed.end()) {
-        LTRY(row_delete(v, sh->second));
+        TRY(row_delete(v, sh->second));
         v->gid_of_row[(size_t)sh->second] = -1;
         v->shadowed.erase(sh);
     }
@@ -313,7 +278,7 @@ void leaf_after_build(V* v, bool had_buffer) {
 int leaf_build(V* v) {
     if (v->kind == PYROPE_FLAT) return PYROPE_OK;
     const bool had_buffer = !v->buffered.empty();
-    LTRY(row_build(v));
+    TRY(row_build(v));
     leaf_after_build(v, had_buffer);
     return PYROPE_OK;
 }
@@ -328,7 +293,7 @@ void leaf_after_extend(V* v) {
 }
 
 int leaf_extend(V* v) {
-    LTRY(row_extend(v));  // FLAT -> UNSUPPORTED, not built -> INVALID_STATE
+    TRY(row_extend(v));  // FLAT -> UNSUPPORTED, not built -> INVALID_STATE
     leaf_after_extend(v);
     return PYROPE_OK;
 }
@@ -343,10 +308,10 @@ int delta_move_with_ids(V* v) {
         if (hd->gid_of_row[r] >= 0) moved_gids.push_back(hd->gid_of_row[r]);
     std::vector<int64_t> tail_rows(moved_gids.size() + 1, -1);
     int64_t moved = 0;
-    VTRY(pyrope_delta_move(v->d, &moved, tail_rows.data()));
+    TRY(pyrope_delta_move(v->d, &moved, tail_rows.data()));
     if (moved != (int64_t)moved_gids.size())
-        return vfail(PYROPE_ERR_INVALID_STATE, "compaction moved %lld rows, the id table expected %zu", (long long)moved,
-                     moved_gids.size());
+        return fail(PYROPE_ERR_INVALID_STATE, "compaction moved %lld rows, the id table expected %zu", (long long)moved,
+                    moved_gids.size());
     for (size_t i = 0; i < moved_gids.size(); ++i) {  // what _tail.Add(id, vec) does to the tail's tables
         const int64_t gid = moved_gids[i], row = tail_rows[i];
         auto it = tl->row_of.find(gid);
@@ -374,7 +339,7 @@ bool get64(FILE* f, int64_t* x) { return fread(x, 8, 1, f) == 1; }
 int leaf_save_ids(const V* v, const std::string& path) {
     const std::string tmp = path + ".tmp";
     FILE* f = fopen(tmp.c_str(), "wb");
-    if (!f) return vfail(PYROPE_ERR_INVALID_ARG, "cannot open %s for writing", tmp.c_str());
+    if (!f) return fail(PYROPE_ERR_INVALID_ARG, "cannot open %s for writing", tmp.c_str());
     bool ok = put64(f, 0x5044495650ll) && put64(f, (int64_t)v->gid_of_row.size()) && put64(f, v->built ? 1 : 0);
     int64_t live = 0;
     for (int64_t g : v->gid_of_row) live += g >= 0;
@@ -393,8 +358,8 @@ int leaf_save_ids(const V* v, const std::string& path) {
                  (s.empty() || fwrite(s.data(), 1, s.size(), f) == s.size());
         }
     }
-    if (fclose(f) != 0 || !ok) { remove(tmp.c_str()); return vfail(PYROPE_ERR_INVALID_ARG, "short write to %s", tmp.c_str()); }
-    if (rename(tmp.c_str(), path.c_str()) != 0) { remove(tmp.c_str()); return vfail(PYROPE_ERR_INVALID_ARG, "cannot move %s into place", tmp.c_str()); }
+    if (fclose(f) != 0 || !ok) { remove(tmp.c_str()); return fail(PYROPE_ERR_INVALID_ARG, "short write to %s", tmp.c_str()); }
+    if (rename(tmp.c_str(), path.c_str()) != 0) { remove(tmp.c_str()); return fail(PYROPE_ERR_INVALID_ARG, "cannot move %s into place", tmp.c_str()); }
     return PYROPE_OK;
 }
 
@@ -407,7 +372,7 @@ struct LoadedIds {
 };
 int leaf_parse_ids(const std::string& path, LoadedIds& L) {
     FILE* f = fopen(path.c_str(), "rb");
-    if (!f) return vfail(PYROPE_ERR_NOT_FOUND, "Snapshot file not found. (%s)", path.c_str());
+    if (!f) return fail(PYROPE_ERR_NOT_FOUND, "Snapshot file not found. (%s)", path.c_str());
     int64_t magic = 0, live = 0;
     bool ok = get64(f, &magic) && magic == 0x5044495650ll && get64(f, &L.nrows) && get64(f, &L.built) && get64(f, &live) &&
               L.nrows >= 0 && live >= 0 && live <= L.nrows;
@@ -426,7 +391,7 @@ int leaf_parse_ids(const std::string& path, LoadedIds& L) {
         L.state.push_back(state);
     }
     fclose(f);
-    if (!ok) return vfail(PYROPE_ERR_INVALID_ARG, "%s is not a pyrope id table", path.c_str());
+    if (!ok) return fail(PYROPE_ERR_INVALID_ARG, "%s is not a pyrope id table", path.c_str());
     return PYROPE_OK;
 }
 int leaf_apply_ids(V* v, const LoadedIds& L) {
@@ -466,11 +431,11 @@ int leaf_load(V* v, const std::string& path) {
     int r = leaf_parse_ids(path + ".ids", L);
     if (r != PYROPE_OK) return r;
     int64_t next_row = -1;
-    LTRY(row_snapshot_next_row(v, path.c_str(), &next_row));
+    TRY(row_snapshot_next_row(v, path.c_str(), &next_row));
     if (L.nrows < next_row)
-        return vfail(PYROPE_ERR_INVALID_ARG, "%s.ids covers %lld rows, the snapshot holds %lld", path.c_str(), (long long)L.nrows,
-                     (long long)next_row);
-    LTRY(row_load(v, path.c_str()));
+        return fail(PYROPE_ERR_INVALID_ARG, "%s.ids covers %lld rows, the snapshot holds %lld", path.c_str(), (long long)L.nrows,
+                    (long long)next_row);
+    TRY(row_load(v, path.c_str()));
     return leaf_apply_ids(v, L);
 }
 
@@ -478,17 +443,15 @@ int leaf_load(V* v, const std::string& path) {
 
 extern "C" {
 
-const char* pyrope_vindex_last_error(void) { return g_verr.c_str(); }
-
 int pyrope_vindex_create(int kind, int dim, int metric, int nlist, int pq_m, int pq_k, pyrope_vindex** out) {
-    if (!out) return vfail(PYROPE_ERR_INVALID_ARG, "out is null");
+    if (!out) return fail(PYROPE_ERR_INVALID_ARG, "out is null");
     *out = nullptr;
     V* v = new (std::nothrow) V();
-    if (!v) return vfail(PYROPE_ERR_OOM, "out of host memory");
+    if (!v) return fail(PYROPE_ERR_OOM, "out of host memory");
     int rc = pyrope_index_create(kind, dim, metric, nlist, pq_m, pq_k, &v->h);
     if (rc != PYROPE_OK) {
         delete v;
-        return vpass(rc);
+        return rc;
     }
     v->kind = kind; v->dim = dim; v->metric = metric;
     *out = v;
@@ -497,15 +460,15 @@ int pyrope_vindex_create(int kind, int dim, int metric, int nlist, int pq_m, int
 
 int pyrope_vindex_create_sharded(int n_devices, const int* devices, int kind, int dim, int metric, int nlist, int pq_m, int pq_k,
                                  pyrope_vindex** out) {
-    if (!out) return vfail(PYROPE_ERR_INVALID_ARG, "out is null");
+    if (!out) return fail(PYROPE_ERR_INVALID_ARG, "out is null");
     *out = nullptr;
-    if (kind != PYROPE_IVF_FLAT && kind != PYROPE_IVF_PQ) return vfail(PYROPE_ERR_UNSUPPORTED, "a sharded index must be IVF_FLAT or IVF_PQ");
+    if (kind != PYROPE_IVF_FLAT && kind != PYROPE_IVF_PQ) return fail(PYROPE_ERR_UNSUPPORTED, "a sharded index must be IVF_FLAT or IVF_PQ");
     V* v = new (std::nothrow) V();
-    if (!v) return vfail(PYROPE_ERR_OOM, "out of host memory");
+    if (!v) return fail(PYROPE_ERR_OOM, "out of host memory");
     int rc = pyrope_sharded_create(n_devices, devices, kind, dim, metric, nlist, pq_m, pq_k, &v->sh);
     if (rc != PYROPE_OK) {
         delete v;
-        return spass(rc);
+        return rc;
     }
     v->kind = kind; v->dim = dim; v->metric = metric;
     *out = v;
@@ -513,17 +476,17 @@ int pyrope_vindex_create_sharded(int n_devices, const int* devices, int kind, in
 }
 
 int pyrope_vindex_create_delta(pyrope_vindex* head, pyrope_vindex* tail, pyrope_vindex** out) {
-    if (!out) return vfail(PYROPE_ERR_INVALID_ARG, "out is null");
+    if (!out) return fail(PYROPE_ERR_INVALID_ARG, "out is null");
     *out = nullptr;
-    if (!head || !tail || head->d || tail->d) return vfail(PYROPE_ERR_INVALID_ARG, "head and tail must be leaf indexes");
-    if (head->sh) return vfail(PYROPE_ERR_UNSUPPORTED, "the head must be a one-device FLAT index");
+    if (!head || !tail || head->d || tail->d) return fail(PYROPE_ERR_INVALID_ARG, "head and tail must be leaf indexes");
+    if (head->sh) return fail(PYROPE_ERR_UNSUPPORTED, "the head must be a one-device FLAT index");
     V* v = new (std::nothrow) V();
-    if (!v) return vfail(PYROPE_ERR_OOM, "out of host memory");
+    if (!v) return fail(PYROPE_ERR_OOM, "out of host memory");
     int rc = tail->sh ? pyrope_delta_create_sharded(head->h, tail->sh, &v->d)  // DeltaVectorIndex..ctor :18-28
                       : pyrope_delta_create(head->h, tail->h, &v->d);
     if (rc != PYROPE_OK) {
         delete v;
-        return vpass(rc);
+        return rc;
     }
     v->kind = -1; v->dim = head->dim; v->metric = head->metric;
     v->head = head; v->tail = tail;
@@ -542,20 +505,20 @@ int pyrope_vindex_destroy(pyrope_vindex* v) {
 }
 
 int pyrope_vindex_native(pyrope_vindex* v, pyrope_index** out) {
-    if (!v || !out) return vfail(PYROPE_ERR_INVALID_ARG, "null argument");
+    if (!v || !out) return fail(PYROPE_ERR_INVALID_ARG, "null argument");
     *out = v->h;
     return PYROPE_OK;
 }
 
 int pyrope_vindex_set_quantization(pyrope_vindex* v, int enable) {
-    if (!v) return vfail(PYROPE_ERR_INVALID_ARG, "index handle is null");
-    if (v->d || v->kind != PYROPE_FLAT) return vfail(PYROPE_ERR_INVALID_STATE, "EnableQuantization exists on BruteForceVectorIndex only");
+    if (!v) return fail(PYROPE_ERR_INVALID_ARG, "index handle is null");
+    if (v->d || v->kind != PYROPE_FLAT) return fail(PYROPE_ERR_INVALID_STATE, "EnableQuantization exists on BruteForceVectorIndex only");
     std::unique_lock<std::shared_mutex> g(v->lock);
-    return vpass(pyrope_index_set_quantization(v->h, enable));
+    return pyrope_index_set_quantization(v->h, enable);
 }
 
 int pyrope_vindex_add(pyrope_vindex* v, const char* id, const float* vec, int len) {
-    if (!v) return vfail(PYROPE_ERR_INVALID_ARG, "index handle is null");
+    if (!v) return fail(PYROPE_ERR_INVALID_ARG, "index handle is null");
     std::unique_lock<std::shared_mutex> g(v->lock);
     if (!v->d) return leaf_add(v, id, vec, len, false);
     std::unique_lock<std::shared_mutex> gh(v->head->lock);
@@ -563,7 +526,7 @@ int pyrope_vindex_add(pyrope_vindex* v, const char* id, const float* vec, int le
 }
 
 int pyrope_vindex_upsert(pyrope_vindex* v, const char* id, const float* vec, int len) {
-    if (!v) return vfail(PYROPE_ERR_INVALID_ARG, "index handle is null");
+    if (!v) return fail(PYROPE_ERR_INVALID_ARG, "index handle is null");
     std::unique_lock<std::shared_mutex> g(v->lock);
     if (!v->d) return leaf_add(v, id, vec, len, true);
     std::unique_lock<std::shared_mutex> gh(v->head->lock);
@@ -571,7 +534,7 @@ int pyrope_vindex_upsert(pyrope_vindex* v, const char* id, const float* vec, int
 }
 
 int pyrope_vindex_delete(pyrope_vindex* v, const char* id, int* removed_out) {
-    if (!v) return vfail(PYROPE_ERR_INVALID_ARG, "index handle is null");
+    if (!v) return fail(PYROPE_ERR_INVALID_ARG, "index handle is null");
     if (removed_out) *removed_out = 0;
     std::unique_lock<std::shared_mutex> g(v->lock);
     bool a = false, b = false;
@@ -591,7 +554,7 @@ int pyrope_vindex_delete(pyrope_vindex* v, const char* id, int* removed_out) {
 }
 
 int pyrope_vindex_build(pyrope_vindex* v) {
-    if (!v) return vfail(PYROPE_ERR_INVALID_ARG, "index handle is null");
+    if (!v) return fail(PYROPE_ERR_INVALID_ARG, "index handle is null");
     std::unique_lock<std::shared_mutex> g(v->lock);
     if (!v->d) return leaf_build(v);
     // DeltaVectorIndex.Build :124-158 — compaction: head rows move to the tail device-to-device
@@ -602,14 +565,14 @@ int pyrope_vindex_build(pyrope_vindex* v) {
     const bool had_buffer = !tl->buffered.empty() || !hd->row_of.empty();
     // move first, book-keeping second, the tail's Build last: if the build fails (out of memory in k-means, say) the id
     // tables already describe where every row is, so Delete / Upsert / Snapshot keep working and Build can be retried
-    LTRY(delta_move_with_ids(v));
-    VTRY(pyrope_delta_build_tail(v->d));
+    TRY(delta_move_with_ids(v));
+    TRY(pyrope_delta_build_tail(v->d));
     leaf_after_build(tl, had_buffer);
     return PYROPE_OK;
 }
 
 int pyrope_vindex_extend(pyrope_vindex* v) {
-    if (!v) return vfail(PYROPE_ERR_INVALID_ARG, "index handle is null");
+    if (!v) return fail(PYROPE_ERR_INVALID_ARG, "index handle is null");
     std::unique_lock<std::shared_mutex> g(v->lock);
     if (!v->d) return leaf_extend(v);
     // compaction by Extend: the move of pyrope_vindex_build, then the tail's Extend instead of its Build
@@ -618,43 +581,43 @@ int pyrope_vindex_extend(pyrope_vindex* v) {
     std::unique_lock<std::shared_mutex> gh(hd->lock);
     std::unique_lock<std::shared_mutex> gt(tl->lock);
     // a tail that cannot be extended refuses before any row moves
-    if (tl->kind == PYROPE_FLAT) return vfail(PYROPE_ERR_UNSUPPORTED, "Extend needs an IVF tail: FLAT has no inverted lists");
+    if (tl->kind == PYROPE_FLAT) return fail(PYROPE_ERR_UNSUPPORTED, "Extend needs an IVF tail: FLAT has no inverted lists");
     int built = 0;
-    LTRY(row_is_built(tl, &built));
-    if (!built) return vfail(PYROPE_ERR_INVALID_STATE, "Extend needs a built tail: call Build first");
-    LTRY(delta_move_with_ids(v));
-    VTRY(pyrope_delta_extend_tail(v->d));
+    TRY(row_is_built(tl, &built));
+    if (!built) return fail(PYROPE_ERR_INVALID_STATE, "Extend needs a built tail: call Build first");
+    TRY(delta_move_with_ids(v));
+    TRY(pyrope_delta_extend_tail(v->d));
     leaf_after_extend(tl);
     return PYROPE_OK;
 }
 
 int pyrope_vindex_search(pyrope_vindex* v, int64_t nq, const float* Q, int len, int topk, int64_t max_scans, int nprobe,
                          float* scores_out, int64_t* gids_out, int32_t* counts_out) {
-    if (!v) return vfail(PYROPE_ERR_INVALID_ARG, "index handle is null");
+    if (!v) return fail(PYROPE_ERR_INVALID_ARG, "index handle is null");
     const int kind = v->d ? (int)PYROPE_FLAT : v->kind;  // a delta validates like its FLAT head, which runs first
     if (kind != PYROPE_IVF_PQ) {                          // IvfPqVectorIndex.Search validates nothing (:118-125)
         int r = check_vec(v, Q, len);
         if (r != PYROPE_OK) return r;
     } else if (!Q || len != v->dim) {
-        return vfail(PYROPE_ERR_DIMENSION, "Vector dimension mismatch");
+        return fail(PYROPE_ERR_DIMENSION, "Vector dimension mismatch");
     }
     std::shared_lock<std::shared_mutex> g(v->lock);
-    if (v->d) return vpass(pyrope_delta_search_batch(v->d, nq, Q, topk, max_scans, nprobe, scores_out, gids_out, counts_out));
-    if (v->sh) return spass(pyrope_sharded_search_batch(v->sh, nq, Q, topk, max_scans, nprobe, scores_out, gids_out, counts_out));
-    return vpass(pyrope_index_search_batch(v->h, nq, Q, topk, max_scans, nprobe, scores_out, gids_out, counts_out));
+    if (v->d) return pyrope_delta_search_batch(v->d, nq, Q, topk, max_scans, nprobe, scores_out, gids_out, counts_out);
+    if (v->sh) return pyrope_sharded_search_batch(v->sh, nq, Q, topk, max_scans, nprobe, scores_out, gids_out, counts_out);
+    return pyrope_index_search_batch(v->h, nq, Q, topk, max_scans, nprobe, scores_out, gids_out, counts_out);
 }
 
 // csrc/batcher.cu (internal): what a Search with topK <= 0 or a large topK gives on this index, so the batcher can answer
 // such a caller alone.  max_topk: the largest topK Search accepts; nonpos_empty: topK <= 0 returns an empty result
 // (an IVF leaf) rather than OUT_OF_RANGE (a FLAT leaf, or a delta whose FLAT head validates first).
 int pyrope_internal_vindex_limits(pyrope_vindex* v, int* dim_out, int* max_topk_out, int* nonpos_empty_out) {
-    if (!v) return vfail(PYROPE_ERR_INVALID_ARG, "index handle is null");
+    if (!v) return fail(PYROPE_ERR_INVALID_ARG, "index handle is null");
     int lim = 1024, empty = 0;
     if (v->d) {
-        VTRY(pyrope_internal_delta_limits(v->d, nullptr, &lim));
+        TRY(pyrope_internal_delta_limits(v->d, nullptr, &lim));
     } else if (v->sh) {
         int n = 1;
-        LTRY(spass(pyrope_sharded_device_count(v->sh, &n)));
+        TRY(pyrope_sharded_device_count(v->sh, &n));
         lim = std::min(1024, 4096 / n);  // pyrope_sharded_search_batch: n x topK candidates in one merge
         empty = 1;
     } else {
@@ -672,20 +635,20 @@ int pyrope_internal_vindex_limits(pyrope_vindex* v, int* dim_out, int* max_topk_
 // query's own top topks[i] — the caller keeps those.
 int pyrope_internal_vindex_search_topk(pyrope_vindex* v, int64_t nq, const float* Q, const int32_t* topks, int64_t max_scans,
                                        int nprobe, float* scores_out, int64_t* gids_out, int32_t* counts_out) {
-    if (!v) return vfail(PYROPE_ERR_INVALID_ARG, "index handle is null");
-    if (nq > 0 && (!Q || !topks)) return vfail(PYROPE_ERR_INVALID_ARG, "null argument");
+    if (!v) return fail(PYROPE_ERR_INVALID_ARG, "index handle is null");
+    if (nq > 0 && (!Q || !topks)) return fail(PYROPE_ERR_INVALID_ARG, "null argument");
     std::shared_lock<std::shared_mutex> g(v->lock);
-    if (v->d) return vpass(pyrope_delta_search_batch_topk(v->d, nq, Q, topks, max_scans, nprobe, scores_out, gids_out, counts_out));
+    if (v->d) return pyrope_delta_search_batch_topk(v->d, nq, Q, topks, max_scans, nprobe, scores_out, gids_out, counts_out);
     int kmax = 1;
     for (int64_t i = 0; i < nq; ++i) kmax = std::max(kmax, (int)topks[i]);
-    if (v->sh) return spass(pyrope_sharded_search_batch(v->sh, nq, Q, kmax, max_scans, nprobe, scores_out, gids_out, counts_out));
-    return vpass(pyrope_index_search_batch(v->h, nq, Q, kmax, max_scans, nprobe, scores_out, gids_out, counts_out));
+    if (v->sh) return pyrope_sharded_search_batch(v->sh, nq, Q, kmax, max_scans, nprobe, scores_out, gids_out, counts_out);
+    return pyrope_index_search_batch(v->h, nq, Q, kmax, max_scans, nprobe, scores_out, gids_out, counts_out);
 }
 
 int pyrope_vindex_id(int64_t gid, char* buf, int cap, int* len_out) {
     std::lock_guard<std::mutex> g(g_id_mu);
     if (gid < 0 || gid >= (int64_t)g_ids.size() || !g_ids[(size_t)gid].used)
-        return vfail(PYROPE_ERR_NOT_FOUND, "unknown id ordinal %lld", (long long)gid);
+        return fail(PYROPE_ERR_NOT_FOUND, "unknown id ordinal %lld", (long long)gid);
     const std::string& s = g_ids[(size_t)gid].s;
     if (len_out) *len_out = (int)s.size();
     if (buf && cap > 0) {
@@ -697,7 +660,7 @@ int pyrope_vindex_id(int64_t gid, char* buf, int cap, int* len_out) {
 }
 
 int pyrope_vindex_ids(const int64_t* gids, int64_t n, char* buf, int64_t cap, int64_t* offsets_out, int64_t* bytes_out) {
-    if (n < 0 || (n > 0 && (!gids || !offsets_out))) return vfail(PYROPE_ERR_INVALID_ARG, "null argument");
+    if (n < 0 || (n > 0 && (!gids || !offsets_out))) return fail(PYROPE_ERR_INVALID_ARG, "null argument");
     std::lock_guard<std::mutex> g(g_id_mu);  // one lock for the whole result list
     int64_t o = 0;
     for (int64_t i = 0; i < n; ++i) {
@@ -705,7 +668,7 @@ int pyrope_vindex_ids(const int64_t* gids, int64_t n, char* buf, int64_t cap, in
         const int64_t gid = gids[i];
         if (gid < 0) continue;  // an empty result slot: zero-length string
         if (gid >= (int64_t)g_ids.size() || !g_ids[(size_t)gid].used)
-            return vfail(PYROPE_ERR_NOT_FOUND, "unknown id ordinal %lld", (long long)gid);
+            return fail(PYROPE_ERR_NOT_FOUND, "unknown id ordinal %lld", (long long)gid);
         const std::string& s = g_ids[(size_t)gid].s;
         if (buf && o + (int64_t)s.size() <= cap) memcpy(buf + o, s.data(), s.size());
         o += (int64_t)s.size();
@@ -723,7 +686,7 @@ int pyrope_vindex_id_table_size(int64_t* live_out, int64_t* slots_out) {
 }
 
 int pyrope_vindex_stats(pyrope_vindex* v, int64_t* count_out, int* dim_out, int* metric_out) {
-    if (!v) return vfail(PYROPE_ERR_INVALID_ARG, "index handle is null");
+    if (!v) return fail(PYROPE_ERR_INVALID_ARG, "index handle is null");
     std::shared_lock<std::shared_mutex> g(v->lock);
     if (count_out) *count_out = v->d ? leaf_count(v->head) + leaf_count(v->tail) : leaf_count(v);  // DeltaVectorIndex.cs:232-236
     if (dim_out) *dim_out = v->dim;
@@ -732,33 +695,33 @@ int pyrope_vindex_stats(pyrope_vindex* v, int64_t* count_out, int* dim_out, int*
 }
 
 int pyrope_vindex_get_centroids(pyrope_vindex* v, float* centroids_out, int* n_out) {
-    if (!v || !n_out) return vfail(PYROPE_ERR_INVALID_ARG, "null argument");
+    if (!v || !n_out) return fail(PYROPE_ERR_INVALID_ARG, "null argument");
     std::shared_lock<std::shared_mutex> g(v->lock);
     V* leaf = v->d ? v->tail : v;  // DeltaVectorIndex.cs:241-252: the tail's, if it has any
     *n_out = 0;
     if (leaf->kind == PYROPE_FLAT) return PYROPE_OK;  // not an ICentroidsProvider -> null
-    if (leaf->sh) return spass(pyrope_sharded_get_centroids(leaf->sh, centroids_out, n_out));
-    return vpass(pyrope_index_get_centroids(leaf->h, centroids_out, n_out));
+    if (leaf->sh) return pyrope_sharded_get_centroids(leaf->sh, centroids_out, n_out);
+    return pyrope_index_get_centroids(leaf->h, centroids_out, n_out);
 }
 
 int pyrope_vindex_snapshot(pyrope_vindex* v, const char* path) {
-    if (!v) return vfail(PYROPE_ERR_INVALID_ARG, "index handle is null");
-    if (blank(path)) return vfail(PYROPE_ERR_INVALID_ARG, "Path cannot be empty. (Parameter 'path')");  // BruteForceVectorIndex.cs:60
+    if (!v) return fail(PYROPE_ERR_INVALID_ARG, "index handle is null");
+    if (blank(path)) return fail(PYROPE_ERR_INVALID_ARG, "Path cannot be empty. (Parameter 'path')");  // BruteForceVectorIndex.cs:60
     std::shared_lock<std::shared_mutex> g(v->lock);
     const std::string base(path);
     if (!v->d) {
-        LTRY(row_snapshot(v, path));
+        TRY(row_snapshot(v, path));
         return leaf_save_ids(v, base + ".ids");
     }
-    VTRY(pyrope_delta_snapshot(v->d, path));
+    TRY(pyrope_delta_snapshot(v->d, path));
     int r = leaf_save_ids(v->head, base + ".head.ids");
     if (r != PYROPE_OK) return r;
     return leaf_save_ids(v->tail, base + ".tail.ids");
 }
 
 int pyrope_vindex_load(pyrope_vindex* v, const char* path) {
-    if (!v) return vfail(PYROPE_ERR_INVALID_ARG, "index handle is null");
-    if (blank(path)) return vfail(PYROPE_ERR_INVALID_ARG, "Path cannot be empty. (Parameter 'path')");
+    if (!v) return fail(PYROPE_ERR_INVALID_ARG, "index handle is null");
+    if (blank(path)) return fail(PYROPE_ERR_INVALID_ARG, "Path cannot be empty. (Parameter 'path')");
     std::unique_lock<std::shared_mutex> g(v->lock);
     const std::string base(path);
     if (!v->d) return leaf_load(v, base);

@@ -16,7 +16,7 @@ class FormatException(ValueError):
 
 
 def _err():
-    return (_lib.load().pyrope_formats_last_error() or b"").decode("utf-8", "replace")
+    return (_lib.load().pyrope_last_error() or b"").decode("utf-8", "replace")
 
 
 def _ck(rc):

@@ -79,7 +79,7 @@ def _raise_msg(rc: int, msg: str):
 
 
 def _raise(rc: int):
-    _raise_msg(rc, (_lib.load().pyrope_vindex_last_error() or b"").decode("utf-8", "replace"))
+    _raise_msg(rc, (_lib.load().pyrope_last_error() or b"").decode("utf-8", "replace"))
 
 
 def _id_string(ordinal: int) -> str:
@@ -353,10 +353,7 @@ class VectorIndexBatcher:
         ms, npb = _options(options)
         kk = max(int(topK), 1)
         scores, ids, cnt = np.zeros(kk, np.float32), np.full(kk, -1, np.int64), C.c_int32(0)
-        L = _lib.load()
-        rc = L.pyrope_batcher_search(self._b._b, _p(q), int(topK), ms, npb, _p(scores), _p(ids), C.byref(cnt))
-        if rc != _lib.OK:
-            _raise_msg(rc, (L.pyrope_batcher_last_error() or b"").decode("utf-8", "replace"))
+        _ck(_lib.load().pyrope_batcher_search(self._b._b, _p(q), int(topK), ms, npb, _p(scores), _p(ids), C.byref(cnt)))
         n = cnt.value
         names = _id_strings(ids[:n]) if n else []
         return [SearchResult(names[j], float(scores[j])) for j in range(n)]
