@@ -1330,7 +1330,7 @@ int search_device(Index* h, int64_t nq, const float* dQ, int topk, int64_t max_s
             launches += 2;
         }
         // IvfFlatVectorIndex.cs:186-198 / IvfPqVectorIndex.cs:141-150: rank by the reference's own arithmetic
-        CK(launch_coarse_rerank_exact(h->metric, dim, nq, dQ, h->centroids.as<float>(), h->cnorms.as<float>(),
+        CK(launch_coarse_rerank_exact(h->metric, dim, nq, dQ, h->centroids.as<float>(), h->cnorms.as<float>(), h->nc,
                                       ws.probes_raw.as<int64_t>(), ws.probe_scores.as<float>(), Pc, ws.probes.as<int64_t>(),
                                       nullptr, P, (h->kind == PYROPE_IVF_FLAT && max_scans >= 0) ? 1 : 0, st));
         ++launches;

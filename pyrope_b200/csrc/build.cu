@@ -135,22 +135,30 @@ __global__ void scatter_i32_kernel(const int32_t* src, const int64_t* idx, int64
 // (VectorMath.L2Squared / DotProduct / Cosine, single 8-lane accumulator) and the best P_out are emitted in
 // descending order (ties to the lower list index), so the probed set equals the oracle's even when two
 // centroids score within a rounding error of each other.  One CTA per query.
+//
+// The stage-one scores (fp32, another summation order) settle the probed SET when the P_out-th and (P_out+1)-th are
+// further apart than both their errors.  For L2 the summed terms are non-negative and the error is relative to the
+// score; for IP and Cosine it is gamma * sum|q_i c_i|, at most gamma |q| |c| (Cosine: gamma), whatever the score, so near
+// 0 (centroids orthogonal to the query) a relative margin settles nothing.  When even the last candidate lies within
+// that band of the P_out-th, a centroid the stage left out may belong to the set: every centroid is ranked exactly.
 template <int METRIC>
 __global__ void __launch_bounds__(128) coarse_rerank_kernel(const float* __restrict__ Q, int dim,
                                                             const float* __restrict__ C, const float* __restrict__ cnorms,
-                                                            const int64_t* __restrict__ pin,
+                                                            int nc, const int64_t* __restrict__ pin,
                                                             const float* __restrict__ sin, int P_in,
-                                                            int64_t* pout, float* sout, int P_out, int Psort, int need_order) {
+                                                            int64_t* pout, float* sout, int P_out, int Psort, int H,
+                                                            int need_order) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
-    uint64_t* keys = reinterpret_cast<uint64_t*>(smem_raw);   // [Psort]
-    float* qs = reinterpret_cast<float*>(keys + Psort);       // [dim]
+    uint64_t* keys = reinterpret_cast<uint64_t*>(smem_raw);   // [max(Psort, 2 H)]
+    float* qs = reinterpret_cast<float*>(keys + max(Psort, 2 * H));  // [dim]
     __shared__ float s_qn;
+    __shared__ unsigned s_cmax;
     const int64_t q = blockIdx.x;
     const int tid = threadIdx.x;
-    // Fast path: the stage-one scores (fp32, accurate to ~1e-6 relative, sorted descending) already separate the
-    // P_out-th from the (P_out+1)-th candidate by far more than their rounding error, so the probed SET is
-    // settled; unless the caller needs the exact order too (MaxScans budgets walk lists in rank order), copy.
-    if (!need_order && sin && !sout) {
+    // L2 fast path: the stage-one scores (accurate to ~1e-6 relative, sorted descending) already separate the
+    // P_out-th from the (P_out+1)-th candidate by far more than their rounding error, so the probed SET is settled;
+    // unless the caller needs the exact order too (MaxScans budgets walk lists in rank order), copy.
+    if (METRIC == 0 && !need_order && sin && !sout) {
         bool settled = P_in <= P_out;
         if (!settled) {
             const float a = sin[q * P_in + P_out - 1], b = sin[q * P_in + P_out];
@@ -162,31 +170,62 @@ __global__ void __launch_bounds__(128) coarse_rerank_kernel(const float* __restr
         }
     }
     for (int d = tid; d < dim; d += blockDim.x) qs[d] = Q[q * dim + d];
+    if (tid == 0) s_cmax = 0u;
     __syncthreads();
-    if (METRIC == 2 && tid == 0) s_qn = norm_eval(qs, dim);
-    __syncthreads();
-    for (int i = tid; i < Psort; i += blockDim.x) {
-        uint64_t key = 0ull;
-        if (i < P_in) {
-            const int64_t l = pin[q * P_in + i];
-            if (l >= 0) {
-                const float* cv = C + l * dim;
-                float s;
-                if (METRIC == 0) s = -a2_eval<0>(qs, cv, dim);
-                else if (METRIC == 1) s = a2_eval<1>(qs, cv, dim);
-                else {
-                    const float cn = cnorms[l];
-                    s = (s_qn < 1e-6f || cn < 1e-6f) ? 0.f : __fdiv_rn(a2_eval<1>(qs, cv, dim), __fmul_rn(s_qn, cn));
-                }
-                key = make_key(s, (uint32_t)l);
+    if (METRIC != 0 && tid == 0) s_qn = norm_eval(qs, dim);
+    bool exhaustive = false;
+    if (METRIC != 0 && sin && P_in > P_out) {
+        if (METRIC == 1) {  // |c| of the candidates (fp32, rounded up below)
+            for (int i = tid; i < P_in; i += blockDim.x) {
+                const int64_t l = pin[q * P_in + i];
+                if (l >= 0) atomicMax(&s_cmax, __float_as_uint(norm_eval(C + l * dim, dim)));
             }
         }
-        keys[i] = key;
+        __syncthreads();
+        // two orders of at most dim terms differ by <= (dim / 4 + 24) 2^-24 sum|term| (as ivf_lm.cu's fl_gamma)
+        const float gam = (float)(dim / 4 + 24) * 0x1p-24f;
+        const float e = METRIC == 2 ? gam : gam * s_qn * __uint_as_float(s_cmax) * (1.f + 0x1p-10f);
+        const float a = sin[q * P_in + P_out - 1], b = sin[q * P_in + P_out], last = sin[q * P_in + P_in - 1];
+        exhaustive = P_in < nc && pin[q * P_in + P_in - 1] >= 0 && last >= a - 2.f * e - 1e-30f;
+        if (!exhaustive && !need_order && !sout && (pin[q * P_in + P_out] < 0 || a - b > 2.f * e + 1e-30f)) {
+            for (int i = tid; i < P_out; i += blockDim.x) pout[q * P_out + i] = pin[q * P_in + i];
+            return;  // block-uniform
+        }
     }
     __syncthreads();
-    bitonic_sort_desc<false>(keys, Psort, tid, blockDim.x);
+    auto exact_key = [&](int64_t l) -> uint64_t {
+        const float* cv = C + l * dim;
+        float s;
+        if (METRIC == 0) s = -a2_eval<0>(qs, cv, dim);
+        else if (METRIC == 1) s = a2_eval<1>(qs, cv, dim);
+        else {
+            const float cn = cnorms[l];
+            s = (s_qn < 1e-6f || cn < 1e-6f) ? 0.f : __fdiv_rn(a2_eval<1>(qs, cv, dim), __fmul_rn(s_qn, cn));
+        }
+        return make_key(s, (uint32_t)l);
+    };
+    int P;
+    if (exhaustive) {  // every centroid, H at a time, merged into the best H
+        P = 2 * H;
+        for (int i = tid; i < H; i += blockDim.x) keys[i] = 0ull;
+        for (int c0 = 0; c0 < nc; c0 += H) {
+            for (int i = tid; i < H; i += blockDim.x) keys[H + i] = c0 + i < nc ? exact_key(c0 + i) : 0ull;
+            __syncthreads();
+            bitonic_sort_desc<false>(keys, P, tid, blockDim.x);
+            __syncthreads();
+        }
+    } else {
+        P = Psort;
+        for (int i = tid; i < Psort; i += blockDim.x) {
+            const int64_t l = i < P_in ? pin[q * P_in + i] : -1;
+            keys[i] = l >= 0 ? exact_key(l) : 0ull;
+        }
+        __syncthreads();
+        bitonic_sort_desc<false>(keys, P, tid, blockDim.x);
+        __syncthreads();
+    }
     for (int i = tid; i < P_out; i += blockDim.x) {
-        const uint64_t key = keys[i];
+        const uint64_t key = i < P ? keys[i] : 0ull;
         pout[q * P_out + i] = key ? (int64_t)key_pos(key) : -1;
         if (sout) sout[q * P_out + i] = key ? key_score(key) : 0.f;
     }
@@ -358,17 +397,19 @@ cudaError_t launch_scatter_i32(const int32_t* src, const int64_t* idx, int64_t n
 }
 
 cudaError_t launch_coarse_rerank_exact(int metric, int dim, int64_t nq, const float* Q, const float* centroids,
-                                       const float* cnorms, const int64_t* probes_in, const float* scores_in, int P_in,
+                                       const float* cnorms, int nc, const int64_t* probes_in, const float* scores_in, int P_in,
                                        int64_t* probes_out, float* scores_out, int P_out, int need_order, cudaStream_t st) {
     if (nq <= 0) return cudaSuccess;
     const int Psort = next_pow2(P_in < 2 ? 2 : P_in);
-    const size_t smem = sizeof(uint64_t) * (size_t)Psort + sizeof(float) * (size_t)dim;
+    const int H = metric == kL2 ? 0 : next_pow2(P_out < 64 ? 64 : P_out);  // the exhaustive ranking's merge width
+    const size_t smem = sizeof(uint64_t) * (size_t)std::max(Psort, 2 * H) + sizeof(float) * (size_t)dim;
+    if (smem > 48 * 1024) return cudaErrorInvalidValue;
     if (metric == kL2)
-        coarse_rerank_kernel<0><<<(unsigned)nq, 128, smem, st>>>(Q, dim, centroids, cnorms, probes_in, scores_in, P_in, probes_out, scores_out, P_out, Psort, need_order);
+        coarse_rerank_kernel<0><<<(unsigned)nq, 128, smem, st>>>(Q, dim, centroids, cnorms, nc, probes_in, scores_in, P_in, probes_out, scores_out, P_out, Psort, H, need_order);
     else if (metric == kIP)
-        coarse_rerank_kernel<1><<<(unsigned)nq, 128, smem, st>>>(Q, dim, centroids, cnorms, probes_in, scores_in, P_in, probes_out, scores_out, P_out, Psort, need_order);
+        coarse_rerank_kernel<1><<<(unsigned)nq, 128, smem, st>>>(Q, dim, centroids, cnorms, nc, probes_in, scores_in, P_in, probes_out, scores_out, P_out, Psort, H, need_order);
     else
-        coarse_rerank_kernel<2><<<(unsigned)nq, 128, smem, st>>>(Q, dim, centroids, cnorms, probes_in, scores_in, P_in, probes_out, scores_out, P_out, Psort, need_order);
+        coarse_rerank_kernel<2><<<(unsigned)nq, 128, smem, st>>>(Q, dim, centroids, cnorms, nc, probes_in, scores_in, P_in, probes_out, scores_out, P_out, Psort, H, need_order);
     return cudaGetLastError();
 }
 

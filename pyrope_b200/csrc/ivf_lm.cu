@@ -6,8 +6,8 @@
 // device, same scheme as pq_lm.cu) and one work item is one inverted list x up to 16 of the queries that
 // probe it, so a row fetched from L2/HBM is scored against 16 queries.
 //
-//   ivf_lm_seed_kernel   per query, a lower bound of its k-th best score from a sample of its nearest list
-//                        (exact fp32), so no item starts without a threshold;
+//   ivf_lm_seed_kernel   per query, a lower bound of its k-th best score from a sample of its nearest list, less the
+//                        slack two summation orders can differ by (fl_gamma), so no item starts without a threshold;
 //   ivf_lm_scan_kernel   persistent CTAs, static item striding, 8 warps.  Lane l holds dimensions 4l..4l+3 of
 //                        the item's 16 queries in registers (packed pairs for FFMA2/FADD2); a warp takes two
 //                        rows at a time (one coalesced 128-bit load per lane and row, prefetched), forms the
@@ -16,10 +16,11 @@
 //                        against that query's threshold.  Candidates go to a per-slot queue; after the item
 //                        one warp per slot hands at most k of them to the pair's private pool region and
 //                        tightens the query's threshold (atomicMax);
-//   ivf_lm_redo_kernel   plain scan of a (query, list) whose queue overflowed;
-//   ivf_lm_final_kernel  best k of the pool, RE-SCORED in the reference's evaluation order
-//                        (VectorMath.L2Squared / DotProduct, VectorMath.cs:8-70) so reported scores are the
-//                        oracle's bit for bit, then ordered.
+//   ivf_lm_redo_kernel   plain scan, in the reference's order, of a (query, list) whose queue overflowed or whose
+//                        best k could not be told from the rest within the slack;
+//   ivf_lm_final_kernel  every pool entry within the slack of the k-th, RE-SCORED in the reference's evaluation order
+//                        (VectorMath.L2Squared / DotProduct, VectorMath.cs:8-70), the best k of them reported: the
+//                        oracle's rows and scores bit for bit.
 // Shapes: L2 / inner product / cosine, dim % 4 == 0 and dim <= 1024 (rows wider than 128 floats take the *_wide kernels),
 // no MaxScans budget; everything else takes ivf.cu.
 #include <cub/cub.cuh>
@@ -117,12 +118,28 @@ __device__ __forceinline__ float inv_norm(const float* __restrict__ norms, int64
     return n < 1e-6f ? 0.f : 1.f / n;
 }
 
+// The seed, the scan, the redo and VectorMath (the reference) sum a row's products in different orders.  Each order is
+// within gamma_n sum|term| of the exact sum, n its depth: d/8 + 8 for the reference, at most d/32 + 9 here; two of them
+// differ by at most fl_gamma(d) sum|term| (the slack also covers the 1 / (1 - n u) factors and Cosine's scaling).  L2's
+// terms are non-negative, so sum|term| is the score's magnitude; for IP and the Cosine proxy it is not bounded by the
+// score at all (rows orthogonal to the query score rounding noise), and the seed bounds it (FlSeed::band).
+__host__ __device__ __forceinline__ float fl_gamma(int dim) { return (float)(dim / 4 + 24) * 0x1p-24f; }
+// how far below a score t another order can put a row that ranks with t in the reference's order, twice over (the row's
+// own error and the error of the row that set t): band = fl_gamma * max sum|term| (0 for L2)
+__device__ __forceinline__ float fl_slack(float t, float band, float gam) { return 2.f * (band + gam * fabsf(t)) + 1e-30f; }
+
+__device__ __forceinline__ float warp_abs(const float4 qv, const float4 xv) {
+    return warp_sum(fmaf(fabsf(qv.x), fabsf(xv.x), fmaf(fabsf(qv.y), fabsf(xv.y), fmaf(fabsf(qv.z), fabsf(xv.z), fabsf(qv.w * xv.w)))));
+}
+
 // ---- seed: a lower bound of every query's k-th best score -------------------------------------------------
 struct FlSeed {
     const float* Q; int64_t nq; int dim; const int64_t* probes; int P;
     const float* vecs; const uint8_t* dead; const int64_t* list_off;
     uint32_t* pool_thr; int k;
     const float* norms;  // Cosine: |x| per list entry
+    float* band;         // per query, fl_gamma times a bound of sum|q_i x_i|: IP, the largest over the rows sampled;
+                         // Cosine (the proxy divides by |x|), |q| (Cauchy-Schwarz)
 };
 template <int METRIC>
 __global__ void __launch_bounds__(256) ivf_lm_seed_kernel(FlSeed a) {
@@ -136,7 +153,8 @@ __global__ void __launch_bounds__(256) ivf_lm_seed_kernel(FlSeed a) {
 #pragma unroll
     for (int u = 0; u < U; ++u) sc[u] = -INFINITY;
     int got = 0;
-    for (int pr = 0; pr < a.P && got < max(a.k, 32); ++pr) {
+    float amax = 0.f;
+    for (int pr = 0; pr < a.P && got < min(max(a.k, 32), FSEED); ++pr) {
         const int64_t l = a.probes[q * a.P + pr];
         if (l < 0) continue;
         const int64_t beg = a.list_off[l], len = a.list_off[l + 1] - beg;
@@ -155,6 +173,7 @@ __global__ void __launch_bounds__(256) ivf_lm_seed_kernel(FlSeed a) {
                 if (ok[u] && got < FSEED) {
                     float s = warp_score<METRIC>(qv, xv[u]);
                     if (METRIC == kCosine) s *= inv_norm(a.norms, beg + v0 + u);
+                    if (METRIC == kIP) amax = fmaxf(amax, warp_abs(qv, xv[u]));
 #pragma unroll
                     for (int w = 0; w < U; ++w)
                         if ((got >> 5) == w && (got & 31) == lane) sc[w] = s;
@@ -163,6 +182,9 @@ __global__ void __launch_bounds__(256) ivf_lm_seed_kernel(FlSeed a) {
             }
         }
     }
+    if (METRIC == kCosine) amax = sqrtf(warp_abs(qv, qv));  // sum|q_i x_i| / |x| <= |q| for every row
+    const float gam = fl_gamma(a.dim), band = gam * amax * (1.f + 0x1p-10f);
+    if (lane == 0) a.band[q] = band;
     if (got < a.k) return;  // fewer candidates than k so far: no threshold (everything is kept)
     // k-th largest of the sampled scores by bisection on the ordered bits
     uint32_t o[U], lo = 0xffffffffu, hi = 0u;
@@ -182,9 +204,9 @@ __global__ void __launch_bounds__(256) ivf_lm_seed_kernel(FlSeed a) {
         if (c >= a.k) lo = mid; else hi = mid - 1u;
     }
     if (lane == 0) {
-        // the scan kernel sums the same products in another order: leave room for its rounding
+        // the scan sums the same products in another order, the final ranking in the reference's: leave room for both
         const float t = ord_to_score(lo);
-        const float tl = t - 2e-5f * fabsf(t) - 1e-30f;
+        const float tl = t - fl_slack(t, band, gam);
         a.pool_thr[q] = score_to_ord(tl) - 1u;  // accept iff score >= tl
     }
 }
@@ -196,11 +218,16 @@ struct FlParams {
     unsigned long long* pool; int32_t* pool_cnt; uint32_t* pool_thr; int pslots; int k;
     int2* redo; int32_t* redo_cnt;
     const float* norms;  // Cosine: |x| per list entry
+    const float* band;   // FlSeed::band
 };
 
 // ---- after an item: hand at most k candidates per slot to the pair's private pool region, tighten the threshold ------
+// The pool keeps the best k of a pair by the scan's scores.  When the best one left out is within the slack of the k-th,
+// the cut may disagree with the reference's order: the pair goes to the redo kernel, which ranks in that order.  The
+// published threshold trails the k-th by the slack, so no row the reference ranks above it is turned away.
+template <int METRIC>
 __device__ __forceinline__ void fl_hand_over(const FlParams& p, int it, uint64_t* qkeys, int* s_qcnt, const int* s_qid,
-                                             const int* s_psl, int warp, int lane) {
+                                             const int* s_psl, int warp, int lane, float gam) {
     for (int j = warp; j < FG; j += FT / 32) {
         const int n = s_qcnt[j];
         const int q = s_qid[j];
@@ -211,7 +238,7 @@ __device__ __forceinline__ void fl_hand_over(const FlParams& p, int it, uint64_t
             } else {
                 const size_t ps = (size_t)q * p.pslots + s_psl[j];
                 unsigned long long* dst = p.pool + ps * p.k;
-                uint64_t mink = ~0ull;
+                uint64_t mink = ~0ull, next = 0ull;  // the k-th kept, the best left out
                 int kept;
                 if (n > p.k && n <= 64) {  // select by rank counting inside the warp
                     const uint64_t a = lane < n ? kq[lane] : 0ull, b = lane + 32 < n ? kq[lane + 32] : 0ull;
@@ -227,6 +254,8 @@ __device__ __forceinline__ void fl_hand_over(const FlParams& p, int it, uint64_t
                     const unsigned below = (1u << lane) - 1u;
                     if (ka) { dst[__popc(ma & below)] = a; mink = a; }
                     if (kb) { dst[__popc(ma) + __popc(mb & below)] = b; mink = b < mink ? b : mink; }
+                    if (lane < n && !ka) next = a;
+                    if (lane + 32 < n && !kb) next = b > next ? b : next;
                 } else {
                     if (n > p.k) {
                         const int P2 = next_pow2(n);
@@ -240,15 +269,23 @@ __device__ __forceinline__ void fl_hand_over(const FlParams& p, int it, uint64_t
                         dst[i] = x;
                         mink = x < mink ? x : mink;
                     }
+                    if (n > p.k) next = kq[p.k];
                 }
                 if (lane == 0) p.pool_cnt[ps] = kept;
                 if (kept >= p.k) {
 #pragma unroll
                     for (int o = 16; o > 0; o >>= 1) {
-                        const uint64_t x = __shfl_xor_sync(0xffffffffu, mink, o);
+                        const uint64_t x = __shfl_xor_sync(0xffffffffu, mink, o), y = __shfl_xor_sync(0xffffffffu, next, o);
                         mink = x < mink ? x : mink;
+                        next = y > next ? y : next;
                     }
-                    if (lane == 0) atomicMax(p.pool_thr + q, (uint32_t)(mink >> 32));
+                    if (lane == 0) {
+                        const float m = key_score(mink), band = p.band[q];
+                        const float lim = m - fl_slack(m, band, gam);
+                        atomicMax(p.pool_thr + q, score_to_ord(lim) - 1u);
+                        // L2's slack is relative: a cut inside it is a tie within 2 fl_gamma of the score
+                        if (METRIC != kL2 && next && key_score(next) >= lim) p.redo[atomicAdd(p.redo_cnt, 1)] = make_int2(q, it * FG + j);
+                    }
                 }
             }
         }
@@ -266,6 +303,7 @@ __global__ void __launch_bounds__(FT, 2) ivf_lm_scan_kernel(FlParams p) {
     const int n_items = *p.n_items;
     const int dim = p.dim;
     const bool lane_on = lane * 4 < dim;
+    const float gam = fl_gamma(dim);
     if (tid < FG) s_qcnt[tid] = 0;
     __syncthreads();
 
@@ -354,7 +392,7 @@ __global__ void __launch_bounds__(FT, 2) ivf_lm_scan_kernel(FlParams p) {
             }
         }
         __syncthreads();
-        fl_hand_over(p, it, qkeys, s_qcnt, s_qid, s_psl, warp, lane);
+        fl_hand_over<METRIC>(p, it, qkeys, s_qcnt, s_qid, s_psl, warp, lane, gam);
         __syncthreads();
     }
 }
@@ -386,6 +424,14 @@ __device__ __forceinline__ float warp_score_wide(const float* __restrict__ q, co
     a = warp_sum(a);
     return METRIC == kL2 ? -a : a;
 }
+__device__ __forceinline__ float warp_abs_wide(const float* __restrict__ q, const float* __restrict__ x, int dim, int lane) {
+    float a = 0.f;
+    for (int c = lane * 4; c < dim; c += 128) {
+        const float4 qv = __ldg(reinterpret_cast<const float4*>(q + c)), xv = __ldg(reinterpret_cast<const float4*>(x + c));
+        a = fmaf(fabsf(qv.x), fabsf(xv.x), fmaf(fabsf(qv.y), fabsf(xv.y), fmaf(fabsf(qv.z), fabsf(xv.z), fmaf(fabsf(qv.w), fabsf(xv.w), a))));
+    }
+    return warp_sum(a);
+}
 
 template <int METRIC>
 __global__ void __launch_bounds__(256) ivf_lm_seed_wide_kernel(FlSeed a) {
@@ -398,6 +444,7 @@ __global__ void __launch_bounds__(256) ivf_lm_seed_wide_kernel(FlSeed a) {
     for (int u = 0; u < U; ++u) sc[u] = -INFINITY;
     const int want = FSEEDW;
     int got = 0;
+    float amax = 0.f;
     for (int pr = 0; pr < a.P && got < want; ++pr) {
         const int64_t l = a.probes[q * a.P + pr];
         if (l < 0) continue;
@@ -406,12 +453,16 @@ __global__ void __launch_bounds__(256) ivf_lm_seed_wide_kernel(FlSeed a) {
             if (a.dead && a.dead[beg + v]) continue;  // warp-uniform
             float s = warp_score_wide<METRIC>(a.Q + q * a.dim, a.vecs + (beg + v) * a.dim, a.dim, lane);
             if (METRIC == kCosine) s *= inv_norm(a.norms, beg + v);
+            if (METRIC == kIP) amax = fmaxf(amax, warp_abs_wide(a.Q + q * a.dim, a.vecs + (beg + v) * a.dim, a.dim, lane));
 #pragma unroll
             for (int w = 0; w < U; ++w)
                 if ((got >> 5) == w && (got & 31) == lane) sc[w] = s;
             ++got;
         }
     }
+    if (METRIC == kCosine) amax = sqrtf(warp_abs_wide(a.Q + q * a.dim, a.Q + q * a.dim, a.dim, lane));  // |q|
+    const float gam = fl_gamma(a.dim), band = gam * amax * (1.f + 0x1p-10f);
+    if (lane == 0) a.band[q] = band;
     if (got < a.k) return;  // fewer candidates than k so far: no threshold (everything is kept)
     uint32_t o[U], lo = 0xffffffffu, hi = 0u;
 #pragma unroll
@@ -431,7 +482,7 @@ __global__ void __launch_bounds__(256) ivf_lm_seed_wide_kernel(FlSeed a) {
     }
     if (lane == 0) {
         const float t = ord_to_score(lo);
-        const float tl = t - 2e-5f * fabsf(t) - 1e-30f;  // the scan kernel sums the same products in another order
+        const float tl = t - fl_slack(t, band, gam);  // room for the scan's and the reference's summation orders
         a.pool_thr[q] = score_to_ord(tl) - 1u;
     }
 }
@@ -447,6 +498,7 @@ __global__ void __launch_bounds__(FT, 2) ivf_lm_scan_wide_kernel(FlParams p, int
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int n_items = *p.n_items;
     const int dim = p.dim;
+    const float gam = fl_gamma(dim);
     if (tid < FG) s_qcnt[tid] = 0;
     __syncthreads();
 
@@ -555,12 +607,14 @@ __global__ void __launch_bounds__(FT, 2) ivf_lm_scan_wide_kernel(FlParams p, int
             }
         }
         __syncthreads();
-        fl_hand_over(p, it, qkeys, s_qcnt, s_qid, s_psl, warp, lane);
+        fl_hand_over<METRIC>(p, it, qkeys, s_qcnt, s_qid, s_psl, warp, lane, gam);
         __syncthreads();
     }
 }
 
-// ---- redo: plain scan of one (query, list) whose queue overflowed -------------------------------------------
+// ---- redo: plain scan of one (query, list) whose queue overflowed or whose cut fell inside the slack -------------
+// IP / Cosine: one thread per row, in the reference's summation order, so the best k it keeps are the reference's (the
+// Cosine proxy divides by the row's norm as the scan does).  L2: one warp per row in the scan's order.
 struct FlRedo {
     const float* Q; int dim; const float* vecs; const uint8_t* dead; const int64_t* list_off;
     const int2* items; const int32_t* pair_off; const int32_t* pairp;
@@ -573,6 +627,7 @@ template <int METRIC>
 __global__ void __launch_bounds__(256) ivf_lm_redo_kernel(FlRedo a) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     uint64_t* keys = reinterpret_cast<uint64_t*>(smem_raw);  // [FREDO_QCAP]
+    float* qs = reinterpret_cast<float*>(keys + FREDO_QCAP);  // [dim]
     __shared__ int s_cnt;
     __shared__ uint64_t s_thr;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -588,19 +643,30 @@ __global__ void __launch_bounds__(256) ivf_lm_redo_kernel(FlRedo a) {
         Qu.reset(tid);
         __syncthreads();
         if (tid == 0) s_thr = (uint64_t)__ldcg(a.pool_thr + en.x) << 32;  // keys at or below it cannot be in the top k
+        for (int d = tid; d < a.dim; d += 256) qs[d] = a.Q[(size_t)en.x * a.dim + d];
         __syncthreads();
-        float4 qv = make_float4(0.f, 0.f, 0.f, 0.f);
-        const bool wide = a.dim > 128;
-        if (!wide && lane * 4 < a.dim) qv = __ldg(reinterpret_cast<const float4*>(a.Q + (size_t)en.x * a.dim) + lane);
         for (int64_t c0 = 0; c0 < len; c0 += 256) {
             if (s_cnt + 256 > FREDO_QCAP) Qu.prune(tid, 256);
-            for (int64_t v = c0 + warp; v < min(len, c0 + 256); v += 8) {
-                float4 xv = make_float4(0.f, 0.f, 0.f, 0.f);
-                if (!wide && lane * 4 < a.dim) xv = __ldg(reinterpret_cast<const float4*>(a.vecs + (beg + v) * a.dim) + lane);
-                float s = wide ? warp_score_wide<METRIC>(a.Q + (size_t)en.x * a.dim, a.vecs + (beg + v) * a.dim, a.dim, lane)
-                               : warp_score<METRIC>(qv, xv);
+            if (METRIC == kL2) {
+                const bool wide = a.dim > 128;
+                float4 qv = make_float4(0.f, 0.f, 0.f, 0.f);
+                if (!wide && lane * 4 < a.dim) qv = reinterpret_cast<const float4*>(qs)[lane];
+                for (int64_t v = c0 + warp; v < min(len, c0 + 256); v += 8) {
+                    float4 xv = make_float4(0.f, 0.f, 0.f, 0.f);
+                    if (!wide && lane * 4 < a.dim) xv = __ldg(reinterpret_cast<const float4*>(a.vecs + (beg + v) * a.dim) + lane);
+                    const float s = wide ? warp_score_wide<kL2>(a.Q + (size_t)en.x * a.dim, a.vecs + (beg + v) * a.dim, a.dim, lane)
+                                         : warp_score<kL2>(qv, xv);
+                    if (lane == 0 && !(a.dead && a.dead[beg + v])) Qu.push(make_key(s, (uint32_t)(beg + v)));
+                }
+                __syncthreads();
+                continue;
+            }
+            const int64_t v = c0 + tid;
+            if (v < len && !(a.dead && a.dead[beg + v])) {
+                const float* x = a.vecs + (beg + v) * a.dim;
+                float s = METRIC == kL2 ? -exact::a2_eval<0>(qs, x, a.dim) : exact::a2_eval<1>(qs, x, a.dim);
                 if (METRIC == kCosine) s *= inv_norm(a.norms, beg + v);
-                if (lane == 0 && !(a.dead && a.dead[beg + v])) Qu.push(make_key(s, (uint32_t)(beg + v)));
+                Qu.push(make_key(s, (uint32_t)(beg + v)));
             }
             __syncthreads();
         }
@@ -611,11 +677,14 @@ __global__ void __launch_bounds__(256) ivf_lm_redo_kernel(FlRedo a) {
     }
 }
 
-// ---- pool -> best k, exact re-score in the reference's order, final order ------------------------------------
+// ---- pool -> best k in the reference's order, final order ----------------------------------------------------
+// The pool's keys hold the scan's scores.  Every entry within the slack of the k-th of them is re-scored in the
+// reference's order (no entry below can reach the reference's k-th), and the best k of those are reported.
 struct FlFinal {
     const float* Q; int dim; const float* vecs; const int64_t* labels;
     const unsigned long long* pool; const int32_t* pool_cnt; int pslots; int k; int metric;
     const float* norms; const float* qnorm;  // Cosine
+    const float* band;                       // FlSeed::band
     PairOut out;
 };
 __global__ void __launch_bounds__(256) ivf_lm_final_kernel(FlFinal p) {
@@ -636,18 +705,28 @@ __global__ void __launch_bounds__(256) ivf_lm_final_kernel(FlFinal p) {
             for (int i = 0; i < c; ++i) keys[base + i] = p.pool[ps * p.k + i];
         }
     }
+    __shared__ int s_nr;
+    if (tid == 0) s_nr = 0;
     __syncthreads();
     const int n = s_n;
     const int kk = min(n, p.k);
+    int nr = n;  // entries to re-score
     if (n > kk) {
         const int P2 = next_pow2(max(n, 2));
         for (int i = n + tid; i < P2; i += blockDim.x) keys[i] = 0ull;
         __syncthreads();
         bitonic_sort_desc<false>(keys, P2, tid, blockDim.x);
+        const float m = key_score(keys[kk - 1]);
+        const float lim = m - fl_slack(m, p.band[q], fl_gamma(p.dim));
+        int c = 0;
+        for (int i = kk + tid; i < n; i += blockDim.x) c += key_score(keys[i]) >= lim;
+        if (c) atomicAdd(&s_nr, c);
+        __syncthreads();
+        nr = kk + s_nr;
     }
     __syncthreads();
     // IvfFlatVectorIndex.ComputeScore (:351-360): -L2Squared / DotProduct in VectorMath's single-accumulator order
-    for (int i = tid; i < kk; i += blockDim.x) {
+    for (int i = tid; i < nr; i += blockDim.x) {
         const uint32_t pos = key_pos(keys[i]);
         const float* x = p.vecs + (size_t)pos * p.dim;
         float s = p.metric == kL2 ? -exact::a2_eval<0>(qs, x, p.dim) : exact::a2_eval<1>(qs, x, p.dim);
@@ -658,8 +737,8 @@ __global__ void __launch_bounds__(256) ivf_lm_final_kernel(FlFinal p) {
         keys[i] = make_key(s, pos);
     }
     __syncthreads();
-    const int P3 = next_pow2(max(kk, 2));
-    for (int i = kk + tid; i < P3; i += blockDim.x) keys[i] = 0ull;
+    const int P3 = next_pow2(max(nr, 2));
+    for (int i = nr + tid; i < P3; i += blockDim.x) keys[i] = 0ull;
     __syncthreads();
     bitonic_sort_desc<false>(keys, P3, tid, blockDim.x);
     const int64_t ob = (q * p.out.parts_total + p.out.part_base) * (int64_t)p.k;
@@ -679,7 +758,7 @@ inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
 struct FlLayout {
     size_t zero_bytes;
-    size_t lcnt, lcur, pool_cnt, pool_thr, redo_cnt, scanned, loff, nit, ioff, pairq, pairp, items, redo, pool, temp, total;
+    size_t lcnt, lcur, pool_cnt, pool_thr, band, redo_cnt, scanned, loff, nit, ioff, pairq, pairp, items, redo, pool, temp, total;
     size_t temp_bytes;
     int64_t max_items;
 };
@@ -691,6 +770,7 @@ FlLayout fl_layout(int64_t nq, int P, int k, int nlist) {
     L.lcur = o; o += align_up(sizeof(int32_t) * ((size_t)nlist + 1), 256);
     L.pool_cnt = o; o += align_up(sizeof(int32_t) * (size_t)nq * P, 256);
     L.pool_thr = o; o += align_up(sizeof(uint32_t) * (size_t)nq, 256);
+    L.band = o; o += align_up(sizeof(float) * (size_t)nq, 256);
     L.redo_cnt = o; o += 256;
     L.scanned = o; o += 256;
     L.zero_bytes = o;
@@ -721,6 +801,7 @@ cudaError_t launch_fl(const IvfFlatScanParams& p, int nlist, void* scratch, int 
     int32_t* lcur = reinterpret_cast<int32_t*>(base + L.lcur);
     int32_t* pool_cnt = reinterpret_cast<int32_t*>(base + L.pool_cnt);
     uint32_t* pool_thr = reinterpret_cast<uint32_t*>(base + L.pool_thr);
+    float* band = reinterpret_cast<float*>(base + L.band);
     int32_t* redo_cnt = reinterpret_cast<int32_t*>(base + L.redo_cnt);
     unsigned long long* scanned = reinterpret_cast<unsigned long long*>(base + L.scanned);
     int32_t* loff = reinterpret_cast<int32_t*>(base + L.loff);
@@ -748,19 +829,17 @@ cudaError_t launch_fl(const IvfFlatScanParams& p, int nlist, void* scratch, int 
 
     FlSeed sd{};
     sd.Q = p.Q; sd.nq = p.nq; sd.dim = p.dim; sd.probes = p.probes; sd.P = P; sd.vecs = p.vecs; sd.dead = p.dead;
-    sd.list_off = p.list_off; sd.pool_thr = pool_thr; sd.k = p.k; sd.norms = p.norms;
+    sd.list_off = p.list_off; sd.pool_thr = pool_thr; sd.k = p.k; sd.norms = p.norms; sd.band = band;
     const bool wide = p.dim > 128;
-    if (wide) {
-        if (p.k <= FSEEDW) ivf_lm_seed_wide_kernel<METRIC><<<(unsigned)((p.nq + 7) / 8), 256, 0, st>>>(sd);
-    } else if (p.k <= FSEED) {
-        ivf_lm_seed_kernel<METRIC><<<(unsigned)((p.nq + 7) / 8), 256, 0, st>>>(sd);
-    }
+    // k > the sample: no starting threshold, but the sample still measures the slack the hand-over and the final need
+    if (wide) ivf_lm_seed_wide_kernel<METRIC><<<(unsigned)((p.nq + 7) / 8), 256, 0, st>>>(sd);
+    else ivf_lm_seed_kernel<METRIC><<<(unsigned)((p.nq + 7) / 8), 256, 0, st>>>(sd);
 
     FlParams sp{};
     sp.Q = p.Q; sp.dim = p.dim; sp.vecs = p.vecs; sp.dead = p.dead; sp.list_off = p.list_off;
     sp.items = items; sp.n_items = ioff + nlist; sp.pair_off = loff; sp.pairq = pairq; sp.pairp = pairp;
     sp.pool = pool; sp.pool_cnt = pool_cnt; sp.pool_thr = pool_thr; sp.pslots = P; sp.k = p.k;
-    sp.redo = redo; sp.redo_cnt = redo_cnt; sp.norms = p.norms;
+    sp.redo = redo; sp.redo_cnt = redo_cnt; sp.norms = p.norms; sp.band = band;
     if (p.ev_k0) cudaEventRecord(p.ev_k0, st);
     if (wide) {
         const int nchunk = (p.dim + 127) / 128;
@@ -777,11 +856,11 @@ cudaError_t launch_fl(const IvfFlatScanParams& p, int nlist, void* scratch, int 
     rd.Q = p.Q; rd.dim = p.dim; rd.vecs = p.vecs; rd.dead = p.dead; rd.list_off = p.list_off; rd.items = items;
     rd.pair_off = loff; rd.pairp = pairp; rd.redo = redo; rd.redo_cnt = redo_cnt; rd.pool = pool; rd.pool_cnt = pool_cnt;
     rd.pslots = P; rd.k = p.k; rd.pool_thr = pool_thr; rd.norms = p.norms;
-    ivf_lm_redo_kernel<METRIC><<<(unsigned)(2 * num_sms), 256, sizeof(uint64_t) * FREDO_QCAP, st>>>(rd);
+    ivf_lm_redo_kernel<METRIC><<<(unsigned)(2 * num_sms), 256, sizeof(uint64_t) * FREDO_QCAP + sizeof(float) * p.dim, st>>>(rd);
 
     FlFinal fp{};
     fp.Q = p.Q; fp.dim = p.dim; fp.vecs = p.vecs; fp.labels = p.labels; fp.pool = pool; fp.pool_cnt = pool_cnt;
-    fp.pslots = P; fp.k = p.k; fp.metric = METRIC; fp.out = p.out; fp.norms = p.norms; fp.qnorm = p.qnorm;
+    fp.pslots = P; fp.k = p.k; fp.metric = METRIC; fp.out = p.out; fp.norms = p.norms; fp.qnorm = p.qnorm; fp.band = band;
     const size_t fsm = sizeof(uint64_t) * (size_t)next_pow2(std::max(2, P * p.k)) + sizeof(float) * (size_t)p.dim;
     e = cudaFuncSetAttribute(ivf_lm_final_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fsm);
     if (e != cudaSuccess) return e;

@@ -227,9 +227,9 @@ cudaError_t launch_assign_exact(int metric, int dim, int64_t n, const float* X, 
                                 int32_t* assign, cudaStream_t st);
 // exact-order re-ranking of the coarse stage's candidate lists (P_in >= P_out), best first, ties to the lower index;
 // scores_in (stage-one scores, sorted descending) lets queries whose probed set is already settled skip it
-// unless need_order is set
+// unless need_order is set; for IP / Cosine, when the candidates may miss a centroid of the set, all nc are ranked
 cudaError_t launch_coarse_rerank_exact(int metric, int dim, int64_t nq, const float* Q, const float* centroids,
-                                       const float* cnorms, const int64_t* probes_in, const float* scores_in, int P_in,
+                                       const float* cnorms, int nc, const int64_t* probes_in, const float* scores_in, int P_in,
                                        int64_t* probes_out, float* scores_out, int P_out, int need_order, cudaStream_t st);
 // ComputeNorm:72-100 in the reference's order, one row per thread group
 cudaError_t launch_row_norms_exact(const float* X, int64_t n, int dim, int64_t ldx, float* out,
