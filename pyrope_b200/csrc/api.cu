@@ -466,7 +466,8 @@ struct AssignScratch {
 // KMeansUtils.FindNearestCentroid for n rows, bit-exact.  Small tables: exhaustive exact kernel.
 // Large tables (>= 2048 centroids): tensor-core proxy scores shortlist k' = 17 centroids per row, the
 // shortlist is re-evaluated in the reference's fp32 order (first index wins ties), and any row whose
-// shortlist cannot be proven complete (proxy spread below 1e-4 relative) is redone exhaustively.
+// shortlist cannot be proven complete (its proxy spread within twice the proxy's and the reference's
+// rounding bound, from |x| and the table's max |scale_c| |c|: assign_shortlist_kernel) is redone exhaustively.
 int assign_rows(int metric, int dim, int64_t n, const float* X, int64_t ldx, int nc, const float* centroids,
                 const float* cnorms, int32_t* assign, AssignScratch& sc, bool centroids_changed, cudaStream_t st) {
     if (n <= 0) return PYROPE_OK;
@@ -496,8 +497,9 @@ int assign_rows(int metric, int dim, int64_t n, const float* X, int64_t ldx, int
         tp.metric = metric; tp.k = 1; tp.kprime = kprime; tp.cap = cap; tp.splits = 1;
         tp.queue = sc.tcq.as<uint64_t>(); tp.counts = sc.tcc.as<int32_t>();
         CK(launch_flat_tc_select(tp, st));
-        CK(launch_assign_from_shortlist(metric, dim, cn, Xc, ldx, centroids, cnorms, sc.tcq.as<uint64_t>(),
-                                        sc.tcc.as<int32_t>(), cap, kprime, assign + c0, sc.flag.as<uint8_t>() + c0, st));
+        CK(launch_assign_from_shortlist(metric, dim, cn, Xc, ldx, centroids, cnorms, sc.cent.amax.as<float>(),
+                                        sc.tcq.as<uint64_t>(), sc.tcc.as<int32_t>(), cap, kprime, assign + c0,
+                                        sc.flag.as<uint8_t>() + c0, st));
     }
     // rows whose shortlist may be incomplete: redo exhaustively
     TRY(sc.idx.ensure(sizeof(int64_t) * (size_t)n, 0, st, true));

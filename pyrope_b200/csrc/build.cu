@@ -68,10 +68,27 @@ __global__ void __launch_bounds__(256) nearest_exact_kernel(const float* __restr
 }
 
 // Shortlist variant of nearest_exact_kernel: lanes take the (<= 32) shortlisted centroids of the row.
+//
+// The shortlist holds the k' best 3xTF32 proxy scores p_c (flat_tc.cu: scale_c D + bias_c), so every centroid left out
+// has p_j <= plast.  It settles the reference's arg-best when no centroid left out can reach the best re-evaluated one:
+// with T_c the exact score in proxy units (L2: 2 x.c - |c|^2 = |x|^2 - |x - c|^2, IP: x.c, Cosine: x.c / |c|), the
+// proxy within E_p of T_c and the reference's fp32 score (shifted by |x|^2 for L2, scaled by |x| for Cosine) within E_r,
+//     ref_j <= plast + E_p + E_r   and   ref_best >= p0 - E_p - E_r,
+// so plast < p0 - 2 (E_p + E_r) puts every left-out centroid strictly below the best (a tie could fall to a lower index
+// outside the shortlist: the comparison stays strict).  Both errors are bounded per row from |x| and
+// A = max_c |scale_c| |c| (TcOperand.amax; Cauchy-Schwarz: sum|x_i c_i| scale_c <= |x| A):
+//   E_p = g_p sum|terms|, g_p = (d + 64) 2^-24: the dropped lo.lo product and the tf32-truncated lo operands (< 1.3 2^-20)
+//         plus fp32 accumulation over 3 d / 8 MMA steps (2^-23 each); the slack covers the epilogue's rounding and L2's
+//         fp32 |c|^2 bias (sum|terms| <= |x| A + A^2 / 4);
+//   E_r = g_r sum|terms|, g_r = fl_gamma(d) (ivf_lm.cu); L2's reference sums (x_i - c_i)^2 <= (|x| + A / 2)^2, Cosine's
+//         adds the rounding of the norms and the division (2 g_r |x| A).
+// Neither depends on the score: near 0 (centroids orthogonal to the row) a margin relative to the best proxy accepts a
+// shortlist whose order is rounding noise.  A Cosine row with |x| < 1e-6 scores 0 against every centroid: index 0.
 template <int MODE>
 __global__ void __launch_bounds__(256) assign_shortlist_kernel(const float* __restrict__ X, int64_t n, int64_t ldx,
                                                                int dd, const float* __restrict__ C,
                                                                const float* __restrict__ cnorms,
+                                                               const float* __restrict__ amax,
                                                                const uint64_t* __restrict__ queue,
                                                                const int32_t* __restrict__ counts, int cap, int kprime,
                                                                int32_t* assign, uint8_t* flag) {
@@ -86,6 +103,9 @@ __global__ void __launch_bounds__(256) assign_shortlist_kernel(const float* __re
     const int c = min(counts[row], 32);
     float vnorm = 0.f;
     if (MODE == 2) vnorm = norm_eval(v, dd);
+    float xx = 0.f;
+    for (int i = lane; i < dd; i += 32) xx = fmaf(v[i], v[i], xx);
+    xx = warp_sum(xx);
     float best = -FLT_MAX;
     int besti = 0x7fffffff;
     float proxy = 0.f;
@@ -118,9 +138,16 @@ __global__ void __launch_bounds__(256) assign_shortlist_kernel(const float* __re
         if (os > best || (os == best && oi < besti)) { best = os; besti = oi; }
     }
     if (lane == 0) {
-        const bool incomplete = (c == 0) || besti == 0x7fffffff ||
-                                (c >= kprime && !(plast < p0 - 1e-4f * (fabsf(p0) + 1.f)));
-        assign[row] = incomplete ? 0 : besti;
+        const float A = __ldg(amax), xn = sqrtf(xx) * (1.f + 0x1p-10f);
+        const float gp = (float)(dd + 64) * 0x1p-24f, gr = (float)(dd / 4 + 24) * 0x1p-24f;
+        float e;
+        if (MODE == 0) e = gp * (xn * A + A * A) + gr * (xn + 0.5f * A) * (xn + 0.5f * A);
+        else if (MODE == 1) e = (gp + gr) * xn * A;
+        else e = (gp + 2.f * gr) * xn * A;
+        const float band = 2.f * e * (1.f + 0x1p-10f);
+        const bool zero_row = MODE == 2 && vnorm < 1e-6f;
+        const bool incomplete = !zero_row && ((c == 0) || besti == 0x7fffffff || (c >= kprime && !(plast < p0 - band)));
+        assign[row] = incomplete || zero_row ? 0 : besti;
         flag[row] = incomplete ? 1 : 0;
     }
 }
@@ -375,18 +402,18 @@ cudaError_t launch_assign_exact(int metric, int dim, int64_t n, const float* X, 
 }
 
 cudaError_t launch_assign_from_shortlist(int metric, int dim, int64_t n, const float* X, int64_t ldx,
-                                         const float* centroids, const float* cnorms, const uint64_t* queue,
-                                         const int32_t* counts, int cap, int kprime, int32_t* assign,
-                                         uint8_t* flag, cudaStream_t st) {
+                                         const float* centroids, const float* cnorms, const float* amax,
+                                         const uint64_t* queue, const int32_t* counts, int cap, int kprime,
+                                         int32_t* assign, uint8_t* flag, cudaStream_t st) {
     if (n <= 0) return cudaSuccess;
     const unsigned grid = blocks_for(n, 8);
     const size_t smem = sizeof(float) * 8 * (size_t)dim;
     if (metric == kL2)
-        assign_shortlist_kernel<0><<<grid, 256, smem, st>>>(X, n, ldx, dim, centroids, cnorms, queue, counts, cap, kprime, assign, flag);
+        assign_shortlist_kernel<0><<<grid, 256, smem, st>>>(X, n, ldx, dim, centroids, cnorms, amax, queue, counts, cap, kprime, assign, flag);
     else if (metric == kIP)
-        assign_shortlist_kernel<1><<<grid, 256, smem, st>>>(X, n, ldx, dim, centroids, cnorms, queue, counts, cap, kprime, assign, flag);
+        assign_shortlist_kernel<1><<<grid, 256, smem, st>>>(X, n, ldx, dim, centroids, cnorms, amax, queue, counts, cap, kprime, assign, flag);
     else
-        assign_shortlist_kernel<2><<<grid, 256, smem, st>>>(X, n, ldx, dim, centroids, cnorms, queue, counts, cap, kprime, assign, flag);
+        assign_shortlist_kernel<2><<<grid, 256, smem, st>>>(X, n, ldx, dim, centroids, cnorms, amax, queue, counts, cap, kprime, assign, flag);
     return cudaGetLastError();
 }
 

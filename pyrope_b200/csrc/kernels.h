@@ -84,12 +84,13 @@ cudaError_t launch_flat_tc(const FlatTcParams& p, cudaStream_t st);
 // selection only: leaves the k' best proxy candidates per (split, query) sorted in queue/counts
 cudaError_t launch_flat_tc_select(const FlatTcParams& p, cudaStream_t st);
 // bit-exact arg-best among the shortlisted centroids of each row (split 0 of queue/counts), in the
-// reference's evaluation order; flag[row] = 1 when the shortlist may be incomplete (full and its
-// last proxy score within eps of the first) so the caller re-runs that row exhaustively.
+// reference's evaluation order; flag[row] = 1 when the shortlist may be incomplete (full and its last proxy
+// score within twice the proxy's and the reference's rounding bound of the first; amax: the centroid
+// operand's TcOperand.amax) so the caller re-runs that row exhaustively.
 cudaError_t launch_assign_from_shortlist(int metric, int dim, int64_t n, const float* X, int64_t ldx,
-                                         const float* centroids, const float* cnorms, const uint64_t* queue,
-                                         const int32_t* counts, int cap, int kprime, int32_t* assign,
-                                         uint8_t* flag, cudaStream_t st);
+                                         const float* centroids, const float* cnorms, const float* amax,
+                                         const uint64_t* queue, const int32_t* counts, int cap, int kprime,
+                                         int32_t* assign, uint8_t* flag, cudaStream_t st);
 // scatter: dst[idx[i]] = src[i]
 cudaError_t launch_scatter_i32(const int32_t* src, const int64_t* idx, int64_t n, int32_t* dst, cudaStream_t st);
 
